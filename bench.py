@@ -35,6 +35,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 import numpy as np  # noqa: E402
 
@@ -134,6 +135,17 @@ class ClockSampler(threading.Thread):
         return out
 
 
+def oracle_quantized(frame, T_):
+    """The quantised images of a frame, every level and modality, from the C oracle: templates are planted on them, so that the
+    benchmark's inputs are the same whichever build of the CUDA path runs (that path's own images are bit-identical)."""
+    sys.path.insert(0, os.path.join(ROOT, "oracle"))
+    import fl_oracle_py as F
+    det = F.Detector(T_)
+    if det.process(*frame) != 0:
+        raise SystemExit("bench.py: the C oracle rejected the synthetic frame")
+    return [det.quantized(l, m) for l in range(len(T_)) for m in range(2)]
+
+
 def make_inputs(n_templates: int, seed: int = 1):
     """Frames + a template set with ~1 % planted templates.  The quantised images used for planting come from the product's
     own front end when a GPU is present (our arm) or from the CPU path (reference arm); both are bit-identical."""
@@ -151,7 +163,7 @@ def cpu_time_frames(frames, tset, n_threads: int, steps: int, warmup: int):
     det = F.Detector(T)
     det.set_templates(tset)
     times = []
-    n_matches = 0
+    last = None
     for i in range(warmup + steps):
         b, d = frames[i % len(frames)]
         t0 = time.perf_counter()
@@ -160,8 +172,8 @@ def cpu_time_frames(frames, tset, n_threads: int, steps: int, warmup: int):
         t1 = time.perf_counter()
         if i >= warmup:
             times.append(t1 - t0)
-            n_matches = len(m)
-    return times, n_matches
+            last = m
+    return times, last
 
 
 def ref_time_frames(frames, tset, steps: int, warmup: int):
@@ -192,6 +204,16 @@ def ref_time_frames(frames, tset, steps: int, warmup: int):
     return times, last, prims
 
 
+def dump_outputs(out_dir: str, **outputs) -> None:
+    """What a caller receives for the last timed frame, so that two builds can be compared output for output: every field of
+    every record array as out_dir/<name>_<field>.npy, a plain array as out_dir/<name>.npy, all float64 (exact for the int32
+    and float32 values)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        for f in a.dtype.names or [None]:
+            np.save(os.path.join(out_dir, name + ("_" + f if f else "") + ".npy"), np.ascontiguousarray(a[f] if f else a, np.float64))
+
+
 def match_list_sha(m) -> str:
     import hashlib
     return hashlib.sha256(np.ascontiguousarray(m).tobytes()).hexdigest()[:16]
@@ -212,16 +234,18 @@ def run_reference(args):
     cores_all = os.cpu_count() or 1
     steps = args.steps
     if R.available():
-        steps = min(args.steps, 60)                                      # ~0.12 s per step on one thread: bounded so the run ends within a minute
-        times, last, prims = ref_time_frames(frames, tset, steps, min(args.warmup, 3))
-        kind, cores, n_matches = "reference", 1, len(last)
+        times, last, prims = ref_time_frames(frames, tset, steps, min(args.warmup, 3))    # ~0.12 s per step on one thread
+        kind, cores = "reference", 1
         sample = ("the reference's own Detector::match (linemod.cpp compiled unmodified, oracle/_ref) on ONE thread - its real execution "
                   "model - over %d whole frames x all %d templates; OpenCV supplied by %s" % (steps, args.templates, prims))
     else:
-        times, n_matches = cpu_time_frames(frames, tset, cores_all, steps, args.warmup)
+        times, last = cpu_time_frames(frames, tset, cores_all, steps, args.warmup)
         kind, cores = "port", cores_all
         sample = ("oracle/_ref not in this checkout: the C restatement, %d whole frames x all %d templates; front end single-threaded, "
                   "matchClass OpenMP over templates" % (steps, args.templates))
+    n_matches = len(last)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, matches=last)
     tot = float(np.sum(times))
     v = args.templates * CELLS * steps / tot
     # for context: the OpenMP restatement on every host core (NOT the reference's execution model)
@@ -276,12 +300,7 @@ def run_ours(args):
 
     def make_handle():
         return fb.Handle(T, (0, 1), W, H, max_candidates=max(1 << 16, world * (cap + 1) + 16), device=local)
-    # quantised images for planting come from the product's own front end (empty template set)
-    h0 = make_handle()
-    h0.upload_templates(synth.make_templates(0))
-    rc, _, q = h0.match(frames[0][0], frames[0][1], THRESHOLD, want_quantized=True)
-    assert rc == 0
-    h0.close()
+    q = oracle_quantized(frames[0], T)          # the inputs do not depend on the build under test
     tset = synth.make_templates(n_total, W, H, T, seed=1, quantized=q, planted_fraction=0.01)
     # `depth` frames in flight per GPU: depth handles (own stream, linear memories, candidate / result blocks, exchange buffer),
     # frames dealt round-robin, lists collected in order (fealess_b200.sharded.ShardedPipe; fl_pipe is the same schedule in C)
@@ -366,6 +385,8 @@ def run_ours(args):
     launches = pipe.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
     n_matches = len(last.fetch())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, matches=last.fetch())
     dev_ms = float(e_start.elapsed_time(e_end))
     t = torch.tensor([dev_ms], dtype=torch.float64, device=dev)
     if world > 1:
@@ -750,9 +771,7 @@ def run_pipeline(args):
     frames = [synth.make_frame(Wp, Hp, i) for i in range(2)]
     cap = 4096
     h = fb.Handle(Tp, (0, 1), Wp, Hp, max_candidates=max(1 << 16, world * (cap + 1) + 16), device=local)
-    h.upload_templates(synth.make_templates(0, Wp, Hp, Tp))
-    rc, _, q = h.match(frames[0][0], frames[0][1], THRESHOLD, want_quantized=True)
-    assert rc == 0
+    q = oracle_quantized(frames[0], Tp)
     tset = synth.make_templates(n_total, Wp, Hp, Tp, n_classes=cfg["classes"], seed=1, quantized=q, planted_fraction=0.004)
     sm = sharded.ShardedMatcher(h, tset, rank, world, capacity=cap, device=dev, exchange=args.exchange)
     stream = sm.stream
@@ -921,7 +940,7 @@ def run_pipeline(args):
             smk.match_device(d_frames[f][0].data_ptr(), d_frames[f][1].data_ptr(), Wp, Hp, THRESHOLD)
             refine_local(hk, smk.fetch(), d_frames[f][1].data_ptr())
         hk.sync()
-    n_tp = max(args.steps, 4 * depth)
+    n_tp = args.steps
     run_threads(0, 2 * depth)
     torch.cuda.synchronize()
     if world > 1:
@@ -933,6 +952,7 @@ def run_pipeline(args):
     run_threads(2 * depth, n_tp)
     torch.cuda.synchronize()
     ev1.record(); ev1.synchronize()
+    timed_last = last_of[(n_tp - 1) % depth]                         # the slot that took the last timed frame, 2 * depth + n_tp - 1
     tw1 = time.perf_counter()
     launches_tp = sum(s_[0].launch_count() for s_ in slots) - launches_tp0
     tp = torch.tensor([float(ev0.elapsed_time(ev1))], dtype=torch.float64, device=dev)
@@ -976,6 +996,9 @@ def run_pipeline(args):
     if world > 1:
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
     m = last_of[0][0] if last_of[0] is not None else got0
+    if args.dump_outputs and rank == 0:
+        m_last, res_last, keep_last = timed_last
+        dump_outputs(args.dump_outputs, matches=m_last, icp=res_last, nms_keep=keep_last)
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()
@@ -1235,7 +1258,7 @@ def bench_icp(h, synth, n_hyp: int = 256, cpu: bool = True):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=500)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (frames); default 500 for C2, 100 for C4 / C5")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--templates", type=int, default=8000, help="templates per GPU")
@@ -1246,11 +1269,17 @@ def main():
     ap.add_argument("--no-icp", action="store_true", help="skip the ICP side benchmark")
     ap.add_argument("--config", default="C2", choices=["C2", "C4", "C5"], help="C2: the headline match-only benchmark (weak scaling); C4 / C5: the "
                     "strong-scaling pipeline benchmark (fixed template set sharded over the GPUs, match + top-5 ICP + NMS, frames/s)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed frame returned to DIR as "
+                    "float64 .npy files: its match list (matches_<field>.npy) and, for C4 / C5, its ICP results (icp_<field>.npy) "
+                    "and the NMS keep-list (nms_keep.npy)")
     args = ap.parse_args()
+    pipeline = args.config != "C2" and args.impl == "ours"
+    if args.steps is None:
+        args.steps = 100 if pipeline else 500
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
-    if args.config != "C2" and args.impl == "ours":
-        if args.steps == 500:
-            args.steps = 100
+    if pipeline:
         run_pipeline(args)
     elif args.impl == "reference":
         run_reference(args)            # ~0.1 s per step on 8 host threads: the default run ends within seconds

@@ -134,3 +134,14 @@ def test_nms_matches_golden(golden_dir):
     assert np.array_equal(F.nms(z["nms_t3"], z["nms_n"], z["nms_dist"], 25.0), z["nms_out_th25"])
     assert np.array_equal(F.nms(z["nms_t3"], z["nms_n"], z["nms_dist"], 8.0), z["nms_out_th8"])
     assert len(F.nms(np.zeros((0, 3)), [], [], 1.0)) == 0
+
+
+def test_reference_cases_fixture(golden_dir):
+    """tests/golden/reference_cases.npz, the reference's results that the GPU reference tests compare with (oracle/make_ref_golden.py):
+    the C oracle reproduces every entry, so the oracle stays pinned on the reference's results where oracle/_ref is not built."""
+    import make_ref_golden as G
+    z = np.load(os.path.join(golden_dir, "reference_cases.npz"))
+    got = G.compute(F)
+    assert sorted(got) == sorted(z.files)
+    for k in z.files:
+        assert np.array_equal(got[k], z[k]), k

@@ -420,6 +420,29 @@ def test_training_fixture_is_what_the_reference_returns():
             assert np.array_equal(hdr, g["hdr%d" % i]) and np.array_equal(ft, g["ft%d" % i]) and np.array_equal(bb, g["bb%d" % i])
 
 
+def test_reference_cases_fixture_is_what_the_reference_returns(golden_dir):
+    """tests/golden/reference_cases.npz (oracle/make_ref_golden.py) = the reference's own code on the inputs of tests/test_gpu_ref.py
+    and of the reference cases of tests/test_gpu_train.py, entry for entry; and the real Detector::match (its own std::sort /
+    std::unique) returns the stored lists as sets, with the same best match and the stored `quantized_images`."""
+    import make_ref_golden as G
+    from helpers import sha
+    z = np.load(os.path.join(golden_dir, "reference_cases.npz"))
+    got = G.compute(R)
+    assert sorted(got) == sorted(z.files)
+    for k in z.files:
+        assert np.array_equal(got[k], z[k]), k
+    for k, c in enumerate(G.MATCH_CFGS):
+        b, d, ts, det = G.match_setup(R, c["W"], c["H"], c["T"], c["n"], c["classes"])
+        for thr in (75, 60):
+            want = z["m%d_final_%d" % (k, thr)]
+            rc, full = det.match_full(b, d, float(thr))
+            assert rc == 0 and set(map(tuple, full.tolist())) == set(map(tuple, want.tolist()))
+            if len(want):
+                assert tuple(full[0])[:4] == tuple(want[0])[:4]
+            L = len(c["T"])
+            assert [sha(det.match_quantized(l, m)) for l in range(L) for m in range(2)] == [str(x) for x in z["m%d_quantized_sha" % k]]
+
+
 def test_c_oracle_training_equals_the_reference():
     """flo_add_template (oracle/fl_oracle.c) == the reference's own Detector::addTemplate: every feature, cropped box and bounding box, for
     masks of several shapes and values, no mask, two and three pyramid levels, and the too-few-candidates case; its erode / distance
