@@ -38,6 +38,10 @@ FL_DBG_QUANTIZED, FL_DBG_SPREAD, FL_DBG_LINEAR_MEMORY, FL_DBG_SIMILARITY, FL_DBG
 MATCH_DTYPE = np.dtype([("x", "<i4"), ("y", "<i4"), ("similarity", "<f4"), ("class_idx", "<i4"), ("template_id", "<i4")])
 ICP_RESULT_DTYPE = np.dtype([("R", "<f4", (9,)), ("T", "<f4", (3,)), ("dist_mean", "<f4"), ("inlier_ratio", "<f4"),
                              ("iterations", "<i4"), ("n_points", "<i4"), ("status", "<i4")])
+# fl_reco_result_t: one recognised object of fl_recognize* (the match it came from, its hypothesis index, [R | T; 0 0 0 1], the ICP record)
+RECO_RESULT_DTYPE = np.dtype([("class_idx", "<i4"), ("template_id", "<i4"), ("x", "<i4"), ("y", "<i4"), ("similarity", "<f4"),
+                              ("hypothesis", "<i4"), ("world2cam", "<f4", (16,)), ("icp", ICP_RESULT_DTYPE)])
+RECO_MAX_HYP = 256                                                # FL_RECO_MAX_HYP
 
 # every symbol include/fealess_b200.h declares (tests check that the built library exports all of them)
 EXPORTED_SYMBOLS = [
@@ -49,6 +53,8 @@ EXPORTED_SYMBOLS = [
     "fl_group_create", "fl_group_destroy", "fl_group_size", "fl_group_handle", "fl_group_upload_templates", "fl_group_match",
     "fl_match_async", "fl_set_blocking_wait", "fl_match_shard_exchange_async", "fl_pipe_create", "fl_pipe_destroy", "fl_pipe_depth", "fl_pipe_in_flight", "fl_pipe_handle", "fl_pipe_upload_templates",
     "fl_pipe_submit", "fl_pipe_collect", "fl_pipe_match_batch", "fl_pipe_set_exchange", "fl_default_train_params", "fl_add_template",
+    "fl_default_reco_params", "fl_set_recognition", "fl_recognize_async", "fl_recognize_wait", "fl_recognize", "fl_pipe_upload_model_depths",
+    "fl_pipe_set_recognition", "fl_pipe_submit_recognition", "fl_pipe_collect_recognition",
 ]
 
 
@@ -74,6 +80,31 @@ class Rect(C.Structure):
 
 class IcpParams(C.Structure):
     _fields_ = [("icp_it_thr", C.c_int32), ("dist_mean_thr", C.c_float), ("dist_diff_thr", C.c_float)]
+
+
+class RecoParams(C.Structure):
+    _fields_ = [("threshold", C.c_float), ("icp", IcpParams), ("top_k", C.c_int32), ("per_class", C.c_int32), ("th_obj_dist", C.c_float)]
+
+
+class RecoSummary(C.Structure):
+    _fields_ = [("n_matches", C.c_int32), ("n_hypotheses", C.c_int32), ("n_roi", C.c_int32), ("n_results", C.c_int32)]
+
+
+def reco_params(threshold: float = 75.0, icp=(10, 0.5, 0.01), top_k: int = 1, per_class: bool = False, th_obj_dist: float = 0.0) -> RecoParams:
+    """fl_reco_params_t; the defaults are fl_default_reco_params (the reference's Recognition)."""
+    return RecoParams(float(threshold), IcpParams(*icp), int(top_k), int(bool(per_class)), float(th_obj_dist))
+
+
+def _reco_args(bgr, depth, W, H):
+    """(bgr, depth, src_W, src_H, W, H) of fl_recognize*: dense numpy frames; W x H defaults to the frame's own size."""
+    b = None if bgr is None else np.ascontiguousarray(bgr, np.uint8)
+    d = np.ascontiguousarray(depth, np.uint16)
+    sH, sW = d.shape[:2]
+    return b, d, sW, sH, int(W or sW), int(H or sH)
+
+
+def _summary(s: RecoSummary) -> dict:
+    return dict(n_matches=s.n_matches, n_hypotheses=s.n_hypotheses, n_roi=s.n_roi, n_results=s.n_results)
 
 
 def library_path() -> str:
@@ -523,6 +554,35 @@ class Handle:
             _check(n, "fl_nms")
         return out[:n].copy()
 
+    # ---- Recognition on the device ---------------------------------------------------------------
+    def set_recognition(self, crop_of_template, pose12=None, params: Optional[RecoParams] = None) -> None:
+        """fl_set_recognition: crop index per uploaded template (-1 = none), pose table (n_templates x 12, None = the uploaded pose13)."""
+        crop = np.ascontiguousarray(crop_of_template, np.int32)
+        pose = None if pose12 is None else np.ascontiguousarray(pose12, np.float32).reshape(-1, 12)
+        _check(lib().fl_set_recognition(self._h, C.byref(params or reco_params()), _p(crop), _p(pose)), "fl_set_recognition")
+
+    def recognize_async(self, bgr, depth, K, W: Optional[int] = None, H: Optional[int] = None) -> None:
+        """fl_recognize_async: the frame (rescaled on the device to W x H when that differs) is matched, refined and suppressed in one
+        enqueue.  The arrays must stay alive until ``recognize_wait`` (page-locked ones are read by DMA)."""
+        b, d, sW, sH, W, H = _reco_args(bgr, depth, W, H)
+        _check(lib().fl_recognize_async(self._h, _p(b), C.c_size_t(sW * 3), _p(d), C.c_size_t(sW * 2), sW, sH, W, H,
+                                        Intrinsics(*[float(v) for v in K])), "fl_recognize_async")
+        self._reco_keep = (b, d)
+
+    def recognize_wait(self, capacity: int = RECO_MAX_HYP):
+        """(rc, results RECO_RESULT_DTYPE, summary dict); rc is FL_OK or FL_ERR_CAPACITY (truncated, or a candidate overflow: no results)."""
+        out = np.zeros(max(capacity, 1), RECO_RESULT_DTYPE)
+        s = RecoSummary()
+        rc = lib().fl_recognize_wait(self._h, _p(out), int(capacity), C.byref(s))
+        self._reco_keep = None
+        if rc not in (FL_OK, FL_ERR_CAPACITY):
+            _check(rc, "fl_recognize_wait")
+        return rc, out[:min(s.n_results, capacity)].copy(), _summary(s)
+
+    def recognize(self, bgr, depth, K, W: Optional[int] = None, H: Optional[int] = None, capacity: int = RECO_MAX_HYP):
+        self.recognize_async(bgr, depth, K, W, H)
+        return self.recognize_wait(capacity)
+
 
 class Group:
     """fl_group: Detector::match over N handles of this process (``devices`` may repeat a device), templates sharded gid % N."""
@@ -714,6 +774,42 @@ class Pipe:
         views = [out[f * capacity_per_frame:f * capacity_per_frame + min(int(counts[f]), capacity_per_frame)] for f in range(n)]
         return rc, ([v.copy() for v in views] if copy else views)
 
+    # ---- Recognition over the pipe ----------------------------------------------------------------
+    def upload_model_depths(self, model_depths: Sequence[np.ndarray], rects_model) -> None:
+        """fl_pipe_upload_model_depths: ``Handle.upload_model_depths`` on every slot."""
+        n = len(model_depths)
+        mds = [np.ascontiguousarray(m, np.uint16) for m in model_depths]
+        H, W = mds[0].shape if n else (1, 1)
+        ptrs = (C.c_void_p * max(n, 1))(*[m.ctypes.data for m in mds])
+        strides = (C.c_size_t * max(n, 1))(*[m.strides[0] for m in mds])
+        rm = np.ascontiguousarray(rects_model, np.int32).reshape(-1, 4)
+        _check(lib().fl_pipe_upload_model_depths(self._p, n, ptrs, strides, _p(rm), W, H), "fl_pipe_upload_model_depths")
+
+    def set_recognition(self, crop_of_template, pose12=None, params: Optional[RecoParams] = None) -> None:
+        """fl_pipe_set_recognition: ``Handle.set_recognition`` on every slot."""
+        crop = np.ascontiguousarray(crop_of_template, np.int32)
+        pose = None if pose12 is None else np.ascontiguousarray(pose12, np.float32).reshape(-1, 12)
+        _check(lib().fl_pipe_set_recognition(self._p, C.byref(params or reco_params()), _p(crop), _p(pose)), "fl_pipe_set_recognition")
+
+    def submit_recognition(self, bgr, depth, K, W: Optional[int] = None, H: Optional[int] = None) -> None:
+        """fl_pipe_submit_recognition (host frame; page-locked arrays are read by DMA while in flight, so they are kept referenced)."""
+        b, d, sW, sH, W, H = _reco_args(bgr, depth, W, H)
+        _check(lib().fl_pipe_submit_recognition(self._p, _p(b), C.c_size_t(sW * 3), _p(d), C.c_size_t(sW * 2), sW, sH, W, H,
+                                                Intrinsics(*[float(v) for v in K])), "fl_pipe_submit_recognition")
+        self._keep[self._seq % self.depth] = (b, d)
+        self._seq += 1
+
+    def collect_recognition(self, capacity: int = RECO_MAX_HYP):
+        """(rc, results, summary) of the oldest frame in flight, as ``Handle.recognize_wait``."""
+        out = self._out.get(("reco", capacity))
+        if out is None:
+            out = self._out[("reco", capacity)] = np.zeros(max(capacity, 1), RECO_RESULT_DTYPE)
+        s = RecoSummary()
+        rc = lib().fl_pipe_collect_recognition(self._p, _p(out), int(capacity), C.byref(s))
+        if rc not in (FL_OK, FL_ERR_CAPACITY):
+            _check(rc, "fl_pipe_collect_recognition")
+        return rc, out[:min(s.n_results, capacity)].copy(), _summary(s)
+
 
 # --------------------------------------------------------------------------------------------------
 # mirrors of the reference interface
@@ -749,6 +845,7 @@ class Detector:
         self._classes = {}          # class_id -> list of template pyramids
         self._poses = {}            # class_id -> list of 13-float arrays
         self._dirty = True
+        self._revision = 0          # bumped by every template change (consumers with their own copy of the templates compare it)
         self._class_order: List[str] = []
 
     @property
@@ -808,6 +905,7 @@ class Detector:
         self._poses.setdefault(class_id, []).append(np.zeros(13, np.float32) if pose_info is None else np.asarray(pose_info, np.float32))
         lst.append(templates)
         self._dirty = True
+        self._revision += 1
         return len(lst) - 1
 
     def add_template_set(self, tset) -> None:
@@ -820,6 +918,12 @@ class Detector:
             self.addSyntheticTemplate(pyr, tset.class_names[int(tset.class_of[t])], tset.pose13[t])
 
     def _upload(self):
+        self._handle.upload_templates(self.template_set())
+        self._class_order = self.classIds()
+        self._dirty = False
+
+    def template_set(self):
+        """The flattened template database in upload order (classes sorted by name, templates by id) as a ``synth.TemplateSet``."""
         names = self.classIds()
         hdrs, feats, class_of, poses, pos = [], [], [], [], 0
         for ci, name in enumerate(names):
@@ -831,13 +935,10 @@ class Detector:
                     pos += len(f)
                 class_of.append(ci)
                 poses.append(self._poses[name][tid])
-        ts = synth.TemplateSet(len(self.T_at_level), len(self.modalities), tuple(self.T_at_level), names,
-                               np.array(hdrs, np.int32).reshape(-1, 7),
-                               np.concatenate(feats).astype(np.int32) if feats else np.zeros((0, 3), np.int32),
-                               np.array(class_of, np.int32), np.array(poses, np.float32).reshape(-1, 13))
-        self._handle.upload_templates(ts)
-        self._class_order = names
-        self._dirty = False
+        return synth.TemplateSet(len(self.T_at_level), len(self.modalities), tuple(self.T_at_level), names,
+                                 np.array(hdrs, np.int32).reshape(-1, 7),
+                                 np.concatenate(feats).astype(np.int32) if feats else np.zeros((0, 3), np.int32),
+                                 np.array(class_of, np.int32), np.array(poses, np.float32).reshape(-1, 13))
 
     def match(self, sources: Sequence[np.ndarray], threshold: float, class_ids: Sequence[str] = (),
               quantized_images: Optional[list] = None, masks: Sequence[Optional[np.ndarray]] = ()):

@@ -12,7 +12,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libfealess_b200.so")
-SOURCES = ["frontend.cu", "similarity.cu", "similarity_staged.cu", "icp.cu", "resize.cu", "api.cu", "group.cu", "pipe.cu", "train.cu"]
+SOURCES = ["frontend.cu", "similarity.cu", "similarity_staged.cu", "icp.cu", "resize.cu", "api.cu", "group.cu", "pipe.cu", "train.cu", "reco.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-fmad=false", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-O2", "--expt-relaxed-constexpr"]
 

@@ -80,6 +80,11 @@ struct fl_handle {
   // input rescale: device tables of the current (source -> destination) geometry, source-frame staging
   fl_resize_tables rz; int rz_sW, rz_sH, rz_dW, rz_dH;
   uint8_t* d_src_bgr; uint16_t* d_src_depth; size_t src_cap;
+  // Recognition on the device (fl_set_recognition, fl_recognize_*): per-template table, per-frame selection state, mapped host block
+  // [summary | records] (+ its device alias); the frame in flight (pend_reco) and its geometry and intrinsics
+  bool custom_tids, reco_set, reco_any_crop, pend_reco; fl_reco_params_t reco; int reco_max_hyp;
+  fl_reco_tmpl* d_reco_tmpl; int* d_reco_sel; int* h_reco; int* d_reco_host;
+  int reco_W, reco_H; fl_intrinsics_t reco_K;
 };
 
 // The host waits for the handle's stream.  Default: cudaStreamSynchronize (the runtime spins - lowest latency, one busy core per
@@ -157,6 +162,8 @@ extern "C" int fl_create(const fl_params_t* params, fl_handle** out) {
   memset(h->d_bgr, 0, sizeof h->d_bgr); memset(h->d_q, 0, sizeof h->d_q); memset(h->d_qm, 0, sizeof h->d_qm);
   memset(h->d_mask, 0, sizeof h->d_mask); memset(h->d_spread, 0, sizeof h->d_spread); memset(h->d_lm, 0, sizeof h->d_lm); h->d_lm4 = nullptr; h->d_nms = nullptr; h->nms_cap = 0; h->blocking_wait = false; h->ev_block = nullptr; h->d_train = nullptr;
   memset(h->used_mask, 0, sizeof h->used_mask); memset(h->stage_ms, 0, sizeof h->stage_ms); h->icp_ms = 0.f;
+  h->custom_tids = h->reco_set = h->reco_any_crop = h->pend_reco = false; h->reco_max_hyp = 0; fl_default_reco_params(&h->reco);
+  h->d_reco_tmpl = nullptr; h->d_reco_sel = nullptr; h->h_reco = nullptr; h->d_reco_host = nullptr; h->reco_W = h->reco_H = 0; memset(&h->reco_K, 0, sizeof h->reco_K);
   *out = h;
   FL_CUDA(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
   for (int i = 0; i < 5; ++i) FL_CUDA(cudaEventCreate(&h->ev[i]));
@@ -232,6 +239,7 @@ extern "C" int fl_destroy(fl_handle* h) {
   cudaFree(h->d_ref_depth); cudaFree(h->d_resident); cudaFree(h->d_nms); cudaFree(h->d_train); if (h->ev_block) cudaEventDestroy(h->ev_block);
   cudaFree(h->rz.xofs); cudaFree(h->rz.yofs); cudaFree(h->rz.ialpha); cudaFree(h->rz.ibeta); cudaFree(h->rz.alpha); cudaFree(h->rz.beta);
   cudaFree(h->d_src_bgr); cudaFree(h->d_src_depth);
+  cudaFree(h->d_reco_tmpl); cudaFree(h->d_reco_sel); cudaFreeHost(h->h_reco);
   cudaFree(h->d_in_bgr); cudaFree(h->d_in_depth); cudaFree(h->d_geom);
   for (int l = 0; l < FL_MAX_LEVELS; ++l) {
     cudaFree(h->d_bgr[l]); cudaFree(h->d_lm[l]); if (l == 0) cudaFree(h->d_lm4);
@@ -262,6 +270,7 @@ extern "C" int fl_sync(fl_handle* h) { if (!h) return FL_ERR_ARG; FL_CUDA(cudaSt
 extern "C" void* fl_stream(fl_handle* h) { return h ? (void*)h->stream : nullptr; }
 extern "C" int64_t fl_launch_count(fl_handle* h) { return h ? h->launches : 0; }
 int fl_entries_per_template(const fl_handle* h) { return h ? h->p.n_levels * h->p.n_modalities : 0; }
+bool fl_recognition_pending(const fl_handle* h) { return h && h->pend_reco; }
 extern "C" int fl_profile(fl_handle* h, int enable) { if (!h) return FL_ERR_ARG; h->profile = enable != 0; return FL_OK; }
 extern "C" int fl_last_icp_ms(fl_handle* h, float* ms) { if (!h || !ms) return FL_ERR_ARG; *ms = h->icp_ms; return FL_OK; }
 extern "C" int fl_debug_icp_trace(fl_handle* h, uint64_t* out, int32_t n_hyp) {
@@ -350,7 +359,7 @@ extern "C" int fl_upload_templates(fl_handle* h, int32_t n_templates, const fl_t
   h->pose13_h.clear();
   if (pose13) h->pose13_h.assign(pose13, pose13 + (size_t)n_templates * 13);
   h->class_enabled_h.assign((size_t)std::max(nc, 1), 1); h->class_enabled_valid = false;
-  h->packed = false;
+  h->packed = false; h->custom_tids = false; h->reco_set = false;
   return FL_OK;
 }
 
@@ -361,6 +370,7 @@ extern "C" int fl_set_template_ids(fl_handle* h, const int32_t* template_ids) {
   FL_CUDA(cudaStreamSynchronize(h->stream));
   for (int t = 0; t < h->n_templates; ++t) if (template_ids[t] < 0) return FL_ERR_ARG;
   h->tid_of_h.assign(template_ids, template_ids + h->n_templates);
+  h->custom_tids = true; h->reco_set = false;
   FL_CUDA(cudaMemcpy(h->d_tid_of, template_ids, (size_t)h->n_templates * sizeof(int32_t), cudaMemcpyHostToDevice));
   return FL_OK;
 }
@@ -812,8 +822,7 @@ extern "C" int fl_match_device_async(fl_handle* h, const void* d_bgr, const void
   return FL_OK;
 }
 
-extern "C" int fl_match_wait(fl_handle* h) {
-  if (!h) return FL_ERR_ARG;
+static int match_wait(fl_handle* h) {
   if (!h->pend_sort) return FL_ERR_STATE;
   const bool was_match = h->pend_match;
   h->pend_match = false;
@@ -837,6 +846,11 @@ extern "C" int fl_match_wait(fl_handle* h) {
   if (h->h_small[15]) { fl_set_error("peer exchange timed out waiting for rank %d", h->h_small[15] - 1); return FL_ERR_STATE; }
   h->have_result = true;
   return FL_OK;
+}
+extern "C" int fl_match_wait(fl_handle* h) {
+  if (!h) return FL_ERR_ARG;
+  h->pend_reco = false;                 // a recognition frame waited for this way has no results to collect
+  return match_wait(h);
 }
 
 extern "C" int fl_match_device(fl_handle* h, const void* d_bgr, const void* d_depth, int32_t W, int32_t H, const void* const* d_masks,
@@ -1306,6 +1320,27 @@ extern "C" int fl_resize_linear(fl_handle* h, const void* src, size_t src_stride
   return FL_OK;
 }
 
+// upload of a src_W x src_H frame and its INTER_LINEAR rescale into d_in_bgr / d_in_depth (the host-input staging of W x H frames)
+static int stage_rescaled(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int sW, int sH, int W, int H,
+                          const uint8_t** d_bgr_out, const uint16_t** d_depth_out) {
+  *d_bgr_out = nullptr; *d_depth_out = nullptr;
+  if ((bgr && bgr_stride < (size_t)sW * 3) || (depth && depth_stride < (size_t)sW * 2)) return FL_ERR_SIZE;
+  cudaStream_t s = h->stream;
+  TRY(resize_tables(h, sW, sH, W, H));
+  TRY(resize_staging(h, (size_t)sW * sH));
+  if (depth) {
+    FL_CUDA(cudaMemcpy2DAsync(h->d_src_depth, (size_t)sW * 2, depth, depth_stride, (size_t)sW * 2, sH, cudaMemcpyHostToDevice, s));
+    fl_launch_resize_linear(h->d_src_depth, sW, sH, FL_IMG_16UC1, h->d_in_depth, W, H, h->rz, s); ++h->launches;
+    *d_depth_out = h->d_in_depth;
+  }
+  if (bgr) {
+    FL_CUDA(cudaMemcpy2DAsync(h->d_src_bgr, (size_t)sW * 3, bgr, bgr_stride, (size_t)sW * 3, sH, cudaMemcpyHostToDevice, s));
+    fl_launch_resize_linear(h->d_src_bgr, sW, sH, FL_IMG_8UC3, h->d_in_bgr, W, H, h->rz, s); ++h->launches;
+    *d_bgr_out = h->d_in_bgr;
+  }
+  return FL_OK;
+}
+
 extern "C" int fl_match_rescaled(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int32_t sW, int32_t sH,
                                  int32_t W, int32_t H, float threshold, const int32_t* class_filter, int32_t n_filter, fl_match_t* out, int32_t capacity,
                                  int32_t* count, uint16_t* rescaled_depth_out) {
@@ -1320,23 +1355,10 @@ extern "C" int fl_match_rescaled(fl_handle* h, const uint8_t* bgr, size_t bgr_st
     if (rescaled_depth_out && depth) for (int y = 0; y < H; ++y) memcpy(rescaled_depth_out + (size_t)y * W, (const uint8_t*)depth + (size_t)y * depth_stride, (size_t)W * 2);
     return rc;
   }
-  if ((bgr && bgr_stride < (size_t)sW * 3) || (depth && depth_stride < (size_t)sW * 2)) return FL_ERR_SIZE;
   FL_CUDA(cudaSetDevice(p.device));
-  cudaStream_t s = h->stream;
-  TRY(resize_tables(h, sW, sH, W, H));
-  TRY(resize_staging(h, (size_t)sW * sH));
   const uint8_t* d_bgr = nullptr; const uint16_t* d_depth = nullptr;
-  if (depth) {
-    FL_CUDA(cudaMemcpy2DAsync(h->d_src_depth, (size_t)sW * 2, depth, depth_stride, (size_t)sW * 2, sH, cudaMemcpyHostToDevice, s));
-    fl_launch_resize_linear(h->d_src_depth, sW, sH, FL_IMG_16UC1, h->d_in_depth, W, H, h->rz, s); ++h->launches;
-    d_depth = h->d_in_depth;
-    if (rescaled_depth_out) FL_CUDA(cudaMemcpyAsync(rescaled_depth_out, h->d_in_depth, (size_t)W * H * 2, cudaMemcpyDeviceToHost, s));
-  }
-  if (bgr) {
-    FL_CUDA(cudaMemcpy2DAsync(h->d_src_bgr, (size_t)sW * 3, bgr, bgr_stride, (size_t)sW * 3, sH, cudaMemcpyHostToDevice, s));
-    fl_launch_resize_linear(h->d_src_bgr, sW, sH, FL_IMG_8UC3, h->d_in_bgr, W, H, h->rz, s); ++h->launches;
-    d_bgr = h->d_in_bgr;
-  }
+  TRY(stage_rescaled(h, bgr, bgr_stride, depth, depth_stride, sW, sH, W, H, &d_bgr, &d_depth));
+  if (d_depth && rescaled_depth_out) FL_CUDA(cudaMemcpyAsync(rescaled_depth_out, h->d_in_depth, (size_t)W * H * 2, cudaMemcpyDeviceToHost, h->stream));
   int rc = fl_match_device(h, d_bgr, d_depth, W, H, nullptr, threshold, class_filter, n_filter);
   if (rc != FL_OK) return rc;
   if (d_depth) { h->in_depth_W = W; h->in_depth_H = H; }
@@ -1502,7 +1524,7 @@ extern "C" int fl_upload_model_depths(fl_handle* h, int32_t n_models, const uint
   FL_CUDA(cudaMemcpy(h->d_resident, packed.data(), packed.size() * 2, cudaMemcpyHostToDevice));
   h->res_off.assign(off.begin(), off.end() - 1);
   h->res_rect.assign(rect_model, rect_model + n_models);
-  h->res_W = W; h->res_H = H;
+  h->res_W = W; h->res_H = H; h->reco_set = false;
   // size the ICP workspace for the largest crop now (8 hypotheses; more grow it again): growing it later means cudaFree / cudaMalloc,
   // which synchronise the whole device - harmless for one handle, a stall for the other frames in flight on this GPU, and with a
   // peer-memory exchange in flight on another handle a cross-rank stall until that exchange times out
@@ -1601,4 +1623,141 @@ extern "C" int fl_nms_ex(fl_handle* h, const float* t3, const int32_t* n_model_p
 
 extern "C" int fl_nms(fl_handle* h, const float* t3, const int32_t* n_model_pts, const float* icp_dist, int32_t n, float th, int32_t* out_idx) {
   return fl_nms_ex(h, t3, n_model_pts, icp_dist, n, th, out_idx, nullptr);
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Recognition on the device (CObjRecoLmICP::Recognition, CadReco/obj_reco_lmicp.cpp:86-204)
+// ---------------------------------------------------------------------------------------------------
+extern "C" void fl_default_reco_params(fl_reco_params_t* p) {
+  if (!p) return;
+  p->threshold = 75.0f;                                                           // :52-55
+  p->icp.icp_it_thr = 10; p->icp.dist_mean_thr = 0.5f; p->icp.dist_diff_thr = 0.01f;
+  p->top_k = 1; p->per_class = 0; p->th_obj_dist = 0.f;                           // matches[0] only (:111)
+}
+
+extern "C" int fl_set_recognition(fl_handle* h, const fl_reco_params_t* prm, const int32_t* crop_of_template, const float* pose12) {
+  if (!h || !prm || !crop_of_template || prm->top_k < 1) return FL_ERR_ARG;
+  if (h->pend_sort) { fl_set_error("fl_set_recognition: a frame is in flight on this handle"); return FL_ERR_STATE; }
+  if (h->n_templates == 0) { fl_set_error("fl_set_recognition: no templates uploaded"); return FL_ERR_STATE; }
+  // matches carry the ids of fl_set_template_ids (a shard's global ids): the template behind a match is not class_first + template_id
+  if (h->custom_tids) { fl_set_error("fl_set_recognition: not available on a handle with fl_set_template_ids (template shards)"); return FL_ERR_STATE; }
+  if (!pose12 && h->pose13_h.empty()) { fl_set_error("fl_set_recognition: no pose table (pose12 NULL and no pose13 uploaded)"); return FL_ERR_ARG; }
+  const int64_t max_hyp = (int64_t)prm->top_k * (prm->per_class ? h->n_classes : 1);
+  if (max_hyp > FL_RECO_MAX_HYP) { fl_set_error("fl_set_recognition: %lld hypotheses per frame > FL_RECO_MAX_HYP", (long long)max_hyp); return FL_ERR_CAPACITY; }
+  FL_CUDA(cudaSetDevice(h->p.device));
+  const size_t per = (size_t)h->p.n_levels * h->p.n_modalities;
+  std::vector<fl_template_hdr_t> hdr((size_t)h->n_templates * per);
+  FL_CUDA(cudaMemcpy(hdr.data(), h->d_hdr, hdr.size() * sizeof(fl_template_hdr_t), cudaMemcpyDeviceToHost));
+  std::vector<fl_reco_tmpl> tab((size_t)h->n_templates);
+  int max_pts = 16;
+  bool any_crop = false;
+  for (int t = 0; t < h->n_templates; ++t) {
+    fl_reco_tmpl& e = tab[t];
+    memset(&e, 0, sizeof e);
+    const int c = crop_of_template[t];
+    if (c < -1 || c >= (int)h->res_rect.size()) { fl_set_error("fl_set_recognition: crop %d of template %d is not in the uploaded set", c, t); return FL_ERR_ARG; }
+    if (c >= 0) {
+      const fl_template_hdr_t& b = hdr[(size_t)t * per];                           // current_template[0] (:111, :127-132)
+      const fl_rect_t& r = h->res_rect[c];
+      if (r.x != b.offset_x || r.y != b.offset_y || r.width != b.width || r.height != b.height) {
+        fl_set_error("fl_set_recognition: crop %d was uploaded with a rect other than template %d's level-0 box", c, t); return FL_ERR_ARG;
+      }
+      e.crop = h->d_resident + h->res_off[c]; e.rect = r;
+      max_pts = std::max(max_pts, r.width * r.height);
+      any_crop = true;
+    }
+    memcpy(e.pose, pose12 ? pose12 + (size_t)t * 12 : &h->pose13_h[(size_t)t * 13], 12 * sizeof(float));
+  }
+  h->reco_set = false;
+  TRY(icp_reserve(h, (int)max_hyp, max_pts));                                     // now, so that no frame allocates
+  cudaFree(h->d_reco_tmpl); h->d_reco_tmpl = nullptr;
+  TRY(dalloc(&h->d_reco_tmpl, tab.size()));
+  FL_CUDA(cudaMemcpy(h->d_reco_tmpl, tab.data(), tab.size() * sizeof(fl_reco_tmpl), cudaMemcpyHostToDevice));
+  if (!h->d_reco_sel) TRY(dalloc(&h->d_reco_sel, FL_RECO_SEL_HDR + FL_RECO_MAX_HYP));
+  if (!h->h_reco) {
+    FL_CUDA(cudaHostAlloc((void**)&h->h_reco, FL_RECO_SUMMARY_WORDS * sizeof(int) + FL_RECO_MAX_HYP * sizeof(fl_reco_result_t), cudaHostAllocMapped));
+    FL_CUDA(cudaHostGetDevicePointer((void**)&h->d_reco_host, h->h_reco, 0));
+  }
+  h->reco = *prm; h->reco_max_hyp = (int)max_hyp; h->reco_any_crop = any_crop; h->reco_set = true;
+  return FL_OK;
+}
+
+// selection -> ICP -> finish on the sorted list in d_out.  check_big: the list came from the fused refinement + sort, which leaves
+// lists of more than 1,024 records unsorted and flagged (k_reco_select then selects nothing and reports the frame deferred)
+static int reco_enqueue(fl_handle* h, bool check_big) {
+  cudaStream_t s = h->stream;
+  const int max_hyp = h->reco_max_hyp;
+  int nl = fl_launch_reco_select(h->d_out, reinterpret_cast<const int*>(h->d_outblk), h->p.max_candidates, check_big ? 1 : 0, h->d_class_first, h->n_classes,
+                                 h->n_templates, h->d_reco_tmpl, h->reco.top_k, h->reco.per_class, max_hyp, h->reco_W, h->reco_H, h->d_hyps, h->d_reco_sel, s);
+  if (nl < 0) { fl_set_error("hypothesis selection launch failed: %s", cudaGetErrorString(cudaGetLastError())); return FL_ERR_CUDA; }
+  h->launches += nl;
+  fl_icp_ws ws = h->icp;
+  ws.n_hyp = max_hyp;                                                              // padding hypotheses are skipped by the kernel
+  nl = fl_launch_icp(ws, h->reco.icp, h->d_hyps, h->d_in_depth, h->reco_W, h->reco_H, h->reco_K, h->d_results, h->d_icp_ticket, nullptr, h->n_sm, s);
+  if (nl < 0) { fl_set_error("ICP kernel launch failed: %s", cudaGetErrorString(cudaGetLastError())); return FL_ERR_CUDA; }
+  h->launches += nl;
+  nl = fl_launch_reco_finish(h->d_out, h->d_reco_sel, h->d_results, max_hyp, h->reco.th_obj_dist, h->d_reco_host, s);
+  if (nl < 0) { fl_set_error("recognition finish launch failed: %s", cudaGetErrorString(cudaGetLastError())); return FL_ERR_CUDA; }
+  h->launches += nl;
+  return FL_OK;
+}
+
+extern "C" int fl_recognize_async(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
+                                  int32_t sW, int32_t sH, int32_t W, int32_t H, fl_intrinsics_t K_ref) {
+  if (!h || !depth || sW <= 0 || sH <= 0) return FL_ERR_ARG;
+  const fl_params_t& p = h->p;
+  if (h->pend_sort) { fl_set_error("the previous frame of this handle has not been waited for"); return FL_ERR_STATE; }
+  if (!h->reco_set) { fl_set_error("fl_recognize: call fl_set_recognition after the template and crop uploads"); return FL_ERR_STATE; }
+  h->in_depth_W = h->in_depth_H = 0;
+  if (W <= 0 || H <= 0 || W > p.max_width || H > p.max_height) return FL_ERR_SIZE;
+  if (h->reco_any_crop && (W != h->res_W || H != h->res_H)) { fl_set_error("model depth crops were uploaded for %d x %d frames, not %d x %d", h->res_W, h->res_H, W, H); return FL_ERR_STATE; }
+  FL_CUDA(cudaSetDevice(p.device));
+  const uint8_t* d_bgr; const uint16_t* d_depth;
+  if (sW == W && sH == H) {                                                      // TImage2Mat resizes only when the size differs (:42)
+    const void* d_masks[FL_MAX_MODALITIES];
+    bool any_mask;
+    TRY(stage_frame(h, bgr, bgr_stride, depth, depth_stride, W, H, nullptr, &d_bgr, &d_depth, d_masks, &any_mask));
+  } else {
+    TRY(stage_rescaled(h, bgr, bgr_stride, depth, depth_stride, sW, sH, W, H, &d_bgr, &d_depth));
+  }
+  TRY(fl_match_device_async(h, d_bgr, d_depth, W, H, nullptr, h->reco.threshold, nullptr, 0));
+  h->in_depth_W = W; h->in_depth_H = H;
+  h->reco_W = W; h->reco_H = H; h->reco_K = K_ref;
+  TRY(reco_enqueue(h, true));
+  h->pend_reco = true;
+  return FL_OK;
+}
+
+extern "C" int fl_recognize_wait(fl_handle* h, fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary) {
+  if (!h || capacity < 0 || (capacity > 0 && !out)) return FL_ERR_ARG;
+  if (summary) memset(summary, 0, sizeof *summary);
+  if (!h->pend_reco) { fl_set_error("fl_recognize_wait: no recognition frame in flight on this handle"); return FL_ERR_STATE; }
+  h->pend_reco = false;
+  const bool forced_before = h->fe_force_waves;
+  // the frame's one wait; the rare > 1,024-record sorts and the re-run after a front-end dependency time-out are fl_match_wait's
+  TRY(match_wait(h));
+  const volatile int* blk = h->h_reco;
+  if ((blk[4] & FL_RECO_DEFERRED) || (h->fe_force_waves && !forced_before)) {
+    // the selection ran on a list that was not sorted yet, or on a frame that has been re-run since: once more on the final list
+    TRY(reco_enqueue(h, false));
+    FL_CUDA(wait_stream(h));
+  }
+  FL_CUDA(cudaGetLastError());
+  if (h->overflow) {                                                             // matchClass produced more candidates than the buffers hold
+    if (summary) summary->n_matches = h->h_small[0];
+    fl_set_error("fl_recognize: more candidates than the handle's buffers hold (max_candidates)");
+    return FL_ERR_CAPACITY;
+  }
+  const int n = blk[3];
+  if (summary) { summary->n_matches = blk[0]; summary->n_hypotheses = blk[1]; summary->n_roi = blk[2]; summary->n_results = n; }
+  if (std::min(n, (int)capacity) > 0) memcpy(out, h->h_reco + FL_RECO_SUMMARY_WORDS, sizeof(fl_reco_result_t) * (size_t)std::min(n, (int)capacity));
+  return n > capacity ? FL_ERR_CAPACITY : FL_OK;
+}
+
+extern "C" int fl_recognize(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
+                            int32_t sW, int32_t sH, int32_t W, int32_t H, fl_intrinsics_t K_ref,
+                            fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary) {
+  if (summary) memset(summary, 0, sizeof *summary);
+  TRY(fl_recognize_async(h, bgr, bgr_stride, depth, depth_stride, sW, sH, W, H, K_ref));
+  return fl_recognize_wait(h, out, capacity, summary);
 }

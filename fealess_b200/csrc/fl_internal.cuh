@@ -26,6 +26,7 @@ struct fl_sort_key { unsigned long long hi, lo; };
 
 void fl_set_error(const char* fmt, ...);
 int fl_entries_per_template(const fl_handle* h);   // n_levels * n_modalities of the handle (api.cu)
+bool fl_recognition_pending(const fl_handle* h);   // a fl_recognize_async frame is in flight on the handle (api.cu)
 
 // ---- programmatic dependent launch (PDL) -------------------------------------------------------------------------
 // A kernel launched with cudaLaunchAttributeProgrammaticStreamSerialization may have its CTAs resident while the previous kernel
@@ -218,3 +219,46 @@ int fl_launch_icp(fl_icp_ws ws, fl_icp_params_t p, const fl_icp_hyp* hyps_or_nul
                   fl_icp_result_t* results, int* ticket, unsigned long long* trace, int n_sm, cudaStream_t s);
 void fl_launch_nms(const float* t3, const int32_t* n_model, const float* icp_dist, int n, float th, int32_t* out_idx,
                    int32_t* out_count, cudaStream_t s);
+#ifdef __CUDACC__
+// greedy nonMaximumSuppression (order dependent, n is small): ONE thread walks the list exactly like NMS.cpp:6-39.  out_idx[k] = the
+// object emitted k-th, done[i] = 1 for every object the reference marks check_done (:27).  Shared by k_nms and k_reco_finish.
+__device__ inline int fl_nms_greedy(const float* __restrict__ t3, const int32_t* __restrict__ n_model, const float* __restrict__ icp_dist, int n,
+                                    float th, int32_t* __restrict__ out_idx, uint8_t* __restrict__ done) {
+  int cnt = 0;
+  for (int i = 0; i < n; ++i) done[i] = 0;
+  for (int i = 0; i < n; ++i) {
+    if (done[i]) continue;
+    int win = i;
+    const int size_th = (int)((double)(float)n_model[i] * 0.85);   // static_cast<int>((float)size * 0.85) (:17)
+    for (int j = i + 1; j < n; ++j) {
+      if (done[j]) continue;
+      double s = 0;
+      for (int k = 0; k < 3; ++k) { double d = (double)__fsub_rn(t3[3 * win + k], t3[3 * j + k]); s += d * d; }   // cv::norm(Mat, Mat): fp32 difference, fp64 squares
+      if (sqrt(s) < (double)th) {
+        done[j] = 1;
+        if (n_model[j] > size_th && icp_dist[j] < icp_dist[win]) win = j;
+      }
+    }
+    out_idx[cnt++] = win;
+  }
+  return cnt;
+}
+#endif
+
+// ---- Recognition on the device (reco.cu) -----------------------------------------------------------
+// per-template record of fl_set_recognition: the template's depth crop (NULL = none) with the rect it was uploaded with (= the
+// template's level-0 modality-0 box) and the pose the mirrors look up for it, rows of (R | t)
+struct fl_reco_tmpl { const uint16_t* crop; fl_rect_t rect; float pose[12]; };
+// per-frame selection state written by k_reco_select: {n_matches, n_hyp, deferred, 0, match index of hypothesis 0 .. max_hyp - 1}
+#define FL_RECO_SEL_HDR 4
+// summary words at the head of the mapped host block: {n_matches, n_hyp, n_roi, n_results, flags, ...}, records behind them
+#define FL_RECO_SUMMARY_WORDS 16
+#define FL_RECO_DEFERRED 1        // flags: the list was not sorted yet when the selection ran (more records than the fused sort holds)
+// hypothesis selection after the sort: hyps[0, max_hyp) (padding: status FL_ERR_STATE), sel as above.  check_big: honour the sort's
+// "list not sorted" flag (d_hdr[2]); 0 when the host has just sorted the list itself.
+int fl_launch_reco_select(const fl_match_t* matches, const int* d_hdr, int out_cap, int check_big, const int32_t* class_first, int n_classes,
+                          int n_templates, const fl_reco_tmpl* tmpl, int top_k, int per_class, int max_hyp, int W, int H,
+                          fl_icp_hyp* hyps, int* sel, cudaStream_t s);
+// objects that came out of ICP -> [NMS] -> fl_reco_result_t records + summary posted to mapped host memory (host_block)
+int fl_launch_reco_finish(const fl_match_t* matches, const int* sel, const fl_icp_result_t* results, int max_hyp, float th_obj_dist,
+                          int* host_block, cudaStream_t s);

@@ -876,24 +876,7 @@ int fl_launch_icp(fl_icp_ws ws, fl_icp_params_t p, const fl_icp_hyp* hyps_or_nul
 __global__ void k_nms(const float* __restrict__ t3, const int32_t* __restrict__ n_model, const float* __restrict__ icp_dist, int n, float th,
                       int32_t* __restrict__ out_idx, int32_t* __restrict__ out_count, uint8_t* __restrict__ done) {
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
-  int cnt = 0;
-  for (int i = 0; i < n; ++i) done[i] = 0;
-  for (int i = 0; i < n; ++i) {
-    if (done[i]) continue;
-    int win = i;
-    const int size_th = (int)((double)(float)n_model[i] * 0.85);   // static_cast<int>((float)size * 0.85) (:17)
-    for (int j = i + 1; j < n; ++j) {
-      if (done[j]) continue;
-      double s = 0;
-      for (int k = 0; k < 3; ++k) { double d = (double)__fsub_rn(t3[3 * win + k], t3[3 * j + k]); s += d * d; }   // cv::norm(Mat, Mat): fp32 difference, fp64 squares
-      if (sqrt(s) < (double)th) {
-        done[j] = 1;
-        if (n_model[j] > size_th && icp_dist[j] < icp_dist[win]) win = j;
-      }
-    }
-    out_idx[cnt++] = win;
-  }
-  *out_count = cnt;
+  *out_count = fl_nms_greedy(t3, n_model, icp_dist, n, th, out_idx, done);
 }
 
 void fl_launch_nms(const float* t3, const int32_t* n_model, const float* icp_dist, int n, float th, int32_t* out_idx, int32_t* out_count,

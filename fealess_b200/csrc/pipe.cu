@@ -138,3 +138,49 @@ extern "C" int fl_pipe_match_batch(fl_pipe* p, int32_t n_frames, const void* con
   while (fl_pipe_in_flight(p)) { const int rc = collect(); if (rc != FL_OK) { while (fl_pipe_in_flight(p)) { int32_t c; fl_pipe_collect(p, nullptr, 0, &c); } return rc; } }
   return status;
 }
+
+// Recognition over the pipe (fl_recognize_async / fl_recognize_wait per slot): one host thread keeps `depth` whole frames - match, ICP,
+// suppression - in flight, and takes their results back in submission order.  The crops and the recognition setup go to every slot.
+extern "C" int fl_pipe_upload_model_depths(fl_pipe* p, int32_t n_models, const uint16_t* const* model_depth, const size_t* model_stride,
+                                           const fl_rect_t* rect_model, int32_t W, int32_t H) {
+  if (!p) return FL_ERR_ARG;
+  if (p->submitted != p->collected) { fl_set_error("fl_pipe_upload_model_depths: %lld frame(s) still in flight", p->submitted - p->collected); return FL_ERR_STATE; }
+  for (fl_handle* h : p->h) {
+    const int rc = fl_upload_model_depths(h, n_models, model_depth, model_stride, rect_model, W, H);
+    if (rc != FL_OK) return rc;
+  }
+  return FL_OK;
+}
+
+extern "C" int fl_pipe_set_recognition(fl_pipe* p, const fl_reco_params_t* params, const int32_t* crop_of_template, const float* pose12) {
+  if (!p) return FL_ERR_ARG;
+  if (p->world > 1) { fl_set_error("fl_pipe_set_recognition: not available on a template-sharded pipe"); return FL_ERR_STATE; }
+  if (p->submitted != p->collected) { fl_set_error("fl_pipe_set_recognition: %lld frame(s) still in flight", p->submitted - p->collected); return FL_ERR_STATE; }
+  for (fl_handle* h : p->h) {
+    const int rc = fl_set_recognition(h, params, crop_of_template, pose12);
+    if (rc != FL_OK) return rc;
+  }
+  return FL_OK;
+}
+
+extern "C" int fl_pipe_submit_recognition(fl_pipe* p, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
+                                          int32_t src_W, int32_t src_H, int32_t W, int32_t H, fl_intrinsics_t K_ref) {
+  if (!p) return FL_ERR_ARG;
+  if (p->world > 1) { fl_set_error("fl_pipe_submit_recognition: not available on a template-sharded pipe"); return FL_ERR_STATE; }
+  if (p->submitted - p->collected >= p->depth) { fl_set_error("fl_pipe_submit_recognition: %d frames in flight already - collect one first", p->depth); return FL_ERR_STATE; }
+  const int rc = fl_recognize_async(p->h[p->submitted % p->depth], bgr, bgr_stride, depth, depth_stride, src_W, src_H, W, H, K_ref);
+  if (rc != FL_OK) return rc;
+  ++p->submitted;
+  return FL_OK;
+}
+
+extern "C" int fl_pipe_collect_recognition(fl_pipe* p, fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary) {
+  if (!p) return FL_ERR_ARG;
+  if (summary) memset(summary, 0, sizeof *summary);
+  if (p->submitted == p->collected) { fl_set_error("fl_pipe_collect_recognition: no frame in flight"); return FL_ERR_STATE; }
+  fl_handle* h = p->h[p->collected % p->depth];
+  // the oldest frame came from fl_pipe_submit: it stays in flight for fl_pipe_collect (waiting for it here would leave nothing to fetch)
+  if (!fl_recognition_pending(h)) { fl_set_error("fl_pipe_collect_recognition: the oldest frame in flight is a match frame - fl_pipe_collect it"); return FL_ERR_STATE; }
+  ++p->collected;                                               // the slot is free again whatever the frame's status
+  return fl_recognize_wait(h, out, capacity, summary);
+}

@@ -19,6 +19,11 @@
 launch (``fl_detection_batch``) and filtered by the reference's ``nonMaximumSuppression`` (ICP/NMS.cpp:6-39).  The defaults
 (``top_k=1``, no NMS) are exactly the reference's behaviour.
 
+``submit`` / ``collect`` (not in the reference) are the same Recognition as a stream: each frame is ONE enqueue on the device
+(``fl_pipe_submit_recognition``: rescale, match, hypothesis selection, ICP and suppression with no host round trip in between), up to
+``frames_in_flight`` frames are in flight from the calling thread, and ``collect`` returns what ``Recognition`` returns for the
+oldest one.
+
 Kept from the reference on purpose (``SURVEY.md`` A.6 v): ``detection`` receives the CALLER's intrinsics, not the zoomed ones.
 """
 from __future__ import annotations
@@ -53,7 +58,7 @@ def select_hypotheses(matches, top_k: int = 1, per_class: bool = False):
 
 
 class ObjRecoLmICP:
-    def __init__(self, device: int = 0, max_width: int = 640, max_height: int = 480):
+    def __init__(self, device: int = 0, max_width: int = 640, max_height: int = 480, frames_in_flight: int = 1):
         self.m_matching_threshold = 75.0                             # :52-55
         self.m_icp_it_thr, self.m_dist_mean_thr, self.m_dist_diff_thr = 10, 0.5, 0.01
         self._args = (device, max_width, max_height)
@@ -62,6 +67,10 @@ class ObjRecoLmICP:
         self._resident: Optional[Tuple[tuple, Dict[Tuple[str, int], int]]] = None     # (frame shape, crop index) once uploaded
         self.m_cam = None
         self.last_icp_path = None                                    # "resident" / "per-call": which ICP entry the last Recognition took
+        self.frames_in_flight = int(frames_in_flight)                # submit / collect: frames one thread keeps on the device
+        self._pipe = None
+        self._stream_key = None                                      # what the pipe is set up for (_stream_setup)
+        self.last_summary = None
 
     # ---- AddObj ----
     def AddObj(self, str_feature_path: str) -> int:
@@ -83,14 +92,23 @@ class ObjRecoLmICP:
                 if img is not None:
                     depths[(None, tid)] = model_depth_to_mm(img)     # the reference keys the file by template_id alone (:156)
         self.m_lm_detector, self._model_depth, self._resident = det, depths, None
+        self._close_stream()
         return 0
 
     def add_detector(self, detector, model_depths_mm: Dict[Tuple[Optional[str], int], np.ndarray]) -> None:
         """Programmatic alternative to ``AddObj``: a ready detector + model depth images in mm keyed by (class_id or None, template_id)."""
         self.m_lm_detector, self._model_depth, self._resident = detector, dict(model_depths_mm), None
+        self._close_stream()
 
     def _upload_model_crops(self, frame_shape) -> Dict[Tuple[str, int], int]:
         """(class_id, template_id) -> index of the template's depth crop on the device; uploaded once per detector."""
+        index, images, rects = self._crop_table(frame_shape)
+        if images:
+            self.m_lm_detector._handle.upload_model_depths(images, rects)
+        return index
+
+    def _crop_table(self, frame_shape):
+        """(class_id, template_id) -> crop index, and the crops' images and rects (the templates' level-0 boxes)."""
         det, index, images, rects = self.m_lm_detector, {}, [], []
         for cid in det.classIds():
             for tid in range(det.numTemplates(cid)):
@@ -102,9 +120,7 @@ class ObjRecoLmICP:
                     continue                                          # such a hypothesis takes the per-call path (and its ROI error)
                 index[(cid, tid)] = len(images)
                 images.append(md); rects.append((ox, oy, w, h))
-        if images:
-            det._handle.upload_model_depths(images, rects)
-        return index
+        return index, images, rects
 
     # ---- PrepareInputData ----
     def _prepare(self, rgb, depth, K) -> Optional[Tuple[np.ndarray, np.ndarray]]:
@@ -193,3 +209,79 @@ class ObjRecoLmICP:
             keep = nonMaximumSuppression(objs, th_obj_dist, det._handle)
             out = [out[k["index"]] for k in keep]
         return 0, out
+
+    # ---- Recognition as a stream (submit / collect) ----
+    def submit(self, rgb: np.ndarray, depth: np.ndarray, K: dict, top_k: int = 1, th_obj_dist: Optional[float] = None, per_class: bool = False) -> int:
+        """Queues ``Recognition(rgb, depth, K, top_k, th_obj_dist, per_class)`` as one enqueue on the device and returns 0 (the result
+        comes from ``collect``), or ERROR_INVALID_PARAM without queueing where ``Recognition`` returns it before matching.  The arrays
+        must not change until the frame has been collected (page-locked ones are read by DMA).  Changing the hypothesis settings, the
+        matching threshold or ICP attributes, the detector's templates or the frame size needs an empty stream.
+        One difference from ``Recognition``: a template whose depth image does not have the processing size (or does not hold the
+        template's level-0 box) has no crop on the device and its hypothesis is dropped; ``Recognition`` refines such a template through
+        the per-call ``detection_batch`` path instead."""
+        if self.m_lm_detector is None:
+            return ERROR_INVALID_PARAM
+        prep = self._prepare(rgb, depth, K)
+        if prep is None:
+            return ERROR_INVALID_PARAM
+        m_rgb, m_depth = prep
+        fw, fh = self.m_cam["width"], self.m_cam["height"]
+        if m_rgb.shape[1] == fw and len(self.m_lm_detector.getModalities()) != 2:
+            return ERROR_INVALID_PARAM                                # Recognition's match() gets two sources: -1 (linemod.cpp:1364-1367)
+        self._stream_setup((fh, fw), max(1, int(top_k)), bool(per_class), th_obj_dist)
+        from . import FL_ERR_SIZE, FealessError
+        Kc = (float(K["fx"]), float(K["fy"]), float(K["cx"]), float(K["cy"]))   # the caller's intrinsics (:188)
+        bgr = m_rgb if "ColorGradient" in self.m_lm_detector.getModalities() else None
+        try:
+            self._pipe.submit_recognition(bgr, m_depth, Kc, fw, fh)
+        except FealessError as e:
+            if e.rc == FL_ERR_SIZE:                                   # match() returns -1 (linemod.cpp:1364-1378)
+                return ERROR_INVALID_PARAM
+            raise
+        return 0
+
+    def collect(self):
+        """(status, results) of the oldest submitted frame: what ``Recognition`` returns for it, result for result and bit for bit."""
+        from . import FL_ERR_STATE, FL_OK, FealessError
+        if self._pipe is None:
+            raise FealessError(FL_ERR_STATE, "ObjRecoLmICP.collect", "no frame in flight")
+        rc, recs, self.last_summary = self._pipe.collect_recognition()   # {n_matches, n_hypotheses, n_roi, n_results} of that frame
+        if rc != FL_OK:                                               # more candidates than the device buffers hold: Detector.match raises too
+            raise FealessError(rc, "ObjRecoLmICP.collect", "capacity")
+        names = self.m_lm_detector.classIds()
+        return 0, [dict(strObjTag=names[int(r["class_idx"])], tWorld2Cam=r["world2cam"].reshape(4, 4).copy(), similarity=float(r["similarity"]),
+                        template_id=int(r["template_id"]), icp=r["icp"].copy()) for r in recs]
+
+    def in_flight(self) -> int:
+        return 0 if self._pipe is None else self._pipe.in_flight()
+
+    def _stream_setup(self, frame_shape, top_k: int, per_class: bool, th_obj_dist: Optional[float]) -> None:
+        """The pipe behind submit / collect: the detector's templates, the crops of ``frame_shape`` and the recognition setup on every slot.
+        Crop index and pose table are Recognition's: crops keyed by (class, template_id), pose = getPoseInfo(template_id, class_id)."""
+        from . import FL_ERR_STATE, FealessError, Pipe, reco_params
+        det = self.m_lm_detector
+        key = (frame_shape, det._revision, top_k, per_class, th_obj_dist, float(self.m_matching_threshold), int(self.m_icp_it_thr),
+               float(self.m_dist_mean_thr), float(self.m_dist_diff_thr))
+        if self._pipe is not None and self._stream_key == key:
+            return
+        if self.in_flight():
+            raise FealessError(FL_ERR_STATE, "ObjRecoLmICP.submit", "frame size, templates or recognition settings changed with frames in flight")
+        if self._pipe is None:
+            T, kinds, max_w, max_h, max_cand, device = det._handle_args
+            self._pipe = Pipe(self.frames_in_flight, T, kinds, max_w, max_h, device, max_cand)
+        new_templates = self._stream_key is None or self._stream_key[1] != det._revision
+        if new_templates:
+            self._pipe.upload_templates(det.template_set())
+        if new_templates or self._stream_key[0] != frame_shape:
+            index, images, rects = self._crop_table(frame_shape)
+            self._pipe.upload_model_depths(images, rects)
+            self._stream_crop = np.array([index.get((cid, tid), -1) for cid in det.classIds() for tid in range(det.numTemplates(cid))], np.int32)
+        th = 0.0 if th_obj_dist is None else float(th_obj_dist)       # <= 0: no suppression, what NMS over distance th <= 0 keeps anyway
+        self._pipe.set_recognition(self._stream_crop, None, reco_params(self.m_matching_threshold, (self.m_icp_it_thr, self.m_dist_mean_thr,
+                                                                                                     self.m_dist_diff_thr), top_k, per_class, th))
+        self._stream_key = key
+
+    def _close_stream(self) -> None:
+        if self._pipe is not None:
+            self._pipe.close()
+        self._pipe, self._stream_key = None, None

@@ -325,6 +325,59 @@ int fl_nms(fl_handle* h, const float* t3, const int32_t* n_model_pts, const floa
 int fl_nms_ex(fl_handle* h, const float* t3, const int32_t* n_model_pts, const float* icp_dist, int32_t n,
               float th_obj_dist, int32_t* out_idx, uint8_t* absorbed);
 
+/* ---- Recognition on the device (CObjRecoLmICP::Recognition, CadReco/obj_reco_lmicp.cpp:86-204) ----------------------------------
+ * The whole frame as ONE enqueue: [INTER_LINEAR rescale] + front end + similarity + refinement / sort + hypothesis selection + ICP +
+ * nonMaximumSuppression + pose packing, with the results posted to mapped pinned host memory, so that fl_recognize_wait is the
+ * frame's only host wait (a frame whose unique list exceeds 1,024 records, or whose front end timed out, takes the recovery of
+ * fl_match_wait and one more wait).  Selection, hypotheses and results are those of the mirrors (fealess_b200/reco.py,
+ * include/fealess_b200/obj_reco.hpp): the first top_k matches, or the first top_k of every class (per_class), in list order;
+ * model rect = the template's level-0 modality-0 box, reference rect = that box moved to the match position; a selected match
+ * whose template has no depth crop is dropped (it still counts toward top_k); a reference rect outside the W x H frame gives
+ * FL_ERR_ROI for that hypothesis and no result; nonMaximumSuppression over the refined objects when th_obj_dist > 0. */
+#define FL_RECO_MAX_HYP 256
+typedef struct {
+  float threshold;            /* matching threshold, default 75 (:52-55) */
+  fl_icp_params_t icp;        /* default {10, 0.5, 0.01} (:52-55) */
+  int32_t top_k, per_class;   /* default 1, 0: ICP of matches[0] (:111) */
+  float th_obj_dist;          /* mm; <= 0 (default): no suppression */
+} fl_reco_params_t;
+void fl_default_reco_params(fl_reco_params_t* p);
+/* After fl_upload_templates and fl_upload_model_depths: crop_of_template[n_templates] = index of template t's crop in the uploaded
+ * set (-1 = no crop; the crop's rect must be the template's level-0 modality-0 box), pose12 (nullable: the first 12 floats of the
+ * uploaded pose13) = 12 floats per template, rows of (R | t).  Sizes the ICP workspace for top_k * (per_class ? n_classes : 1)
+ * hypotheses now, so that no frame allocates.  FL_ERR_CAPACITY above FL_RECO_MAX_HYP; FL_ERR_STATE on a handle with
+ * fl_set_template_ids, with a frame in flight, or without templates.  A later fl_upload_templates / fl_upload_model_depths /
+ * fl_set_template_ids clears the setup. */
+int fl_set_recognition(fl_handle* h, const fl_reco_params_t* p, const int32_t* crop_of_template, const float* pose12);
+typedef struct {
+  int32_t class_idx, template_id, x, y;   /* the match the object came from */
+  float similarity;
+  int32_t hypothesis;                     /* its index among the frame's hypotheses */
+  float world2cam[16];                    /* [R | T; 0 0 0 1] row-major (Convert, :20-30) */
+  fl_icp_result_t icp;
+} fl_reco_result_t;
+typedef struct { int32_t n_matches, n_hypotheses, n_roi, n_results; } fl_reco_summary_t;
+/* enqueue-only half: the src_W x src_H frame is uploaded, rescaled on the device to W x H when the sizes differ (as
+ * fl_match_rescaled), and recognised.  depth is required (ICP reads it), bgr as in fl_match.  K_ref = the CALLER's intrinsics,
+ * which the mirrors pass to detection() (:188).  Page-locked caller buffers must stay valid until fl_recognize_wait; pageable
+ * ones are copied before this returns.  One frame in flight per handle. */
+int fl_recognize_async(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
+                       int32_t src_W, int32_t src_H, int32_t W, int32_t H, fl_intrinsics_t K_ref);
+/* waits for the frame, writes min(n_results, capacity) results and the summary (nullable).  FL_ERR_CAPACITY: more results than
+ * capacity, or more candidates than the handle's buffers hold (then no results, as fl_match_fetch). */
+int fl_recognize_wait(fl_handle* h, fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary);
+int fl_recognize(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
+                 int32_t src_W, int32_t src_H, int32_t W, int32_t H, fl_intrinsics_t K_ref,
+                 fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary);
+/* The same over a pipe: one host thread keeps up to `depth` frames in flight; results come back in submission order.  Setup on
+ * every slot (FL_ERR_STATE while frames are in flight); FL_ERR_STATE on a template-sharded pipe (fl_pipe_set_exchange). */
+int fl_pipe_upload_model_depths(fl_pipe* p, int32_t n_models, const uint16_t* const* model_depth, const size_t* model_stride,
+                                const fl_rect_t* rect_model, int32_t W, int32_t H);
+int fl_pipe_set_recognition(fl_pipe* p, const fl_reco_params_t* params, const int32_t* crop_of_template, const float* pose12);
+int fl_pipe_submit_recognition(fl_pipe* p, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
+                               int32_t src_W, int32_t src_H, int32_t W, int32_t H, fl_intrinsics_t K_ref);
+int fl_pipe_collect_recognition(fl_pipe* p, fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary);
+
 /* ---- stage-level debug exports (host copies of device intermediates of the LAST match call) -------- */
 enum {
   FL_DBG_QUANTIZED = 0,     /* (level, modality)         -> (W>>l)*(H>>l) u8 */

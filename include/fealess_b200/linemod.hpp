@@ -296,6 +296,22 @@ class Detector {
   // the C-ABI handle behind this detector (created on first match), e.g. for fl_profile / fl_last_stage_ms
   fl_handle* handle() const { return handle_; }
 
+  // mirror-only: a pipe of `depth` handles for frames up to W x H that hold this detector's templates in the order match() uploads them
+  // (classes by id, templates by template_id), on the detector's device.  The caller owns it (fl_pipe_destroy).
+  fl_pipe* createPipe(int depth, int W, int H) const {
+    if (devices_.size() > 1) throw cv::Exception("Detector::createPipe is not available together with useDevices()");
+    fl_params_t p = device_params(W, H);
+    if (devices_.size() == 1) p.device = devices_[0];
+    fl_pipe* pipe = nullptr;
+    fealess_b200::check_status(fl_pipe_create(&p, depth, &pipe), "fl_pipe_create");
+    std::vector<fl_template_hdr_t> hdr; std::vector<fl_feature_t> feat; std::vector<int32_t> class_of;
+    flatten(hdr, feat, class_of);
+    const int rc = fl_pipe_upload_templates(pipe, (int32_t)class_of.size(), hdr.data(), feat.data(), (int32_t)feat.size(), class_of.data(), nullptr);
+    if (rc != FL_OK) fl_pipe_destroy(pipe);
+    fealess_b200::check_status(rc, "fl_pipe_upload_templates");
+    return pipe;
+  }
+
  protected:
   std::vector<Ptr<Modality> > modalities;
   int pyramid_levels;
@@ -310,19 +326,7 @@ class Detector {
   void ensure_uploaded(int W, int H) const {
     if (!handle_ || W > cap_w_ || H > cap_h_) {
       release_device();
-      fl_params_t p;
-      fl_default_params(&p);
-      p.n_levels = pyramid_levels;
-      if (pyramid_levels < 1 || pyramid_levels > FL_MAX_LEVELS || modalities.empty() || (int)modalities.size() > FL_MAX_MODALITIES) throw cv::Exception("Detector: unsupported number of pyramid levels / modalities");
-      for (int l = 0; l < pyramid_levels; ++l) p.T[l] = T_at_level[l];
-      p.n_modalities = (int)modalities.size();
-      for (int m = 0; m < p.n_modalities; ++m) {
-        p.modality_kind[m] = modalities[m]->kind();
-        if (const ColorGradient* cg = dynamic_cast<const ColorGradient*>(modalities[m].get())) p.weak_threshold = cg->weak_threshold;
-        if (const DepthNormal* dn = dynamic_cast<const DepthNormal*>(modalities[m].get())) { p.distance_threshold = dn->distance_threshold; p.difference_threshold = dn->difference_threshold; }
-      }
-      p.max_width = std::max(W, cap_w_); p.max_height = std::max(H, cap_h_);
-      p.device = fealess_b200::device_ordinal();
+      fl_params_t p = device_params(std::max(W, cap_w_), std::max(H, cap_h_));
       if (devices_.size() > 1) {
         std::vector<int32_t> dv(devices_.begin(), devices_.end());
         fealess_b200::check_status(fl_group_create(&p, dv.data(), (int32_t)dv.size(), xcap_, &group_), "fl_group_create");
@@ -337,8 +341,31 @@ class Detector {
     const size_t fingerprint = (size_t)numTemplates() * 4099u + class_templates.size();
     if (!dirty_ && fingerprint == uploaded_fingerprint_) return;
     uploaded_fingerprint_ = fingerprint;
-    // flatten in std::map (sorted class id) order = the order Detector::match visits the classes (:1418-1423)
     std::vector<fl_template_hdr_t> hdr; std::vector<fl_feature_t> feat; std::vector<int32_t> class_of;
+    flatten(hdr, feat, class_of);
+    if (group_) fealess_b200::check_status(fl_group_upload_templates(group_, (int32_t)class_of.size(), hdr.data(), feat.data(), (int32_t)feat.size(), class_of.data(), nullptr), "fl_group_upload_templates");
+    else fealess_b200::check_status(fl_upload_templates(handle_, (int32_t)class_of.size(), hdr.data(), feat.data(), (int32_t)feat.size(), class_of.data(), nullptr), "fl_upload_templates");
+    dirty_ = false;
+  }
+  // handle parameters of this detector's modalities for frames up to W x H on device_ordinal()
+  fl_params_t device_params(int W, int H) const {
+    fl_params_t p;
+    fl_default_params(&p);
+    p.n_levels = pyramid_levels;
+    if (pyramid_levels < 1 || pyramid_levels > FL_MAX_LEVELS || modalities.empty() || (int)modalities.size() > FL_MAX_MODALITIES) throw cv::Exception("Detector: unsupported number of pyramid levels / modalities");
+    for (int l = 0; l < pyramid_levels; ++l) p.T[l] = T_at_level[l];
+    p.n_modalities = (int)modalities.size();
+    for (int m = 0; m < p.n_modalities; ++m) {
+      p.modality_kind[m] = modalities[m]->kind();
+      if (const ColorGradient* cg = dynamic_cast<const ColorGradient*>(modalities[m].get())) p.weak_threshold = cg->weak_threshold;
+      if (const DepthNormal* dn = dynamic_cast<const DepthNormal*>(modalities[m].get())) { p.distance_threshold = dn->distance_threshold; p.difference_threshold = dn->difference_threshold; }
+    }
+    p.max_width = W; p.max_height = H;
+    p.device = fealess_b200::device_ordinal();
+    return p;
+  }
+  // the template database flattened in std::map (sorted class id) order = the order Detector::match visits the classes (:1418-1423)
+  void flatten(std::vector<fl_template_hdr_t>& hdr, std::vector<fl_feature_t>& feat, std::vector<int32_t>& class_of) const {
     class_names_.clear(); class_index_.clear();
     const size_t per = (size_t)pyramid_levels * modalities.size();
     for (TemplatesMap::const_iterator it = class_templates.begin(); it != class_templates.end(); ++it) {
@@ -357,9 +384,6 @@ class Detector {
         class_of.push_back(ci);
       }
     }
-    if (group_) fealess_b200::check_status(fl_group_upload_templates(group_, (int32_t)class_of.size(), hdr.data(), feat.data(), (int32_t)feat.size(), class_of.data(), nullptr), "fl_group_upload_templates");
-    else fealess_b200::check_status(fl_upload_templates(handle_, (int32_t)class_of.size(), hdr.data(), feat.data(), (int32_t)feat.size(), class_of.data(), nullptr), "fl_upload_templates");
-    dirty_ = false;
   }
   // class filter named only unknown classes: nothing is matched, but the quantised images are still produced (:1411-1412)
   void fill_quantized_only(const uint8_t* bgr, size_t bgr_step, const uint16_t* depth, size_t depth_step, int W, int H, const uint8_t* const* masks,

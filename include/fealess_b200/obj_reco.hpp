@@ -13,6 +13,9 @@
 //                                   fl_match_rescaled), then detection() on matches[0] (:111-189) against the depth frame that is
 //                                   already on the device (fl_detection_batch_resident), pose packed by Convert (:20-30).
 //   Train / ClearObj / SetROI / Set-/GetAdvancedParam: return 0 without doing anything, exactly like the reference (:62-84, 206-214).
+//   SetFramesInFlight / SubmitRecognition / CollectRecognition (not in the reference): the same Recognition as a stream - every frame
+//                                   is ONE enqueue on the device (fl_pipe_submit_recognition: rescale, match, hypothesis selection, ICP,
+//                                   suppression), up to k frames are in flight from one thread, results come back in submission order.
 //
 // Kept from the reference on purpose: detection() receives the CALLER's intrinsics, not the zoomed ones (:188, SURVEY.md A.6 v);
 // only matches[0] is refined (:111).  A rect that leaves the frame raises cv::Exception (the reference's cv::Mat ROI assert,
@@ -80,6 +83,7 @@ class CObjRecoCAD {
 class CObjRecoLmICP : public CObjRecoCAD {
  public:
   CObjRecoLmICP() : m_matching_threshold(75.0f), m_icp_it_thr(10), m_dist_mean_thr(0.5f), m_dist_diff_thr(0.01f), m_proc_w(0), m_proc_h(0), m_crops_w(0), m_crops_h(0) {}   // :47-56
+  virtual ~CObjRecoLmICP() { close_stream(); }
   virtual int Train(const string&, const TScanPackage&, const TTrainParam&) { return 0; }
   virtual int ClearObj() { return 0; }
   virtual int SetROI(const TImageU&) { return 0; }
@@ -90,6 +94,7 @@ class CObjRecoLmICP : public CObjRecoCAD {
     m_str_lm_feature_path = str_feature_path;
     m_lm_detector = readLinemod(m_str_lm_feature_path + string("/linemod_templates.yml"));
     m_model_depth.clear(); m_crop_index.clear(); m_crops_w = m_crops_h = 0;
+    close_stream();
     if (0 == m_lm_detector->numClasses()) return (int)ERROR_OPEN_FILE_FAILED;
     // the reference names the file by template_id alone (:156), so one image serves that id in every class
     int max_templates = 0;
@@ -176,6 +181,42 @@ class CObjRecoLmICP : public CObjRecoCAD {
   // distance (mm) under which nonMaximumSuppression merges refined objects (0 = no suppression).
   void SetHypotheses(int top_k, bool per_class = false, float th_obj_dist = 0.f) { m_top_k = top_k < 1 ? 1 : top_k; m_per_class = per_class; m_th_obj_dist = th_obj_dist; }
 
+  // NOT in the reference: Recognition as a stream.  SubmitRecognition queues what Recognition computes for the frame (same checks and
+  // statuses before matching; the images must stay unchanged until the frame has been collected); CollectRecognition returns the
+  // results of the oldest queued frame, equal to Recognition's, and throws where Recognition throws.  Up to k frames
+  // (<= FL_PIPE_MAX_DEPTH) are in flight; SetFramesInFlight, SetHypotheses and a new frame size take effect on an empty stream.
+  void SetFramesInFlight(int k) {
+    if (m_pipe && fl_pipe_in_flight(m_pipe)) throw std::runtime_error("SetFramesInFlight: frames are in flight");
+    m_frames_in_flight = k < 1 ? 1 : k > FL_PIPE_MAX_DEPTH ? FL_PIPE_MAX_DEPTH : k;
+    close_stream();
+  }
+  int SubmitRecognition(const TImageU& tRGB, const TImageU16& tDepth, const TCamIntrinsicParam& tCamIntrinsic) {
+    if (!m_lm_detector || 0 != PrepareInputData(tRGB, tDepth, tCamIntrinsic)) return (int)ERROR_INVALID_PARAM;
+    if (m_lm_detector->getModalities().size() != 2) return (int)ERROR_INVALID_PARAM;   // as Recognition
+    stream_setup();
+    const fl_intrinsics_t K = {(float)tCamIntrinsic.dFx, (float)tCamIntrinsic.dFy, (float)tCamIntrinsic.dCx, (float)tCamIntrinsic.dCy};   // the caller's (:188)
+    const int rc = fl_pipe_submit_recognition(m_pipe, tRGB.pData, (size_t)tRGB.nWidth * 3, tDepth.pData, (size_t)tDepth.nWidth * 2, tRGB.nWidth, tRGB.nHeight,
+                                              m_proc_w, m_proc_h, K);
+    if (rc == FL_ERR_SIZE) return (int)ERROR_INVALID_PARAM;
+    fealess_b200::check_status(rc, "SubmitRecognition");
+    return 0;
+  }
+  int CollectRecognition(vector<TObjRecoResult>& vtResult) {
+    vtResult.clear();
+    if (!m_pipe) fealess_b200::check_status(FL_ERR_STATE, "CollectRecognition: no frame in flight");
+    std::vector<fl_reco_result_t> res(FL_RECO_MAX_HYP);
+    fl_reco_summary_t sum;
+    fealess_b200::check_status(fl_pipe_collect_recognition(m_pipe, res.data(), (int32_t)res.size(), &sum), "CollectRecognition");
+    if (sum.n_hypotheses == 1 && sum.n_roi == 1) fealess_b200::check_status(FL_ERR_ROI, "detection");   // Recognition's single detection() throws (detection.cpp:43-44)
+    for (int k = 0; k < sum.n_results; ++k) {
+      TObjRecoResult cur_result;
+      cur_result.strObjTag = m_stream_classes[(size_t)res[k].class_idx];
+      std::memcpy(cur_result.tWorld2Cam, res[k].world2cam, sizeof cur_result.tWorld2Cam);
+      vtResult.push_back(cur_result);
+    }
+    return 0;
+  }
+
   // mirror-only accessors (tests, callers that want the zoomed intrinsics PrepareInputData stored)
   const TCamIntrinsicParam& processingIntrinsics() const { return m_tCamParam; }
   cv::Ptr<cup_linemod::Detector> detector() const { return m_lm_detector; }
@@ -225,8 +266,15 @@ class CObjRecoLmICP : public CObjRecoCAD {
   // crop every template's depth image to its level-0 box and keep the crops on the device; once per detector and frame size
   void upload_crops() {
     if (m_crops_w == m_proc_w && m_crops_h == m_proc_h) return;
-    m_crop_index.clear();
     std::vector<const uint16_t*> ptr; std::vector<size_t> stride; std::vector<fl_rect_t> rect;
+    crop_table(m_crop_index, ptr, stride, rect);
+    fealess_b200::check_status(fl_upload_model_depths(m_lm_detector->handle(), (int32_t)ptr.size(), ptr.data(), stride.data(), rect.data(), m_proc_w, m_proc_h),
+                               "fl_upload_model_depths");
+    m_crops_w = m_proc_w; m_crops_h = m_proc_h;
+  }
+  // the templates whose depth image has the processing size and holds their level-0 box: (class, template_id) -> crop index, crops
+  void crop_table(std::map<std::pair<cv::String, int>, int>& index, std::vector<const uint16_t*>& ptr, std::vector<size_t>& stride, std::vector<fl_rect_t>& rect) const {
+    index.clear();
     const vector<cv::String> ids = m_lm_detector->classIds();
     for (size_t c = 0; c < ids.size(); ++c)
       for (int tid = 0; tid < m_lm_detector->numTemplates(ids[c]); ++tid) {
@@ -235,14 +283,55 @@ class CObjRecoLmICP : public CObjRecoCAD {
         if (!md || md->width != m_proc_w || md->height != m_proc_h || t0.offset_x < 0 || t0.offset_y < 0 || t0.offset_x + t0.width > md->width ||
             t0.offset_y + t0.height > md->height)
           continue;
-        m_crop_index[std::make_pair(ids[c], tid)] = (int)ptr.size();
+        index[std::make_pair(ids[c], tid)] = (int)ptr.size();
         ptr.push_back(md->mm.data()); stride.push_back((size_t)md->width * 2);
         const fl_rect_t r = {t0.offset_x, t0.offset_y, t0.width, t0.height};
         rect.push_back(r);
       }
-    fealess_b200::check_status(fl_upload_model_depths(m_lm_detector->handle(), (int32_t)ptr.size(), ptr.data(), stride.data(), rect.data(), m_proc_w, m_proc_h),
-                               "fl_upload_model_depths");
-    m_crops_w = m_proc_w; m_crops_h = m_proc_h;
+  }
+
+  // the pipe behind SubmitRecognition for the current frame size and hypothesis settings: the detector's templates and the crops on every
+  // slot, the crop index and Recognition's pose rule per template (getPoseInfo(template_id) in the reference's mode top_k = 1 without
+  // per_class, the class-keyed lookup otherwise)
+  void stream_setup() {
+    // templates added to the detector since the pipe was built: the same count check Detector::match uses before it re-uploads
+    const size_t fingerprint = (size_t)m_lm_detector->numTemplates() * 4099u + (size_t)m_lm_detector->numClasses();
+    const bool same_size = m_pipe && m_stream_w == m_proc_w && m_stream_h == m_proc_h && m_stream_fingerprint == fingerprint;
+    if (same_size && m_stream_top_k == m_top_k && m_stream_per_class == m_per_class && m_stream_th == m_th_obj_dist) return;
+    if (m_pipe && fl_pipe_in_flight(m_pipe)) throw std::runtime_error("SubmitRecognition: frame size, templates or hypotheses changed with frames in flight");
+    if (!same_size) {
+      close_stream();
+      m_pipe = m_lm_detector->createPipe(m_frames_in_flight, m_proc_w, m_proc_h);
+      std::map<std::pair<cv::String, int>, int> index;
+      std::vector<const uint16_t*> ptr; std::vector<size_t> stride; std::vector<fl_rect_t> rect;
+      crop_table(index, ptr, stride, rect);
+      fealess_b200::check_status(fl_pipe_upload_model_depths(m_pipe, (int32_t)ptr.size(), ptr.data(), stride.data(), rect.data(), m_proc_w, m_proc_h),
+                                 "fl_pipe_upload_model_depths");
+      m_stream_classes = m_lm_detector->classIds();
+      m_stream_crop.clear();
+      for (size_t c = 0; c < m_stream_classes.size(); ++c)
+        for (int tid = 0; tid < m_lm_detector->numTemplates(m_stream_classes[c]); ++tid) {
+          std::map<std::pair<cv::String, int>, int>::const_iterator it = index.find(std::make_pair(m_stream_classes[c], tid));
+          m_stream_crop.push_back(it == index.end() ? -1 : it->second);
+        }
+      m_stream_w = m_proc_w; m_stream_h = m_proc_h; m_stream_fingerprint = fingerprint;
+    }
+    std::vector<float> pose12;
+    for (size_t c = 0; c < m_stream_classes.size(); ++c)
+      for (int tid = 0; tid < m_lm_detector->numTemplates(m_stream_classes[c]); ++tid) {
+        const std::vector<float> pose = (m_top_k == 1 && !m_per_class) ? m_lm_detector->getPoseInfo(tid) : m_lm_detector->getPoseInfo(m_stream_classes[c], tid);
+        pose12.insert(pose12.end(), pose.begin(), pose.begin() + 12);
+      }
+    fl_reco_params_t prm;
+    fl_default_reco_params(&prm);
+    prm.threshold = m_matching_threshold; prm.icp.icp_it_thr = m_icp_it_thr; prm.icp.dist_mean_thr = m_dist_mean_thr; prm.icp.dist_diff_thr = m_dist_diff_thr;
+    prm.top_k = m_top_k; prm.per_class = m_per_class ? 1 : 0; prm.th_obj_dist = m_th_obj_dist;
+    fealess_b200::check_status(fl_pipe_set_recognition(m_pipe, &prm, m_stream_crop.data(), pose12.data()), "fl_pipe_set_recognition");
+    m_stream_top_k = m_top_k; m_stream_per_class = m_per_class; m_stream_th = m_th_obj_dist;
+  }
+  void close_stream() {
+    if (m_pipe) fl_pipe_destroy(m_pipe);
+    m_pipe = nullptr; m_stream_w = m_stream_h = 0;
   }
 
   string m_str_lm_feature_path;
@@ -254,6 +343,14 @@ class CObjRecoLmICP : public CObjRecoCAD {
   std::map<std::pair<cv::String, int>, int> m_crop_index;        // (class, template_id) -> crop on the device
   int m_crops_w, m_crops_h;
   int m_top_k = 1; bool m_per_class = false; float m_th_obj_dist = 0.f;   // SetHypotheses
+  // SubmitRecognition / CollectRecognition: the pipe and what it was set up for
+  int m_frames_in_flight = 1;
+  fl_pipe* m_pipe = nullptr;
+  int m_stream_w = 0, m_stream_h = 0, m_stream_top_k = 0; bool m_stream_per_class = false; float m_stream_th = 0.f; size_t m_stream_fingerprint = 0;
+  std::vector<cv::String> m_stream_classes;
+  std::vector<int32_t> m_stream_crop;
+  CObjRecoLmICP(const CObjRecoLmICP&) = delete;
+  CObjRecoLmICP& operator=(const CObjRecoLmICP&) = delete;
 };
 
 inline CObjRecoCAD* CObjRecoCAD::Create(EObjRecoType eType) { return eType == EObjReco_LmICP ? new CObjRecoLmICP() : nullptr; }   // obj_reco_temp.cpp:13-30
