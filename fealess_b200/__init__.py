@@ -48,7 +48,7 @@ EXPORTED_SYMBOLS = [
     "fl_default_params", "fl_create", "fl_destroy", "fl_last_error", "fl_version", "fl_sync", "fl_stream",
     "fl_upload_templates", "fl_set_template_ids", "fl_num_templates", "fl_get_pose_info", "fl_match", "fl_match_device", "fl_match_device_async", "fl_match_wait", "fl_match_fetch",
     "fl_resize_linear", "fl_match_rescaled", "fl_match_shard_device", "fl_sort_unique_device", "fl_sort_unique_blocks_device", "fl_exchange_buffer_bytes", "fl_exchange_sort_unique_device", "fl_exchange_sort_unique_device_async", "fl_match_shard_exchange_device_async", "fl_depth_to_3d", "fl_icp_cloud_to_cloud_ex",
-    "fl_detection_batch", "fl_upload_model_depths", "fl_detection_batch_resident", "fl_detection_batch_resident_device", "fl_detection", "fl_nms", "fl_nms_ex", "fl_debug_option", "fl_debug_keep_spread", "fl_debug_force_baseline", "fl_debug_uses_staged", "fl_debug_get", "fl_debug_icp_trace", "fl_launch_count",
+    "fl_detection_batch", "fl_upload_model_depths", "fl_detection_batch_resident", "fl_detection_batch_resident_device", "fl_detection", "fl_nms", "fl_nms_ex", "fl_debug_option", "fl_debug_keep_spread", "fl_debug_force_baseline", "fl_debug_uses_staged", "fl_debug_plan_staged", "fl_debug_get", "fl_debug_icp_trace", "fl_launch_count",
     "fl_profile", "fl_last_stage_ms", "fl_last_icp_ms",
     "fl_group_create", "fl_group_destroy", "fl_group_size", "fl_group_handle", "fl_group_upload_templates", "fl_group_match",
     "fl_match_async", "fl_set_blocking_wait", "fl_match_shard_exchange_async", "fl_pipe_create", "fl_pipe_destroy", "fl_pipe_depth", "fl_pipe_in_flight", "fl_pipe_handle", "fl_pipe_upload_templates",
@@ -141,6 +141,19 @@ def _check(rc: int, where: str, ok=(FL_OK,)):
     if rc not in ok:
         raise FealessError(rc, where, lib().fl_last_error().decode(errors="replace"))
     return rc
+
+
+STAGED_PLAN_FIELDS = ("nw_template", "tpw", "tpc", "n_cta", "block_threads", "phase_rows", "n_rowblocks", "labels_per_phase",
+                      "n_phases", "n_buf", "buf_bytes", "halo_bytes", "smem_bytes")
+
+
+def plan_staged(W: int, H: int, T: int, n_modalities: int, n_templates: int, max_positions: int, n_sm: int) -> Optional[dict]:
+    """fl_debug_plan_staged: the staged similarity kernel's plan for a W x H coarsest level with step T (a dict keyed by
+    STAGED_PLAN_FIELDS), or None where the planner refuses the geometry and the baseline kernel runs.  No device needed."""
+    out = (C.c_int32 * 16)()
+    rc = lib().fl_debug_plan_staged(int(W), int(H), int(T), int(n_modalities), int(n_templates), int(max_positions), int(n_sm), out)
+    _check(rc, "fl_debug_plan_staged", ok=(0, 1))
+    return dict(zip(STAGED_PLAN_FIELDS, out)) if rc == 1 else None
 
 
 class Handle:

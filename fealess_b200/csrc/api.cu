@@ -222,6 +222,23 @@ extern "C" int fl_last_stage_ms(fl_handle* h, float out4[4]) { if (!h || !out4) 
 // 1 = always use the baseline (L1/L2-fed) global similarity kernel; 0 = use the shared-memory-staged kernel when eligible
 extern "C" int fl_debug_force_baseline(fl_handle* h, int enable) { if (!h) return FL_ERR_ARG; h->force_baseline = enable != 0; h->packed = false; return FL_OK; }
 extern "C" int fl_debug_uses_staged(fl_handle* h) { return h ? (h->use_staged ? 1 : 0) : FL_ERR_ARG; }
+extern "C" int fl_debug_plan_staged(int W, int H, int T, int n_modalities, int n_templates, int max_positions, int n_sm, int32_t out[16]) {
+  if (!out || T < 1 || T > FL_MAX_T || W < T || H < T || W % T || H % T || (int64_t)W * H > INT32_MAX || n_modalities < 1 ||
+      n_modalities > FL_MAX_MODALITIES || n_sm < 1)
+    return FL_ERR_ARG;
+  memset(out, 0, 16 * sizeof(int32_t));
+  fl_params_t p;
+  fl_default_params(&p);
+  p.n_levels = 1; p.T[0] = T; p.n_modalities = n_modalities;
+  fl_level_geom g;
+  level_lm_bytes(p, 0, W, H, &g);                              // the geometry ensure_geometry builds for the coarsest level
+  fl_staged_plan pl;
+  if (!fl_plan_staged(g, n_modalities, n_templates, max_positions, n_sm, &pl)) return 0;
+  const int32_t v[] = {pl.nw_template, pl.tpw, pl.tpc, pl.n_cta, pl.block_threads, pl.phase_rows, pl.n_rowblocks, pl.labels_per_phase,
+                       pl.n_phases, pl.n_buf, pl.buf_bytes, pl.halo_bytes, pl.smem_bytes};
+  memcpy(out, v, sizeof v);
+  return 1;
+}
 // developer options of one handle (all off by default; each one is exercised by tests/test_gpu_match.py::test_debug_options)
 extern "C" int fl_debug_option(fl_handle* h, int option, int value) {
   if (!h) return FL_ERR_ARG;

@@ -310,12 +310,13 @@ __device__ __forceinline__ void dev_spread_lm(const uint8_t* __restrict__ q, con
       else for (int k = 0; k < nvalid; ++k) dst[k] = (uint8_t)(w >> (8 * k));
       if (lm4) {
         // the same four responses (each 0, 1, 2 or 4) as nibbles, cell j of the label in nibble j: what the staged similarity
-        // kernel reads (half the bytes).  Only passed for grids of even width, so `off` is even and nvalid is 2 or 4.
+        // kernel reads (half the bytes).  Only passed for grids of even width, so `off` is even and nvalid is 2 or 4.  `off` is
+        // a multiple of 4 only when Wd and cells are: a grid width of 2 mod 4 cells puts every other row at an odd byte.
         const uint32_t p2 = (w | (w >> 4)) & 0x00FF00FFu;
         const uint32_t p4 = (p2 | (p2 >> 8)) & 0xFFFFu;
         uint8_t* d4 = lm4 + (((size_t)lab * g.label_stride + off) >> 1);
-        if (nvalid == 4) *reinterpret_cast<uint16_t*>(d4) = (uint16_t)p4;
-        else *d4 = (uint8_t)p4;
+        if (nvalid == 4 && (((uintptr_t)d4) & 1) == 0) *reinterpret_cast<uint16_t*>(d4) = (uint16_t)p4;
+        else { d4[0] = (uint8_t)p4; if (nvalid == 4) d4[1] = (uint8_t)(p4 >> 8); }
       }
     }
   }

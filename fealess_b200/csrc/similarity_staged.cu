@@ -207,11 +207,13 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
       if (t < t_end) {
         m = plan.gmeta[t];
         m.w = db.L == 1 ? db.tid_of[t] : t;                   // the id candidates carry (see k_similarity_global)
-        if (!db.class_enabled[m.z]) m.x = 0;                  // no positions -> no candidates
-        // raw threshold int(2 nf + (threshold / 100) 2 nf + 0.5f) in fp32 (:1487); stored biased by 1, clamped to [-1, 255]
+        const bool on = db.class_enabled[m.z];
+        if (!on) m.x = 0;                                     // no positions -> no candidates
+        // raw threshold int(2 nf + (threshold / 100) 2 nf + 0.5f) in fp32 (:1487); stored biased by 1, clamped to [-1, 255];
+        // a disabled class gets 255, which no u8 total exceeds
         const int nf = m.y;
         const int rt = (int)__fadd_rn(__fadd_rn((float)(2 * nf), __fmul_rn(__fdiv_rn(threshold, 100.f), (float)(2 * nf))), 0.5f);
-        m.y = nf | ((min(max(rt, -1), 255) + 1) << 8);
+        m.y = nf | ((on ? min(max(rt, -1), 255) + 1 : 256) << 8);
       }
       s_meta[i] = m;
     }
@@ -425,6 +427,28 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
       __syncwarp();
       if (lane == 0) { __threadfence_block(); atomicExch(&s_emit_lock, 0); }
     }
+    // Below a zero raw threshold (only a threshold under -100 gives one) every cell of the map is a candidate (:1497-1504), also
+    // the cells at and past template_positions - where the reference's map holds 0 - and every cell of a template without
+    // positions.  The accumulators cover template_positions only, so these candidates are written here with a raw score of 0.
+#pragma unroll
+    for (int s = 0; s < TPW; ++s) {
+      const int slot = warp + s * n_cwarps;
+      if (slot >= plan.tpc || t_begin + slot >= t_end) continue;      // warp-uniform
+      const int4 meta = s_meta[slot];
+      const int nf = meta.y & 0xFF, raw_thr = (meta.y >> 8) - 1;
+      const int j0 = max(meta.x, 0), n = g.cells - j0;
+      if (raw_thr >= 0 || n <= 0) continue;
+      int base = 0;
+      if (lane == 0) base = atomicAdd(d_count, n);
+      base = __shfl_sync(0xffffffffu, base, 0);
+      const float msim = __fadd_rn(__fdiv_rn(__fmul_rn(0.f, 100.f), (float)(4 * nf)), 0.5f);
+      for (int k = lane; k < n && base + k < cap; k += 32) {
+        const int j = j0 + k, r = j / g.Wd, c = j - r * g.Wd;
+        fl_match_t mt;
+        mt.x = c * g.T + off; mt.y = r * g.T + off; mt.similarity = msim; mt.class_idx = meta.z; mt.template_id = meta.w;
+        cand[base + k] = mt;
+      }
+    }
     if (trace && lane == 0) { atomicMax(&trace[6], globaltimer()); plan.trace[(size_t)plan.n_cta * 8 + 8 + ((size_t)blockIdx.x * 32 + warp) * 4 + 1] = globaltimer(); }
   }
   if (trace && tid == 0) trace[4] = globaltimer();
@@ -467,7 +491,9 @@ static int launch_staged(fl_tdb db, fl_level_geom g, const uint8_t* lm4_level, f
 // template_positions (linemod.cpp:1155) over the uploaded templates: only that many cells of a similarity map are ever
 // looked at, so the per-lane accumulator count NW is sized for it rather than for the whole grid.
 bool fl_plan_staged(const fl_level_geom& g, int M, int n_templates, int max_positions, int n_sm, fl_staged_plan* plan) {
-  static const int kNW[] = {3, 5, 7, 9, 11, 13, 15, 19};
+  // NW <= 15 covers 32 x 15 x 8 = 3,840 positions.  A larger NW would need a halo of 32 NW 4 + 16 bytes past the last row,
+  // more than the FL_LM_PAD / 2 bytes of zero pad behind a label's 4-bit linear memory: larger grids use the baseline kernel.
+  static const int kNW[] = {3, 5, 7, 9, 11, 13, 15};
   fl_staged_plan p;
   memset(&p, 0, sizeof p);
   const int T2 = g.T * g.T;
@@ -478,7 +504,7 @@ bool fl_plan_staged(const fl_level_geom& g, int M, int n_templates, int max_posi
   const int nw_min = (p.n_words + 31) / 32;
   p.nw_template = 0;
   for (int nw : kNW) if (nw >= nw_min) { p.nw_template = nw; break; }
-  if (!p.nw_template) return false;                            // accumulators would not fit the register budget
+  if (!p.nw_template) return false;                            // more than 3,840 positions (see kNW)
   p.tpw = p.nw_template > 5 ? 1 : 2;                           // register budget: 64 per thread at 1,024 threads, 3 NW accumulator words per slot
   // bytes staged past the last row of a phase: a window starts at most at the last cell of the last row and the loads run
   // unconditionally over 32 * NW + 1 words
@@ -545,7 +571,6 @@ int fl_launch_similarity_staged(fl_tdb db, fl_level_geom g, const uint8_t* lm4_l
     case 11: return launch_staged<11, 1>(db, g, lm4_level, threshold, cand, cap, d_count, plan, s);
     case 13: return launch_staged<13, 1>(db, g, lm4_level, threshold, cand, cap, d_count, plan, s);
     case 15: return launch_staged<15, 1>(db, g, lm4_level, threshold, cand, cap, d_count, plan, s);
-    case 19: return launch_staged<19, 1>(db, g, lm4_level, threshold, cand, cap, d_count, plan, s);
   }
   return -1;
 }

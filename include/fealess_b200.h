@@ -408,6 +408,14 @@ int fl_debug_keep_spread(fl_handle* h, int enable);
  * choice made for the last frame geometry (1 / 0). */
 int fl_debug_force_baseline(fl_handle* h, int enable);
 int fl_debug_uses_staged(fl_handle* h);
+/* the plan of the staged kernel for one coarsest level: W x H pixels (multiples of T), step T, n_modalities, n_templates,
+ * max_positions = the largest template_positions of the set at that level, n_sm multiprocessors.  Host code, no device
+ * needed.  Returns 1 and fills out[0..12] = {NW (accumulator words per lane), templates per warp, templates per CTA, CTAs,
+ * threads per CTA, linear-memory rows per phase, row blocks per label, labels per phase, phases, ring buffers,
+ * bytes per buffer, halo bytes, dynamic shared memory bytes} (out[13..15] = 0) when the staged kernel would run; 0 when
+ * the planner refuses the geometry (a handle then runs the baseline kernel); FL_ERR_ARG for a bad argument.  A handle also
+ * needs 256 or more eligible templates before it plans. */
+int fl_debug_plan_staged(int W, int H, int T, int n_modalities, int n_templates, int max_positions, int n_sm, int32_t out[16]);
 int fl_debug_get(fl_handle* h, int what, int32_t a, int32_t b, int32_t c, void* host_out, size_t bytes);
 /* number of kernels launched by this handle since creation (bench.py reports the per-step delta) */
 int64_t fl_launch_count(fl_handle* h);
