@@ -55,6 +55,8 @@ EXPORTED_SYMBOLS = [
     "fl_pipe_submit", "fl_pipe_collect", "fl_pipe_match_batch", "fl_pipe_set_exchange", "fl_default_train_params", "fl_add_template",
     "fl_default_reco_params", "fl_set_recognition", "fl_recognize_async", "fl_recognize_wait", "fl_recognize", "fl_pipe_upload_model_depths",
     "fl_pipe_set_recognition", "fl_pipe_submit_recognition", "fl_pipe_collect_recognition",
+    "fl_group_create_pipe", "fl_group_depth", "fl_group_in_flight", "fl_group_upload_model_depths", "fl_group_set_recognition",
+    "fl_group_submit_recognition", "fl_group_collect_recognition", "fl_group_recognize",
 ]
 
 
@@ -595,10 +597,11 @@ class Handle:
 
 
 class Group:
-    """fl_group: Detector::match over N handles of this process (``devices`` may repeat a device), templates sharded gid % N."""
+    """fl_group: Detector::match over N handles of this process (``devices`` may repeat a device), templates sharded gid % N.  With
+    ``depth`` > 1 (fl_group_create_pipe) up to ``depth`` recognition frames are in flight; handle i = slot * N + member."""
 
     def __init__(self, devices: Sequence[int], T: Sequence[int] = (5, 8), modality_kind: Sequence[int] = (0, 1), max_width=640, max_height=480,
-                 exchange_capacity: int = 2048):
+                 exchange_capacity: int = 2048, depth: int = 1):
         L = lib()
         p = Params()
         L.fl_default_params(C.byref(p))
@@ -611,10 +614,13 @@ class Group:
         p.max_width, p.max_height = max_width, max_height
         self._g = C.c_void_p()
         dv = np.ascontiguousarray(devices, np.int32)
-        rc = L.fl_group_create(C.byref(p), _p(dv), len(dv), exchange_capacity, C.byref(self._g))
+        rc = L.fl_group_create_pipe(C.byref(p), _p(dv), len(dv), exchange_capacity, int(depth), C.byref(self._g))
         if rc != FL_OK:
             self._g = None
-            raise FealessError(rc, "fl_group_create", L.fl_last_error().decode(errors="replace"))
+            raise FealessError(rc, "fl_group_create_pipe", L.fl_last_error().decode(errors="replace"))
+        self.n, self.depth = len(dv), int(depth)
+        self._keep = {}                                          # frames in flight: the arrays the DMA reads stay referenced
+        self._seq = 0
 
     def close(self):
         if getattr(self, "_g", None):
@@ -627,17 +633,27 @@ class Group:
         except Exception:  # noqa: BLE001
             pass
 
-    def member_option(self, i: int, option: int, value: int = 1) -> int:
-        """fl_debug_option on member handle ``i`` (fl_group_handle)."""
+    def _handle(self, i: int) -> C.c_void_p:
         L = lib()
         L.fl_group_handle.restype = C.c_void_p
         hp = L.fl_group_handle(self._g, int(i))
         if not hp:
             raise FealessError(FL_ERR_ARG, "fl_group_handle")
-        rc = L.fl_debug_option(C.c_void_p(hp), int(option), int(value))
+        return C.c_void_p(hp)
+
+    def member_option(self, i: int, option: int, value: int = 1) -> int:
+        """fl_debug_option on handle ``i`` (fl_group_handle: slot * N + member)."""
+        rc = lib().fl_debug_option(self._handle(i), int(option), int(value))
         if rc < 0:
             _check(rc, "fl_debug_option")
         return rc
+
+    def launch_counts(self) -> np.ndarray:
+        """fl_launch_count of every handle, shape (depth, N)."""
+        return np.array([int(lib().fl_launch_count(self._handle(i))) for i in range(self.n * self.depth)], np.int64).reshape(self.depth, self.n)
+
+    def in_flight(self) -> int:
+        return int(lib().fl_group_in_flight(self._g))
 
     def upload_templates(self, tset) -> None:
         hdr = np.ascontiguousarray(tset.headers, np.int32)
@@ -658,6 +674,51 @@ class Group:
         if rc not in (FL_OK, FL_ERR_CAPACITY):
             _check(rc, "fl_group_match")
         return rc, out[:min(cnt.value, capacity)].copy()
+
+    # ---- Recognition over the group ---------------------------------------------------------------
+    def upload_model_depths(self, model_depths: Sequence[np.ndarray], rects_model) -> None:
+        """fl_group_upload_model_depths: ``Handle.upload_model_depths`` on every slot of every member."""
+        n = len(model_depths)
+        mds = [np.ascontiguousarray(m, np.uint16) for m in model_depths]
+        H, W = mds[0].shape if n else (1, 1)
+        ptrs = (C.c_void_p * max(n, 1))(*[m.ctypes.data for m in mds])
+        strides = (C.c_size_t * max(n, 1))(*[m.strides[0] for m in mds])
+        rm = np.ascontiguousarray(rects_model, np.int32).reshape(-1, 4)
+        _check(lib().fl_group_upload_model_depths(self._g, n, ptrs, strides, _p(rm), W, H), "fl_group_upload_model_depths")
+
+    def set_recognition(self, crop_of_template, pose12=None, params: Optional[RecoParams] = None) -> None:
+        """fl_group_set_recognition: crop index and pose of every template of the whole set (order of ``upload_templates``)."""
+        crop = np.ascontiguousarray(crop_of_template, np.int32)
+        pose = None if pose12 is None else np.ascontiguousarray(pose12, np.float32).reshape(-1, 12)
+        _check(lib().fl_group_set_recognition(self._g, C.byref(params or reco_params()), _p(crop), _p(pose)), "fl_group_set_recognition")
+
+    def submit_recognition(self, bgr, depth, K, W: Optional[int] = None, H: Optional[int] = None) -> None:
+        """fl_group_submit_recognition (host frame; page-locked arrays are read by DMA while in flight, so they are kept referenced)."""
+        b, d, sW, sH, W, H = _reco_args(bgr, depth, W, H)
+        _check(lib().fl_group_submit_recognition(self._g, _p(b), C.c_size_t(sW * 3), _p(d), C.c_size_t(sW * 2), sW, sH, W, H,
+                                                 Intrinsics(*[float(v) for v in K])), "fl_group_submit_recognition")
+        self._keep[self._seq % self.depth] = (b, d)
+        self._seq += 1
+
+    def collect_recognition(self, capacity: int = RECO_MAX_HYP):
+        """(rc, results, summary) of the oldest frame in flight, as ``Handle.recognize_wait``."""
+        out = np.zeros(max(capacity, 1), RECO_RESULT_DTYPE)
+        s = RecoSummary()
+        rc = lib().fl_group_collect_recognition(self._g, _p(out), int(capacity), C.byref(s))
+        if rc not in (FL_OK, FL_ERR_CAPACITY):
+            _check(rc, "fl_group_collect_recognition")
+        return rc, out[:min(s.n_results, capacity)].copy(), _summary(s)
+
+    def recognize(self, bgr, depth, K, W: Optional[int] = None, H: Optional[int] = None, capacity: int = RECO_MAX_HYP):
+        """fl_group_recognize: one frame, submitted and collected (nothing else may be in flight)."""
+        b, d, sW, sH, W, H = _reco_args(bgr, depth, W, H)
+        out = np.zeros(max(capacity, 1), RECO_RESULT_DTYPE)
+        s = RecoSummary()
+        rc = lib().fl_group_recognize(self._g, _p(b), C.c_size_t(sW * 3), _p(d), C.c_size_t(sW * 2), sW, sH, W, H,
+                                      Intrinsics(*[float(v) for v in K]), _p(out), int(capacity), C.byref(s))
+        if rc not in (FL_OK, FL_ERR_CAPACITY):
+            _check(rc, "fl_group_recognize")
+        return rc, out[:min(s.n_results, capacity)].copy(), _summary(s)
 
 
 class Pipe:

@@ -95,6 +95,9 @@ struct fl_handle {
   bool custom_tids = false, reco_set = false, reco_any_crop = false, pend_reco = false; fl_reco_params_t reco = {}; int reco_max_hyp = 0;
   fl_dev_buf<fl_reco_tmpl> d_reco_tmpl; fl_dev_buf<int> d_reco_sel; fl_mapped_buf<int> h_reco; int* d_reco_host = nullptr;
   int reco_W = 0, reco_H = 0; fl_intrinsics_t reco_K = {};
+  // the template set the selection table covers: the handle's own upload, or the whole set of a template-sharded group, whose merged
+  // list this handle selects from (fl_group_set_recognition)
+  int reco_n_templates = 0, reco_n_classes = 0; fl_dev_buf<int32_t> d_reco_class_first; bool reco_bgr = false;   // reco_bgr: the staged frame has colour
 };
 
 // The host waits for the handle's stream.  Default: cudaStreamSynchronize (the runtime spins - lowest latency, one busy core per
@@ -1588,48 +1591,70 @@ extern "C" void fl_default_reco_params(fl_reco_params_t* p) {
   p->top_k = 1; p->per_class = 0; p->th_obj_dist = 0.f;                           // matches[0] only (:111)
 }
 
-extern "C" int fl_set_recognition(fl_handle* h, const fl_reco_params_t* prm, const int32_t* crop_of_template, const float* pose12) {
-  if (!h || !prm || !crop_of_template || prm->top_k < 1) return FL_ERR_ARG;
+// The one builder of a recognition set-up: the selection table of `set` (crop and pose of every template, in the order of the set) and
+// the set's class_first, installed on the handle together with an ICP workspace sized for the frame's hypotheses.  fl_set_recognition
+// passes the handle's own upload; fl_group_set_recognition passes the whole set of a template-sharded group, whose merged list every
+// member's handle selects from.
+int fl_reco_setup(fl_handle* h, const fl_reco_params_t* prm, const fl_reco_set& set, const int32_t* crop_of_template, const float* pose12) {
+  if (!h || !prm || !crop_of_template || prm->top_k < 1 || set.n_templates < 0 || (set.n_templates > 0 && (!set.class_of || !set.box0))) return FL_ERR_ARG;
   if (h->pend_sort) { fl_set_error("fl_set_recognition: a frame is in flight on this handle"); return FL_ERR_STATE; }
-  if (h->n_templates == 0) { fl_set_error("fl_set_recognition: no templates uploaded"); return FL_ERR_STATE; }
-  // matches carry the ids of fl_set_template_ids (a shard's global ids): the template behind a match is not class_first + template_id
-  if (h->custom_tids) { fl_set_error("fl_set_recognition: not available on a handle with fl_set_template_ids (template shards)"); return FL_ERR_STATE; }
-  if (!pose12 && h->pose13_h.empty()) { fl_set_error("fl_set_recognition: no pose table (pose12 NULL and no pose13 uploaded)"); return FL_ERR_ARG; }
-  const int64_t max_hyp = (int64_t)prm->top_k * (prm->per_class ? h->n_classes : 1);
+  if (set.n_templates == 0) { fl_set_error("fl_set_recognition: no templates uploaded"); return FL_ERR_STATE; }
+  if (!pose12 && !set.pose13) { fl_set_error("fl_set_recognition: no pose table (pose12 NULL and no pose13 uploaded)"); return FL_ERR_ARG; }
+  int nc = 0;
+  for (int t = 0; t < set.n_templates; ++t) { if (set.class_of[t] < 0) return FL_ERR_ARG; nc = std::max(nc, set.class_of[t] + 1); }
+  std::vector<int32_t> first((size_t)nc, -1);                                      // as fl_upload_templates numbers them (matchClass, :1458)
+  for (int t = 0; t < set.n_templates; ++t) if (first[set.class_of[t]] < 0) first[set.class_of[t]] = t;
+  const int64_t max_hyp = (int64_t)prm->top_k * (prm->per_class ? nc : 1);
   if (max_hyp > FL_RECO_MAX_HYP) { fl_set_error("fl_set_recognition: %lld hypotheses per frame > FL_RECO_MAX_HYP", (long long)max_hyp); return FL_ERR_CAPACITY; }
   FL_CUDA(cudaSetDevice(h->p.device));
-  const size_t per = (size_t)h->p.n_levels * h->p.n_modalities;
-  std::vector<fl_template_hdr_t> hdr((size_t)h->n_templates * per);
-  FL_CUDA(cudaMemcpy(hdr.data(), h->d_hdr.get(), hdr.size() * sizeof(fl_template_hdr_t), cudaMemcpyDeviceToHost));
-  std::vector<fl_reco_tmpl> tab((size_t)h->n_templates);
+  std::vector<fl_reco_tmpl> tab((size_t)set.n_templates);
   int max_pts = 16;
   bool any_crop = false;
-  for (int t = 0; t < h->n_templates; ++t) {
+  for (int t = 0; t < set.n_templates; ++t) {
     fl_reco_tmpl& e = tab[t];
     memset(&e, 0, sizeof e);
     const int c = crop_of_template[t];
     if (c < -1 || c >= (int)h->res_rect.size()) { fl_set_error("fl_set_recognition: crop %d of template %d is not in the uploaded set", c, t); return FL_ERR_ARG; }
     if (c >= 0) {
-      const fl_template_hdr_t& b = hdr[(size_t)t * per];                           // current_template[0] (:111, :127-132)
+      const fl_rect_t& b = set.box0[t];                                             // current_template[0] (:111, :127-132)
       const fl_rect_t& r = h->res_rect[c];
-      if (r.x != b.offset_x || r.y != b.offset_y || r.width != b.width || r.height != b.height) {
+      if (r.x != b.x || r.y != b.y || r.width != b.width || r.height != b.height) {
         fl_set_error("fl_set_recognition: crop %d was uploaded with a rect other than template %d's level-0 box", c, t); return FL_ERR_ARG;
       }
       e.crop = h->d_resident.get() + h->res_off[c]; e.rect = r;
       max_pts = std::max(max_pts, r.width * r.height);
       any_crop = true;
     }
-    memcpy(e.pose, pose12 ? pose12 + (size_t)t * 12 : &h->pose13_h[(size_t)t * 13], 12 * sizeof(float));
+    memcpy(e.pose, pose12 ? pose12 + (size_t)t * 12 : set.pose13 + (size_t)t * 13, 12 * sizeof(float));
   }
   h->reco_set = false;
   TRY(icp_reserve(h, (int)max_hyp, max_pts));                                     // now, so that no frame allocates
   TRY(h->d_reco_tmpl.alloc(tab.size()));
   FL_CUDA(cudaMemcpy(h->d_reco_tmpl.get(), tab.data(), tab.size() * sizeof(fl_reco_tmpl), cudaMemcpyHostToDevice));
+  TRY(h->d_reco_class_first.alloc((size_t)nc));
+  FL_CUDA(cudaMemcpy(h->d_reco_class_first.get(), first.data(), first.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
   TRY(h->d_reco_sel.grow(FL_RECO_SEL_HDR + FL_RECO_MAX_HYP));
   TRY(h->h_reco.grow(FL_RECO_SUMMARY_WORDS + FL_RECO_MAX_HYP * sizeof(fl_reco_result_t) / sizeof(int)));
   FL_CUDA(cudaHostGetDevicePointer((void**)&h->d_reco_host, h->h_reco.get(), 0));
-  h->reco = *prm; h->reco_max_hyp = (int)max_hyp; h->reco_any_crop = any_crop; h->reco_set = true;
+  h->reco = *prm; h->reco_max_hyp = (int)max_hyp; h->reco_any_crop = any_crop;
+  h->reco_n_templates = set.n_templates; h->reco_n_classes = nc; h->reco_set = true;
   return FL_OK;
+}
+
+extern "C" int fl_set_recognition(fl_handle* h, const fl_reco_params_t* prm, const int32_t* crop_of_template, const float* pose12) {
+  if (!h || !prm || !crop_of_template || prm->top_k < 1) return FL_ERR_ARG;
+  if (h->pend_sort) { fl_set_error("fl_set_recognition: a frame is in flight on this handle"); return FL_ERR_STATE; }
+  if (h->n_templates == 0) { fl_set_error("fl_set_recognition: no templates uploaded"); return FL_ERR_STATE; }
+  // matches carry the ids of fl_set_template_ids (a shard's global ids): the template behind a match is not class_first + template_id
+  if (h->custom_tids) { fl_set_error("fl_set_recognition: not available on a handle with fl_set_template_ids (template shards)"); return FL_ERR_STATE; }
+  FL_CUDA(cudaSetDevice(h->p.device));
+  const size_t per = (size_t)h->p.n_levels * h->p.n_modalities;
+  std::vector<fl_template_hdr_t> hdr((size_t)h->n_templates * per);
+  FL_CUDA(cudaMemcpy(hdr.data(), h->d_hdr.get(), hdr.size() * sizeof(fl_template_hdr_t), cudaMemcpyDeviceToHost));
+  std::vector<fl_rect_t> box0((size_t)h->n_templates);
+  for (int t = 0; t < h->n_templates; ++t) { const fl_template_hdr_t& b = hdr[(size_t)t * per]; box0[t] = {b.offset_x, b.offset_y, b.width, b.height}; }
+  const fl_reco_set set = {h->n_templates, h->class_of_h.data(), box0.data(), h->pose13_h.empty() ? nullptr : h->pose13_h.data()};
+  return fl_reco_setup(h, prm, set, crop_of_template, pose12);
 }
 
 // selection -> ICP -> finish on the sorted list in d_out.  check_big: the list came from the fused refinement + sort, which leaves
@@ -1637,8 +1662,9 @@ extern "C" int fl_set_recognition(fl_handle* h, const fl_reco_params_t* prm, con
 static int reco_enqueue(fl_handle* h, bool check_big) {
   cudaStream_t s = h->stream.get();
   const int max_hyp = h->reco_max_hyp;
-  int nl = fl_launch_reco_select(h->d_out, reinterpret_cast<const int*>(h->d_outblk.get()), h->p.max_candidates, check_big ? 1 : 0, h->d_class_first.get(), h->n_classes,
-                                 h->n_templates, h->d_reco_tmpl.get(), h->reco.top_k, h->reco.per_class, max_hyp, h->reco_W, h->reco_H, h->icpw.d_hyps.get(), h->d_reco_sel.get(), s);
+  int nl = fl_launch_reco_select(h->d_out, reinterpret_cast<const int*>(h->d_outblk.get()), h->p.max_candidates, check_big ? 1 : 0, h->d_reco_class_first.get(),
+                                 h->reco_n_classes, h->reco_n_templates, h->d_reco_tmpl.get(), h->reco.top_k, h->reco.per_class, max_hyp, h->reco_W, h->reco_H,
+                                 h->icpw.d_hyps.get(), h->d_reco_sel.get(), s);
   if (nl < 0) { fl_set_error("hypothesis selection launch failed: %s", cudaGetErrorString(cudaGetLastError())); return FL_ERR_CUDA; }
   h->launches += nl;
   fl_icp_ws ws = h->icp;
@@ -1652,9 +1678,9 @@ static int reco_enqueue(fl_handle* h, bool check_big) {
   return FL_OK;
 }
 
-extern "C" int fl_recognize_async(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
-                                  int32_t sW, int32_t sH, int32_t W, int32_t H, fl_intrinsics_t K_ref) {
-  if (!h || !depth || sW <= 0 || sH <= 0) return FL_ERR_ARG;
+// the upload of a recognition frame into d_in_bgr / d_in_depth, rescaled on the device when src_W x src_H differs from W x H
+static int reco_stage(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int sW, int sH, int W, int H,
+                      fl_intrinsics_t K_ref, const uint8_t** d_bgr, const uint16_t** d_depth) {
   const fl_params_t& p = h->p;
   if (h->pend_sort) { fl_set_error("the previous frame of this handle has not been waited for"); return FL_ERR_STATE; }
   if (!h->reco_set) { fl_set_error("fl_recognize: call fl_set_recognition after the template and crop uploads"); return FL_ERR_STATE; }
@@ -1662,20 +1688,91 @@ extern "C" int fl_recognize_async(fl_handle* h, const uint8_t* bgr, size_t bgr_s
   if (W <= 0 || H <= 0 || W > p.max_width || H > p.max_height) return FL_ERR_SIZE;
   if (h->reco_any_crop && (W != h->res_W || H != h->res_H)) { fl_set_error("model depth crops were uploaded for %d x %d frames, not %d x %d", h->res_W, h->res_H, W, H); return FL_ERR_STATE; }
   FL_CUDA(cudaSetDevice(p.device));
-  const uint8_t* d_bgr; const uint16_t* d_depth;
   if (sW == W && sH == H) {                                                      // TImage2Mat resizes only when the size differs (:42)
     const void* d_masks[FL_MAX_MODALITIES];
     bool any_mask;
-    TRY(stage_frame(h, bgr, bgr_stride, depth, depth_stride, W, H, nullptr, &d_bgr, &d_depth, d_masks, &any_mask));
+    TRY(stage_frame(h, bgr, bgr_stride, depth, depth_stride, W, H, nullptr, d_bgr, d_depth, d_masks, &any_mask));
   } else {
-    TRY(stage_rescaled(h, bgr, bgr_stride, depth, depth_stride, sW, sH, W, H, &d_bgr, &d_depth));
+    TRY(stage_rescaled(h, bgr, bgr_stride, depth, depth_stride, sW, sH, W, H, d_bgr, d_depth));
   }
+  h->reco_W = W; h->reco_H = H; h->reco_K = K_ref; h->reco_bgr = *d_bgr != nullptr;
+  return FL_OK;
+}
+
+extern "C" int fl_recognize_async(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
+                                  int32_t sW, int32_t sH, int32_t W, int32_t H, fl_intrinsics_t K_ref) {
+  if (!h || !depth || sW <= 0 || sH <= 0) return FL_ERR_ARG;
+  const uint8_t* d_bgr; const uint16_t* d_depth;
+  TRY(reco_stage(h, bgr, bgr_stride, depth, depth_stride, sW, sH, W, H, K_ref, &d_bgr, &d_depth));
   TRY(fl_match_device_async(h, d_bgr, d_depth, W, H, nullptr, h->reco.threshold, nullptr, 0));
   h->in_depth_W = W; h->in_depth_H = H;
-  h->reco_W = W; h->reco_H = H; h->reco_K = K_ref;
   TRY(reco_enqueue(h, true));
   h->pend_reco = true;
   return FL_OK;
+}
+
+// One member's part of a frame of a template-sharded group (fl_group_submit_recognition), in three steps that the group runs over all
+// members in turn: fl_reco_shard_stage (upload [+ rescale] of the frame), fl_reco_shard_match (local match over the member's shard + the
+// fused refinement / peer-memory exchange / sort of the staged frame, after which every member holds the merged list) and, on the
+// frame's owner only, fl_reco_shard_tail (selection, ICP, finish on that list).  Nothing that may wait for the device - an allocation,
+// the first launch of a kernel under lazy module loading - may run between one member's exchange launch and the last member's: the
+// exchange kernel spins until every peer has published the frame.  The re-run after a front-end time-out calls the last two steps
+// again on the frames already staged.
+int fl_reco_shard_stage(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int sW, int sH, int W, int H,
+                        fl_intrinsics_t K_ref) {
+  if (!h || !depth || sW <= 0 || sH <= 0) return FL_ERR_ARG;
+  const uint8_t* d_bgr; const uint16_t* d_depth;
+  TRY(reco_stage(h, bgr, bgr_stride, depth, depth_stride, sW, sH, W, H, K_ref, &d_bgr, &d_depth));
+  return FL_OK;
+}
+
+int fl_reco_shard_match(fl_handle* h, int rank, int world, void* const* peers, int capacity, fl_match_t* block, uint32_t epoch) {
+  if (!h) return FL_ERR_ARG;
+  if (h->pend_sort || !h->reco_set || h->reco_W == 0) { fl_set_error("no staged recognition frame on this handle"); return FL_ERR_STATE; }
+  FL_CUDA(cudaSetDevice(h->p.device));
+  h->pend_reco = false;
+  const uint8_t* d_bgr = h->reco_bgr ? h->d_in_bgr.get() : nullptr;
+  TRY(fl_match_shard_exchange_device_async(h, d_bgr, h->d_in_depth.get(), h->reco_W, h->reco_H, h->reco.threshold, nullptr, 0, rank, world, peers, capacity,
+                                           block, epoch));
+  h->in_depth_W = h->reco_W; h->in_depth_H = h->reco_H;
+  return FL_OK;
+}
+
+int fl_reco_shard_tail(fl_handle* h) {
+  if (!h) return FL_ERR_ARG;
+  if (!h->pend_sort || !h->reco_set) { fl_set_error("no matched recognition frame on this handle"); return FL_ERR_STATE; }
+  FL_CUDA(cudaSetDevice(h->p.device));
+  TRY(reco_enqueue(h, true));
+  h->pend_reco = true;
+  return FL_OK;
+}
+
+// after the frame's match wait: the tail once more on the final list when the selection ran on a list that was not sorted yet (or on a
+// frame that has been re-run since), then the results and the summary
+static int reco_results(fl_handle* h, bool rerun, fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary) {
+  const volatile int* blk = h->h_reco.get();
+  if ((blk[4] & FL_RECO_DEFERRED) || rerun) {
+    TRY(reco_enqueue(h, false));
+    FL_CUDA(wait_stream(h));
+  }
+  FL_CUDA(cudaGetLastError());
+  if (h->overflow) {                                                             // matchClass produced more candidates than the buffers hold
+    if (summary) summary->n_matches = h->h_small[0];
+    fl_set_error("fl_recognize: more candidates than the handle's buffers hold (max_candidates, or the exchange capacity of a group)");
+    return FL_ERR_CAPACITY;
+  }
+  const int n = blk[3];
+  if (summary) { summary->n_matches = blk[0]; summary->n_hypotheses = blk[1]; summary->n_roi = blk[2]; summary->n_results = n; }
+  if (std::min(n, (int)capacity) > 0) memcpy(out, h->h_reco.get() + FL_RECO_SUMMARY_WORDS, sizeof(fl_reco_result_t) * (size_t)std::min(n, (int)capacity));
+  return n > capacity ? FL_ERR_CAPACITY : FL_OK;
+}
+
+// the owner's results of a group frame whose members have all been waited for (fl_match_wait)
+int fl_reco_shard_results(fl_handle* h, fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary) {
+  if (!h || capacity < 0 || (capacity > 0 && !out)) return FL_ERR_ARG;
+  if (summary) memset(summary, 0, sizeof *summary);
+  FL_CUDA(cudaSetDevice(h->p.device));
+  return reco_results(h, false, out, capacity, summary);
 }
 
 extern "C" int fl_recognize_wait(fl_handle* h, fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary) {
@@ -1686,22 +1783,7 @@ extern "C" int fl_recognize_wait(fl_handle* h, fl_reco_result_t* out, int32_t ca
   const bool forced_before = h->fe_force_waves;
   // the frame's one wait; the rare > 1,024-record sorts and the re-run after a front-end dependency time-out are fl_match_wait's
   TRY(match_wait(h));
-  const volatile int* blk = h->h_reco.get();
-  if ((blk[4] & FL_RECO_DEFERRED) || (h->fe_force_waves && !forced_before)) {
-    // the selection ran on a list that was not sorted yet, or on a frame that has been re-run since: once more on the final list
-    TRY(reco_enqueue(h, false));
-    FL_CUDA(wait_stream(h));
-  }
-  FL_CUDA(cudaGetLastError());
-  if (h->overflow) {                                                             // matchClass produced more candidates than the buffers hold
-    if (summary) summary->n_matches = h->h_small[0];
-    fl_set_error("fl_recognize: more candidates than the handle's buffers hold (max_candidates)");
-    return FL_ERR_CAPACITY;
-  }
-  const int n = blk[3];
-  if (summary) { summary->n_matches = blk[0]; summary->n_hypotheses = blk[1]; summary->n_roi = blk[2]; summary->n_results = n; }
-  if (std::min(n, (int)capacity) > 0) memcpy(out, h->h_reco.get() + FL_RECO_SUMMARY_WORDS, sizeof(fl_reco_result_t) * (size_t)std::min(n, (int)capacity));
-  return n > capacity ? FL_ERR_CAPACITY : FL_OK;
+  return reco_results(h, h->fe_force_waves && !forced_before, out, capacity, summary);
 }
 
 extern "C" int fl_recognize(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,

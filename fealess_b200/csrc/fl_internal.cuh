@@ -262,3 +262,16 @@ int fl_launch_reco_select(const fl_match_t* matches, const int* d_hdr, int out_c
 // objects that came out of ICP -> [NMS] -> fl_reco_result_t records + summary posted to mapped host memory (host_block)
 int fl_launch_reco_finish(const fl_match_t* matches, const int* sel, const fl_icp_result_t* results, int max_hyp, float th_obj_dist,
                           int* host_block, cudaStream_t s);
+// the template set a recognition set-up covers, in upload order: class, level-0 modality-0 box and pose13 (nullable) of every template.
+// fl_set_recognition passes the handle's own upload, fl_group_set_recognition the whole set of a template-sharded group (api.cu).
+struct fl_reco_set { int n_templates; const int32_t* class_of; const fl_rect_t* box0; const float* pose13; };
+int fl_reco_setup(fl_handle* h, const fl_reco_params_t* prm, const fl_reco_set& set, const int32_t* crop_of_template, const float* pose12);
+// one member's part of a group frame (api.cu): stage the frame (rescaled when src != W x H); match the staged frame over the member's shard
+// + exchange + sort; on the frame's owner, the recognition tail.  The group runs each step on every member before the next one (no
+// member's enqueue may wait for the device while a peer's exchange kernel spins).  Finish with fl_match_wait on every member, then
+// fl_reco_shard_results on the owner.
+int fl_reco_shard_stage(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int src_W, int src_H, int W, int H,
+                        fl_intrinsics_t K_ref);
+int fl_reco_shard_match(fl_handle* h, int rank, int world, void* const* peers, int capacity, fl_match_t* block, uint32_t epoch);
+int fl_reco_shard_tail(fl_handle* h);
+int fl_reco_shard_results(fl_handle* h, fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary);

@@ -16,7 +16,8 @@
  *   fl_icp_cloud_to_cloud_ex ............. icpCloudToCloud_Ex ICP/ICP.h:165-172, ICP/ICP.cpp:617-809
  *   fl_detection / fl_detection_batch .... detection() ICP/detection.h:9-11, ICP/detection.cpp:11-254
  *   fl_nms ............................... nonMaximumSuppression ICP/NMS.h:14-16, ICP/NMS.cpp:6-39
- *   fl_group_* ........................... the same Detector::match over N GPUs of one process (templates sharded)
+ *   fl_group_* ........................... the same Detector::match, and Recognition with several frames in flight, over N GPUs
+ *                                          of one process (templates sharded)
  *   fl_debug_get ......................... stage-level exports for bit-exact parity checks (no reference equivalent)
  *
  * The library is CUDA-only (sm_100a): there is no CPU fallback; every call fails with FL_ERR_CUDA if no
@@ -256,11 +257,20 @@ int fl_exchange_sort_unique_device_async(fl_handle* h, int32_t rank, int32_t wor
  * handle's list.  exchange_capacity = candidate records one handle may emit per frame (more -> FL_ERR_CAPACITY). */
 typedef struct fl_group fl_group;
 int fl_group_create(const fl_params_t* params, const int32_t* devices, int32_t n, int32_t exchange_capacity, fl_group** out);
+/* the same with `depth` slots (1 .. FL_PIPE_MAX_DEPTH; fl_group_create = depth 1): every (member, slot) pair has its own handle,
+ * exchange buffer, candidate block and epoch sequence, so that up to `depth` recognition frames are in flight (fl_group_submit_recognition).
+ * FL_ERR_ARG for depth or n out of range (n <= 8) and NULL pointers; on failure *out is NULL. */
+int fl_group_create_pipe(const fl_params_t* params, const int32_t* devices, int32_t n, int32_t exchange_capacity, int32_t depth, fl_group** out);
 int fl_group_destroy(fl_group* g);
-int32_t fl_group_size(const fl_group* g);
-fl_handle* fl_group_handle(fl_group* g, int32_t i);          /* handle i (e.g. for fl_get_pose_info, fl_detection_batch*) */
+int32_t fl_group_size(const fl_group* g);                     /* members (n) */
+int32_t fl_group_depth(const fl_group* g);
+int32_t fl_group_in_flight(const fl_group* g);                /* recognition frames submitted and not collected */
+/* handle i = slot * n + member, i in [0, n * depth) (e.g. for fl_get_pose_info, fl_detection_batch*, fl_launch_count); fl_group_match
+ * runs on slot 0 */
+fl_handle* fl_group_handle(fl_group* g, int32_t i);
 int fl_group_upload_templates(fl_group* g, int32_t n_templates, const fl_template_hdr_t* headers, const fl_feature_t* features,
-                              int32_t n_features, const int32_t* class_of, const float* pose13);   /* layout of fl_upload_templates */
+                              int32_t n_features, const int32_t* class_of, const float* pose13);   /* layout of fl_upload_templates, every slot */
+/* FL_ERR_STATE while recognition frames are in flight */
 int fl_group_match(fl_group* g, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int32_t W, int32_t H,
                    float threshold, const int32_t* class_filter, int32_t n_filter, fl_match_t* out, int32_t capacity, int32_t* count);
 
@@ -378,6 +388,27 @@ int fl_pipe_set_recognition(fl_pipe* p, const fl_reco_params_t* params, const in
 int fl_pipe_submit_recognition(fl_pipe* p, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
                                int32_t src_W, int32_t src_H, int32_t W, int32_t H, fl_intrinsics_t K_ref);
 int fl_pipe_collect_recognition(fl_pipe* p, fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary);
+/* The same over a template-sharded group (fl_group_create_pipe): frame f goes to slot f % depth of every member; each member uploads
+ * [and rescales] the frame, matches its shard and takes part in the peer-memory exchange, after which every member holds the merged
+ * list; only the frame's owner, member f % n, runs the selection, ICP and suppression on it.  One host thread, results in submission
+ * order, equal to a single handle's fl_recognize over the whole set.
+ * fl_group_upload_model_depths: layout of fl_upload_model_depths; the crops go to every slot of every member (any member can own a
+ * frame).  fl_group_set_recognition: crop_of_template and pose12 (nullable: the uploaded pose13) cover the whole set in the order of
+ * fl_group_upload_templates; checks and statuses of fl_set_recognition; cleared by a later template or crop upload.  Memory: every
+ * slot of every member holds all crops and a 72-byte selection record per template of the set.
+ * Submit / collect / recognize: arguments and statuses of their fl_pipe_* / fl_recognize counterparts; FL_ERR_STATE with `depth`
+ * frames in flight, before the set-up, or on collect with nothing in flight.  Collecting frees the slot whatever the frame's status:
+ * a missing peer (FL_ERR_STATE) or an overflowing exchange block (FL_ERR_CAPACITY) is that frame's status only.  A front-end time-out
+ * on a member re-runs the frame on every member of its slot from the frames already staged there. */
+int fl_group_upload_model_depths(fl_group* g, int32_t n_models, const uint16_t* const* model_depth, const size_t* model_stride,
+                                 const fl_rect_t* rect_model, int32_t W, int32_t H);
+int fl_group_set_recognition(fl_group* g, const fl_reco_params_t* params, const int32_t* crop_of_template, const float* pose12);
+int fl_group_submit_recognition(fl_group* g, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
+                                int32_t src_W, int32_t src_H, int32_t W, int32_t H, fl_intrinsics_t K_ref);
+int fl_group_collect_recognition(fl_group* g, fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary);
+int fl_group_recognize(fl_group* g, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
+                       int32_t src_W, int32_t src_H, int32_t W, int32_t H, fl_intrinsics_t K_ref,
+                       fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary);
 
 /* ---- stage-level debug exports (host copies of device intermediates of the LAST match call) -------- */
 enum {

@@ -311,6 +311,24 @@ class Detector {
     fealess_b200::check_status(rc, "fl_pipe_upload_templates");
     return pipe;
   }
+  // mirror-only: the multi-device counterpart of createPipe - a group over the useDevices() list with `depth` slots (fl_group_create_pipe)
+  // for frames up to W x H, holding this detector's templates in the order match() uploads them, dealt gid % n.  The caller owns it
+  // (fl_group_destroy).
+  fl_group* createGroupPipe(int depth, int W, int H) const {
+    if (devices_.size() < 2) throw cv::Exception("Detector::createGroupPipe needs useDevices() with two or more devices");
+    fl_params_t p = device_params(W, H);
+    std::vector<int32_t> dv(devices_.begin(), devices_.end());
+    fl_group* group = nullptr;
+    fealess_b200::check_status(fl_group_create_pipe(&p, dv.data(), (int32_t)dv.size(), xcap_, depth, &group), "fl_group_create_pipe");
+    std::vector<fl_template_hdr_t> hdr; std::vector<fl_feature_t> feat; std::vector<int32_t> class_of;
+    flatten(hdr, feat, class_of);
+    const int rc = fl_group_upload_templates(group, (int32_t)class_of.size(), hdr.data(), feat.data(), (int32_t)feat.size(), class_of.data(), nullptr);
+    if (rc != FL_OK) fl_group_destroy(group);
+    fealess_b200::check_status(rc, "fl_group_upload_templates");
+    return group;
+  }
+  // mirror-only: the device list of useDevices() (empty: the default device)
+  const std::vector<int>& devices() const { return devices_; }
 
  protected:
   std::vector<Ptr<Modality> > modalities;

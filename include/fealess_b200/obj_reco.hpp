@@ -16,6 +16,9 @@
 //   SetFramesInFlight / SubmitRecognition / CollectRecognition (not in the reference): the same Recognition as a stream - every frame
 //                                   is ONE enqueue on the device (fl_pipe_submit_recognition: rescale, match, hypothesis selection, ICP,
 //                                   suppression), up to k frames are in flight from one thread, results come back in submission order.
+//   SetDevices (not in the reference): the detector's templates are sharded over several GPUs of this process (Detector::useDevices);
+//                                   Recognition and the stream then run over a template-sharded group (fl_group_*_recognition), with the
+//                                   single-GPU class's results.
 //
 // Kept from the reference on purpose: detection() receives the CALLER's intrinsics, not the zoomed ones (:188, SURVEY.md A.6 v);
 // only matches[0] is refined (:111).  A rect that leaves the frame raises cv::Exception (the reference's cv::Mat ROI assert,
@@ -83,7 +86,7 @@ class CObjRecoCAD {
 class CObjRecoLmICP : public CObjRecoCAD {
  public:
   CObjRecoLmICP() : m_matching_threshold(75.0f), m_icp_it_thr(10), m_dist_mean_thr(0.5f), m_dist_diff_thr(0.01f), m_proc_w(0), m_proc_h(0), m_crops_w(0), m_crops_h(0) {}   // :47-56
-  virtual ~CObjRecoLmICP() { close_stream(); }
+  virtual ~CObjRecoLmICP() { close_stream(m_stream); close_stream(m_sync); }
   virtual int Train(const string&, const TScanPackage&, const TTrainParam&) { return 0; }
   virtual int ClearObj() { return 0; }
   virtual int SetROI(const TImageU&) { return 0; }
@@ -94,7 +97,8 @@ class CObjRecoLmICP : public CObjRecoCAD {
     m_str_lm_feature_path = str_feature_path;
     m_lm_detector = readLinemod(m_str_lm_feature_path + string("/linemod_templates.yml"));
     m_model_depth.clear(); m_crop_index.clear(); m_crops_w = m_crops_h = 0;
-    close_stream();
+    close_stream(m_stream); close_stream(m_sync);
+    if (!m_devices.empty()) m_lm_detector->useDevices(m_devices, m_xcap);   // SetDevices outlives the detector it was first applied to
     if (0 == m_lm_detector->numClasses()) return (int)ERROR_OPEN_FILE_FAILED;
     // the reference names the file by template_id alone (:156), so one image serves that id in every class
     int max_templates = 0;
@@ -113,6 +117,7 @@ class CObjRecoLmICP : public CObjRecoCAD {
     vtResult.clear();
     if (!m_lm_detector || 0 != PrepareInputData(tRGB, tDepth, tCamIntrinsic)) return (int)ERROR_INVALID_PARAM;
     if (m_lm_detector->getModalities().size() != 2) return (int)ERROR_INVALID_PARAM;   // match() == -1: two sources are passed (:94-96, linemod.cpp:1364)
+    if (multi_device()) return recognition_on_group(tRGB, tDepth, tCamIntrinsic, vtResult);
     std::vector<cup_linemod::Match> matches;
     if (0 != m_lm_detector->matchRescaled(tRGB.pData, (size_t)tRGB.nWidth * 3, tDepth.pData, (size_t)tDepth.nWidth * 2, tRGB.nWidth, tRGB.nHeight,
                                           m_proc_w, m_proc_h, m_matching_threshold, matches))
@@ -186,35 +191,44 @@ class CObjRecoLmICP : public CObjRecoCAD {
   // results of the oldest queued frame, equal to Recognition's, and throws where Recognition throws.  Up to k frames
   // (<= FL_PIPE_MAX_DEPTH) are in flight; SetFramesInFlight, SetHypotheses and a new frame size take effect on an empty stream.
   void SetFramesInFlight(int k) {
-    if (m_pipe && fl_pipe_in_flight(m_pipe)) throw std::runtime_error("SetFramesInFlight: frames are in flight");
+    if (in_flight(m_stream)) throw std::runtime_error("SetFramesInFlight: frames are in flight");
     m_frames_in_flight = k < 1 ? 1 : k > FL_PIPE_MAX_DEPTH ? FL_PIPE_MAX_DEPTH : k;
-    close_stream();
+    close_stream(m_stream);
   }
   int SubmitRecognition(const TImageU& tRGB, const TImageU16& tDepth, const TCamIntrinsicParam& tCamIntrinsic) {
     if (!m_lm_detector || 0 != PrepareInputData(tRGB, tDepth, tCamIntrinsic)) return (int)ERROR_INVALID_PARAM;
     if (m_lm_detector->getModalities().size() != 2) return (int)ERROR_INVALID_PARAM;   // as Recognition
-    stream_setup();
+    stream_setup(m_stream, m_frames_in_flight);
     const fl_intrinsics_t K = {(float)tCamIntrinsic.dFx, (float)tCamIntrinsic.dFy, (float)tCamIntrinsic.dCx, (float)tCamIntrinsic.dCy};   // the caller's (:188)
-    const int rc = fl_pipe_submit_recognition(m_pipe, tRGB.pData, (size_t)tRGB.nWidth * 3, tDepth.pData, (size_t)tDepth.nWidth * 2, tRGB.nWidth, tRGB.nHeight,
-                                              m_proc_w, m_proc_h, K);
+    const int rc = m_stream.group ? fl_group_submit_recognition(m_stream.group, tRGB.pData, (size_t)tRGB.nWidth * 3, tDepth.pData, (size_t)tDepth.nWidth * 2,
+                                                                tRGB.nWidth, tRGB.nHeight, m_proc_w, m_proc_h, K)
+                                  : fl_pipe_submit_recognition(m_stream.pipe, tRGB.pData, (size_t)tRGB.nWidth * 3, tDepth.pData, (size_t)tDepth.nWidth * 2,
+                                                               tRGB.nWidth, tRGB.nHeight, m_proc_w, m_proc_h, K);
     if (rc == FL_ERR_SIZE) return (int)ERROR_INVALID_PARAM;
     fealess_b200::check_status(rc, "SubmitRecognition");
     return 0;
   }
   int CollectRecognition(vector<TObjRecoResult>& vtResult) {
     vtResult.clear();
-    if (!m_pipe) fealess_b200::check_status(FL_ERR_STATE, "CollectRecognition: no frame in flight");
+    if (!m_stream.pipe && !m_stream.group) fealess_b200::check_status(FL_ERR_STATE, "CollectRecognition: no frame in flight");
     std::vector<fl_reco_result_t> res(FL_RECO_MAX_HYP);
     fl_reco_summary_t sum;
-    fealess_b200::check_status(fl_pipe_collect_recognition(m_pipe, res.data(), (int32_t)res.size(), &sum), "CollectRecognition");
-    if (sum.n_hypotheses == 1 && sum.n_roi == 1) fealess_b200::check_status(FL_ERR_ROI, "detection");   // Recognition's single detection() throws (detection.cpp:43-44)
-    for (int k = 0; k < sum.n_results; ++k) {
-      TObjRecoResult cur_result;
-      cur_result.strObjTag = m_stream_classes[(size_t)res[k].class_idx];
-      std::memcpy(cur_result.tWorld2Cam, res[k].world2cam, sizeof cur_result.tWorld2Cam);
-      vtResult.push_back(cur_result);
-    }
+    fealess_b200::check_status(m_stream.group ? fl_group_collect_recognition(m_stream.group, res.data(), (int32_t)res.size(), &sum)
+                                              : fl_pipe_collect_recognition(m_stream.pipe, res.data(), (int32_t)res.size(), &sum), "CollectRecognition");
+    convert_results(m_stream, res, sum, vtResult);
     return 0;
+  }
+
+  // NOT in the reference: shard the detector's templates over these GPUs of this process (Detector::useDevices; exchange_capacity =
+  // candidates one GPU may emit per frame).  Kept across AddObj, which replaces the detector.  With more than one device Recognition runs
+  // its frame through a depth-1 template-sharded group of its own and SubmitRecognition / CollectRecognition run over a group with
+  // SetFramesInFlight slots; results, exceptions and status codes are those of one GPU.  Masks are not supported there (SetROI is a stub).
+  void SetDevices(const std::vector<int>& devices, int exchange_capacity = 2048) {
+    if (in_flight(m_stream)) throw std::runtime_error("SetDevices: frames are in flight");
+    close_stream(m_stream); close_stream(m_sync);
+    m_devices = devices; m_xcap = exchange_capacity;
+    m_crops_w = m_crops_h = 0;                                   // the crops of the per-call path live on the detector's (new) handle
+    if (m_lm_detector) m_lm_detector->useDevices(m_devices, m_xcap);
   }
 
   // mirror-only accessors (tests, callers that want the zoomed intrinsics PrepareInputData stored)
@@ -290,48 +304,90 @@ class CObjRecoLmICP : public CObjRecoCAD {
       }
   }
 
-  // the pipe behind SubmitRecognition for the current frame size and hypothesis settings: the detector's templates and the crops on every
-  // slot, the crop index and Recognition's pose rule per template (getPoseInfo(template_id) in the reference's mode top_k = 1 without
-  // per_class, the class-keyed lookup otherwise)
-  void stream_setup() {
+  // what a stream was built for, and the pipe (one GPU) or template-sharded group (SetDevices with more than one device) behind it
+  struct Stream {
+    fl_pipe* pipe = nullptr; fl_group* group = nullptr;
+    int w = 0, h = 0, top_k = 0; bool per_class = false; float th = 0.f; size_t fingerprint = 0;
+    std::vector<cv::String> classes;
+    std::vector<int32_t> crop;
+  };
+  bool multi_device() const { return m_lm_detector && m_lm_detector->devices().size() > 1; }
+  static int in_flight(const Stream& st) { return st.group ? fl_group_in_flight(st.group) : st.pipe ? fl_pipe_in_flight(st.pipe) : 0; }
+
+  // the pipe (or group) behind SubmitRecognition / the multi-device Recognition for the current frame size and hypothesis settings: the
+  // detector's templates and the crops on every slot, the crop index and Recognition's pose rule per template (getPoseInfo(template_id)
+  // in the reference's mode top_k = 1 without per_class, the class-keyed lookup otherwise)
+  void stream_setup(Stream& st, int depth) {
     // templates added to the detector since the pipe was built: the same count check Detector::match uses before it re-uploads
     const size_t fingerprint = (size_t)m_lm_detector->numTemplates() * 4099u + (size_t)m_lm_detector->numClasses();
-    const bool same_size = m_pipe && m_stream_w == m_proc_w && m_stream_h == m_proc_h && m_stream_fingerprint == fingerprint;
-    if (same_size && m_stream_top_k == m_top_k && m_stream_per_class == m_per_class && m_stream_th == m_th_obj_dist) return;
-    if (m_pipe && fl_pipe_in_flight(m_pipe)) throw std::runtime_error("SubmitRecognition: frame size, templates or hypotheses changed with frames in flight");
+    const bool same_size = (st.pipe || st.group) && st.w == m_proc_w && st.h == m_proc_h && st.fingerprint == fingerprint;
+    if (same_size && st.top_k == m_top_k && st.per_class == m_per_class && st.th == m_th_obj_dist) return;
+    if (in_flight(st)) throw std::runtime_error("SubmitRecognition: frame size, templates or hypotheses changed with frames in flight");
     if (!same_size) {
-      close_stream();
-      m_pipe = m_lm_detector->createPipe(m_frames_in_flight, m_proc_w, m_proc_h);
+      close_stream(st);
       std::map<std::pair<cv::String, int>, int> index;
       std::vector<const uint16_t*> ptr; std::vector<size_t> stride; std::vector<fl_rect_t> rect;
       crop_table(index, ptr, stride, rect);
-      fealess_b200::check_status(fl_pipe_upload_model_depths(m_pipe, (int32_t)ptr.size(), ptr.data(), stride.data(), rect.data(), m_proc_w, m_proc_h),
-                                 "fl_pipe_upload_model_depths");
-      m_stream_classes = m_lm_detector->classIds();
-      m_stream_crop.clear();
-      for (size_t c = 0; c < m_stream_classes.size(); ++c)
-        for (int tid = 0; tid < m_lm_detector->numTemplates(m_stream_classes[c]); ++tid) {
-          std::map<std::pair<cv::String, int>, int>::const_iterator it = index.find(std::make_pair(m_stream_classes[c], tid));
-          m_stream_crop.push_back(it == index.end() ? -1 : it->second);
+      if (multi_device()) {
+        st.group = m_lm_detector->createGroupPipe(depth, m_proc_w, m_proc_h);
+        fealess_b200::check_status(fl_group_upload_model_depths(st.group, (int32_t)ptr.size(), ptr.data(), stride.data(), rect.data(), m_proc_w, m_proc_h),
+                                   "fl_group_upload_model_depths");
+      } else {
+        st.pipe = m_lm_detector->createPipe(depth, m_proc_w, m_proc_h);
+        fealess_b200::check_status(fl_pipe_upload_model_depths(st.pipe, (int32_t)ptr.size(), ptr.data(), stride.data(), rect.data(), m_proc_w, m_proc_h),
+                                   "fl_pipe_upload_model_depths");
+      }
+      st.classes = m_lm_detector->classIds();
+      st.crop.clear();
+      for (size_t c = 0; c < st.classes.size(); ++c)
+        for (int tid = 0; tid < m_lm_detector->numTemplates(st.classes[c]); ++tid) {
+          std::map<std::pair<cv::String, int>, int>::const_iterator it = index.find(std::make_pair(st.classes[c], tid));
+          st.crop.push_back(it == index.end() ? -1 : it->second);
         }
-      m_stream_w = m_proc_w; m_stream_h = m_proc_h; m_stream_fingerprint = fingerprint;
+      st.w = m_proc_w; st.h = m_proc_h; st.fingerprint = fingerprint;
     }
     std::vector<float> pose12;
-    for (size_t c = 0; c < m_stream_classes.size(); ++c)
-      for (int tid = 0; tid < m_lm_detector->numTemplates(m_stream_classes[c]); ++tid) {
-        const std::vector<float> pose = (m_top_k == 1 && !m_per_class) ? m_lm_detector->getPoseInfo(tid) : m_lm_detector->getPoseInfo(m_stream_classes[c], tid);
+    for (size_t c = 0; c < st.classes.size(); ++c)
+      for (int tid = 0; tid < m_lm_detector->numTemplates(st.classes[c]); ++tid) {
+        const std::vector<float> pose = (m_top_k == 1 && !m_per_class) ? m_lm_detector->getPoseInfo(tid) : m_lm_detector->getPoseInfo(st.classes[c], tid);
         pose12.insert(pose12.end(), pose.begin(), pose.begin() + 12);
       }
     fl_reco_params_t prm;
     fl_default_reco_params(&prm);
     prm.threshold = m_matching_threshold; prm.icp.icp_it_thr = m_icp_it_thr; prm.icp.dist_mean_thr = m_dist_mean_thr; prm.icp.dist_diff_thr = m_dist_diff_thr;
     prm.top_k = m_top_k; prm.per_class = m_per_class ? 1 : 0; prm.th_obj_dist = m_th_obj_dist;
-    fealess_b200::check_status(fl_pipe_set_recognition(m_pipe, &prm, m_stream_crop.data(), pose12.data()), "fl_pipe_set_recognition");
-    m_stream_top_k = m_top_k; m_stream_per_class = m_per_class; m_stream_th = m_th_obj_dist;
+    if (st.group) fealess_b200::check_status(fl_group_set_recognition(st.group, &prm, st.crop.data(), pose12.data()), "fl_group_set_recognition");
+    else fealess_b200::check_status(fl_pipe_set_recognition(st.pipe, &prm, st.crop.data(), pose12.data()), "fl_pipe_set_recognition");
+    st.top_k = m_top_k; st.per_class = m_per_class; st.th = m_th_obj_dist;
   }
-  void close_stream() {
-    if (m_pipe) fl_pipe_destroy(m_pipe);
-    m_pipe = nullptr; m_stream_w = m_stream_h = 0;
+  static void close_stream(Stream& st) {
+    if (st.pipe) fl_pipe_destroy(st.pipe);
+    if (st.group) fl_group_destroy(st.group);
+    st.pipe = nullptr; st.group = nullptr; st.w = st.h = 0;
+  }
+  // device results -> TObjRecoResult; throws where Recognition's single detection() throws (detection.cpp:43-44)
+  static void convert_results(const Stream& st, const std::vector<fl_reco_result_t>& res, const fl_reco_summary_t& sum, vector<TObjRecoResult>& vtResult) {
+    if (sum.n_hypotheses == 1 && sum.n_roi == 1) fealess_b200::check_status(FL_ERR_ROI, "detection");
+    for (int k = 0; k < sum.n_results; ++k) {
+      TObjRecoResult cur_result;
+      cur_result.strObjTag = st.classes[(size_t)res[k].class_idx];
+      std::memcpy(cur_result.tWorld2Cam, res[k].world2cam, sizeof cur_result.tWorld2Cam);
+      vtResult.push_back(cur_result);
+    }
+  }
+  // Recognition over several GPUs: the frame through a depth-1 group of this object's own (rescale, sharded match, selection, ICP and
+  // suppression on the device), rebuilt under the conditions that rebuild the stream
+  int recognition_on_group(const TImageU& tRGB, const TImageU16& tDepth, const TCamIntrinsicParam& tCamIntrinsic, vector<TObjRecoResult>& vtResult) {
+    stream_setup(m_sync, 1);
+    const fl_intrinsics_t K = {(float)tCamIntrinsic.dFx, (float)tCamIntrinsic.dFy, (float)tCamIntrinsic.dCx, (float)tCamIntrinsic.dCy};   // the caller's (:188)
+    std::vector<fl_reco_result_t> res(FL_RECO_MAX_HYP);
+    fl_reco_summary_t sum;
+    const int rc = fl_group_recognize(m_sync.group, tRGB.pData, (size_t)tRGB.nWidth * 3, tDepth.pData, (size_t)tDepth.nWidth * 2, tRGB.nWidth, tRGB.nHeight,
+                                      m_proc_w, m_proc_h, K, res.data(), (int32_t)res.size(), &sum);
+    if (rc == FL_ERR_SIZE) return (int)ERROR_INVALID_PARAM;     // matchRescaled's -1
+    fealess_b200::check_status(rc, "Recognition");
+    convert_results(m_sync, res, sum, vtResult);
+    return 0;
   }
 
   string m_str_lm_feature_path;
@@ -343,12 +399,10 @@ class CObjRecoLmICP : public CObjRecoCAD {
   std::map<std::pair<cv::String, int>, int> m_crop_index;        // (class, template_id) -> crop on the device
   int m_crops_w, m_crops_h;
   int m_top_k = 1; bool m_per_class = false; float m_th_obj_dist = 0.f;   // SetHypotheses
-  // SubmitRecognition / CollectRecognition: the pipe and what it was set up for
+  // SubmitRecognition / CollectRecognition (m_stream) and the multi-device Recognition (m_sync, one slot)
   int m_frames_in_flight = 1;
-  fl_pipe* m_pipe = nullptr;
-  int m_stream_w = 0, m_stream_h = 0, m_stream_top_k = 0; bool m_stream_per_class = false; float m_stream_th = 0.f; size_t m_stream_fingerprint = 0;
-  std::vector<cv::String> m_stream_classes;
-  std::vector<int32_t> m_stream_crop;
+  Stream m_stream, m_sync;
+  std::vector<int> m_devices; int m_xcap = 2048;                 // SetDevices
   CObjRecoLmICP(const CObjRecoLmICP&) = delete;
   CObjRecoLmICP& operator=(const CObjRecoLmICP&) = delete;
 };
