@@ -32,7 +32,7 @@ _SO = os.path.join(_HERE, "libfealess_b200.so")
 
 FL_OK, FL_ERR_SIZE, FL_ERR_GEOMETRY, FL_ERR_ROI, FL_ERR_FEATURES = 0, -1, -2, -3, -4
 FL_ERR_ARG, FL_ERR_CAPACITY, FL_ERR_CUDA, FL_ERR_STATE, FL_ERR_TRAIN = -5, -6, -7, -8, -9
-FL_OPT_FE_WAVES, FL_OPT_SPLIT_REFINE, FL_OPT_TRACE, FL_OPT_FE_DEP_TIMEOUT_TEST, FL_OPT_FE_FORCED_WAVES = 0, 1, 2, 3, 4
+FL_OPT_FE_WAVES, FL_OPT_SPLIT_REFINE, FL_OPT_TRACE, FL_OPT_FE_DEP_TIMEOUT_TEST, FL_OPT_FE_FORCED_WAVES, FL_OPT_SIM_NO_PRUNE = 0, 1, 2, 3, 4, 5
 FL_DBG_QUANTIZED, FL_DBG_SPREAD, FL_DBG_LINEAR_MEMORY, FL_DBG_SIMILARITY, FL_DBG_STAGED_TRACE, FL_DBG_LAST_COUNTS, FL_DBG_FE_TRACE = 0, 1, 2, 3, 4, 5, 6
 
 MATCH_DTYPE = np.dtype([("x", "<i4"), ("y", "<i4"), ("similarity", "<f4"), ("class_idx", "<i4"), ("template_id", "<i4")])

@@ -66,7 +66,7 @@ struct fl_handle {
   bool pend_sort = false, pend_match = false, pend_own = false, pend_masks_valid = false, pend_small_fused = false; fl_lists pend_lists = {}; fl_match_t* pend_out = nullptr; int pend_out_cap = 0; int* pend_out_count = nullptr;
   const void* pend_bgr = nullptr; const void* pend_depth = nullptr; int pend_W = 0, pend_H = 0; float pend_threshold = 0.f; const void* pend_masks[FL_MAX_MODALITIES] = {}; std::vector<int32_t> pend_filter;
   fl_dev_buf<unsigned long long> d_fe_trace; int fe_trace_jobs = 0, fe_trace_kind[FL_FE_MAX_JOBS] = {}, fe_trace_ctas[FL_FE_MAX_JOBS] = {};
-  bool opt_fe_waves = false, opt_split_refine = false, opt_trace = false, opt_dep_test = false;   // fl_debug_option
+  bool opt_fe_waves = false, opt_split_refine = false, opt_trace = false, opt_dep_test = false, opt_no_prune = false;   // fl_debug_option
   fl_mapped_buf<int> h_fe_err; int* d_fe_err_host = nullptr; bool fe_force_waves = false;   // in-grid dependency time-out: mapped host flag (+ its device alias); true = this handle launches one kernel per wave from now on
   fl_dev_buf<unsigned> d_fe_counters; unsigned fe_counter_base[FL_FE_MAX_JOBS] = {}; unsigned fe_row_base[FL_FE_MAX_JOBS] = {};   // in-grid dependency counters of the single-launch front end (+ 1 error word)
   // candidates / matches
@@ -251,6 +251,7 @@ extern "C" int fl_debug_option(fl_handle* h, int option, int value) {
     case FL_OPT_TRACE: h->opt_trace = value != 0; h->packed = false; return FL_OK;     // (the staged plan allocates its timeline at planning time)
     case FL_OPT_FE_DEP_TIMEOUT_TEST: h->opt_dep_test = value != 0; return FL_OK;
     case FL_OPT_FE_FORCED_WAVES: return h->fe_force_waves ? 1 : 0;                      // query: has a dependency time-out switched this handle to wave launches?
+    case FL_OPT_SIM_NO_PRUNE: h->opt_no_prune = value != 0; return FL_OK;
   }
   return FL_ERR_ARG;
 }
@@ -658,6 +659,7 @@ static int run_match_stages(fl_handle* h, const uint8_t* d_bgr, const uint16_t* 
     fl_tdb db = make_tdb(h);
     const int lowest = p.n_levels - 1;
     if (h->use_staged) {
+      h->plan.prune = h->opt_no_prune ? 0 : 1;
       if (fl_launch_similarity_staged(db, h->geom[lowest], h->d_lm4.get(), threshold, cand, cap, d_count, h->plan, s) != 0) {
         fl_set_error("staged similarity kernel could not be configured"); return FL_ERR_CUDA;
       }

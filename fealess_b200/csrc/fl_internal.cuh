@@ -136,6 +136,7 @@ struct fl_staged_plan {
   int tpc, n_cta, block_threads;           // templates per CTA, grid, block
   int smem_bytes, pre_stride;              // dynamic shared memory; bytes per gpre row
   int stage_off;                           // emission staging area (one similarity map, nw_template x 32 words)
+  int prune;                               // 1: drop a template once no position can reach the threshold (off: FL_OPT_SIM_NO_PRUNE)
   uint32_t* gfeat;                         // [n_templates][64] feature words sorted by phase: word offset in the phase buffer << 5 | 8 * byte misalignment
   uint8_t* gpre;                           // [n_templates][pre_stride] prefix counts per phase
   int4* gmeta;                             // [n_templates] {template_positions, n_features, class, 0}

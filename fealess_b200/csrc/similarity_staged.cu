@@ -167,6 +167,28 @@ __device__ __forceinline__ void accumulate_features(const uint8_t* __restrict__ 
   }
 }
 
+// per-byte maxima of packed u8 values, two 16-bit lanes at a time: the high byte of each lane of max.u16x2 is the larger of the two
+// high bytes (the high byte decides a 16-bit comparison); the low bytes are garbage and ignored
+__device__ __forceinline__ uint32_t vmax_u16x2(uint32_t a, uint32_t b) { uint32_t d; asm("max.u16x2 %0, %1, %2;" : "=r"(d) : "r"(a), "r"(b)); return d; }
+
+// Early exit (DESIGN.md 4.1): after a phase, a slot whose every position p < template_positions has partial(p) + 4 x (features
+// left) <= raw_thr can produce no candidate (a response is at most 4) and is dropped.  "Any byte >= t" over the lane's accumulator
+// words: the even cells are lo - 16 hi (see accumulate_features), the odd ones hi; words wholly at or past template_positions
+// (nvw = the lane's words that hold a valid cell) are left out.  Per word: 1 IMAD, 2 shifts, 4 max.u16x2.
+template <int NW>
+__device__ __forceinline__ bool any_byte_at_least(const uint32_t (&lo)[NW], const uint32_t (&hi)[NW], int nvw, int t) {
+  uint32_t mh = 0, ml = 0;                                   // maxima of bytes 1, 3 / of bytes 0, 2 (shifted up by 8), in the high bytes
+#pragma unroll
+  for (int i = 0; i < NW; ++i)
+    if (i < nvw) {
+      const uint32_t e = lo[i] - (hi[i] << 4);
+      mh = vmax_u16x2(vmax_u16x2(mh, e), hi[i]);
+      ml = vmax_u16x2(vmax_u16x2(ml, e << 8), hi[i] << 8);
+    }
+  const uint32_t m = vmax_u16x2(mh, ml);
+  return (int)max((m >> 8) & 0xFFu, m >> 24) >= t;
+}
+
 // (Refining the candidates in this kernel's own tail was measured much slower than the separate launch - stage 143 us vs 43 + 11 us:
 // candidates cluster in the few CTAs that own a matching template while the other 140 CTAs idle - and was removed.)
 template <int NW, int TPW>
@@ -175,9 +197,13 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
   extern __shared__ __align__(128) uint8_t s_dyn[];          // [n_buf x buf_bytes][tpc x int4 meta][tpc x 64 feature words + 4][tpc x pre_stride][emission staging]
   __shared__ __align__(8) uint64_t s_full[SS_NBUF_MAX], s_empty[SS_NBUF_MAX];
   __shared__ int s_emit_lock;                                 // the CTA's emission staging area is taken by one warp at a time
+  __shared__ int s_live;                                      // template slots of this CTA that may still produce a candidate (early exit)
+  __shared__ int s_stop;                                      // set by the producer when it issues no more phases (see the producer)
   __shared__ __align__(8) uint64_t s_aux;                     // completion of the bulk copy of this CTA's feature lists
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int n_cwarps = (blockDim.x >> 5) - 1;                 // consumer warps; the last warp is the TMA producer
+  // early exit (see any_byte_at_least); NW = 15 has no registers left for its test (ptxas spills), so it accumulates every template
+  const bool prune = NW < 15 && plan.prune;
   const int t_begin = blockIdx.x * plan.tpc;
   const int t_end = min(t_begin + plan.tpc, db.n_templates);
   const int n_phases = plan.n_phases, n_buf = plan.n_buf;
@@ -193,6 +219,8 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
 
   if (tid == 0) {
     s_emit_lock = 0;
+    s_live = max(t_end - t_begin, 0);                         // slots without positions are taken off by the consumers' prologue
+    s_stop = 0;
     for (int b = 0; b < n_buf; ++b) { mbar_init(&s_full[b], 1); mbar_init(&s_empty[b], n_cwarps); }
     mbar_init(&s_aux, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -250,6 +278,21 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
       for (int q = 0; q < n_phases; ++q) {
         const int b = q % n_buf;
         if (q >= n_buf) mbar_wait(&s_empty[b], ((q / n_buf) - 1) & 1);
+        // Early exit: no live slot left -> no more phases.  The consumers wait on s_full[b] for phase q whatever happens, so the stop
+        // is announced through that barrier: s_stop is written first and a plain arrive (count 1, no bytes) completes phase q of
+        // s_full[b]; the arrive releases and the consumers' wait acquires, so every consumer that sees phase q complete reads
+        // s_stop = 1 and leaves the loop without arriving on s_empty (a warp still behind, at an earlier phase, may see it sooner and
+        // skip that phase's work: it has no live slot either).  Nothing waits on s_empty after that.  Copies still in
+        // flight are those of phases q - n_buf + 1 .. q - 1 (phase q - n_buf completed before s_empty[b] could); their buffers are
+        // this CTA's shared memory, so they are waited for here before the thread exits (each of those s_full barriers completes
+        // once more at most: the next use of its buffer would be a phase >= q, never issued).  s_live is read without ordering:
+        // a decrement seen one phase late only costs one more phase.
+        if (prune && *(volatile int*)&s_live == 0) {
+          *(volatile int*)&s_stop = 1;
+          mbar_arrive(&s_full[b]);
+          for (int r = max(q - n_buf + 1, 0); r < q; ++r) mbar_wait(&s_full[r % n_buf], (r / n_buf) & 1);
+          break;
+        }
         int p = q + rot; if (p >= n_phases) p -= n_phases;
         const int grp = p / plan.n_rowblocks, rb = p - grp * plan.n_rowblocks;
         const int ml = grp * plan.labels_per_phase;             // first (modality, label) of the group; a group never straddles modalities
@@ -265,7 +308,7 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
     }
   } else {
     // ===== consumers =====
-    bool live[TPW];
+    bool live[TPW];                                           // false: no positions, or dropped by the early exit (pre[s] is then NULL too)
     const uint8_t* pre[TPW];
     const uint32_t* fl[TPW];
     uint32_t lo[TPW][NW], hi[TPW][NW];
@@ -274,6 +317,7 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
       const int slot = warp + s * n_cwarps;
       const int t = t_begin + slot;
       const bool in = slot < plan.tpc && t < t_end && s_meta[slot < plan.tpc ? slot : 0].x > 0;   // no positions (or disabled class): no work at all
+      if (slot < plan.tpc && t < t_end && !in && lane == 0) atomicSub(&s_live, 1);
       live[s] = in;
       pre[s] = s_pre + (in ? slot : 0) * plan.pre_stride;
       fl[s] = s_feat + (in ? slot : 0) * SS_MAXF;
@@ -301,6 +345,7 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
           "bra CWAIT_LOOP;\n"
           "CWAIT_DONE:\n"
           "}\n" ::"r"(full_a), "r"(par) : "memory");
+      if (*(volatile int*)&s_stop) break;                     // the producer issued no phase q (early exit, see the producer)
       if (trace && tid == 0 && q == 0) trace[2] = globaltimer();
 #pragma unroll
       for (int s = 0; s < TPW; ++s) {
@@ -326,6 +371,28 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
       }
       __syncwarp();
       if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(empty_a) : "memory");   // this warp is done with the buffer
+      // early exit, after the release so that the producer never waits for it.  The bound only bites once raw_thr + 1 > 4 x
+      // (features left); a slot without new features keeps its verdict.  A dropped slot does no more feature work and emits nothing;
+      // its warp stays in step with the ring (wait on s_full, arrive on s_empty), which costs a wait and an arrive per phase.
+      // (The features left are re-read from the prefix counts - phases rot .. p are done - rather than kept in registers: the
+      // accumulators leave no room for them.)
+      if (prune) {
+#pragma unroll
+        for (int s = 0; s < TPW; ++s) {
+          if (!pre[s]) continue;
+          const int k1 = pre[s][p + 1];
+          if (pre[s][p] == k1) continue;                      // warp-uniform
+          const int k_rot = pre[s][rot];
+          const int rem = p >= rot ? pre[s][n_phases] - k1 + k_rot : k_rot - k1;
+          const int4 meta = s_meta[warp + s * n_cwarps];
+          const int t = (meta.y >> 8) - 4 * rem;              // (meta.y >> 8) = raw_thr + 1
+          if (t <= 0) continue;
+          const int nvw = min(max((meta.x - lane * (NW * 8) + 7) >> 3, 0), NW);
+          if (__any_sync(0xffffffffu, any_byte_at_least<NW>(lo[s], hi[s], nvw, t))) continue;
+          pre[s] = nullptr; live[s] = false;
+          if (lane == 0) atomicSub(&s_live, 1);
+        }
+      }
       full_a += 8; empty_a += 8; lane_base += buf_bytes;
       if (full_a == ring_end) { full_a -= 8u * (uint32_t)n_buf; empty_a -= 8u * (uint32_t)n_buf; lane_base -= (size_t)n_buf * buf_bytes; par ^= 1; }
       if (++p == n_phases) p = 0;
@@ -557,6 +624,7 @@ bool fl_plan_staged(const fl_level_geom& g, int M, int n_templates, int max_posi
   p.stage_off = (p.smem_bytes + 15) & ~15;
   p.smem_bytes = p.stage_off + (int)stage_bytes;
   if (p.smem_bytes > 227 * 1024 - 512) return false;
+  p.prune = 1;
   *plan = p;
   return true;
 }

@@ -430,7 +430,9 @@ enum {
   FL_OPT_SPLIT_REFINE = 1,        /* refinement and sort + unique as separate launches instead of one */
   FL_OPT_TRACE = 2,               /* record the in-kernel timelines (FL_DBG_STAGED_TRACE, front-end job timeline); slows the frame down */
   FL_OPT_FE_DEP_TIMEOUT_TEST = 3, /* the next frame's first in-grid dependency can never be satisfied: exercises the time-out fallback (takes ~1 s) */
-  FL_OPT_FE_FORCED_WAVES = 4      /* query (value ignored): 1 if a dependency time-out has switched this handle to per-wave launches */
+  FL_OPT_FE_FORCED_WAVES = 4,     /* query (value ignored): 1 if a dependency time-out has switched this handle to per-wave launches */
+  FL_OPT_SIM_NO_PRUNE = 5         /* the staged similarity kernel accumulates every template in full instead of dropping one once no
+                                     position can reach the threshold (same results; for A/B measurements and tests) */
 };
 int fl_debug_option(fl_handle* h, int option, int value);
 int fl_debug_keep_spread(fl_handle* h, int enable);
