@@ -33,7 +33,9 @@ _SO = os.path.join(_HERE, "libfealess_b200.so")
 FL_OK, FL_ERR_SIZE, FL_ERR_GEOMETRY, FL_ERR_ROI, FL_ERR_FEATURES = 0, -1, -2, -3, -4
 FL_ERR_ARG, FL_ERR_CAPACITY, FL_ERR_CUDA, FL_ERR_STATE, FL_ERR_TRAIN = -5, -6, -7, -8, -9
 FL_OPT_FE_WAVES, FL_OPT_SPLIT_REFINE, FL_OPT_TRACE, FL_OPT_FE_DEP_TIMEOUT_TEST, FL_OPT_FE_FORCED_WAVES, FL_OPT_SIM_NO_PRUNE = 0, 1, 2, 3, 4, 5
+FL_OPT_SIM_ROTATE = 6
 FL_DBG_QUANTIZED, FL_DBG_SPREAD, FL_DBG_LINEAR_MEMORY, FL_DBG_SIMILARITY, FL_DBG_STAGED_TRACE, FL_DBG_LAST_COUNTS, FL_DBG_FE_TRACE = 0, 1, 2, 3, 4, 5, 6
+FL_DBG_STAGED_ORDER = 7
 
 MATCH_DTYPE = np.dtype([("x", "<i4"), ("y", "<i4"), ("similarity", "<f4"), ("class_idx", "<i4"), ("template_id", "<i4")])
 ICP_RESULT_DTYPE = np.dtype([("R", "<f4", (9,)), ("T", "<f4", (3,)), ("dist_mean", "<f4"), ("inlier_ratio", "<f4"),
@@ -440,6 +442,15 @@ class Handle:
         if n < 0:
             _check(n, "fl_debug_get(FL_DBG_STAGED_TRACE)")
         return buf[:n * 8].reshape(n, 8).astype(np.int64)
+
+    def staged_order(self):
+        """FL_DBG_STAGED_ORDER: (order, mass) of the last staged similarity launch: order[q] = the phase CTA 0 visited at step q,
+        mass[8 m + l] = the coarsest level's response sum of (modality m, label l) the order was derived from."""
+        buf = np.zeros(32 * 4 + 256, np.uint8)
+        n = lib().fl_debug_get(self._h, FL_DBG_STAGED_ORDER, 0, 0, 0, C.c_void_p(buf.ctypes.data), C.c_size_t(buf.nbytes))
+        if n < 0:
+            _check(n, "fl_debug_get(FL_DBG_STAGED_ORDER)")
+        return buf[128:128 + n].astype(np.int64), buf[:128].view(np.uint32).astype(np.int64)
 
     def fe_trace(self):
         """FL_DBG_FE_TRACE: [n_jobs, 4] int64 {kind, CTAs, first start ns, last end ns} of the front end of the last frame."""

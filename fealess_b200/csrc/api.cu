@@ -61,12 +61,13 @@ struct fl_handle {
   fl_dev_buf<uint8_t> d_mask[FL_MAX_LEVELS][FL_MAX_MODALITIES];
   fl_dev_buf<uint8_t> d_spread[FL_MAX_LEVELS][FL_MAX_MODALITIES];  // debug only
   fl_dev_buf<uint8_t> d_lm[FL_MAX_LEVELS]; fl_dev_buf<uint8_t> d_lm4;   // d_lm4: 4-bit copy of the coarsest level's linear memories
+  fl_dev_buf<uint32_t> d_mass;                                         // response mass of the coarsest level (FL_MASS_*): the staged kernel's phase order
   bool used_mask[FL_MAX_MODALITIES] = {}; bool keep_spread = false;
   // state between the enqueue half (fl_match_device_async, ..._async) and fl_match_wait
   bool pend_sort = false, pend_match = false, pend_own = false, pend_masks_valid = false, pend_small_fused = false; fl_lists pend_lists = {}; fl_match_t* pend_out = nullptr; int pend_out_cap = 0; int* pend_out_count = nullptr;
   const void* pend_bgr = nullptr; const void* pend_depth = nullptr; int pend_W = 0, pend_H = 0; float pend_threshold = 0.f; const void* pend_masks[FL_MAX_MODALITIES] = {}; std::vector<int32_t> pend_filter;
   fl_dev_buf<unsigned long long> d_fe_trace; int fe_trace_jobs = 0, fe_trace_kind[FL_FE_MAX_JOBS] = {}, fe_trace_ctas[FL_FE_MAX_JOBS] = {};
-  bool opt_fe_waves = false, opt_split_refine = false, opt_trace = false, opt_dep_test = false, opt_no_prune = false;   // fl_debug_option
+  bool opt_fe_waves = false, opt_split_refine = false, opt_trace = false, opt_dep_test = false, opt_no_prune = false, opt_rotate = false;   // fl_debug_option
   fl_mapped_buf<int> h_fe_err; int* d_fe_err_host = nullptr; bool fe_force_waves = false;   // in-grid dependency time-out: mapped host flag (+ its device alias); true = this handle launches one kernel per wave from now on
   fl_dev_buf<unsigned> d_fe_counters; unsigned fe_counter_base[FL_FE_MAX_JOBS] = {}; unsigned fe_row_base[FL_FE_MAX_JOBS] = {};   // in-grid dependency counters of the single-launch front end (+ 1 error word)
   // candidates / matches
@@ -167,6 +168,8 @@ extern "C" int fl_create(const fl_params_t* params, fl_handle** out) {
       FL_CUDA(cudaMemset(h->d_lm4.get(), 0, h->d_lm4.capacity()));
     }
   }
+  TRY(h->d_mass.alloc(FL_MASS_WORDS));
+  FL_CUDA(cudaMemset(h->d_mass.get(), 0, FL_MASS_WORDS * sizeof(uint32_t)));
   TRY(h->d_cand.alloc((size_t)p.max_candidates)); TRY(h->d_count.alloc(4));   // [0] candidate count, [1] CTA ticket counter of k_refine_sort
   FL_CUDA(cudaMemset(h->d_count.get(), 0, 4 * sizeof(int)));
   // [FL_FE_MAX_JOBS job counters][1 error word][FL_FE_MAX_JOBS x FL_FE_MAX_TILE_ROWS tile-row counters]
@@ -252,6 +255,7 @@ extern "C" int fl_debug_option(fl_handle* h, int option, int value) {
     case FL_OPT_FE_DEP_TIMEOUT_TEST: h->opt_dep_test = value != 0; return FL_OK;
     case FL_OPT_FE_FORCED_WAVES: return h->fe_force_waves ? 1 : 0;                      // query: has a dependency time-out switched this handle to wave launches?
     case FL_OPT_SIM_NO_PRUNE: h->opt_no_prune = value != 0; return FL_OK;
+    case FL_OPT_SIM_ROTATE: h->opt_rotate = value != 0; return FL_OK;
   }
   return FL_ERR_ARG;
 }
@@ -424,6 +428,11 @@ static int ensure_geometry(fl_handle* h, int W, int H) {
 static uint8_t* lm4_of(fl_handle* h, int l, int m) {
   return (l == h->p.n_levels - 1 && (h->geom[l].Wd & 1) == 0) ? h->d_lm4.get() + (((size_t)m * h->geom[l].mod_stride) >> 1) : nullptr;
 }
+// the response sums of (level, modality) that order the staged kernel's phases: only the coarsest level, and only when that kernel runs
+// (it clears them; nothing else would)
+static uint32_t* mass_of(fl_handle* h, int l, int m) {
+  return (l == h->p.n_levels - 1 && h->use_staged && h->n_templates > 0) ? h->d_mass.get() + 8 * m : nullptr;
+}
 static void fe_wave_init(fl_fe_wave* w) { memset(w, 0, sizeof *w); }   // an empty launch description (no jobs, no in-grid dependencies)
 
 // front end + matchClass on the handle's templates; candidates land in (cand, count)
@@ -553,7 +562,7 @@ static int run_match_stages(fl_handle* h, const uint8_t* d_bgr, const uint16_t* 
         for (int m = 0; m < p.n_modalities; ++m) {
           uint8_t* spread = nullptr;
           if (h->keep_spread) { TRY(h->d_spread[l][m].grow((size_t)(p.max_width >> l) * (p.max_height >> l))); spread = h->d_spread[l][m].get(); }
-          fl_fe_add_spread(&w, h->d_q[l][m].get(), h->geom[l], h->d_lm[l].get() + (size_t)m * h->geom[l].mod_stride, spread, lm4_of(h, l, m));
+          fl_fe_add_spread(&w, h->d_q[l][m].get(), h->geom[l], h->d_lm[l].get() + (size_t)m * h->geom[l].mod_stride, spread, lm4_of(h, l, m), mass_of(h, l, m));
           const bool is_color = p.modality_kind[m] == FL_MODALITY_COLOR_GRADIENT;
           consume(is_color ? slot_color[l][m] : slot_depth[m]);
           consume_rows(is_color ? slot_color[l][m] : slot_depth[m], is_color ? 0 : l);
@@ -603,7 +612,7 @@ static int run_match_stages(fl_handle* h, const uint8_t* d_bgr, const uint16_t* 
           uint8_t* spread = nullptr;
           if (h->keep_spread) { TRY(h->d_spread[l - 1][m].grow((size_t)(p.max_width >> (l - 1)) * (p.max_height >> (l - 1)))); spread = h->d_spread[l - 1][m].get(); }
           wave_room();
-          fl_fe_add_spread(&w, h->d_q[l - 1][m].get(), g, h->d_lm[l - 1].get() + (size_t)m * g.mod_stride, spread, lm4_of(h, l - 1, m));
+          fl_fe_add_spread(&w, h->d_q[l - 1][m].get(), g, h->d_lm[l - 1].get() + (size_t)m * g.mod_stride, spread, lm4_of(h, l - 1, m), mass_of(h, l - 1, m));
         }
       }
       if (l < L) {
@@ -648,7 +657,7 @@ static int run_match_stages(fl_handle* h, const uint8_t* d_bgr, const uint16_t* 
         }
         uint8_t* spread = nullptr;
         if (h->keep_spread) { TRY(h->d_spread[l][m].grow((size_t)(p.max_width >> l) * (p.max_height >> l))); spread = h->d_spread[l][m].get(); }
-        fl_launch_spread_lm(qsrc, g, h->d_lm[l].get() + (size_t)m * g.mod_stride, spread, lm4_of(h, l, m), s); ++h->launches;
+        fl_launch_spread_lm(qsrc, g, h->d_lm[l].get() + (size_t)m * g.mod_stride, spread, lm4_of(h, l, m), mass_of(h, l, m), s); ++h->launches;
       }
       color_pyr_done = false;
     }
@@ -660,6 +669,8 @@ static int run_match_stages(fl_handle* h, const uint8_t* d_bgr, const uint16_t* 
     const int lowest = p.n_levels - 1;
     if (h->use_staged) {
       h->plan.prune = h->opt_no_prune ? 0 : 1;
+      h->plan.rotate = h->opt_rotate ? 1 : 0;
+      h->plan.mass = h->d_mass.get();
       if (fl_launch_similarity_staged(db, h->geom[lowest], h->d_lm4.get(), threshold, cand, cap, d_count, h->plan, s) != 0) {
         fl_set_error("staged similarity kernel could not be configured"); return FL_ERR_CUDA;
       }
@@ -1220,6 +1231,15 @@ extern "C" int fl_debug_get(fl_handle* h, int what, int32_t a, int32_t b, int32_
     unsigned long long* o = static_cast<unsigned long long*>(host_out);
     for (int i = 0; i < h->fe_trace_jobs; ++i) { o[4 * i] = (unsigned long long)h->fe_trace_kind[i]; o[4 * i + 1] = (unsigned long long)h->fe_trace_ctas[i]; o[4 * i + 2] = raw[2 * i]; o[4 * i + 3] = raw[2 * i + 1]; }
     return h->fe_trace_jobs;
+  }
+  if (what == FL_DBG_STAGED_ORDER) {                                                           // the phase order of the last staged launch
+    if (!h->use_staged) return FL_ERR_STATE;
+    if (bytes < 32 * sizeof(uint32_t) + (size_t)h->plan.n_phases) return FL_ERR_CAPACITY;
+    uint32_t raw[FL_MASS_WORDS];
+    FL_CUDA(cudaMemcpy(raw, h->d_mass.get(), sizeof raw, cudaMemcpyDeviceToHost));
+    memcpy(host_out, raw + FL_MASS_USED, 32 * sizeof(uint32_t));
+    memcpy(static_cast<uint8_t*>(host_out) + 32 * sizeof(uint32_t), raw + FL_MASS_ORDER, (size_t)h->plan.n_phases);
+    return h->plan.n_phases;
   }
   if (what == FL_DBG_STAGED_TRACE) {
     if (!h->use_staged || !h->plan.trace) return FL_ERR_STATE;

@@ -61,7 +61,17 @@ int fl_launch_tables_init();   // uploads the two LUTs to __constant__ memory of
 void fl_launch_pyrdown_bgr(const uint8_t* src, int W, int H, uint8_t* dst, cudaStream_t s);
 void fl_launch_resize_nn_half(const uint8_t* src, int W, int H, uint8_t* dst, cudaStream_t s);
 void fl_launch_apply_mask(const uint8_t* q, const uint8_t* mask, int n, uint8_t* out, cudaStream_t s);
-void fl_launch_spread_lm(const uint8_t* q, fl_level_geom g, uint8_t* lm_mod, uint8_t* spread_or_null, uint8_t* lm4_mod_or_null, cudaStream_t s);
+// mass_or_null: the coarsest level's response sums of this modality (8 words, see FL_MASS_*), or NULL
+void fl_launch_spread_lm(const uint8_t* q, fl_level_geom g, uint8_t* lm_mod, uint8_t* spread_or_null, uint8_t* lm4_mod_or_null, uint32_t* mass_or_null,
+                         cudaStream_t s);
+// Per-handle response mass of the coarsest level, u32 words: the spread jobs of that level add the sum of every linear-memory
+// response of (modality m, label l) into word 8 m + l; k_similarity_staged orders its phases by these sums and its last CTA to
+// read them clears them again (ticket), so every frame starts from zero without a memset.  Behind them: what the last staged
+// launch used (the sums, and CTA 0's phase of every visit step as bytes), for fl_debug_get(FL_DBG_STAGED_ORDER).
+#define FL_MASS_TICKET 32
+#define FL_MASS_USED 64
+#define FL_MASS_ORDER 96
+#define FL_MASS_WORDS (FL_MASS_ORDER + 64)
 
 // one launch = several independent front-end jobs (see k_front_end_wave)
 enum { FL_JOB_PYRDOWN = 2, FL_JOB_RESIZE = 3, FL_JOB_SPREAD = 4, FL_JOB_COLOR2 = 5, FL_JOB_DEPTH2 = 6, FL_JOB_PREFETCH = 7 };
@@ -69,6 +79,7 @@ struct fl_fe_job {
   int kind, cta_begin, gx, W, H, p0, p1;
   float thr_sq;
   const uint8_t* src; uint8_t* dst; uint8_t* dst2; uint8_t* dst3;   // spread job: dst = linear memories, dst2 = spread image (or NULL), dst3 = 4-bit linear memories (or NULL)
+  uint32_t* mass;                                                     // spread job: response sums of the modality's 8 labels (or NULL), see FL_MASS_*
   fl_level_geom g;
   // in-grid dependencies (single-launch front end): a CTA of this job first waits until counters[wait_slot] has reached
   // wait_target (all CTAs of the producing job have finished), and bumps counters[signal_slot] when it is done; -1 = none
@@ -97,7 +108,8 @@ void fl_fe_add_pyrdown(fl_fe_wave* w, const uint8_t* src, int W, int H, uint8_t*
 // in the shadow of the front end so that its prologue does not start with DRAM round trips
 void fl_fe_add_prefetch(fl_fe_wave* w, const void* src, size_t bytes);
 void fl_fe_add_resize(fl_fe_wave* w, const uint8_t* src, int W, int H, uint8_t* dst);
-void fl_fe_add_spread(fl_fe_wave* w, const uint8_t* q, fl_level_geom g, uint8_t* lm_mod, uint8_t* spread_or_null, uint8_t* lm4_mod_or_null);
+void fl_fe_add_spread(fl_fe_wave* w, const uint8_t* q, fl_level_geom g, uint8_t* lm_mod, uint8_t* spread_or_null, uint8_t* lm4_mod_or_null,
+                      uint32_t* mass_or_null);
 cudaError_t fl_launch_fe_wave(const fl_fe_wave& w, cudaStream_t s);
 
 // ---- template training, per-pixel half (train.cu) -----------------------------------------------
@@ -137,6 +149,8 @@ struct fl_staged_plan {
   int smem_bytes, pre_stride;              // dynamic shared memory; bytes per gpre row
   int stage_off;                           // emission staging area (one similarity map, nw_template x 32 words)
   int prune;                               // 1: drop a template once no position can reach the threshold (off: FL_OPT_SIM_NO_PRUNE)
+  int rotate;                              // 1: visit the phases in the rotated order of CTA b (FL_OPT_SIM_ROTATE) instead of by response mass
+  uint32_t* mass;                          // the handle's response mass (FL_MASS_WORDS words, see FL_MASS_*)
   uint32_t* gfeat;                         // [n_templates][64] feature words sorted by phase: word offset in the phase buffer << 5 | 8 * byte misalignment
   uint8_t* gpre;                           // [n_templates][pre_stride] prefix counts per phase
   int4* gmeta;                             // [n_templates] {template_positions, n_features, class, 0}

@@ -214,8 +214,11 @@ __device__ __forceinline__ uint32_t or_window(const uint32_t* __restrict__ w, in
 }
 
 template <int TT>
+// mass (nullable, the coarsest level only): += this CTA's sum of every (row, cell) response of label lab into mass[lab], one atomic per label
+// per CTA - the per-frame weights by which the staged similarity kernel orders its phases (k_similarity_staged)
 __device__ __forceinline__ void dev_spread_lm(const uint8_t* __restrict__ q, const fl_level_geom& g, uint8_t* __restrict__ lm,
-                                              uint8_t* __restrict__ spread_out, uint8_t* __restrict__ lm4, int bx, int by, uint8_t* smem, int cw) {
+                                              uint8_t* __restrict__ spread_out, uint8_t* __restrict__ lm4, uint32_t* __restrict__ mass,
+                                              int bx, int by, uint8_t* smem, int cw) {
   const int T = TT > 0 ? TT : g.T;
   const int W = g.W, H = g.H, Wd = g.Wd;
   const int gy = by, cx0 = bx * cw;                     // cw <= SL_CW cells per CTA (fewer on small levels: more CTAs in flight)
@@ -230,7 +233,9 @@ __device__ __forceinline__ void dev_spread_lm(const uint8_t* __restrict__ q, con
   uint2* s_resp = reinterpret_cast<uint2*>(smem);        // 256 x 8 B
   uint8_t* s_in = smem + 2048;                          // [th][st_in]   input labels (later reused for the final spread)
   uint8_t* s_hor = s_in + (size_t)(2 * T - 1) * spread_stride_in(T);   // [th][st_pw] horizontal OR
+  __shared__ uint32_t s_mass[8];
   for (int i = tid; i < 256; i += SL_THREADS) s_resp[i] = g_resp8[i];
+  if (tid < 8) s_mass[tid] = 0;
   if (((reinterpret_cast<uintptr_t>(q) | (uintptr_t)W | (uintptr_t)px0) & 3) == 0) {
     // word-aligned tile: whole 32-bit words, every load of the tile in flight at once (fixed trip count, unrolled).  A word is
     // either entirely inside the image or entirely outside (W % 4 == 0); bytes past the CTA's own window are real pixels of
@@ -286,6 +291,9 @@ __device__ __forceinline__ void dev_spread_lm(const uint8_t* __restrict__ q, con
   const int items = T * T * ngrp;
   const size_t cells = (size_t)g.cells;
   const uint32_t inv_ngrp = (65536u + ngrp - 1) / ngrp, inv_T = (65536u + T - 1) / T;   // exact for the small ranges used here
+  // response sums of labels {0, 2}, {1, 3}, {4, 6}, {5, 7}, two per word in 16-bit halves (a thread adds at most 16 per item, a warp
+  // at most 32 x 16 x ceil(T^2 SL_CW / 4 / SL_THREADS) <= 8,192 per half for T <= 16)
+  uint32_t m02 = 0, m13 = 0, m46 = 0, m57 = 0;
   for (int i = tid; i < items; i += SL_THREADS) {
     const int rr = (int)(((uint32_t)i * inv_ngrp) >> 16), c4 = i - rr * ngrp;
     const int ry = (int)(((uint32_t)rr * inv_T) >> 16), rx = rr - ry * T;
@@ -295,6 +303,7 @@ __device__ __forceinline__ void dev_spread_lm(const uint8_t* __restrict__ q, con
       const int c = c4 * 4 + k;
       const uint2 r8 = c < ncell ? s_resp[s_sp[ry * st_pw + c * T + rx]] : make_uint2(0, 0);
       lo[k] = r8.x; hi[k] = r8.y;
+      m02 += r8.x & 0x00FF00FFu; m13 += (r8.x >> 8) & 0x00FF00FFu; m46 += r8.y & 0x00FF00FFu; m57 += (r8.y >> 8) & 0x00FF00FFu;
     }
     const size_t off = (size_t)rr * cells + (size_t)gy * Wd + cx0 + c4 * 4;
     const int nvalid = min(4, ncell - c4 * 4);
@@ -320,27 +329,39 @@ __device__ __forceinline__ void dev_spread_lm(const uint8_t* __restrict__ q, con
       }
     }
   }
+  if (mass) {                                           // (uniform over the CTA)
+    m02 = __reduce_add_sync(0xffffffffu, m02); m13 = __reduce_add_sync(0xffffffffu, m13);
+    m46 = __reduce_add_sync(0xffffffffu, m46); m57 = __reduce_add_sync(0xffffffffu, m57);
+    if (lane == 0 && (m02 | m13 | m46 | m57)) {
+      atomicAdd(&s_mass[0], m02 & 0xFFFFu); atomicAdd(&s_mass[2], m02 >> 16); atomicAdd(&s_mass[1], m13 & 0xFFFFu); atomicAdd(&s_mass[3], m13 >> 16);
+      atomicAdd(&s_mass[4], m46 & 0xFFFFu); atomicAdd(&s_mass[6], m46 >> 16); atomicAdd(&s_mass[5], m57 & 0xFFFFu); atomicAdd(&s_mass[7], m57 >> 16);
+    }
+    __syncthreads();
+    if (tid < 8 && s_mass[tid]) atomicAdd(mass + tid, s_mass[tid]);
+  }
 }
 
 __device__ __forceinline__ void dev_spread_lm_any(const uint8_t* __restrict__ q, const fl_level_geom& g, uint8_t* __restrict__ lm,
-                                                  uint8_t* __restrict__ spread_out, uint8_t* __restrict__ lm4, int bx, int by, uint8_t* smem, int cw) {
+                                                  uint8_t* __restrict__ spread_out, uint8_t* __restrict__ lm4, uint32_t* __restrict__ mass,
+                                                  int bx, int by, uint8_t* smem, int cw) {
   switch (g.T) {
-    case 5: dev_spread_lm<5>(q, g, lm, spread_out, lm4, bx, by, smem, cw); break;
-    case 8: dev_spread_lm<8>(q, g, lm, spread_out, lm4, bx, by, smem, cw); break;
-    case 4: dev_spread_lm<4>(q, g, lm, spread_out, lm4, bx, by, smem, cw); break;
-    default: dev_spread_lm<0>(q, g, lm, spread_out, lm4, bx, by, smem, cw); break;
+    case 5: dev_spread_lm<5>(q, g, lm, spread_out, lm4, mass, bx, by, smem, cw); break;
+    case 8: dev_spread_lm<8>(q, g, lm, spread_out, lm4, mass, bx, by, smem, cw); break;
+    case 4: dev_spread_lm<4>(q, g, lm, spread_out, lm4, mass, bx, by, smem, cw); break;
+    default: dev_spread_lm<0>(q, g, lm, spread_out, lm4, mass, bx, by, smem, cw); break;
   }
 }
 
 __global__ void __launch_bounds__(SL_THREADS) k_spread_lm(const uint8_t* __restrict__ q, fl_level_geom g, uint8_t* __restrict__ lm,
-                                                          uint8_t* __restrict__ spread_out, uint8_t* __restrict__ lm4) {
+                                                          uint8_t* __restrict__ spread_out, uint8_t* __restrict__ lm4, uint32_t* __restrict__ mass) {
   extern __shared__ __align__(16) uint8_t smem_dyn[];
-  dev_spread_lm_any(q, g, lm, spread_out, lm4, blockIdx.x, blockIdx.y, smem_dyn, SL_CW);
+  dev_spread_lm_any(q, g, lm, spread_out, lm4, mass, blockIdx.x, blockIdx.y, smem_dyn, SL_CW);
 }
 
-void fl_launch_spread_lm(const uint8_t* q, fl_level_geom g, uint8_t* lm_mod, uint8_t* spread_or_null, uint8_t* lm4_mod_or_null, cudaStream_t s) {
+void fl_launch_spread_lm(const uint8_t* q, fl_level_geom g, uint8_t* lm_mod, uint8_t* spread_or_null, uint8_t* lm4_mod_or_null, uint32_t* mass_or_null,
+                         cudaStream_t s) {
   dim3 grid((g.Wd + SL_CW - 1) / SL_CW, g.Hd);
-  k_spread_lm<<<grid, SL_THREADS, spread_smem_bytes(g.T), s>>>(q, g, lm_mod, spread_or_null, lm4_mod_or_null);
+  k_spread_lm<<<grid, SL_THREADS, spread_smem_bytes(g.T), s>>>(q, g, lm_mod, spread_or_null, lm4_mod_or_null, mass_or_null);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -423,7 +444,7 @@ __global__ void __launch_bounds__(256, 8) k_front_end_wave(fl_fe_wave w) {
   switch (jb.kind) {
     case FL_JOB_PYRDOWN: dev_pyrdown_bgr(jb.src, jb.W, jb.H, jb.dst, local, jb.p0 != 0); break;
     case FL_JOB_RESIZE: dev_resize_nn_half(jb.src, jb.W, jb.H, jb.dst, local); break;
-    case FL_JOB_SPREAD: dev_spread_lm_any(jb.src, jb.g, jb.dst, jb.dst2, jb.dst3, local % jb.gx, local / jb.gx, smem_dyn, jb.p0); break;
+    case FL_JOB_SPREAD: dev_spread_lm_any(jb.src, jb.g, jb.dst, jb.dst2, jb.dst3, jb.mass, local % jb.gx, local / jb.gx, smem_dyn, jb.p0); break;
     case FL_JOB_PREFETCH: {
       const size_t line = (size_t)local * 256 + threadIdx.x;
       if (line * 128 < (size_t)jb.W * 128) asm volatile("prefetch.global.L2 [%0];" ::"l"(jb.src + line * 128));
@@ -490,10 +511,11 @@ void fl_fe_add_resize(fl_fe_wave* w, const uint8_t* src, int W, int H, uint8_t* 
   j.kind = FL_JOB_RESIZE; j.src = src; j.dst = dst; j.dst2 = nullptr; j.W = W; j.H = H; j.gx = 1;
   j.cta_begin = w->n_ctas; w->n_ctas += ((W / 2) * (H / 2) + 255) / 256;
 }
-void fl_fe_add_spread(fl_fe_wave* w, const uint8_t* q, fl_level_geom g, uint8_t* lm_mod, uint8_t* spread_or_null, uint8_t* lm4_mod_or_null) {
+void fl_fe_add_spread(fl_fe_wave* w, const uint8_t* q, fl_level_geom g, uint8_t* lm_mod, uint8_t* spread_or_null, uint8_t* lm4_mod_or_null,
+                      uint32_t* mass_or_null) {
   fl_fe_job& j = w->job[w->n_jobs++];
   j.wait_slot = -1; j.signal_slot = -1; j.wait_target = 0; j.row_base = -1; j.wait_row_base = -1; j.wait_row_shift = 0; j.wait_row_count = 0; j.wait_row_target = 0;
-  j.kind = FL_JOB_SPREAD; j.src = q; j.dst = lm_mod; j.dst2 = spread_or_null; j.dst3 = lm4_mod_or_null; j.g = g; j.W = g.W; j.H = g.H;
+  j.kind = FL_JOB_SPREAD; j.src = q; j.dst = lm_mod; j.dst2 = spread_or_null; j.dst3 = lm4_mod_or_null; j.mass = mass_or_null; j.g = g; j.W = g.W; j.H = g.H;
   int cw = SL_CW;                                       // small levels: narrower CTAs so that the job still fills the SMs
   while (cw > 8 && ((g.Wd + cw - 1) / cw) * g.Hd < 148) cw >>= 1;
   j.p0 = cw;

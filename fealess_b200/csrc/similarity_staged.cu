@@ -189,6 +189,49 @@ __device__ __forceinline__ bool any_byte_at_least(const uint32_t (&lo)[NW], cons
   return (int)max((m >> 8) & 0xFFu, m >> 24) >= t;
 }
 
+// Phase order of one CTA, computed by the producer warp after griddepcontrol.wait (the response sums are written by the front end):
+// s_phase[q] = the phase visited at step q.  With the early exit, a phase whose responses are low adds little to the partial sums
+// and much headroom against the bound (4 per feature it retires), so the lightest phases go first: a group of labels (one phase per
+// row block) weighs the sum of its labels' responses over the frame, groups are sorted by weight, ties by index so that every CTA
+// agrees, and the row blocks of a group keep their order.  Without the exit (NW = 15, FL_OPT_SIM_NO_PRUNE) or with
+// FL_OPT_SIM_ROTATE, CTA b starts at phase 7 b mod n_phases, so that different SMs pull different rows out of L2.  Only the load
+// of the sums stands between griddepcontrol.wait and the first phase copy; the ticket that clears them is taken after the last
+// copy has been issued (release_mass).
+__device__ __forceinline__ void phase_order(const fl_staged_plan& plan, bool by_mass, int lane, uint8_t* s_phase) {
+  const int n_phases = plan.n_phases, nrb = plan.n_rowblocks, lpp = plan.labels_per_phase;
+  const int n_groups = n_phases / nrb;                        // (modality, label) groups: M x 8 / lpp <= 32
+  const uint32_t mv = __ldcg(plan.mass + lane);               // the sums of all FL_MAX_MODALITIES x 8 labels, one per lane
+  uint32_t w = 0;
+  for (int l = 0; l < lpp; ++l) w += __shfl_sync(0xffffffffu, mv, (lane * lpp + l) & 31);
+  int rank = 0;
+  for (int j = 0; j < n_groups; ++j) {
+    const uint32_t wj = __shfl_sync(0xffffffffu, w, j);
+    rank += wj < w || (wj == w && j < lane);
+  }
+  if (by_mass) {
+    if (lane < n_groups)
+      for (int rb = 0; rb < nrb; ++rb) s_phase[rank * nrb + rb] = (uint8_t)(lane * nrb + rb);
+  } else {
+    const int rot = (int)((blockIdx.x * 7u) % (unsigned)n_phases);
+    for (int q = lane; q < n_phases; q += 32) s_phase[q] = (uint8_t)(q + rot < n_phases ? q + rot : q + rot - n_phases);
+  }
+  __syncwarp();
+  if (blockIdx.x == 0) {                                      // for fl_debug_get(FL_DBG_STAGED_ORDER) (stores: nothing waits for them)
+    plan.mass[FL_MASS_USED + lane] = mv;
+    for (int q = lane; q < n_phases; q += 32) reinterpret_cast<uint8_t*>(plan.mass + FL_MASS_ORDER)[q] = s_phase[q];
+  }
+}
+
+// One thread per CTA, once the CTA's sums have been read (phase_order) and its phases issued: the last CTA to get here clears the
+// sums (ticket), so that the next frame's spread jobs start from zero without a memset.  The next front end runs after this kernel.
+__device__ __forceinline__ void release_mass(const fl_staged_plan& plan) {
+  __threadfence();                                            // (the reads of the sums are complete: their values were used)
+  if (atomicAdd(plan.mass + FL_MASS_TICKET, 1u) == gridDim.x - 1) {
+    for (int i = 0; i < FL_MASS_TICKET; ++i) plan.mass[i] = 0;
+    plan.mass[FL_MASS_TICKET] = 0;
+  }
+}
+
 // (Refining the candidates in this kernel's own tail was measured much slower than the separate launch - stage 143 us vs 43 + 11 us:
 // candidates cluster in the few CTAs that own a matching template while the other 140 CTAs idle - and was removed.)
 template <int NW, int TPW>
@@ -200,6 +243,7 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
   __shared__ int s_live;                                      // template slots of this CTA that may still produce a candidate (early exit)
   __shared__ int s_stop;                                      // set by the producer when it issues no more phases (see the producer)
   __shared__ __align__(8) uint64_t s_aux;                     // completion of the bulk copy of this CTA's feature lists
+  __shared__ uint8_t s_phase[SS_MAX_PHASES];                  // the phase visited at each step (phase_order), written before phase 0 is issued
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int n_cwarps = (blockDim.x >> 5) - 1;                 // consumer warps; the last warp is the TMA producer
   // early exit (see any_byte_at_least); NW = 15 has no registers left for its test (ptxas spills), so it accumulates every template
@@ -211,9 +255,6 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
   int4* s_meta = reinterpret_cast<int4*>(s_dyn + (size_t)n_buf * plan.buf_bytes);
   uint32_t* s_feat = reinterpret_cast<uint32_t*>(s_meta + plan.tpc);
   uint8_t* s_pre = reinterpret_cast<uint8_t*>(s_feat + plan.tpc * SS_MAXF + 4);
-  // CTAs walk the phases in rotated order so that, at any moment, different SMs pull different linear-memory rows
-  // out of L2 instead of all hammering the same lines (the sums are order independent)
-  const int rot = (int)((blockIdx.x * 7u) % (unsigned)n_phases);
   unsigned long long* trace = plan.trace ? plan.trace + (size_t)blockIdx.x * 8 : nullptr;
   if (trace && tid == 0) { trace[0] = globaltimer(); unsigned smid; asm volatile("mov.u32 %0, %%smid;" : "=r"(smid)); trace[5] = smid; }
 
@@ -268,13 +309,14 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
 
   if (warp == n_cwarps) {
     // ===== producer: one elected lane streams phase q into buffer q % n_buf as soon as every consumer warp of the cluster released it =====
+    if (lane == 0 && t_end > t_begin) {                       // static data: may be fetched before the previous kernel has finished
+      const uint32_t fbytes = (uint32_t)(t_end - t_begin) * SS_MAXF * 4u;
+      mbar_expect_tx(&s_aux, fbytes);
+      bulk_g2s(s_feat, plan.gfeat + (size_t)t_begin * SS_MAXF, fbytes, &s_aux);
+    }
+    fl_grid_dep_wait();                                       // the linear memories and response sums are written by the previous kernel of the stream
+    phase_order(plan, prune && !plan.rotate, lane, s_phase);   // (the consumers read s_phase after their wait on s_full[0])
     if (lane == 0) {
-      if (t_end > t_begin) {                                  // static data: may be fetched before the previous kernel has finished
-        const uint32_t fbytes = (uint32_t)(t_end - t_begin) * SS_MAXF * 4u;
-        mbar_expect_tx(&s_aux, fbytes);
-        bulk_g2s(s_feat, plan.gfeat + (size_t)t_begin * SS_MAXF, fbytes, &s_aux);
-      }
-      fl_grid_dep_wait();                                     // the linear memories are written by the previous kernel of the stream
       for (int q = 0; q < n_phases; ++q) {
         const int b = q % n_buf;
         if (q >= n_buf) mbar_wait(&s_empty[b], ((q / n_buf) - 1) & 1);
@@ -293,7 +335,7 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
           for (int r = max(q - n_buf + 1, 0); r < q; ++r) mbar_wait(&s_full[r % n_buf], (r / n_buf) & 1);
           break;
         }
-        int p = q + rot; if (p >= n_phases) p -= n_phases;
+        const int p = s_phase[q];
         const int grp = p / plan.n_rowblocks, rb = p - grp * plan.n_rowblocks;
         const int ml = grp * plan.labels_per_phase;             // first (modality, label) of the group; a group never straddles modalities
         const int m = ml >> 3, lab = ml & 7;
@@ -304,11 +346,13 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
         mbar_expect_tx(&s_full[b], bytes);                    // the whole phase lands here, whoever fetches it
         bulk_g2s(s_buf + (size_t)b * plan.buf_bytes, src, bytes, &s_full[b]);
       }
+      release_mass(plan);
       if (trace) trace[7] = globaltimer();
     }
   } else {
     // ===== consumers =====
     bool live[TPW];                                           // false: no positions, or dropped by the early exit (pre[s] is then NULL too)
+    int left[TPW];                                            // features of the slot in the phases not visited yet (early exit)
     const uint8_t* pre[TPW];
     const uint32_t* fl[TPW];
     uint32_t lo[TPW][NW], hi[TPW][NW];
@@ -322,10 +366,10 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
       pre[s] = s_pre + (in ? slot : 0) * plan.pre_stride;
       fl[s] = s_feat + (in ? slot : 0) * SS_MAXF;
       if (!in) pre[s] = nullptr;
+      left[s] = in ? pre[s][n_phases] : 0;
 #pragma unroll
       for (int i = 0; i < NW; ++i) { lo[s][i] = 0; hi[s][i] = 0; }
     }
-    int p = rot;
     uint32_t par = 0;
     // loop-carried shared-memory addresses, kept opaque so that the compiler carries them in registers instead of re-deriving them
     // from the kernel parameters every phase (measured: ~90 -> ~55 instructions of per-phase overhead per warp)
@@ -346,6 +390,7 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
           "CWAIT_DONE:\n"
           "}\n" ::"r"(full_a), "r"(par) : "memory");
       if (*(volatile int*)&s_stop) break;                     // the producer issued no phase q (early exit, see the producer)
+      const int p = s_phase[q];
       if (trace && tid == 0 && q == 0) trace[2] = globaltimer();
 #pragma unroll
       for (int s = 0; s < TPW; ++s) {
@@ -374,16 +419,14 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
       // early exit, after the release so that the producer never waits for it.  The bound only bites once raw_thr + 1 > 4 x
       // (features left); a slot without new features keeps its verdict.  A dropped slot does no more feature work and emits nothing;
       // its warp stays in step with the ring (wait on s_full, arrive on s_empty), which costs a wait and an arrive per phase.
-      // (The features left are re-read from the prefix counts - phases rot .. p are done - rather than kept in registers: the
-      // accumulators leave no room for them.)
       if (prune) {
 #pragma unroll
         for (int s = 0; s < TPW; ++s) {
           if (!pre[s]) continue;
           const int k1 = pre[s][p + 1];
           if (pre[s][p] == k1) continue;                      // warp-uniform
-          const int k_rot = pre[s][rot];
-          const int rem = p >= rot ? pre[s][n_phases] - k1 + k_rot : k_rot - k1;
+          left[s] -= k1 - pre[s][p];
+          const int rem = left[s];
           const int4 meta = s_meta[warp + s * n_cwarps];
           const int t = (meta.y >> 8) - 4 * rem;              // (meta.y >> 8) = raw_thr + 1
           if (t <= 0) continue;
@@ -395,7 +438,6 @@ __global__ void __launch_bounds__(1024, 1) k_similarity_staged(const __grid_cons
       }
       full_a += 8; empty_a += 8; lane_base += buf_bytes;
       if (full_a == ring_end) { full_a -= 8u * (uint32_t)n_buf; empty_a -= 8u * (uint32_t)n_buf; lane_base -= (size_t)n_buf * buf_bytes; par ^= 1; }
-      if (++p == n_phases) p = 0;
     }
     (void)lane_end;
 #pragma unroll

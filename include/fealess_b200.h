@@ -421,8 +421,11 @@ enum {
   FL_DBG_STAGED_TRACE = 4,  /* ()                        -> 8 u64 per CTA of the staged similarity kernel {t_start, t_ready, t_first_data,
                                t_loop_end, t_end (globaltimer ns), smid, 0, 0}; only after fl_debug_option(h, FL_OPT_TRACE, 1);
                                returns the number of CTAs */
-  FL_DBG_FE_TRACE = 6       /* ()                        -> 4 u64 per front-end job {kind, CTAs, first CTA start, last CTA end (globaltimer ns)};
+  FL_DBG_FE_TRACE = 6,      /* ()                        -> 4 u64 per front-end job {kind, CTAs, first CTA start, last CTA end (globaltimer ns)};
                                only after fl_debug_option(h, FL_OPT_TRACE, 1); returns the number of jobs */
+  FL_DBG_STAGED_ORDER = 7   /* ()                        -> the phase order of the last staged similarity launch: 32 u32 response sums of the
+                               coarsest level it ordered by (word 8 m + l = modality m, label l), then one u8 per visit step: the phase
+                               CTA 0 visited at that step; returns the number of phases */
 };
 /* developer options of one handle; every one is off by default and covered by a test */
 enum {
@@ -431,8 +434,10 @@ enum {
   FL_OPT_TRACE = 2,               /* record the in-kernel timelines (FL_DBG_STAGED_TRACE, front-end job timeline); slows the frame down */
   FL_OPT_FE_DEP_TIMEOUT_TEST = 3, /* the next frame's first in-grid dependency can never be satisfied: exercises the time-out fallback (takes ~1 s) */
   FL_OPT_FE_FORCED_WAVES = 4,     /* query (value ignored): 1 if a dependency time-out has switched this handle to per-wave launches */
-  FL_OPT_SIM_NO_PRUNE = 5         /* the staged similarity kernel accumulates every template in full instead of dropping one once no
+  FL_OPT_SIM_NO_PRUNE = 5,        /* the staged similarity kernel accumulates every template in full instead of dropping one once no
                                      position can reach the threshold (same results; for A/B measurements and tests) */
+  FL_OPT_SIM_ROTATE = 6           /* the staged similarity kernel visits the phases in the order rotated by CTA instead of by the frame's
+                                     response mass (same results; for A/B measurements and tests) */
 };
 int fl_debug_option(fl_handle* h, int option, int value);
 int fl_debug_keep_spread(fl_handle* h, int enable);

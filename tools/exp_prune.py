@@ -1,13 +1,16 @@
-"""Developer experiment (GPU): the staged similarity kernel with and without its early exit, in one process on the same handles.
+"""Developer experiment (GPU): the staged similarity kernel with and without its early exit (--ab prune), or with its phases in
+the order of the frame's response mass and in the rotated order of FL_OPT_SIM_ROTATE (--ab order), in one process on the same handles.
 
 bench.py's C2 inputs (640x480, 8,000 templates, seed 1, 1 % planted, threshold 75).  The option FL_OPT_SIM_NO_PRUNE is switched
+(or FL_OPT_SIM_ROTATE) is switched
 off and on in alternation, ROUNDS times, and each time the script measures
   * the similarity stage (the library's own CUDA events, h.profile) over one frame at a time;
   * the stream: microseconds per frame at 4 frames in flight (fealess_b200.sharded.ShardedPipe, as bench.py drives it), inputs
     cycled over 160 device copies (> L2);
   * the in-kernel timeline (FL_OPT_TRACE, a handle of its own): per CTA the end of the phase loop and of the kernel, in us after
     the first CTA started (as tools/exp_warps.py reads it).
-The match list must not depend on the option; the script checks that too.  Usage: python tools/exp_prune.py [--rounds 5] [--json F]"""
+The match list must not depend on the option; the script checks that too.
+Usage: python tools/exp_prune.py [--ab prune|order] [--rounds 5] [--json F]"""
 import argparse
 import ctypes as C
 import json
@@ -41,6 +44,8 @@ def main():
     ap.add_argument("--rounds", type=int, default=5)
     ap.add_argument("--frames", type=int, default=400, help="frames per stream measurement")
     ap.add_argument("--json", help="write the per-round figures here")
+    ap.add_argument("--ab", choices=("prune", "order"), default="prune",
+                    help="prune: FL_OPT_SIM_NO_PRUNE off / on; order: FL_OPT_SIM_ROTATE off (by response mass) / on (rotated)")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("exp_prune.py needs a GPU")
@@ -61,10 +66,13 @@ def main():
     torch.cuda.synchronize()
     seq = [0]
 
+    opt = fb.FL_OPT_SIM_NO_PRUNE if args.ab == "prune" else fb.FL_OPT_SIM_ROTATE
+    names = ("early exit", "FL_OPT_SIM_NO_PRUNE") if args.ab == "prune" else ("by response mass", "FL_OPT_SIM_ROTATE")
+
     def set_opt(v):
         for s in pipe.slots:
-            assert s.h.debug_option(fb.FL_OPT_SIM_NO_PRUNE, v) == 0
-        assert htr.debug_option(fb.FL_OPT_SIM_NO_PRUNE, v) == 0
+            assert s.h.debug_option(opt, v) == 0
+        assert htr.debug_option(opt, v) == 0
 
     def stream(n):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -114,7 +122,7 @@ def main():
         set_opt(v)
         lists[v] = [h0.match(*frames[i], THR)[1] for i in range(8)]
     same = all(np.array_equal(a, b) for a, b in zip(lists[0], lists[1]))
-    print("match lists of the 8 frames identical with and without the early exit:", same)
+    print("match lists of the 8 frames identical with %s and with %s:" % names, same)
 
     set_opt(0)
     stream(200)
@@ -123,13 +131,13 @@ def main():
     for r in range(args.rounds):
         for v in ((0, 1) if r % 2 == 0 else (1, 0)):
             set_opt(v)
-            row = {"round": r, "early_exit": v == 0, "stage_similarity_us": stage(), "stream_us_per_frame": stream(args.frames)}
+            row = {"round": r, "option": names[v], "early_exit": v == 0, "stage_similarity_us": stage(), "stream_us_per_frame": stream(args.frames)}
             row["cta_loop_end_us_mean"], row["cta_loop_end_us_max"], row["cta_end_us_mean"], row["cta_end_us_max"] = timeline()
             rows.append(row)
             print(json.dumps(row))
             sys.stdout.flush()
     set_opt(0)
-    for v, name in ((0, "early exit"), (1, "FL_OPT_SIM_NO_PRUNE")):
+    for v, name in enumerate(names):
         sel = [x for x in rows if x["early_exit"] == (v == 0)]
         print("%-20s median: stage %.1f us, stream %.2f us/frame, CTA loop end mean %.1f / max %.1f us, CTA end max %.1f us" % (
             name, *(float(np.median([x[k] for x in sel])) for k in ("stage_similarity_us", "stream_us_per_frame", "cta_loop_end_us_mean",

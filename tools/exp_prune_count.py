@@ -3,7 +3,9 @@
 The staged kernel drops a template slot after a phase when, at every position p it tests, partial(p) + 4 x (features left) <=
 raw_thr: no candidate is possible any more (a response is at most 4).  This script replays that rule with the C oracle's linear
 memories, on bench.py's frames and 8,000-template set (seed 1, 1 % planted on frame 0), in the kernel's phase order (templates
-per CTA, slot -> warp, rotation rot = 7 x CTA % phases).  The plan comes from fl_debug_plan_staged for the SM count of GPU 0 when
+per CTA, slot -> warp).  Two phase orders (--order, count_frame's visit): "rotation" (CTA b starts at phase 7 b mod phases, what the kernel does without the early
+exit or with FL_OPT_SIM_ROTATE) and "mass" (the kernel's default: label groups by ascending response sum of the frame, ties by index,
+the same in every CTA; see phase_order).  The plan comes from fl_debug_plan_staged for the SM count of GPU 0 when
 a GPU is present, else it is the C2 plan on a 148-SM B200 stated below.
 
 Columns per frame: the share of (template, feature) pairs skipped; templates alive before the first phase and after each phase;
@@ -11,7 +13,7 @@ features of the busiest warp of a CTA (mean over CTAs) without and with the exit
   tp     positions [0, template_positions) - the cells a candidate can come from;
   words  [0, 8 ceil(template_positions / 8)) - what the kernel tests (whole 32-bit accumulator words);
   grid   every cell of the grid - a test without any mask (cells past template_positions hold sums of real data).
-Usage: python tools/exp_prune_count.py [--frames 8] [--threshold 75]"""
+Usage: python tools/exp_prune_count.py [--frames 8] [--threshold 75] [--order rotation|mass]"""
 import argparse
 import os
 import sys
@@ -71,9 +73,27 @@ class Templates:
             self.items.append((np.array(ph, np.int64), np.array(base, np.int64), nf, tp))
 
 
-def count_frame(lm_flat, tmpl, plan, thr, mask):
+def label_mass(lm_flat, cells, n_modalities=2):
+    """The response sum of every (modality, label) of the coarsest level: what the front end's spread jobs add up on the device."""
+    n = T[-1] * T[-1] * cells
+    return np.array([int(lm_flat[i * n:(i + 1) * n].astype(np.int64).sum()) for i in range(8 * n_modalities)], np.int64)
+
+
+def phase_order(mass, plan):
+    """The kernel's visit order by response mass: order[q] = the phase visited at step q.  A group of labels_per_phase labels
+    weighs the sum of their masses; groups ascending by weight, ties by index; the row blocks of a group keep their order."""
+    nrb, lpp = plan["n_rowblocks"], plan["labels_per_phase"]
+    n_groups = plan["n_phases"] // nrb
+    w = np.array([int(mass[g * lpp:(g + 1) * lpp].sum()) for g in range(n_groups)], np.int64)
+    groups = np.argsort(w, kind="stable")
+    return np.array([g * nrb + rb for g in groups for rb in range(nrb)], np.int64)
+
+
+def count_frame(lm_flat, tmpl, plan, thr, mask, visit="rotation"):
     """lm_flat: the coarsest level's linear memories of all (modality, label, row) laid out flat, zero pad behind."""
     nph, tpc = plan["n_phases"], plan["tpc"]
+    if visit == "mass":
+        step_of = np.argsort(phase_order(label_mass(lm_flat, tmpl.cells), plan))   # step_of[phase] = visit step
     ncw = plan["block_threads"] // 32 - 1
     n_cta = (len(tmpl.items) + tpc - 1) // tpc
     alive = np.zeros(nph + 1, np.int64)
@@ -82,7 +102,7 @@ def count_frame(lm_flat, tmpl, plan, thr, mask):
     warp_pr = np.zeros((n_cta, ncw), np.int64)
     for t, (ph, base, nf, tp) in enumerate(tmpl.items):
         b, slot = divmod(t, tpc)
-        warp, rot = slot % ncw, (b * 7) % nph
+        warp = slot % ncw
         n = len(ph)
         total += n
         warp_full[b, warp] += n
@@ -91,7 +111,7 @@ def count_frame(lm_flat, tmpl, plan, thr, mask):
             alive[1:] += 1
             continue
         P = {"tp": tp, "words": min(8 * ((tp + 7) // 8), tmpl.cells), "grid": tmpl.cells}[mask]
-        key = (ph - rot) % nph                                  # the order in which this CTA visits the phases
+        key = (ph - (b * 7) % nph) % nph if visit == "rotation" else step_of[ph]   # the step at which this CTA visits each feature's phase
         order = np.argsort(key, kind="stable")
         A = lm_flat[base[order][:, None] + np.arange(P)[None, :]].astype(np.int32)
         cs = np.cumsum(A, axis=0)
@@ -132,7 +152,7 @@ def linear_memories(det, cells):
     return lm
 
 
-def run(n_frames=8, thr=75.0, masks=MASKS, out=sys.stdout):
+def run(n_frames=8, thr=75.0, masks=MASKS, out=sys.stdout, order="rotation"):
     frames, det, ts = setup()
     Tc = T[-1]
     Wd, Hd = (W >> 1) // Tc, (H >> 1) // Tc
@@ -140,14 +160,14 @@ def run(n_frames=8, thr=75.0, masks=MASKS, out=sys.stdout):
     max_pos = max(min((Hd - ((int(h) - 1) // Tc + 1)) * Wd + (Wd - ((int(w) - 1) // Tc + 1)) + 1, Wd * Hd) for w, h in hd[:, :2])
     plan, src = plan_for(max_pos)
     tmpl = Templates(ts, plan)
-    out.write("plan (%s): %d templates per CTA, %d consumer warps, %d phases of %d label(s); threshold %g\n" % (
-        src, plan["tpc"], plan["block_threads"] // 32 - 1, plan["n_phases"], plan["labels_per_phase"], thr))
+    out.write("plan (%s): %d templates per CTA, %d consumer warps, %d phases of %d label(s); threshold %g; phase order: %s\n" % (
+        src, plan["tpc"], plan["block_threads"] // 32 - 1, plan["n_phases"], plan["labels_per_phase"], thr, order))
     res = {}
     for fi in range(n_frames):
         det.process(*frames[fi])
         lm = linear_memories(det, tmpl.cells)
         for mask in masks:
-            r = count_frame(lm, tmpl, plan, thr, mask)
+            r = count_frame(lm, tmpl, plan, thr, mask, order)
             res[(fi, mask)] = r
             out.write("frame %d  %-5s  skipped %5.1f %%  (needed %d of %d)  alive %s  busiest warp %.1f -> %.1f\n" % (
                 fi, mask, 100 * r["skipped"], r["needed"], r["total"], " ".join(map(str, r["alive"])), r["busiest_warp_full"],
@@ -160,5 +180,6 @@ if __name__ == "__main__":
     ap = argparse.ArgumentParser()
     ap.add_argument("--frames", type=int, default=8)
     ap.add_argument("--threshold", type=float, default=75.0)
+    ap.add_argument("--order", choices=("rotation", "mass"), default="rotation")
     a = ap.parse_args()
-    run(a.frames, a.threshold)
+    run(a.frames, a.threshold, order=a.order)
