@@ -59,6 +59,7 @@ EXPORTED_SYMBOLS = [
     "fl_pipe_set_recognition", "fl_pipe_submit_recognition", "fl_pipe_collect_recognition",
     "fl_group_create_pipe", "fl_group_depth", "fl_group_in_flight", "fl_group_upload_model_depths", "fl_group_set_recognition",
     "fl_group_submit_recognition", "fl_group_collect_recognition", "fl_group_recognize",
+    "fl_pipe_submit_masked", "fl_group_match_masked", "fl_match_shard_exchange_masked_async", "fl_match_shard_exchange_device_masked_async",
 ]
 
 
@@ -145,6 +146,32 @@ def _check(rc: int, where: str, ok=(FL_OK,)):
     if rc not in ok:
         raise FealessError(rc, where, lib().fl_last_error().decode(errors="replace"))
     return rc
+
+
+def host_masks(masks, M: int, W: int, H: int):
+    """``masks=`` of the calls that take a frame in host memory: None / empty = unmasked, else M entries, each None or an H x W array
+    (nonzero = keep).  Returns (ctypes array of M pointers or None, the arrays it points into).  A count other than M or a mask of
+    another size raises FealessError(FL_ERR_SIZE) - the -1 of Detector::match (linemod.cpp:1374-1377)."""
+    if masks is None or len(masks) == 0:
+        return None, []
+    if len(masks) != M:
+        raise FealessError(FL_ERR_SIZE, "masks", "%d masks for %d modalities" % (len(masks), M))
+    keep = [None if m is None else np.ascontiguousarray(m, np.uint8) for m in masks]
+    for k in keep:
+        if k is not None and k.shape != (H, W):
+            raise FealessError(FL_ERR_SIZE, "masks", "a mask of shape %s for a %d x %d frame" % (k.shape, W, H))
+    return (C.c_void_p * M)(*[None if k is None else k.ctypes.data for k in keep]), keep
+
+
+def device_masks(masks, M: int):
+    """``masks=`` of the calls that take a frame in device memory: None / empty = unmasked, else M device pointers (0 / None = that
+    modality unmasked), each a dense W x H u8 image that stays valid until the frame has been waited for.  A count other than M raises
+    FealessError(FL_ERR_SIZE)."""
+    if masks is None or len(masks) == 0:
+        return None
+    if len(masks) != M:
+        raise FealessError(FL_ERR_SIZE, "masks", "%d masks for %d modalities" % (len(masks), M))
+    return (C.c_void_p * M)(*[int(p) if p else None for p in masks])
 
 
 STAGED_PLAN_FIELDS = ("nw_template", "tpw", "tpc", "n_cta", "block_threads", "phase_rows", "n_rowblocks", "labels_per_phase",
@@ -288,24 +315,25 @@ class Handle:
         res = out[:min(cnt.value, capacity)].copy()
         return (rc, res, dout) if want_depth else (rc, res)
 
-    def match_device(self, d_bgr: int, d_depth: int, W: int, H: int, threshold: float, class_filter=None) -> None:
-        """Frame already in device memory (raw device pointers, dense rows); results stay on the device."""
+    def match_device(self, d_bgr: int, d_depth: int, W: int, H: int, threshold: float, class_filter=None, masks=None) -> None:
+        """Frame already in device memory (raw device pointers, dense rows); results stay on the device.  ``masks``: see device_masks."""
         cf = None if not class_filter else np.ascontiguousarray(class_filter, np.int32)
-        _check(lib().fl_match_device(self._h, C.c_void_p(d_bgr), C.c_void_p(d_depth), W, H, None, C.c_float(threshold), _p(cf),
+        _check(lib().fl_match_device(self._h, C.c_void_p(d_bgr), C.c_void_p(d_depth), W, H, device_masks(masks, self.M), C.c_float(threshold), _p(cf),
                                      0 if cf is None else int(cf.size)), "fl_match_device")
 
-    def match_device_async(self, d_bgr: int, d_depth: int, W: int, H: int, threshold: float, class_filter=None) -> None:
+    def match_device_async(self, d_bgr: int, d_depth: int, W: int, H: int, threshold: float, class_filter=None, masks=None) -> None:
         """Enqueue-only half of ``match_device`` (finish with ``match_wait``): nothing but kernel launches on the handle's stream."""
         cf = None if not class_filter else np.ascontiguousarray(class_filter, np.int32)
-        _check(lib().fl_match_device_async(self._h, C.c_void_p(d_bgr), C.c_void_p(d_depth), W, H, None, C.c_float(threshold), _p(cf),
+        _check(lib().fl_match_device_async(self._h, C.c_void_p(d_bgr), C.c_void_p(d_depth), W, H, device_masks(masks, self.M), C.c_float(threshold), _p(cf),
                                            0 if cf is None else int(cf.size)), "fl_match_device_async")
 
-    def match_async(self, bgr, depth, threshold: float, class_filter=None) -> None:
+    def match_async(self, bgr, depth, threshold: float, class_filter=None, masks=None) -> None:
         """fl_match_async: enqueue-only half of ``match`` for a frame in host memory (dense numpy arrays; page-locked ones are read
-        by DMA and have to stay alive until ``match_wait``)."""
+        by DMA and have to stay alive until ``match_wait``; masks, see host_masks, are copied before this returns)."""
         H, W = (depth if depth is not None else bgr).shape[:2]
         cf = None if not class_filter else np.ascontiguousarray(class_filter, np.int32)
-        _check(lib().fl_match_async(self._h, _p(bgr), C.c_size_t(W * 3), _p(depth), C.c_size_t(W * 2), W, H, None, C.c_float(threshold), _p(cf),
+        marr, _keep = host_masks(masks, self.M, W, H)
+        _check(lib().fl_match_async(self._h, _p(bgr), C.c_size_t(W * 3), _p(depth), C.c_size_t(W * 2), W, H, marr, C.c_float(threshold), _p(cf),
                                     0 if cf is None else int(cf.size)), "fl_match_async")
 
     def add_template(self, bgr, depth, mask=None, num_features=None, strong_threshold: float = 55.0, extract_threshold: int = 2,
@@ -356,9 +384,9 @@ class Handle:
         return out[:min(cnt.value, capacity)].copy()
 
     def match_shard_device(self, d_bgr: int, d_depth: int, W: int, H: int, threshold: float, d_candidates: int, capacity: int,
-                           d_count: int, class_filter=None) -> None:
+                           d_count: int, class_filter=None, masks=None) -> None:
         cf = None if not class_filter else np.ascontiguousarray(class_filter, np.int32)
-        _check(lib().fl_match_shard_device(self._h, C.c_void_p(d_bgr), C.c_void_p(d_depth), W, H, None, C.c_float(threshold), _p(cf),
+        _check(lib().fl_match_shard_device(self._h, C.c_void_p(d_bgr), C.c_void_p(d_depth), W, H, device_masks(masks, self.M), C.c_float(threshold), _p(cf),
                                            0 if cf is None else int(cf.size), C.c_void_p(d_candidates), capacity, C.c_void_p(d_count)),
                "fl_match_shard_device")
 
@@ -381,23 +409,27 @@ class Handle:
                "fl_exchange_sort_unique_device_async")
 
     def match_shard_exchange_device_async(self, d_bgr: int, d_depth: int, W: int, H: int, threshold: float, rank: int, world: int,
-                                          peer_buffers: Sequence[int], capacity: int, d_local_block: int, epoch: int, class_filter=None) -> None:
+                                          peer_buffers: Sequence[int], capacity: int, d_local_block: int, epoch: int, class_filter=None,
+                                          masks=None) -> None:
+        """fl_match_shard_exchange_device_masked_async (``masks``: device pointers, see device_masks; None = unmasked)."""
         cf = None if not class_filter else np.ascontiguousarray(class_filter, np.int32)
         arr = peer_buffers if isinstance(peer_buffers, C.Array) else (C.c_void_p * world)(*[int(p) for p in peer_buffers])
-        _check(lib().fl_match_shard_exchange_device_async(self._h, C.c_void_p(d_bgr), C.c_void_p(d_depth), W, H, C.c_float(threshold), _p(cf),
-                                                          0 if cf is None else int(cf.size), rank, world, arr, capacity, C.c_void_p(d_local_block),
-                                                          C.c_uint32(epoch)), "fl_match_shard_exchange_device_async")
+        _check(lib().fl_match_shard_exchange_device_masked_async(self._h, C.c_void_p(d_bgr), C.c_void_p(d_depth), W, H, device_masks(masks, self.M),
+                                                                 C.c_float(threshold), _p(cf), 0 if cf is None else int(cf.size), rank, world, arr,
+                                                                 capacity, C.c_void_p(d_local_block), C.c_uint32(epoch)),
+               "fl_match_shard_exchange_device_masked_async")
 
     def match_shard_exchange_async(self, bgr, depth, threshold: float, rank: int, world: int, peer_buffers: Sequence[int], capacity: int,
-                                   d_local_block: int, epoch: int, class_filter=None) -> None:
-        """fl_match_shard_exchange_async: the frame in HOST memory (numpy arrays, dense rows; page-locked ones are read by DMA and have
-        to stay alive until ``match_wait``)."""
+                                   d_local_block: int, epoch: int, class_filter=None, masks=None) -> None:
+        """fl_match_shard_exchange_masked_async: the frame in HOST memory (numpy arrays, dense rows; page-locked ones are read by DMA and
+        have to stay alive until ``match_wait``; masks, see host_masks, are copied before this returns)."""
         H, W = (depth if depth is not None else bgr).shape[:2]
         cf = None if not class_filter else np.ascontiguousarray(class_filter, np.int32)
+        marr, _keep = host_masks(masks, self.M, W, H)
         arr = peer_buffers if isinstance(peer_buffers, C.Array) else (C.c_void_p * world)(*[int(p) for p in peer_buffers])
-        _check(lib().fl_match_shard_exchange_async(self._h, _p(bgr), C.c_size_t(W * 3), _p(depth), C.c_size_t(W * 2), W, H, C.c_float(threshold), _p(cf),
-                                                   0 if cf is None else int(cf.size), rank, world, arr, capacity, C.c_void_p(d_local_block),
-                                                   C.c_uint32(epoch)), "fl_match_shard_exchange_async")
+        _check(lib().fl_match_shard_exchange_masked_async(self._h, _p(bgr), C.c_size_t(W * 3), _p(depth), C.c_size_t(W * 2), W, H, marr, C.c_float(threshold),
+                                                          _p(cf), 0 if cf is None else int(cf.size), rank, world, arr, capacity, C.c_void_p(d_local_block),
+                                                          C.c_uint32(epoch)), "fl_match_shard_exchange_masked_async")
 
     def sync(self):
         _check(lib().fl_sync(self._h), "fl_sync")
@@ -629,7 +661,7 @@ class Group:
         if rc != FL_OK:
             self._g = None
             raise FealessError(rc, "fl_group_create_pipe", L.fl_last_error().decode(errors="replace"))
-        self.n, self.depth = len(dv), int(depth)
+        self.n, self.depth, self.M = len(dv), int(depth), len(modality_kind)
         self._keep = {}                                          # frames in flight: the arrays the DMA reads stay referenced
         self._seq = 0
 
@@ -673,17 +705,22 @@ class Group:
         pose = np.ascontiguousarray(tset.pose13, np.float32)
         _check(lib().fl_group_upload_templates(self._g, tset.n_templates, _p(hdr), _p(ft), ft.shape[0], _p(co), _p(pose)), "fl_group_upload_templates")
 
-    def match(self, bgr, depth, threshold: float, class_filter=None, capacity: int = 1 << 16):
+    def match(self, bgr, depth, threshold: float, class_filter=None, capacity: int = 1 << 16, masks=None):
+        """fl_group_match_masked: (rc, merged list); ``masks`` as in ``Handle.match`` (a wrong count or size gives rc FL_ERR_SIZE)."""
         H, W = depth.shape[:2]
         b = np.ascontiguousarray(bgr, np.uint8)
         d = np.ascontiguousarray(depth, np.uint16)
         out = np.zeros(capacity, MATCH_DTYPE)
+        try:
+            marr, _keep = host_masks(masks, self.M, W, H)
+        except FealessError as e:
+            return e.rc, out[:0]
         cnt = C.c_int32(0)
         cf = None if not class_filter else np.ascontiguousarray(class_filter, np.int32)
-        rc = lib().fl_group_match(self._g, _p(b), C.c_size_t(W * 3), _p(d), C.c_size_t(W * 2), W, H, C.c_float(threshold), _p(cf),
-                                  0 if cf is None else int(cf.size), _p(out), capacity, C.byref(cnt))
+        rc = lib().fl_group_match_masked(self._g, _p(b), C.c_size_t(W * 3), _p(d), C.c_size_t(W * 2), W, H, marr, C.c_float(threshold), _p(cf),
+                                         0 if cf is None else int(cf.size), _p(out), capacity, C.byref(cnt))
         if rc not in (FL_OK, FL_ERR_CAPACITY):
-            _check(rc, "fl_group_match")
+            _check(rc, "fl_group_match_masked")
         return rc, out[:min(cnt.value, capacity)].copy()
 
     # ---- Recognition over the group ---------------------------------------------------------------
@@ -755,7 +792,7 @@ class Pipe:
         if rc != FL_OK:
             self._p = None
             raise FealessError(rc, "fl_pipe_create", L.fl_last_error().decode(errors="replace"))
-        self.depth = int(depth)
+        self.depth, self.M = int(depth), len(modality_kind)
         self._keep = {}                                          # frames in flight: the arrays the DMA reads stay referenced
         self._seq = 0
         self._out = {}
@@ -803,21 +840,25 @@ class Pipe:
         L.fl_launch_count.restype = C.c_int64
         return sum(int(L.fl_launch_count(C.c_void_p(L.fl_pipe_handle(self._p, i)))) for i in range(self.depth))
 
-    def submit(self, bgr, depth, threshold: float, class_filter=None) -> None:
-        """Host frame (numpy arrays; page-locked ones are read by DMA while in flight)."""
+    def submit(self, bgr, depth, threshold: float, class_filter=None, masks=None) -> None:
+        """Host frame (numpy arrays; page-locked ones are read by DMA while in flight).  ``masks``: see host_masks (copied before this
+        returns)."""
         H, W = (depth if depth is not None else bgr).shape[:2]
         b = None if bgr is None else np.ascontiguousarray(bgr, np.uint8)
         d = None if depth is None else np.ascontiguousarray(depth, np.uint16)
         cf = None if not class_filter else np.ascontiguousarray(class_filter, np.int32)
-        _check(lib().fl_pipe_submit(self._p, _p(b), C.c_size_t(W * 3), _p(d), C.c_size_t(W * 2), W, H, C.c_float(threshold), _p(cf),
-                                    0 if cf is None else int(cf.size), 0), "fl_pipe_submit")
+        marr, _keep = host_masks(masks, self.M, W, H)
+        _check(lib().fl_pipe_submit_masked(self._p, _p(b), C.c_size_t(W * 3), _p(d), C.c_size_t(W * 2), W, H, marr, C.c_float(threshold), _p(cf),
+                                           0 if cf is None else int(cf.size), 0), "fl_pipe_submit_masked")
         self._keep[self._seq % self.depth] = (b, d)
         self._seq += 1
 
-    def submit_device(self, d_bgr: int, d_depth: int, W: int, H: int, threshold: float, class_filter=None) -> None:
+    def submit_device(self, d_bgr: int, d_depth: int, W: int, H: int, threshold: float, class_filter=None, d_masks=None) -> None:
+        """Device frame (dense rows); ``d_masks``: see device_masks."""
         cf = None if not class_filter else np.ascontiguousarray(class_filter, np.int32)
-        _check(lib().fl_pipe_submit(self._p, C.c_void_p(d_bgr), C.c_size_t(W * 3), C.c_void_p(d_depth), C.c_size_t(W * 2), W, H, C.c_float(threshold), _p(cf),
-                                    0 if cf is None else int(cf.size), 1), "fl_pipe_submit")
+        _check(lib().fl_pipe_submit_masked(self._p, C.c_void_p(d_bgr), C.c_size_t(W * 3), C.c_void_p(d_depth), C.c_size_t(W * 2), W, H,
+                                           device_masks(d_masks, self.M), C.c_float(threshold), _p(cf), 0 if cf is None else int(cf.size), 1),
+               "fl_pipe_submit_masked")
         self._seq += 1
 
     def collect(self, capacity: int = 1 << 14, copy: bool = True):

@@ -56,13 +56,15 @@ struct fl_handle {
   // frame-sized buffers
   fl_dev_buf<uint8_t> d_in_bgr; fl_dev_buf<uint16_t> d_in_depth;   // staging for host-input calls
   fl_dev_buf<uint8_t> d_bgr[FL_MAX_LEVELS];                        // colour pyramid, levels >= 1
-  fl_dev_buf<uint8_t> d_q[FL_MAX_LEVELS][FL_MAX_MODALITIES];       // quantised images (unmasked)
-  fl_dev_buf<uint8_t> d_qm[FL_MAX_LEVELS][FL_MAX_MODALITIES];      // masked copies (allocated on first use)
+  fl_dev_buf<uint8_t> d_q[FL_MAX_LEVELS][FL_MAX_MODALITIES];       // quantised images (unmasked: a frame's masks apply in the spread jobs and at read-back)
+  // masks, sized at fl_create: level 0 = the staged masks of host-input frames, levels >= 1 = the NN mask pyramid of a geometry that
+  // does not halve exactly (run_match_stages)
   fl_dev_buf<uint8_t> d_mask[FL_MAX_LEVELS][FL_MAX_MODALITIES];
   fl_dev_buf<uint8_t> d_spread[FL_MAX_LEVELS][FL_MAX_MODALITIES];  // debug only
   fl_dev_buf<uint8_t> d_lm[FL_MAX_LEVELS]; fl_dev_buf<uint8_t> d_lm4;   // d_lm4: 4-bit copy of the coarsest level's linear memories
   fl_dev_buf<uint32_t> d_mass;                                         // response mass of the coarsest level (FL_MASS_*): the staged kernel's phase order
-  bool used_mask[FL_MAX_MODALITIES] = {}; bool keep_spread = false;
+  const uint8_t* frame_mask[FL_MAX_MODALITIES] = {};               // level-0 mask (device memory) of the last frame's modality m, or NULL
+  bool keep_spread = false;
   // state between the enqueue half (fl_match_device_async, ..._async) and fl_match_wait
   bool pend_sort = false, pend_match = false, pend_own = false, pend_masks_valid = false, pend_small_fused = false; fl_lists pend_lists = {}; fl_match_t* pend_out = nullptr; int pend_out_cap = 0; int* pend_out_count = nullptr;
   const void* pend_bgr = nullptr; const void* pend_depth = nullptr; int pend_W = 0, pend_H = 0; float pend_threshold = 0.f; const void* pend_masks[FL_MAX_MODALITIES] = {}; std::vector<int32_t> pend_filter;
@@ -156,7 +158,7 @@ extern "C" int fl_create(const fl_params_t* params, fl_handle** out) {
   for (int l = 0; l < p.n_levels; ++l) {
     size_t n = (size_t)(p.max_width >> l) * (p.max_height >> l);
     if (l > 0) TRY(h->d_bgr[l].alloc(n * 3));
-    for (int m = 0; m < p.n_modalities; ++m) TRY(h->d_q[l][m].alloc(n));
+    for (int m = 0; m < p.n_modalities; ++m) { TRY(h->d_q[l][m].alloc(n)); TRY(h->d_mask[l][m].alloc(n)); }
     // linear memories: T need not divide the maximum size, so bound the cell count from above
     int T = p.T[l];
     size_t cells = (size_t)(((p.max_width >> l) + T - 1) / T) * (((p.max_height >> l) + T - 1) / T);
@@ -433,7 +435,6 @@ static uint8_t* lm4_of(fl_handle* h, int l, int m) {
 static uint32_t* mass_of(fl_handle* h, int l, int m) {
   return (l == h->p.n_levels - 1 && h->use_staged && h->n_templates > 0) ? h->d_mass.get() + 8 * m : nullptr;
 }
-static void fe_wave_init(fl_fe_wave* w) { memset(w, 0, sizeof *w); }   // an empty launch description (no jobs, no in-grid dependencies)
 
 // front end + matchClass on the handle's templates; candidates land in (cand, count)
 // defer_refine: leave the candidates at the coarsest level; the caller refines them in the same launch that sorts (k_refine_sort)
@@ -465,205 +466,170 @@ static int run_match_stages(fl_handle* h, const uint8_t* d_bgr, const uint16_t* 
   }
   if (h->profile) cudaEventRecord(h->ev[0].get(), s);
   const float thr_sq = p.weak_threshold * p.weak_threshold;
-  bool any_mask = false;
-  for (int m = 0; m < p.n_modalities; ++m) { h->used_mask[m] = d_masks && d_masks[m]; any_mask |= h->used_mask[m]; }
+  // the frame's masks (level 0, device memory): applied where the spread jobs read the labels (dev_spread_lm), so a masked frame takes
+  // the same schedule and launches as an unmasked one
+  const uint8_t* mask0[FL_MAX_MODALITIES] = {};
+  for (int m = 0; m < p.n_modalities; ++m) { mask0[m] = d_masks ? static_cast<const uint8_t*>(d_masks[m]) : nullptr; h->frame_mask[m] = mask0[m]; }
   int first_color = -1;
   for (int m = 0; m < p.n_modalities; ++m) if (p.modality_kind[m] == FL_MODALITY_COLOR_GRADIENT && first_color < 0) first_color = m;
-  const bool zero_in_wave = !any_mask;                       // wave 0 resets the candidate counter: no memset node between the kernels
-  if (!any_mask) {
-    // wave schedule (frontend.cu): L + 1 launches for the whole front end; wave l produces the labels of level l and the
-    // linear memories of level l - 1.  Jobs are added longest first: the kernel ends with its slowest CTA, and CTAs are
-    // scheduled in job order.  (Measured alternative: slicing the level-0 colour quantisation over the waves and moving
-    // every spread to the last wave - 16.6 + 10.8 + 9.2 us instead of 17.7 + 9.4 + 6.0 us, i.e. no gain: each wave has a
-    // latency floor of one colour-tile CTA, about 8 us.)
-    const int L = p.n_levels;
-    fl_fe_wave w;
-    auto wave_begin = [&](bool zero) { w.n_jobs = 0; w.n_ctas = 0; w.smem = 0; w.n_pyr = 0; w.zero_me = zero ? d_count : nullptr; w.counters = nullptr; w.dep_error = nullptr; w.dep_error_host = nullptr; w.trace = nullptr; };
-    bool launch_ok = true;
-    auto wave_flush = [&]() { if (w.n_jobs > 0) { launch_ok &= fl_launch_fe_wave(w, s) == cudaSuccess; ++h->launches; } w.n_jobs = 0; w.n_ctas = 0; w.smem = 0; w.n_pyr = 0; w.zero_me = nullptr; };
-    // word-parallel quantisers (frontend_v2.cuh).  The depth job also writes the NN-downsampled label pyramid when every level
-    // halves exactly (then dst_l(y,x) = src(2^l y, 2^l x)).
-    bool depth_pyr_fused[FL_MAX_MODALITIES] = {false, false, false, false};
-    bool halves = true;
-    for (int l = 0; l + 1 < L; ++l) halves &= (h->geom[l].W % 2 == 0) && (h->geom[l].H % 2 == 0);
-    auto wave_room = [&]() { if (w.n_jobs == FL_FE_MAX_JOBS) wave_flush(); };     // jobs of one wave are independent: splitting is always safe
-    // ---- single-launch front end: every job of the frame in ONE grid, producers before consumers, dependencies resolved by
-    // per-job CTA counters inside the kernel (k_front_end_wave).  Removes L launches + their dependency gaps and lets the
-    // level-0 work fill the machine while the short critical chain pyrDown -> colour L(top) -> spread L(top) runs.
-    const bool fe_waves = h->opt_fe_waves;                                       // FL_OPT_FE_WAVES: one launch per wave (also the fallback after a dependency time-out)
-    int n_color = 0, n_depth = 0;
-    for (int m = 0; m < p.n_modalities; ++m) { n_color += p.modality_kind[m] == FL_MODALITY_COLOR_GRADIENT; n_depth += p.modality_kind[m] == FL_MODALITY_DEPTH_NORMAL; }
-    const int n_jobs_single = (n_color ? L - 1 : 0) + n_color * L + n_depth + p.n_modalities * L;
-    const bool single = !fe_waves && !h->fe_force_waves && n_jobs_single <= FL_FE_MAX_JOBS && n_depth <= FL_FE_MAX_DPYR && (L == 1 || (halves && L - 1 <= FL_FE_MAX_PYR));
-    if (single) {
-      wave_begin(zero_in_wave);
-      w.counters = h->d_fe_counters.get(); w.dep_error = reinterpret_cast<int*>(h->d_fe_counters.get() + FL_FE_MAX_JOBS); w.dep_error_host = h->d_fe_err_host;
-      int slot_pyr[FL_MAX_LEVELS], slot_color[FL_MAX_LEVELS][FL_MAX_MODALITIES], slot_depth[FL_MAX_MODALITIES];
-      auto last_job = [&]() -> fl_fe_job& { return w.job[w.n_jobs - 1]; };
-      auto job_ctas = [&](int idx) { return (idx + 1 < w.n_jobs ? w.job[idx + 1].cta_begin : w.n_ctas) - w.job[idx].cta_begin; };
-      auto produce = [&]() { last_job().signal_slot = w.n_jobs - 1; return w.n_jobs - 1; };
-      // tile jobs (32 x 16 tiles) also count per tile row; returns false when the image has more tile rows than counters
-      auto produce_rows = [&](int slot) {
-        fl_fe_job& jb = w.job[slot];
-        const int rows = (jb.H + 15) / 16;
-        if (rows > FL_FE_MAX_TILE_ROWS) return;                 // (then the consumers wait for the whole job)
-        jb.row_base = FL_FE_MAX_JOBS + 1 + slot * FL_FE_MAX_TILE_ROWS;
-      };
-      auto consume_rows = [&](int slot, int shift) {      // spread job: wait per tile row of producer `slot` (level shift for the depth pyramid)
-        const fl_fe_job& pj = w.job[slot];
-        if (pj.row_base < 0) return;
-        fl_fe_job& jb = last_job();
-        jb.wait_row_base = pj.row_base; jb.wait_row_shift = shift; jb.wait_row_count = (pj.H + 15) / 16;
-        jb.wait_row_target = h->fe_row_base[slot] + (unsigned)abs(pj.gx);
-      };
-      // FL_OPT_FE_DEP_TIMEOUT_TEST: the next frame waits for one CTA more than its producer has, i.e. the wait times out (test of the fallback)
-      const unsigned dep_test = h->opt_dep_test ? 1u : 0u;
-      h->opt_dep_test = false;
-      auto consume = [&](int slot) { last_job().wait_slot = slot; last_job().wait_target = h->fe_counter_base[slot] + (unsigned)job_ctas(slot) + dep_test; };
-      // 0. the staged similarity kernel's per-template feature lists -> L2 (they would otherwise cost its prologue DRAM round trips)
-      if (h->use_staged && h->n_templates > 0 && n_jobs_single + 3 <= FL_FE_MAX_JOBS) {
-        fl_fe_add_prefetch(&w, h->plan.gfeat, (size_t)h->n_templates * 64 * sizeof(uint32_t));
-        fl_fe_add_prefetch(&w, h->plan.gpre, (size_t)h->n_templates * h->plan.pre_stride);
-        fl_fe_add_prefetch(&w, h->plan.gmeta, (size_t)h->n_templates * sizeof(int4));
-        if (n_jobs_single + 6 <= FL_FE_MAX_JOBS) {                               // the prologue's dependent lookups: template -> class -> enabled
-          fl_fe_add_prefetch(&w, h->d_class_of.get(), (size_t)h->n_templates * sizeof(int32_t));
-          fl_fe_add_prefetch(&w, h->d_class_enabled.get(), (size_t)std::max(h->n_classes, 1));
-          fl_fe_add_prefetch(&w, h->d_tid_of.get(), (size_t)h->n_templates * sizeof(int32_t));
-        }
+  // wave schedule (frontend.cu): L + 1 launches for the whole front end; wave l produces the labels of level l and the
+  // linear memories of level l - 1.  Jobs are added longest first: the kernel ends with its slowest CTA, and CTAs are
+  // scheduled in job order.  (Measured alternative: slicing the level-0 colour quantisation over the waves and moving
+  // every spread to the last wave - 16.6 + 10.8 + 9.2 us instead of 17.7 + 9.4 + 6.0 us, i.e. no gain: each wave has a
+  // latency floor of one colour-tile CTA, about 8 us.)
+  const int L = p.n_levels;
+  fl_fe_wave w;
+  auto wave_begin = [&](bool zero) { w.n_jobs = 0; w.n_ctas = 0; w.smem = 0; w.n_pyr = 0; w.zero_me = zero ? d_count : nullptr; w.counters = nullptr; w.dep_error = nullptr; w.dep_error_host = nullptr; w.trace = nullptr; };
+  bool launch_ok = true;
+  auto wave_flush = [&]() { if (w.n_jobs > 0) { launch_ok &= fl_launch_fe_wave(w, s) == cudaSuccess; ++h->launches; } w.n_jobs = 0; w.n_ctas = 0; w.smem = 0; w.n_pyr = 0; w.zero_me = nullptr; };
+  // word-parallel quantisers (frontend_v2.cuh).  The depth job also writes the NN-downsampled label pyramid when every level
+  // halves exactly (then dst_l(y,x) = src(2^l y, 2^l x)).
+  bool depth_pyr_fused[FL_MAX_MODALITIES] = {false, false, false, false};
+  bool halves = true;
+  for (int l = 0; l + 1 < L; ++l) halves &= (h->geom[l].W % 2 == 0) && (h->geom[l].H % 2 == 0);
+  auto wave_room = [&]() { if (w.n_jobs == FL_FE_MAX_JOBS) wave_flush(); };     // jobs of one wave are independent: splitting is always safe
+  // spread + response maps + linear memories of (level l, modality m).  A masked modality's spread job reads the level-0 mask at a
+  // shift of l when every level halves exactly (NN-halving then picks src(2y, 2x)); otherwise only the per-wave schedule runs, and it
+  // builds the mask pyramid in d_mask with resize jobs next to the depth labels'.
+  auto add_spread = [&](int l, int m) -> int {
+    uint8_t* spread = nullptr;
+    if (h->keep_spread) { TRY(h->d_spread[l][m].grow((size_t)(p.max_width >> l) * (p.max_height >> l))); spread = h->d_spread[l][m].get(); }
+    const bool pyr = mask0[m] && l > 0 && !halves;
+    fl_fe_add_spread(&w, h->d_q[l][m].get(), h->geom[l], h->d_lm[l].get() + (size_t)m * h->geom[l].mod_stride, spread, lm4_of(h, l, m), mass_of(h, l, m),
+                     pyr ? h->d_mask[l][m].get() : mask0[m], pyr ? h->geom[l].W : h->geom[0].W, pyr ? 0 : l);
+    return FL_OK;
+  };
+  // ---- single-launch front end: every job of the frame in ONE grid, producers before consumers, dependencies resolved by
+  // per-job CTA counters inside the kernel (k_front_end_wave).  Removes L launches + their dependency gaps and lets the
+  // level-0 work fill the machine while the short critical chain pyrDown -> colour L(top) -> spread L(top) runs.
+  const bool fe_waves = h->opt_fe_waves;                                       // FL_OPT_FE_WAVES: one launch per wave (also the fallback after a dependency time-out)
+  int n_color = 0, n_depth = 0;
+  for (int m = 0; m < p.n_modalities; ++m) { n_color += p.modality_kind[m] == FL_MODALITY_COLOR_GRADIENT; n_depth += p.modality_kind[m] == FL_MODALITY_DEPTH_NORMAL; }
+  const int n_jobs_single = (n_color ? L - 1 : 0) + n_color * L + n_depth + p.n_modalities * L;
+  const bool single = !fe_waves && !h->fe_force_waves && n_jobs_single <= FL_FE_MAX_JOBS && n_depth <= FL_FE_MAX_DPYR && (L == 1 || (halves && L - 1 <= FL_FE_MAX_PYR));
+  if (single) {
+    wave_begin(true);                                                            // wave 0 resets the candidate counter: no memset node between the kernels
+    w.counters = h->d_fe_counters.get(); w.dep_error = reinterpret_cast<int*>(h->d_fe_counters.get() + FL_FE_MAX_JOBS); w.dep_error_host = h->d_fe_err_host;
+    int slot_pyr[FL_MAX_LEVELS], slot_color[FL_MAX_LEVELS][FL_MAX_MODALITIES], slot_depth[FL_MAX_MODALITIES];
+    auto last_job = [&]() -> fl_fe_job& { return w.job[w.n_jobs - 1]; };
+    auto job_ctas = [&](int idx) { return (idx + 1 < w.n_jobs ? w.job[idx + 1].cta_begin : w.n_ctas) - w.job[idx].cta_begin; };
+    auto produce = [&]() { last_job().signal_slot = w.n_jobs - 1; return w.n_jobs - 1; };
+    // tile jobs (32 x 16 tiles) also count per tile row; returns false when the image has more tile rows than counters
+    auto produce_rows = [&](int slot) {
+      fl_fe_job& jb = w.job[slot];
+      const int rows = (jb.H + 15) / 16;
+      if (rows > FL_FE_MAX_TILE_ROWS) return;                 // (then the consumers wait for the whole job)
+      jb.row_base = FL_FE_MAX_JOBS + 1 + slot * FL_FE_MAX_TILE_ROWS;
+    };
+    auto consume_rows = [&](int slot, int shift) {      // spread job: wait per tile row of producer `slot` (level shift for the depth pyramid)
+      const fl_fe_job& pj = w.job[slot];
+      if (pj.row_base < 0) return;
+      fl_fe_job& jb = last_job();
+      jb.wait_row_base = pj.row_base; jb.wait_row_shift = shift; jb.wait_row_count = (pj.H + 15) / 16;
+      jb.wait_row_target = h->fe_row_base[slot] + (unsigned)abs(pj.gx);
+    };
+    // FL_OPT_FE_DEP_TIMEOUT_TEST: the next frame waits for one CTA more than its producer has, i.e. the wait times out (test of the fallback)
+    const unsigned dep_test = h->opt_dep_test ? 1u : 0u;
+    h->opt_dep_test = false;
+    auto consume = [&](int slot) { last_job().wait_slot = slot; last_job().wait_target = h->fe_counter_base[slot] + (unsigned)job_ctas(slot) + dep_test; };
+    // 0. the staged similarity kernel's per-template feature lists -> L2 (they would otherwise cost its prologue DRAM round trips)
+    if (h->use_staged && h->n_templates > 0 && n_jobs_single + 3 <= FL_FE_MAX_JOBS) {
+      fl_fe_add_prefetch(&w, h->plan.gfeat, (size_t)h->n_templates * 64 * sizeof(uint32_t));
+      fl_fe_add_prefetch(&w, h->plan.gpre, (size_t)h->n_templates * h->plan.pre_stride);
+      fl_fe_add_prefetch(&w, h->plan.gmeta, (size_t)h->n_templates * sizeof(int4));
+      if (n_jobs_single + 6 <= FL_FE_MAX_JOBS) {                               // the prologue's dependent lookups: template -> class -> enabled
+        fl_fe_add_prefetch(&w, h->d_class_of.get(), (size_t)h->n_templates * sizeof(int32_t));
+        fl_fe_add_prefetch(&w, h->d_class_enabled.get(), (size_t)std::max(h->n_classes, 1));
+        fl_fe_add_prefetch(&w, h->d_tid_of.get(), (size_t)h->n_templates * sizeof(int32_t));
       }
-      // 1. colour pyramid chain (short jobs, on the critical path of the coarsest level)
-      if (first_color >= 0)
-        for (int l = 0; l + 1 < L; ++l) {
-          fl_fe_add_pyrdown(&w, l == 0 ? d_bgr : h->d_bgr[l].get(), h->geom[l].W, h->geom[l].H, h->d_bgr[l + 1].get(), l == 0);
-          slot_pyr[l + 1] = produce();
+    }
+    // 1. colour pyramid chain (short jobs, on the critical path of the coarsest level)
+    if (first_color >= 0)
+      for (int l = 0; l + 1 < L; ++l) {
+        fl_fe_add_pyrdown(&w, l == 0 ? d_bgr : h->d_bgr[l].get(), h->geom[l].W, h->geom[l].H, h->d_bgr[l + 1].get(), l == 0);
+        slot_pyr[l + 1] = produce();
+        if (l > 0) consume(slot_pyr[l]);
+      }
+    // 2. depth labels of every level (one job per depth modality)
+    for (int m = 0; m < p.n_modalities; ++m)
+      if (p.modality_kind[m] == FL_MODALITY_DEPTH_NORMAL) {
+        fl_depth_pyr pyr; memset(&pyr, 0, sizeof pyr);
+        pyr.n = L - 1;
+        for (int k = 1; k < L; ++k) { pyr.W[k - 1] = h->geom[k].W; pyr.H[k - 1] = h->geom[k].H; pyr.dst[k - 1] = h->d_q[k][m].get(); }
+        fl_fe_add_depth_v2(&w, d_depth, h->geom[0].W, h->geom[0].H, p.distance_threshold, p.difference_threshold, h->d_q[0][m].get(), pyr.n > 0 ? &pyr : nullptr);
+        slot_depth[m] = produce();
+        produce_rows(slot_depth[m]);
+      }
+    // 3. colour labels, coarsest level first
+    for (int l = L - 1; l >= 0; --l)
+      for (int m = 0; m < p.n_modalities; ++m)
+        if (p.modality_kind[m] == FL_MODALITY_COLOR_GRADIENT) {
+          fl_fe_add_color_v2(&w, l == 0 ? d_bgr : h->d_bgr[l].get(), h->geom[l].W, h->geom[l].H, thr_sq, h->d_q[l][m].get());
+          slot_color[l][m] = produce();
+          produce_rows(slot_color[l][m]);
           if (l > 0) consume(slot_pyr[l]);
         }
-      // 2. depth labels of every level (one job per depth modality)
-      for (int m = 0; m < p.n_modalities; ++m)
-        if (p.modality_kind[m] == FL_MODALITY_DEPTH_NORMAL) {
-          fl_depth_pyr pyr; memset(&pyr, 0, sizeof pyr);
-          pyr.n = L - 1;
-          for (int k = 1; k < L; ++k) { pyr.W[k - 1] = h->geom[k].W; pyr.H[k - 1] = h->geom[k].H; pyr.dst[k - 1] = h->d_q[k][m].get(); }
-          fl_fe_add_depth_v2(&w, d_depth, h->geom[0].W, h->geom[0].H, p.distance_threshold, p.difference_threshold, h->d_q[0][m].get(), pyr.n > 0 ? &pyr : nullptr);
-          slot_depth[m] = produce();
-          produce_rows(slot_depth[m]);
-        }
-      // 3. colour labels, coarsest level first
-      for (int l = L - 1; l >= 0; --l)
-        for (int m = 0; m < p.n_modalities; ++m)
-          if (p.modality_kind[m] == FL_MODALITY_COLOR_GRADIENT) {
-            fl_fe_add_color_v2(&w, l == 0 ? d_bgr : h->d_bgr[l].get(), h->geom[l].W, h->geom[l].H, thr_sq, h->d_q[l][m].get());
-            slot_color[l][m] = produce();
-            produce_rows(slot_color[l][m]);
-            if (l > 0) consume(slot_pyr[l]);
-          }
-      // 4. spread + response maps + linear memories, coarsest level first (the similarity kernel needs only that one)
-      for (int l = L - 1; l >= 0; --l)
-        for (int m = 0; m < p.n_modalities; ++m) {
-          uint8_t* spread = nullptr;
-          if (h->keep_spread) { TRY(h->d_spread[l][m].grow((size_t)(p.max_width >> l) * (p.max_height >> l))); spread = h->d_spread[l][m].get(); }
-          fl_fe_add_spread(&w, h->d_q[l][m].get(), h->geom[l], h->d_lm[l].get() + (size_t)m * h->geom[l].mod_stride, spread, lm4_of(h, l, m), mass_of(h, l, m));
-          const bool is_color = p.modality_kind[m] == FL_MODALITY_COLOR_GRADIENT;
-          consume(is_color ? slot_color[l][m] : slot_depth[m]);
-          consume_rows(is_color ? slot_color[l][m] : slot_depth[m], is_color ? 0 : l);
-        }
-      if (h->opt_trace) {                                                        // developer timeline: per job first start / last end
-        TRY(h->d_fe_trace.grow(2 * FL_FE_MAX_JOBS + 2 * FL_FE_MAX_JOBS));
-        unsigned long long init[2 * FL_FE_MAX_JOBS];
-        for (int i = 0; i < FL_FE_MAX_JOBS; ++i) { init[2 * i] = ~0ull; init[2 * i + 1] = 0; }
-        FL_CUDA(cudaMemcpyAsync(h->d_fe_trace.get(), init, sizeof init, cudaMemcpyHostToDevice, s));
-        FL_CUDA(cudaStreamSynchronize(s));
-        w.trace = h->d_fe_trace.get();
-        h->fe_trace_jobs = w.n_jobs;
-        for (int i = 0; i < w.n_jobs; ++i) { h->fe_trace_kind[i] = w.job[i].kind; h->fe_trace_ctas[i] = job_ctas(i); }
-      }
-      // the monotonic counter bases advance only when the launch really went out (a failed launch bumps no counter)
-      unsigned add_ctr[FL_FE_MAX_JOBS] = {0}, add_row[FL_FE_MAX_JOBS] = {0};
-      for (int i = 0; i < w.n_jobs; ++i) { if (w.job[i].signal_slot >= 0) add_ctr[i] = (unsigned)job_ctas(i); if (w.job[i].row_base >= 0) add_row[i] = (unsigned)abs(w.job[i].gx); }
-      wave_flush();
-      if (!launch_ok) { fl_set_error("front-end launch failed: %s", cudaGetErrorString(cudaGetLastError())); return FL_ERR_CUDA; }
-      for (int i = 0; i < FL_FE_MAX_JOBS; ++i) { h->fe_counter_base[i] += add_ctr[i]; h->fe_row_base[i] += add_row[i]; }
-    } else
-    for (int wv = 0; wv <= L; ++wv) {
-      wave_begin(wv == 0 && zero_in_wave);                                        // the candidate counter is reset by the first wave
-      const int l = wv;                                                             // level whose labels this wave produces
-      if (l < L) {
-        const fl_level_geom& g = h->geom[l];
-        for (int m = 0; m < p.n_modalities; ++m)
-          if (p.modality_kind[m] == FL_MODALITY_COLOR_GRADIENT) {
-            wave_room();
-            fl_fe_add_color_v2(&w, l == 0 ? d_bgr : h->d_bgr[l].get(), g.W, g.H, thr_sq, h->d_q[l][m].get());
-          }
-        for (int m = 0; m < p.n_modalities; ++m)
-          if (p.modality_kind[m] == FL_MODALITY_DEPTH_NORMAL && l == 0) {
-            wave_room();
-            fl_depth_pyr pyr; memset(&pyr, 0, sizeof pyr);
-            if (halves && L > 1 && L - 1 <= FL_FE_MAX_PYR) {
-              pyr.n = L - 1;
-              for (int k = 1; k < L; ++k) { pyr.W[k - 1] = h->geom[k].W; pyr.H[k - 1] = h->geom[k].H; pyr.dst[k - 1] = h->d_q[k][m].get(); }
-            }
-            if (pyr.n > 0 && fl_fe_add_depth_v2(&w, d_depth, g.W, g.H, p.distance_threshold, p.difference_threshold, h->d_q[0][m].get(), &pyr)) depth_pyr_fused[m] = true;
-            else fl_fe_add_depth_v2(&w, d_depth, g.W, g.H, p.distance_threshold, p.difference_threshold, h->d_q[0][m].get(), nullptr);
-          }
-      }
-      if (l >= 1) {
-        const fl_level_geom& g = h->geom[l - 1];
-        for (int m = 0; m < p.n_modalities; ++m) {
-          uint8_t* spread = nullptr;
-          if (h->keep_spread) { TRY(h->d_spread[l - 1][m].grow((size_t)(p.max_width >> (l - 1)) * (p.max_height >> (l - 1)))); spread = h->d_spread[l - 1][m].get(); }
-          wave_room();
-          fl_fe_add_spread(&w, h->d_q[l - 1][m].get(), g, h->d_lm[l - 1].get() + (size_t)m * g.mod_stride, spread, lm4_of(h, l - 1, m), mass_of(h, l - 1, m));
-        }
-      }
-      if (l < L) {
-        const fl_level_geom& g = h->geom[l];
-        if (first_color >= 0 && l + 1 < L) { wave_room(); fl_fe_add_pyrdown(&w, l == 0 ? d_bgr : h->d_bgr[l].get(), g.W, g.H, h->d_bgr[l + 1].get(), true); }   // shared by all colour modalities
-        for (int m = 0; m < p.n_modalities; ++m)
-          if (p.modality_kind[m] == FL_MODALITY_DEPTH_NORMAL && l > 0 && !depth_pyr_fused[m]) { wave_room(); fl_fe_add_resize(&w, h->d_q[l - 1][m].get(), h->geom[l - 1].W, h->geom[l - 1].H, h->d_q[l][m].get()); }
-      }
-      wave_flush();
-    }
-  } else {
-    // masked path (rare): one kernel per stage, masks NN-downsampled per level and applied before spreading
-    bool color_pyr_done = false;
-    for (int l = 0; l < p.n_levels; ++l) {
-      const fl_level_geom& g = h->geom[l];
-      const size_t npx = (size_t)g.W * g.H;
+    // 4. spread + response maps + linear memories, coarsest level first (the similarity kernel needs only that one)
+    for (int l = L - 1; l >= 0; --l)
       for (int m = 0; m < p.n_modalities; ++m) {
-        const bool has_mask = h->used_mask[m];
-        if (p.modality_kind[m] == FL_MODALITY_COLOR_GRADIENT) {
-          const uint8_t* src = d_bgr;
-          if (l > 0) {
-            if (!color_pyr_done) {
-              const uint8_t* prev = l == 1 ? d_bgr : h->d_bgr[l - 1].get();
-              fl_launch_pyrdown_bgr(prev, h->geom[l - 1].W, h->geom[l - 1].H, h->d_bgr[l].get(), s); ++h->launches;
-              color_pyr_done = true;
-            }
-            src = h->d_bgr[l].get();
-          }
-          { fl_fe_wave w1; fe_wave_init(&w1); fl_fe_add_color_v2(&w1, src, g.W, g.H, thr_sq, h->d_q[l][m].get()); fl_launch_fe_wave(w1, s); ++h->launches; }
-        } else {
-          if (l == 0) { fl_fe_wave w1; fe_wave_init(&w1); fl_fe_add_depth_v2(&w1, d_depth, g.W, g.H, p.distance_threshold, p.difference_threshold, h->d_q[0][m].get(), nullptr); fl_launch_fe_wave(w1, s); ++h->launches; }
-          else { fl_launch_resize_nn_half(h->d_q[l - 1][m].get(), h->geom[l - 1].W, h->geom[l - 1].H, h->d_q[l][m].get(), s); ++h->launches; }
-        }
-        const uint8_t* qsrc = h->d_q[l][m].get();
-        if (has_mask) {
-          const size_t n = (size_t)(p.max_width >> l) * (p.max_height >> l);
-          TRY(h->d_mask[l][m].grow(n)); TRY(h->d_qm[l][m].grow(n));
-          const uint8_t* mk = (const uint8_t*)d_masks[m];
-          if (l > 0) { fl_launch_resize_nn_half(l == 1 ? (const uint8_t*)d_masks[m] : h->d_mask[l - 1][m].get(), h->geom[l - 1].W, h->geom[l - 1].H, h->d_mask[l][m].get(), s); ++h->launches; mk = h->d_mask[l][m].get(); }
-          fl_launch_apply_mask(h->d_q[l][m].get(), mk, (int)npx, h->d_qm[l][m].get(), s); ++h->launches;
-          qsrc = h->d_qm[l][m].get();
-        }
-        uint8_t* spread = nullptr;
-        if (h->keep_spread) { TRY(h->d_spread[l][m].grow((size_t)(p.max_width >> l) * (p.max_height >> l))); spread = h->d_spread[l][m].get(); }
-        fl_launch_spread_lm(qsrc, g, h->d_lm[l].get() + (size_t)m * g.mod_stride, spread, lm4_of(h, l, m), mass_of(h, l, m), s); ++h->launches;
+        TRY(add_spread(l, m));
+        const bool is_color = p.modality_kind[m] == FL_MODALITY_COLOR_GRADIENT;
+        consume(is_color ? slot_color[l][m] : slot_depth[m]);
+        consume_rows(is_color ? slot_color[l][m] : slot_depth[m], is_color ? 0 : l);
       }
-      color_pyr_done = false;
+    if (h->opt_trace) {                                                        // developer timeline: per job first start / last end
+      TRY(h->d_fe_trace.grow(2 * FL_FE_MAX_JOBS + 2 * FL_FE_MAX_JOBS));
+      unsigned long long init[2 * FL_FE_MAX_JOBS];
+      for (int i = 0; i < FL_FE_MAX_JOBS; ++i) { init[2 * i] = ~0ull; init[2 * i + 1] = 0; }
+      FL_CUDA(cudaMemcpyAsync(h->d_fe_trace.get(), init, sizeof init, cudaMemcpyHostToDevice, s));
+      FL_CUDA(cudaStreamSynchronize(s));
+      w.trace = h->d_fe_trace.get();
+      h->fe_trace_jobs = w.n_jobs;
+      for (int i = 0; i < w.n_jobs; ++i) { h->fe_trace_kind[i] = w.job[i].kind; h->fe_trace_ctas[i] = job_ctas(i); }
     }
+    // the monotonic counter bases advance only when the launch really went out (a failed launch bumps no counter)
+    unsigned add_ctr[FL_FE_MAX_JOBS] = {0}, add_row[FL_FE_MAX_JOBS] = {0};
+    for (int i = 0; i < w.n_jobs; ++i) { if (w.job[i].signal_slot >= 0) add_ctr[i] = (unsigned)job_ctas(i); if (w.job[i].row_base >= 0) add_row[i] = (unsigned)abs(w.job[i].gx); }
+    wave_flush();
+    if (!launch_ok) { fl_set_error("front-end launch failed: %s", cudaGetErrorString(cudaGetLastError())); return FL_ERR_CUDA; }
+    for (int i = 0; i < FL_FE_MAX_JOBS; ++i) { h->fe_counter_base[i] += add_ctr[i]; h->fe_row_base[i] += add_row[i]; }
+  } else
+  for (int wv = 0; wv <= L; ++wv) {
+    wave_begin(wv == 0);                                                        // the candidate counter is reset by the first wave
+    const int l = wv;                                                             // level whose labels this wave produces
+    if (l < L) {
+      const fl_level_geom& g = h->geom[l];
+      for (int m = 0; m < p.n_modalities; ++m)
+        if (p.modality_kind[m] == FL_MODALITY_COLOR_GRADIENT) {
+          wave_room();
+          fl_fe_add_color_v2(&w, l == 0 ? d_bgr : h->d_bgr[l].get(), g.W, g.H, thr_sq, h->d_q[l][m].get());
+        }
+      for (int m = 0; m < p.n_modalities; ++m)
+        if (p.modality_kind[m] == FL_MODALITY_DEPTH_NORMAL && l == 0) {
+          wave_room();
+          fl_depth_pyr pyr; memset(&pyr, 0, sizeof pyr);
+          if (halves && L > 1 && L - 1 <= FL_FE_MAX_PYR) {
+            pyr.n = L - 1;
+            for (int k = 1; k < L; ++k) { pyr.W[k - 1] = h->geom[k].W; pyr.H[k - 1] = h->geom[k].H; pyr.dst[k - 1] = h->d_q[k][m].get(); }
+          }
+          if (pyr.n > 0 && fl_fe_add_depth_v2(&w, d_depth, g.W, g.H, p.distance_threshold, p.difference_threshold, h->d_q[0][m].get(), &pyr)) depth_pyr_fused[m] = true;
+          else fl_fe_add_depth_v2(&w, d_depth, g.W, g.H, p.distance_threshold, p.difference_threshold, h->d_q[0][m].get(), nullptr);
+        }
+    }
+    if (l >= 1) {
+      for (int m = 0; m < p.n_modalities; ++m) { wave_room(); TRY(add_spread(l - 1, m)); }
+    }
+    if (l < L) {
+      const fl_level_geom& g = h->geom[l];
+      if (first_color >= 0 && l + 1 < L) { wave_room(); fl_fe_add_pyrdown(&w, l == 0 ? d_bgr : h->d_bgr[l].get(), g.W, g.H, h->d_bgr[l + 1].get(), true); }   // shared by all colour modalities
+      for (int m = 0; m < p.n_modalities; ++m)
+        if (p.modality_kind[m] == FL_MODALITY_DEPTH_NORMAL && l > 0 && !depth_pyr_fused[m]) { wave_room(); fl_fe_add_resize(&w, h->d_q[l - 1][m].get(), h->geom[l - 1].W, h->geom[l - 1].H, h->d_q[l][m].get()); }
+      for (int m = 0; m < p.n_modalities; ++m)
+        if (mask0[m] && l > 0 && !halves) { wave_room(); fl_fe_add_resize(&w, l == 1 ? mask0[m] : h->d_mask[l - 1][m].get(), h->geom[l - 1].W, h->geom[l - 1].H, h->d_mask[l][m].get()); }
+    }
+    wave_flush();
   }
   if (h->profile) cudaEventRecord(h->ev[1].get(), s);
-  if (!zero_in_wave) FL_CUDA(cudaMemsetAsync(d_count, 0, sizeof(int), s));
   if (h->n_templates > 0) {
     fl_tdb db = make_tdb(h);
     const int lowest = p.n_levels - 1;
@@ -892,11 +858,35 @@ static int stage_frame(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, cons
   }
   for (int m = 0; m < FL_MAX_MODALITIES; ++m) d_masks[m] = nullptr;
   if (masks) for (int m = 0; m < p.n_modalities; ++m) if (masks[m]) {
-    TRY(h->d_mask[0][m].grow((size_t)p.max_width * p.max_height)); TRY(h->d_qm[0][m].grow((size_t)p.max_width * p.max_height));
     memcpy(h->h_mask.get() + (size_t)m * W * H, masks[m], (size_t)W * H);
     FL_CUDA(cudaMemcpyAsync(h->d_mask[0][m].get(), h->h_mask.get() + (size_t)m * W * H, (size_t)W * H, cudaMemcpyHostToDevice, s));
     d_masks[m] = h->d_mask[0][m].get(); *any_mask = true;
   }
+  return FL_OK;
+}
+
+// The quantised image of (level l, modality m) of the last frame into host memory, as the reference's quantize() leaves it: a masked
+// modality reads 0 where the level's mask - the level-0 mask NN-halved l times (linemod.cpp:448, 736) - is 0.  The mask is applied here,
+// outside the frame, so that the frame's kernels only AND it into the labels they read (dev_spread_lm).  An unmasked image is only
+// enqueued (the caller synchronises); a masked one is finished before this returns.
+static int read_quantized(fl_handle* h, int l, int m, uint8_t* dst) {
+  cudaStream_t s = h->stream.get();
+  const fl_level_geom* g = h->geom;
+  FL_CUDA(cudaMemcpyAsync(dst, h->d_q[l][m].get(), (size_t)g[l].W * g[l].H, cudaMemcpyDeviceToHost, s));
+  if (!h->frame_mask[m]) return FL_OK;
+  std::vector<uint8_t> mk((size_t)g[0].W * g[0].H), half;
+  FL_CUDA(cudaMemcpyAsync(mk.data(), h->frame_mask[m], mk.size(), cudaMemcpyDeviceToHost, s));
+  FL_CUDA(cudaStreamSynchronize(s));
+  for (int k = 1; k <= l; ++k) {                        // cv::resize INTER_NEAREST to (W/2, H/2): the index arithmetic of dev_resize_nn_half
+    const int sw = g[k - 1].W, sh = g[k - 1].H, dw = g[k].W, dh = g[k].H;
+    half.resize((size_t)dw * dh);
+    for (int y = 0; y < dh; ++y) {
+      const int sy = std::min((int)floor(y * ((double)sh / dh)), sh - 1);
+      for (int x = 0; x < dw; ++x) half[(size_t)y * dw + x] = mk[(size_t)sy * sw + std::min((int)floor(x * ((double)sw / dw)), sw - 1)];
+    }
+    mk.swap(half);
+  }
+  for (size_t i = 0; i < mk.size(); ++i) if (!mk[i]) dst[i] = 0;
   return FL_OK;
 }
 
@@ -929,16 +919,11 @@ extern "C" int fl_match(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, con
   if (rc != FL_OK) return rc;
   rc = fl_match_wait(h);
   if (rc != FL_OK) { h->in_depth_W = h->in_depth_H = 0; return rc; }
-  cudaStream_t s = h->stream.get();
   rc = fl_match_fetch(h, out, capacity, count);
   if (quantized_out) {
-    for (int l = 0; l < p.n_levels; ++l) for (int m = 0; m < p.n_modalities; ++m) {
-      uint8_t* dst = quantized_out[l * p.n_modalities + m];
-      if (!dst) continue;
-      const uint8_t* src = h->used_mask[m] ? h->d_qm[l][m].get() : h->d_q[l][m].get();
-      FL_CUDA(cudaMemcpyAsync(dst, src, (size_t)h->geom[l].W * h->geom[l].H, cudaMemcpyDeviceToHost, s));
-    }
-    FL_CUDA(cudaStreamSynchronize(s));
+    for (int l = 0; l < p.n_levels; ++l) for (int m = 0; m < p.n_modalities; ++m)
+      if (quantized_out[l * p.n_modalities + m]) TRY(read_quantized(h, l, m, quantized_out[l * p.n_modalities + m]));
+    FL_CUDA(cudaStreamSynchronize(h->stream.get()));
   }
   return rc;
 }
@@ -1127,9 +1112,10 @@ extern "C" int fl_exchange_sort_unique_device_async(fl_handle* h, int32_t rank, 
 // Template-sharded frame in one go (enqueue only): front end + matchClass on this handle's shard with the candidates written
 // straight into the caller's block [count | records], then ONE launch that refines them, pushes the block to every peer,
 // waits for the peers' blocks and sorts the union (k_refine_sort<1> with the exchange in its last CTA).
-extern "C" int fl_match_shard_exchange_device_async(fl_handle* h, const void* d_bgr, const void* d_depth, int32_t W, int32_t H, float threshold,
-                                                    const int32_t* class_filter, int32_t n_filter, int32_t rank, int32_t world,
-                                                    void* const* peer_buffers, int32_t capacity, fl_match_t* d_local_block, uint32_t epoch) {
+extern "C" int fl_match_shard_exchange_device_masked_async(fl_handle* h, const void* d_bgr, const void* d_depth, int32_t W, int32_t H,
+                                                           const void* const* d_masks, float threshold, const int32_t* class_filter, int32_t n_filter,
+                                                           int32_t rank, int32_t world, void* const* peer_buffers, int32_t capacity,
+                                                           fl_match_t* d_local_block, uint32_t epoch) {
   if (!h || !peer_buffers || !d_local_block || world < 1 || world > FL_XCHG_MAX_WORLD || rank < 0 || rank >= world || capacity < 1 || epoch == 0) return FL_ERR_ARG;
   FL_CUDA(cudaSetDevice(h->p.device));
   if (h->pend_sort) { fl_set_error("fl_match_wait has not been called for the previous frame"); return FL_ERR_STATE; }
@@ -1137,7 +1123,7 @@ extern "C" int fl_match_shard_exchange_device_async(fl_handle* h, const void* d_
   const bool defer = !h->opt_split_refine && h->n_templates > 0 && h->p.n_levels > 1;
   fl_match_t* recs = d_local_block + 1;
   int* d_cnt = reinterpret_cast<int*>(d_local_block);
-  TRY(run_match_stages(h, (const uint8_t*)d_bgr, (const uint16_t*)d_depth, W, H, nullptr, threshold, class_filter, n_filter, recs, capacity, d_cnt, defer));
+  TRY(run_match_stages(h, (const uint8_t*)d_bgr, (const uint16_t*)d_depth, W, H, d_masks, threshold, class_filter, n_filter, recs, capacity, d_cnt, defer));
   fl_xchg X;
   memset(&X, 0, sizeof X);
   X.world = world; X.rank = rank; X.cap = capacity; X.epoch = epoch; X.local_block = d_local_block;
@@ -1147,10 +1133,17 @@ extern "C" int fl_match_shard_exchange_device_async(fl_handle* h, const void* d_
   const fl_refine_req req = {threshold, recs, capacity, d_cnt};
   return sort_launch(h, lists, h->d_out, h->p.max_candidates, h->d_out_count, true, &X, defer ? &req : nullptr);
 }
+extern "C" int fl_match_shard_exchange_device_async(fl_handle* h, const void* d_bgr, const void* d_depth, int32_t W, int32_t H, float threshold,
+                                                    const int32_t* class_filter, int32_t n_filter, int32_t rank, int32_t world,
+                                                    void* const* peer_buffers, int32_t capacity, fl_match_t* d_local_block, uint32_t epoch) {
+  return fl_match_shard_exchange_device_masked_async(h, d_bgr, d_depth, W, H, nullptr, threshold, class_filter, n_filter, rank, world, peer_buffers, capacity,
+                                                     d_local_block, epoch);
+}
 
-extern "C" int fl_match_shard_exchange_async(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int32_t W, int32_t H,
-                                             float threshold, const int32_t* class_filter, int32_t n_filter, int32_t rank, int32_t world,
-                                             void* const* peer_buffers, int32_t capacity, fl_match_t* d_local_block, uint32_t epoch) {
+extern "C" int fl_match_shard_exchange_masked_async(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
+                                                    int32_t W, int32_t H, const uint8_t* const* masks, float threshold, const int32_t* class_filter,
+                                                    int32_t n_filter, int32_t rank, int32_t world, void* const* peer_buffers, int32_t capacity,
+                                                    fl_match_t* d_local_block, uint32_t epoch) {
   if (!h) return FL_ERR_ARG;
   if (h->pend_sort) { fl_set_error("fl_match_wait has not been called for the previous frame"); return FL_ERR_STATE; }
   h->in_depth_W = h->in_depth_H = 0;
@@ -1159,10 +1152,17 @@ extern "C" int fl_match_shard_exchange_async(fl_handle* h, const uint8_t* bgr, s
   const uint8_t* d_bgr; const uint16_t* d_depth;
   const void* d_masks[FL_MAX_MODALITIES];
   bool any_mask;
-  TRY(stage_frame(h, bgr, bgr_stride, depth, depth_stride, W, H, nullptr, &d_bgr, &d_depth, d_masks, &any_mask));
-  TRY(fl_match_shard_exchange_device_async(h, d_bgr, d_depth, W, H, threshold, class_filter, n_filter, rank, world, peer_buffers, capacity, d_local_block, epoch));
+  TRY(stage_frame(h, bgr, bgr_stride, depth, depth_stride, W, H, masks, &d_bgr, &d_depth, d_masks, &any_mask));
+  TRY(fl_match_shard_exchange_device_masked_async(h, d_bgr, d_depth, W, H, any_mask ? d_masks : nullptr, threshold, class_filter, n_filter, rank, world,
+                                                  peer_buffers, capacity, d_local_block, epoch));
   if (d_depth) { h->in_depth_W = W; h->in_depth_H = H; }
   return FL_OK;
+}
+extern "C" int fl_match_shard_exchange_async(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int32_t W, int32_t H,
+                                             float threshold, const int32_t* class_filter, int32_t n_filter, int32_t rank, int32_t world,
+                                             void* const* peer_buffers, int32_t capacity, fl_match_t* d_local_block, uint32_t epoch) {
+  return fl_match_shard_exchange_masked_async(h, bgr, bgr_stride, depth, depth_stride, W, H, nullptr, threshold, class_filter, n_filter, rank, world,
+                                              peer_buffers, capacity, d_local_block, epoch);
 }
 
 extern "C" int fl_exchange_sort_unique_device(fl_handle* h, int32_t rank, int32_t world, void* const* peer_buffers, int32_t capacity,
@@ -1194,9 +1194,13 @@ extern "C" int fl_debug_get(fl_handle* h, int what, int32_t a, int32_t b, int32_
     if (a < 0 || a >= p.n_levels || b < 0 || b >= p.n_modalities) return FL_ERR_ARG;
     size_t n = (size_t)h->geom[a].W * h->geom[a].H;
     if (bytes < n) return FL_ERR_CAPACITY;
-    const uint8_t* src = what == FL_DBG_SPREAD ? h->d_spread[a][b].get() : (h->used_mask[b] ? h->d_qm[a][b].get() : h->d_q[a][b].get());
-    if (!src) return FL_ERR_STATE;
-    FL_CUDA(cudaMemcpy(host_out, src, n, cudaMemcpyDeviceToHost));
+    if (what == FL_DBG_QUANTIZED) {
+      TRY(read_quantized(h, a, b, static_cast<uint8_t*>(host_out)));
+      FL_CUDA(cudaStreamSynchronize(h->stream.get()));
+      return FL_OK;
+    }
+    if (!h->d_spread[a][b].get()) return FL_ERR_STATE;
+    FL_CUDA(cudaMemcpy(host_out, h->d_spread[a][b].get(), n, cudaMemcpyDeviceToHost));
     return FL_OK;
   }
   if (what == FL_DBG_LINEAR_MEMORY) {

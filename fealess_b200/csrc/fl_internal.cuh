@@ -58,12 +58,7 @@ inline cudaError_t fl_launch(void (*kern)(KArgs...), dim3 grid, dim3 block, size
 
 // ---- front end (frontend.cu) -------------------------------------------------------------------
 int fl_launch_tables_init();   // uploads the two LUTs to __constant__ memory of the current device
-void fl_launch_pyrdown_bgr(const uint8_t* src, int W, int H, uint8_t* dst, cudaStream_t s);
-void fl_launch_resize_nn_half(const uint8_t* src, int W, int H, uint8_t* dst, cudaStream_t s);
-void fl_launch_apply_mask(const uint8_t* q, const uint8_t* mask, int n, uint8_t* out, cudaStream_t s);
-// mass_or_null: the coarsest level's response sums of this modality (8 words, see FL_MASS_*), or NULL
-void fl_launch_spread_lm(const uint8_t* q, fl_level_geom g, uint8_t* lm_mod, uint8_t* spread_or_null, uint8_t* lm4_mod_or_null, uint32_t* mass_or_null,
-                         cudaStream_t s);
+void fl_launch_resize_nn_half(const uint8_t* src, int W, int H, uint8_t* dst, cudaStream_t s);   // training's mask pyramid
 // Per-handle response mass of the coarsest level, u32 words: the spread jobs of that level add the sum of every linear-memory
 // response of (modality m, label l) into word 8 m + l; k_similarity_staged orders its phases by these sums and its last CTA to
 // read them clears them again (ticket), so every frame starts from zero without a memset.  Behind them: what the last staged
@@ -80,6 +75,7 @@ struct fl_fe_job {
   float thr_sq;
   const uint8_t* src; uint8_t* dst; uint8_t* dst2; uint8_t* dst3;   // spread job: dst = linear memories, dst2 = spread image (or NULL), dst3 = 4-bit linear memories (or NULL)
   uint32_t* mass;                                                     // spread job: response sums of the modality's 8 labels (or NULL), see FL_MASS_*
+  const uint8_t* mask; int mask_stride, mask_shift;                   // spread job: the frame's mask of the modality (or NULL), see dev_spread_lm
   fl_level_geom g;
   // in-grid dependencies (single-launch front end): a CTA of this job first waits until counters[wait_slot] has reached
   // wait_target (all CTAs of the producing job have finished), and bumps counters[signal_slot] when it is done; -1 = none
@@ -108,8 +104,10 @@ void fl_fe_add_pyrdown(fl_fe_wave* w, const uint8_t* src, int W, int H, uint8_t*
 // in the shadow of the front end so that its prologue does not start with DRAM round trips
 void fl_fe_add_prefetch(fl_fe_wave* w, const void* src, size_t bytes);
 void fl_fe_add_resize(fl_fe_wave* w, const uint8_t* src, int W, int H, uint8_t* dst);
+// mass_or_null: the coarsest level's response sums of this modality (8 words, see FL_MASS_*), or NULL.  mask_or_null: labels (y, x) are
+// kept where mask[(y << mask_shift) * mask_stride + (x << mask_shift)] != 0
 void fl_fe_add_spread(fl_fe_wave* w, const uint8_t* q, fl_level_geom g, uint8_t* lm_mod, uint8_t* spread_or_null, uint8_t* lm4_mod_or_null,
-                      uint32_t* mass_or_null);
+                      uint32_t* mass_or_null, const uint8_t* mask_or_null, int mask_stride, int mask_shift);
 cudaError_t fl_launch_fe_wave(const fl_fe_wave& w, cudaStream_t s);
 
 // ---- template training, per-pixel half (train.cu) -----------------------------------------------

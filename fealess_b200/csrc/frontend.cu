@@ -133,14 +133,7 @@ __device__ __forceinline__ void dev_pyrdown_bgr(const uint8_t* __restrict__ src,
   o[0] = (uint8_t)((s0 + 128) >> 8); o[1] = (uint8_t)((s1 + 128) >> 8); o[2] = (uint8_t)((s2 + 128) >> 8);
 }
 
-__global__ void __launch_bounds__(256) k_pyrdown_bgr(const uint8_t* __restrict__ src, int W, int H, uint8_t* __restrict__ dst) {
-  dev_pyrdown_bgr(src, W, H, dst, blockIdx.x, false);
-}
-
 static int pyrdown_ctas(int W, int H) { return ((W / 2 + PD_TW - 1) / PD_TW) * ((H / 2 + PD_TH - 1) / PD_TH); }
-void fl_launch_pyrdown_bgr(const uint8_t* src, int W, int H, uint8_t* dst, cudaStream_t s) {
-  if (pyrdown_ctas(W, H) > 0) k_pyrdown_bgr<<<pyrdown_ctas(W, H), 256, 0, s>>>(src, W, H, dst);
-}
 
 // ------------------------------------------------------------------------------------------------
 // K3 depth normals: 8-tap bilateral least squares -> normal -> NORMAL_LUT, then 5x5 median, fused (halo 2 + 5).
@@ -151,7 +144,7 @@ void fl_launch_pyrdown_bgr(const uint8_t* src, int W, int H, uint8_t* dst, cudaS
 
 
 // ------------------------------------------------------------------------------------------------
-// K4 nearest-neighbour x1/2 (cv::resize INTER_NEAREST to (W/2, H/2)) and mask application (copyTo(dst, mask))
+// K4 nearest-neighbour x1/2 (cv::resize INTER_NEAREST to (W/2, H/2)): depth labels and masks of levels that do not halve exactly
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void dev_resize_nn_half(const uint8_t* __restrict__ src, int W, int H, uint8_t* __restrict__ dst, int bx) {
   const int dw = W / 2, dh = H / 2;
@@ -168,15 +161,6 @@ __global__ void __launch_bounds__(256) k_resize_nn_half(const uint8_t* __restric
 void fl_launch_resize_nn_half(const uint8_t* src, int W, int H, uint8_t* dst, cudaStream_t s) {
   int n = (W / 2) * (H / 2);
   k_resize_nn_half<<<(n + 255) / 256, 256, 0, s>>>(src, W, H, dst);
-}
-
-__global__ void __launch_bounds__(256) k_apply_mask(const uint8_t* __restrict__ q, const uint8_t* __restrict__ mask, int n,
-                                                    uint8_t* __restrict__ out) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) out[i] = mask[i] ? q[i] : (uint8_t)0;
-}
-void fl_launch_apply_mask(const uint8_t* q, const uint8_t* mask, int n, uint8_t* out, cudaStream_t s) {
-  k_apply_mask<<<(n + 255) / 256, 256, 0, s>>>(q, mask, n, out);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -216,9 +200,12 @@ __device__ __forceinline__ uint32_t or_window(const uint32_t* __restrict__ w, in
 template <int TT>
 // mass (nullable, the coarsest level only): += this CTA's sum of every (row, cell) response of label lab into mass[lab], one atomic per label
 // per CTA - the per-frame weights by which the staged similarity kernel orders its phases (k_similarity_staged)
+// mk (nullable): the frame's mask of this modality (copyTo(dst, mask), linemod.cpp:455-459, 741-745); label (y, x) of this level is kept
+// where mk[(y << msh) * mst + (x << msh)] != 0.  msh = level with the level-0 mask when every level halves exactly (the NN pyramid
+// then picks src(2y, 2x) at every step), 0 with a mask already resized to this level.
 __device__ __forceinline__ void dev_spread_lm(const uint8_t* __restrict__ q, const fl_level_geom& g, uint8_t* __restrict__ lm,
                                               uint8_t* __restrict__ spread_out, uint8_t* __restrict__ lm4, uint32_t* __restrict__ mass,
-                                              int bx, int by, uint8_t* smem, int cw) {
+                                              const uint8_t* __restrict__ mk, int mst, int msh, int bx, int by, uint8_t* smem, int cw) {
   const int T = TT > 0 ? TT : g.T;
   const int W = g.W, H = g.H, Wd = g.Wd;
   const int gy = by, cx0 = bx * cw;                     // cw <= SL_CW cells per CTA (fewer on small levels: more CTAs in flight)
@@ -260,6 +247,20 @@ __device__ __forceinline__ void dev_spread_lm(const uint8_t* __restrict__ q, con
       const int y = py0 + r;
       const uint8_t* src = q + (size_t)y * W + px0;
       for (int c = lane; c < st_in; c += 32) s_in[r * st_in + c] = (c < tw && px0 + c < W && y < H) ? __ldcg(src + c) : (uint8_t)0;   // clipped window == OR with zeros
+    }
+  }
+  if (mk) {                                             // (uniform over the grid) masked frame: labels under a zero mask byte become 0
+    __syncthreads();
+    const int nwi = st_in >> 2;
+    uint32_t* s_in32 = reinterpret_cast<uint32_t*>(s_in);
+    for (int i = tid; i < th * nwi; i += SL_THREADS) {
+      const int r = i / nwi, y = py0 + r, x = px0 + 4 * (i - r * nwi);
+      if (y >= H || x >= W) continue;                   // outside the image the tile is zero already
+      const uint8_t* mrow = mk + (size_t)(y << msh) * mst;
+      uint32_t mw = 0;
+      if (msh == 0 && x + 3 < W && ((reinterpret_cast<uintptr_t>(mrow) + x) & 3) == 0) mw = __ldg(reinterpret_cast<const uint32_t*>(mrow + x));
+      else for (int k = 0; k < 4 && x + k < W; ++k) mw |= (uint32_t)__ldg(mrow + ((x + k) << msh)) << (8 * k);
+      s_in32[i] &= __vcmpne4(mw, 0u);                   // SWAR: byte != 0 -> 0xFF
     }
   }
   __syncthreads();
@@ -341,27 +342,13 @@ __device__ __forceinline__ void dev_spread_lm(const uint8_t* __restrict__ q, con
   }
 }
 
-__device__ __forceinline__ void dev_spread_lm_any(const uint8_t* __restrict__ q, const fl_level_geom& g, uint8_t* __restrict__ lm,
-                                                  uint8_t* __restrict__ spread_out, uint8_t* __restrict__ lm4, uint32_t* __restrict__ mass,
-                                                  int bx, int by, uint8_t* smem, int cw) {
-  switch (g.T) {
-    case 5: dev_spread_lm<5>(q, g, lm, spread_out, lm4, mass, bx, by, smem, cw); break;
-    case 8: dev_spread_lm<8>(q, g, lm, spread_out, lm4, mass, bx, by, smem, cw); break;
-    case 4: dev_spread_lm<4>(q, g, lm, spread_out, lm4, mass, bx, by, smem, cw); break;
-    default: dev_spread_lm<0>(q, g, lm, spread_out, lm4, mass, bx, by, smem, cw); break;
+__device__ __forceinline__ void dev_spread_lm_any(const fl_fe_job& jb, int bx, int by, uint8_t* smem) {
+  switch (jb.g.T) {
+    case 5: dev_spread_lm<5>(jb.src, jb.g, jb.dst, jb.dst2, jb.dst3, jb.mass, jb.mask, jb.mask_stride, jb.mask_shift, bx, by, smem, jb.p0); break;
+    case 8: dev_spread_lm<8>(jb.src, jb.g, jb.dst, jb.dst2, jb.dst3, jb.mass, jb.mask, jb.mask_stride, jb.mask_shift, bx, by, smem, jb.p0); break;
+    case 4: dev_spread_lm<4>(jb.src, jb.g, jb.dst, jb.dst2, jb.dst3, jb.mass, jb.mask, jb.mask_stride, jb.mask_shift, bx, by, smem, jb.p0); break;
+    default: dev_spread_lm<0>(jb.src, jb.g, jb.dst, jb.dst2, jb.dst3, jb.mass, jb.mask, jb.mask_stride, jb.mask_shift, bx, by, smem, jb.p0); break;
   }
-}
-
-__global__ void __launch_bounds__(SL_THREADS) k_spread_lm(const uint8_t* __restrict__ q, fl_level_geom g, uint8_t* __restrict__ lm,
-                                                          uint8_t* __restrict__ spread_out, uint8_t* __restrict__ lm4, uint32_t* __restrict__ mass) {
-  extern __shared__ __align__(16) uint8_t smem_dyn[];
-  dev_spread_lm_any(q, g, lm, spread_out, lm4, mass, blockIdx.x, blockIdx.y, smem_dyn, SL_CW);
-}
-
-void fl_launch_spread_lm(const uint8_t* q, fl_level_geom g, uint8_t* lm_mod, uint8_t* spread_or_null, uint8_t* lm4_mod_or_null, uint32_t* mass_or_null,
-                         cudaStream_t s) {
-  dim3 grid((g.Wd + SL_CW - 1) / SL_CW, g.Hd);
-  k_spread_lm<<<grid, SL_THREADS, spread_smem_bytes(g.T), s>>>(q, g, lm_mod, spread_or_null, lm4_mod_or_null, mass_or_null);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -444,7 +431,7 @@ __global__ void __launch_bounds__(256, 8) k_front_end_wave(fl_fe_wave w) {
   switch (jb.kind) {
     case FL_JOB_PYRDOWN: dev_pyrdown_bgr(jb.src, jb.W, jb.H, jb.dst, local, jb.p0 != 0); break;
     case FL_JOB_RESIZE: dev_resize_nn_half(jb.src, jb.W, jb.H, jb.dst, local); break;
-    case FL_JOB_SPREAD: dev_spread_lm_any(jb.src, jb.g, jb.dst, jb.dst2, jb.dst3, jb.mass, local % jb.gx, local / jb.gx, smem_dyn, jb.p0); break;
+    case FL_JOB_SPREAD: dev_spread_lm_any(jb, local % jb.gx, local / jb.gx, smem_dyn); break;
     case FL_JOB_PREFETCH: {
       const size_t line = (size_t)local * 256 + threadIdx.x;
       if (line * 128 < (size_t)jb.W * 128) asm volatile("prefetch.global.L2 [%0];" ::"l"(jb.src + line * 128));
@@ -512,10 +499,11 @@ void fl_fe_add_resize(fl_fe_wave* w, const uint8_t* src, int W, int H, uint8_t* 
   j.cta_begin = w->n_ctas; w->n_ctas += ((W / 2) * (H / 2) + 255) / 256;
 }
 void fl_fe_add_spread(fl_fe_wave* w, const uint8_t* q, fl_level_geom g, uint8_t* lm_mod, uint8_t* spread_or_null, uint8_t* lm4_mod_or_null,
-                      uint32_t* mass_or_null) {
+                      uint32_t* mass_or_null, const uint8_t* mask_or_null, int mask_stride, int mask_shift) {
   fl_fe_job& j = w->job[w->n_jobs++];
   j.wait_slot = -1; j.signal_slot = -1; j.wait_target = 0; j.row_base = -1; j.wait_row_base = -1; j.wait_row_shift = 0; j.wait_row_count = 0; j.wait_row_target = 0;
   j.kind = FL_JOB_SPREAD; j.src = q; j.dst = lm_mod; j.dst2 = spread_or_null; j.dst3 = lm4_mod_or_null; j.mass = mass_or_null; j.g = g; j.W = g.W; j.H = g.H;
+  j.mask = mask_or_null; j.mask_stride = mask_stride; j.mask_shift = mask_shift;
   int cw = SL_CW;                                       // small levels: narrower CTAs so that the job still fills the SMs
   while (cw > 8 && ((g.Wd + cw - 1) / cw) * g.Hd < 148) cw >>= 1;
   j.p0 = cw;

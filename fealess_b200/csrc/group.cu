@@ -172,8 +172,11 @@ extern "C" int fl_group_upload_templates(fl_group* g, int32_t n_templates, const
 
 // Detector::match over the whole (sharded) set, on slot 0.  Host buffers in, merged host list out; every handle of the slot ends up
 // with the same list.
-extern "C" int fl_group_match(fl_group* g, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int32_t W, int32_t H,
-                              float threshold, const int32_t* class_filter, int32_t n_filter, fl_match_t* out, int32_t capacity, int32_t* count) {
+// masks (NULL or n_modalities host pointers, layout of fl_match) are staged into every member's own mask buffers (allocated at fl_create):
+// no member allocates between its peers' exchange launches.
+extern "C" int fl_group_match_masked(fl_group* g, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int32_t W, int32_t H,
+                                     const uint8_t* const* masks, float threshold, const int32_t* class_filter, int32_t n_filter, fl_match_t* out,
+                                     int32_t capacity, int32_t* count) {
   if (!g || !count || (!bgr && !depth)) return FL_ERR_ARG;
   *count = 0;
   if (in_flight(g)) { fl_set_error("fl_group_match: %d recognition frame(s) in flight - collect them first", in_flight(g)); return FL_ERR_STATE; }
@@ -188,8 +191,8 @@ extern "C" int fl_group_match(fl_group* g, const uint8_t* bgr, size_t bgr_stride
     int launched = 0;
     for (int i = 0; i < g->n; ++i) {                            // enqueue on every handle; nothing waits until all are under way
       GCUDA(cudaSetDevice(g->device[i]));
-      const int rc = fl_match_shard_exchange_async(g->h[i], bgr, bgr_stride, depth, depth_stride, W, H, threshold, class_filter, n_filter,
-                                                   i, g->n, g->peers.data(), g->cap, g->block[i].get(), e);
+      const int rc = fl_match_shard_exchange_masked_async(g->h[i], bgr, bgr_stride, depth, depth_stride, W, H, masks, threshold, class_filter, n_filter,
+                                                          i, g->n, g->peers.data(), g->cap, g->block[i].get(), e);
       if (rc != FL_OK) { first_err = rc; break; }                // (the ranks already launched report the missing peer instead of hanging)
       ++launched;
     }
@@ -206,6 +209,10 @@ extern "C" int fl_group_match(fl_group* g, const uint8_t* bgr, size_t bgr_stride
   }
   GCUDA(cudaSetDevice(g->device[0]));
   return fl_match_fetch(g->h[0], out, capacity, count);
+}
+extern "C" int fl_group_match(fl_group* g, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int32_t W, int32_t H,
+                              float threshold, const int32_t* class_filter, int32_t n_filter, fl_match_t* out, int32_t capacity, int32_t* count) {
+  return fl_group_match_masked(g, bgr, bgr_stride, depth, depth_stride, W, H, nullptr, threshold, class_filter, n_filter, out, capacity, count);
 }
 
 // ---- Recognition over the group -----------------------------------------------------------------------------------------------

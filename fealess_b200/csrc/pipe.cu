@@ -80,8 +80,8 @@ extern "C" int fl_pipe_set_exchange(fl_pipe* p, int32_t rank, int32_t world, int
   return FL_OK;
 }
 
-extern "C" int fl_pipe_submit(fl_pipe* p, const void* bgr, size_t bgr_stride, const void* depth, size_t depth_stride, int32_t W, int32_t H, float threshold,
-                              const int32_t* class_filter, int32_t n_filter, int32_t on_device) {
+extern "C" int fl_pipe_submit_masked(fl_pipe* p, const void* bgr, size_t bgr_stride, const void* depth, size_t depth_stride, int32_t W, int32_t H,
+                                     const void* const* masks, float threshold, const int32_t* class_filter, int32_t n_filter, int32_t on_device) {
   if (!p || (!bgr && !depth)) return FL_ERR_ARG;
   if (p->submitted - p->collected >= p->depth) { fl_set_error("fl_pipe_submit: %d frames in flight already - collect one first", p->depth); return FL_ERR_STATE; }
   const int slot = (int)(p->submitted % p->depth);
@@ -91,18 +91,25 @@ extern "C" int fl_pipe_submit(fl_pipe* p, const void* bgr, size_t bgr_stride, co
   if (p->world > 1) {                                           // template-sharded: local match + peer-memory exchange + merge, one enqueue
     void* const* peers = p->peers.data() + (size_t)slot * p->world;
     const uint32_t e = p->epoch[slot] + 1;
-    rc = on_device ? fl_match_shard_exchange_device_async(h, bgr, depth, W, H, threshold, class_filter, n_filter, p->rank, p->world, peers, p->xcap, p->blocks[slot], e)
-                   : fl_match_shard_exchange_async(h, static_cast<const uint8_t*>(bgr), bgr_stride, static_cast<const uint16_t*>(depth), depth_stride, W, H, threshold,
-                                                   class_filter, n_filter, p->rank, p->world, peers, p->xcap, p->blocks[slot], e);
+    rc = on_device ? fl_match_shard_exchange_device_masked_async(h, bgr, depth, W, H, masks, threshold, class_filter, n_filter, p->rank, p->world, peers, p->xcap,
+                                                                 p->blocks[slot], e)
+                   : fl_match_shard_exchange_masked_async(h, static_cast<const uint8_t*>(bgr), bgr_stride, static_cast<const uint16_t*>(depth), depth_stride, W, H,
+                                                          reinterpret_cast<const uint8_t* const*>(masks), threshold, class_filter, n_filter, p->rank, p->world,
+                                                          peers, p->xcap, p->blocks[slot], e);
     if (rc == FL_OK) p->epoch[slot] = e;
   } else if (on_device) {
-    rc = fl_match_device_async(h, bgr, depth, W, H, nullptr, threshold, class_filter, n_filter);
+    rc = fl_match_device_async(h, bgr, depth, W, H, masks, threshold, class_filter, n_filter);
   } else {
-    rc = fl_match_async(h, static_cast<const uint8_t*>(bgr), bgr_stride, static_cast<const uint16_t*>(depth), depth_stride, W, H, nullptr, threshold, class_filter, n_filter);
+    rc = fl_match_async(h, static_cast<const uint8_t*>(bgr), bgr_stride, static_cast<const uint16_t*>(depth), depth_stride, W, H,
+                        reinterpret_cast<const uint8_t* const*>(masks), threshold, class_filter, n_filter);
   }
   if (rc != FL_OK) return rc;
   ++p->submitted;
   return FL_OK;
+}
+extern "C" int fl_pipe_submit(fl_pipe* p, const void* bgr, size_t bgr_stride, const void* depth, size_t depth_stride, int32_t W, int32_t H, float threshold,
+                              const int32_t* class_filter, int32_t n_filter, int32_t on_device) {
+  return fl_pipe_submit_masked(p, bgr, bgr_stride, depth, depth_stride, W, H, nullptr, threshold, class_filter, n_filter, on_device);
 }
 
 extern "C" int fl_pipe_collect(fl_pipe* p, fl_match_t* out, int32_t capacity, int32_t* count) {

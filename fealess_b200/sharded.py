@@ -130,37 +130,38 @@ class ShardedMatcher:
             if int(ok.item()) == 0:
                 self.exchange = "nccl"
 
-    def match_device_async(self, d_bgr: int, d_depth: int, W: int, H: int, threshold: float) -> bool:
+    def match_device_async(self, d_bgr: int, d_depth: int, W: int, H: int, threshold: float, masks=None) -> bool:
         """One frame, enqueue only: the local match and (p2p exchange) the exchange + merge kernel go onto the handle's stream.
         Returns True when ``match_wait`` is all that is left (p2p); with the NCCL exchange the collective and the merge are
-        issued by ``match_wait``."""
+        issued by ``match_wait``.  ``masks``: None, or one device pointer (0 = unmasked) per modality, valid until ``match_wait``."""
         if self.world == 1:                                      # nothing to exchange: the plain three-launch frame
-            self.h.match_device_async(d_bgr, d_depth, W, H, threshold)
+            self.h.match_device_async(d_bgr, d_depth, W, H, threshold, masks=masks)
             return True
         if self.exchange == "p2p":
             # front end + matchClass, then ONE launch: refinement, push to the peers, wait, sort of the union
             self.epoch += 1
             self.h.match_shard_exchange_device_async(d_bgr, d_depth, W, H, threshold, self.rank, self.world, self._peers, self.cap,
-                                                     self._block_ptr, self.epoch)
+                                                     self._block_ptr, self.epoch, masks=masks)
             return True
         recs = records_view(self.block)
         # the count lives in the header record of the block, so the candidates + count travel together
-        self.h.match_shard_device(d_bgr, d_depth, W, H, threshold, recs.data_ptr(), self.cap, self.block.data_ptr())
+        self.h.match_shard_device(d_bgr, d_depth, W, H, threshold, recs.data_ptr(), self.cap, self.block.data_ptr(), masks=masks)
         return False
 
-    def match_host_async(self, bgr: np.ndarray, depth: np.ndarray, threshold: float) -> bool:
+    def match_host_async(self, bgr: np.ndarray, depth: np.ndarray, threshold: float, masks=None) -> bool:
         """``match_device_async`` for a frame in host memory: with the p2p exchange ONE C call uploads the frame and enqueues the
-        local match and the exchange (fl_match_shard_exchange_async); with the NCCL exchange the frame is copied into the rank's
-        device buffers first."""
+        local match and the exchange (fl_match_shard_exchange_masked_async); with the NCCL exchange the frame is copied into the rank's
+        device buffers first.  ``masks``: as in ``Handle.match`` (numpy arrays)."""
         H, W = depth.shape[:2]
         if self.world == 1:
             self._host_frame = (bgr, depth)
-            self.h.match_async(bgr, depth, threshold)
+            self.h.match_async(bgr, depth, threshold, masks=masks)
             return True
         if self.exchange == "p2p":
             self.epoch += 1
             self._host_frame = (bgr, depth)                     # page-locked buffers are read by DMA until match_wait
-            self.h.match_shard_exchange_async(bgr, depth, threshold, self.rank, self.world, self._peers, self.cap, self._block_ptr, self.epoch)
+            self.h.match_shard_exchange_async(bgr, depth, threshold, self.rank, self.world, self._peers, self.cap, self._block_ptr, self.epoch,
+                                              masks=masks)
             return True
         torch = self._torch
         if getattr(self, "_d_in", None) is None or self._d_in[0].numel() != H * W * 3:
@@ -171,8 +172,14 @@ class ShardedMatcher:
         cur = torch.cuda.current_stream()
         self._d_in[0].copy_(torch.from_numpy(bgr).view(-1), non_blocking=True)
         self._d_in[1].copy_(torch.from_numpy(depth.view(np.int16)).view(-1), non_blocking=True)
+        d_masks = None
+        if masks:
+            from . import host_masks
+            _, keep = host_masks(masks, self.h.M, W, H)
+            self._d_masks = [None if k is None else torch.from_numpy(k).to(self.block.device, non_blocking=True) for k in keep]
+            d_masks = [0 if t is None else t.data_ptr() for t in self._d_masks]
         self.stream.wait_stream(cur)
-        return self.match_device_async(self._d_in[0].data_ptr(), self._d_in[1].data_ptr(), W, H, threshold)
+        return self.match_device_async(self._d_in[0].data_ptr(), self._d_in[1].data_ptr(), W, H, threshold, masks=d_masks)
 
     def match_wait(self) -> None:
         torch = self._torch
@@ -202,7 +209,7 @@ class ShardedMatcher:
             return
         self._torch.cuda.synchronize()
         self.block = self.gathered = None
-        self._d_in = None
+        self._d_in = self._d_masks = None
         self._host_frame = None
         self._xhdl = None
         self._xbuf = None
@@ -238,14 +245,14 @@ class ShardedPipe:
         self.submitted += 1
         return s
 
-    def submit_device(self, d_bgr: int, d_depth: int, W: int, H: int, threshold: float) -> "ShardedMatcher":
+    def submit_device(self, d_bgr: int, d_depth: int, W: int, H: int, threshold: float, masks=None) -> "ShardedMatcher":
         s = self._next_slot()
-        s.match_device_async(d_bgr, d_depth, W, H, threshold)
+        s.match_device_async(d_bgr, d_depth, W, H, threshold, masks=masks)
         return s
 
-    def submit_host(self, bgr: np.ndarray, depth: np.ndarray, threshold: float) -> "ShardedMatcher":
+    def submit_host(self, bgr: np.ndarray, depth: np.ndarray, threshold: float, masks=None) -> "ShardedMatcher":
         s = self._next_slot()
-        s.match_host_async(bgr, depth, threshold)
+        s.match_host_async(bgr, depth, threshold, masks=masks)
         return s
 
     def collect(self) -> "ShardedMatcher":

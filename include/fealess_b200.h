@@ -142,7 +142,8 @@ int fl_add_template(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const u
  * Host buffers in, host matches out (sorted by the canonical total order, duplicates pruned).
  * bgr: 8UC3 rows of bgr_stride bytes; depth: 16UC1 rows of depth_stride bytes (mm); either may be NULL if no
  * modality of that kind is configured.  masks: NULL or n_modalities pointers (each NULL or W*H dense u8, nonzero =
- * keep).  class_filter: NULL/0 = all classes.  quantized_out: NULL or n_levels*n_modalities host pointers
+ * keep; a masked frame runs the same launches as an unmasked one, and the handle allocates nothing for it: the level-0 masks are
+ * staged in buffers sized at fl_create, (max_width * max_height * 4 / 3) * n_modalities bytes).  class_filter: NULL/0 = all classes.  quantized_out: NULL or n_levels*n_modalities host pointers
  * (index level*n_modalities + modality) receiving the quantised images, each (W>>l)*(H>>l) bytes.
  * *count = number of matches found (may exceed capacity -> FL_ERR_CAPACITY, first `capacity` are written). */
 int fl_match(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
@@ -151,7 +152,7 @@ int fl_match(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t
              fl_match_t* out, int32_t capacity, int32_t* count, uint8_t* const* quantized_out);
 
 /* Same computation with the frame already resident in device memory (dense rows).  d_masks as above but device
- * pointers.  Results stay on the device; fl_match_fetch copies them out (and synchronises). */
+ * pointers (valid until fl_match_wait; fl_debug_get(FL_DBG_QUANTIZED) of such a frame reads them again).  Results stay on the device; fl_match_fetch copies them out (and synchronises). */
 int fl_match_device(fl_handle* h, const void* d_bgr, const void* d_depth, int32_t W, int32_t H,
                     const void* const* d_masks, float threshold, const int32_t* class_filter, int32_t n_filter);
 int fl_match_fetch(fl_handle* h, fl_match_t* out, int32_t capacity, int32_t* count);
@@ -179,7 +180,10 @@ int fl_match_async(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const ui
  * copy of frame i-1 overlap the similarity kernel of frame i.  Lists come back in submission order and equal fl_match's.
  * fl_pipe_submit: FL_ERR_STATE when `depth` frames are in flight already.  on_device != 0: bgr / depth are device pointers with
  * dense rows (the strides must say so); otherwise host pointers as in fl_match_async (page-locked buffers must stay valid until the
- * frame has been collected).  fl_pipe_collect: waits for the OLDEST frame in flight and writes its list (status as fl_match_fetch).
+ * frame has been collected).  fl_pipe_submit_masked: the same with masks (layout of fl_match: NULL or n_modalities pointers, each NULL
+ * or a dense W*H u8 image, nonzero = keep), in device memory when on_device != 0, else host memory (copied before the call returns);
+ * a masked frame takes the same launches as an unmasked one, on plain and on template-sharded pipes.  fl_pipe_submit = masks NULL.
+ * fl_pipe_collect: waits for the OLDEST frame in flight and writes its list (status as fl_match_fetch).
  * fl_pipe_match_batch: n_frames frames of one geometry (arrays of n_frames pointers), frame f's list at out + f *
  * capacity_per_frame and its length in counts[f]; FL_ERR_CAPACITY if some list was truncated. */
 typedef struct fl_pipe fl_pipe;
@@ -200,6 +204,8 @@ int fl_pipe_set_exchange(fl_pipe* p, int32_t rank, int32_t world, int32_t exchan
                          fl_match_t* const* local_blocks);
 int fl_pipe_submit(fl_pipe* p, const void* bgr, size_t bgr_stride, const void* depth, size_t depth_stride, int32_t W, int32_t H,
                    float threshold, const int32_t* class_filter, int32_t n_filter, int32_t on_device);
+int fl_pipe_submit_masked(fl_pipe* p, const void* bgr, size_t bgr_stride, const void* depth, size_t depth_stride, int32_t W, int32_t H,
+                          const void* const* masks, float threshold, const int32_t* class_filter, int32_t n_filter, int32_t on_device);
 int fl_pipe_collect(fl_pipe* p, fl_match_t* out, int32_t capacity, int32_t* count);
 int fl_pipe_match_batch(fl_pipe* p, int32_t n_frames, const void* const* bgr, size_t bgr_stride, const void* const* depth, size_t depth_stride,
                         int32_t W, int32_t H, float threshold, const int32_t* class_filter, int32_t n_filter, int32_t on_device,
@@ -240,11 +246,21 @@ int fl_exchange_sort_unique_device(fl_handle* h, int32_t rank, int32_t world, vo
 int fl_match_shard_exchange_device_async(fl_handle* h, const void* d_bgr, const void* d_depth, int32_t W, int32_t H, float threshold,
                                          const int32_t* class_filter, int32_t n_filter, int32_t rank, int32_t world,
                                          void* const* peer_buffers, int32_t capacity, fl_match_t* d_local_block, uint32_t epoch);
+/* the same with masks in device memory (d_masks as in fl_match_device; the call above = d_masks NULL) */
+int fl_match_shard_exchange_device_masked_async(fl_handle* h, const void* d_bgr, const void* d_depth, int32_t W, int32_t H,
+                                                const void* const* d_masks, float threshold, const int32_t* class_filter, int32_t n_filter,
+                                                int32_t rank, int32_t world, void* const* peer_buffers, int32_t capacity,
+                                                fl_match_t* d_local_block, uint32_t epoch);
 /* the same with the frame in HOST memory (buffers as in fl_match_async): upload + local match + exchange in one call, so that a
  * rank's per-frame host work is this call, fl_match_wait and fl_match_fetch */
 int fl_match_shard_exchange_async(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int32_t W, int32_t H,
                                   float threshold, const int32_t* class_filter, int32_t n_filter, int32_t rank, int32_t world,
                                   void* const* peer_buffers, int32_t capacity, fl_match_t* d_local_block, uint32_t epoch);
+/* the same with host masks (masks as in fl_match; the call above = masks NULL) */
+int fl_match_shard_exchange_masked_async(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
+                                         int32_t W, int32_t H, const uint8_t* const* masks, float threshold, const int32_t* class_filter,
+                                         int32_t n_filter, int32_t rank, int32_t world, void* const* peer_buffers, int32_t capacity,
+                                         fl_match_t* d_local_block, uint32_t epoch);
 /* enqueue-only half; finish with fl_match_wait */
 int fl_exchange_sort_unique_device_async(fl_handle* h, int32_t rank, int32_t world, void* const* peer_buffers, int32_t capacity,
                                          const fl_match_t* d_local_block, uint32_t epoch);
@@ -273,6 +289,10 @@ int fl_group_upload_templates(fl_group* g, int32_t n_templates, const fl_templat
 /* FL_ERR_STATE while recognition frames are in flight */
 int fl_group_match(fl_group* g, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int32_t W, int32_t H,
                    float threshold, const int32_t* class_filter, int32_t n_filter, fl_match_t* out, int32_t capacity, int32_t* count);
+/* the same with host masks (masks as in fl_match; fl_group_match = masks NULL); the merged list equals a single handle's fl_match */
+int fl_group_match_masked(fl_group* g, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int32_t W, int32_t H,
+                          const uint8_t* const* masks, float threshold, const int32_t* class_filter, int32_t n_filter, fl_match_t* out,
+                          int32_t capacity, int32_t* count);
 
 /* ---- input rescale (the caller's PrepareInputData) ------------------------------------------------- */
 enum { FL_IMG_8UC3 = 0, FL_IMG_16UC1 = 1 };

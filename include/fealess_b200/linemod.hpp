@@ -103,7 +103,7 @@ class Detector {
 
   // NOT in the reference: spread match() over several GPUs of this process.  The templates are dealt round-robin over one handle per
   // entry of `devices` (fl_group_*: peer-memory candidate exchange inside the sort kernel, no NCCL / Python involved); match() returns
-  // the same list as on one GPU.  exchange_capacity = candidates one GPU may emit per frame.  Masks are not supported in this mode.
+  // the same list as on one GPU, masks and quantized_images included.  exchange_capacity = candidates one GPU may emit per frame.
   void useDevices(const std::vector<int>& devices, int exchange_capacity = 2048) {
     release_device();
     devices_ = devices; xcap_ = exchange_capacity; dirty_ = true; cap_w_ = cap_h_ = 0;
@@ -148,7 +148,6 @@ class Detector {
       for (int y = 0; y < H; ++y) std::memcpy(&mask_store[m][(size_t)y * W], k.ptr<uint8_t>(y), (size_t)W);
       mask_ptr[m] = mask_store[m].data(); any_mask = true;
     }
-    if (any_mask && devices_.size() > 1) throw cv::Exception("Detector::match: masks are not supported together with useDevices()");
     ensure_uploaded(W, H);
     // class filter: ids the detector does not know are ignored (:1425-1433)
     std::vector<int32_t> filter;
@@ -170,11 +169,12 @@ class Detector {
     int32_t count = 0;
     int rc;
     if (group_) {                                                            // template-sharded over the GPUs of useDevices()
-      rc = fl_group_match(group_, bgr, bgr_step, depth, depth_step, W, H, threshold, filter.empty() ? nullptr : filter.data(), (int32_t)filter.size(),
-                          out.data(), (int32_t)out.size(), &count);
+      rc = fl_group_match_masked(group_, bgr, bgr_step, depth, depth_step, W, H, any_mask ? mask_ptr.data() : nullptr, threshold,
+                                 filter.empty() ? nullptr : filter.data(), (int32_t)filter.size(), out.data(), (int32_t)out.size(), &count);
       if (quantized_images.needed() && (rc == FL_OK || rc == FL_ERR_CAPACITY)) {   // the front end alone, on the first GPU
         const int32_t none = -1; fl_match_t dummy; int32_t c2 = 0;
-        fealess_b200::check_status(fl_match(handle_, bgr, bgr_step, depth, depth_step, W, H, nullptr, 100.0f, &none, 1, &dummy, 1, &c2, qptr.data()), "Detector::match");
+        fealess_b200::check_status(fl_match(handle_, bgr, bgr_step, depth, depth_step, W, H, any_mask ? mask_ptr.data() : nullptr, 100.0f, &none, 1, &dummy, 1,
+                                            &c2, qptr.data()), "Detector::match");
       }
     } else
     rc = fl_match(handle_, bgr, bgr_step, depth, depth_step, W, H, any_mask ? mask_ptr.data() : nullptr, threshold,
