@@ -60,6 +60,7 @@ EXPORTED_SYMBOLS = [
     "fl_group_create_pipe", "fl_group_depth", "fl_group_in_flight", "fl_group_upload_model_depths", "fl_group_set_recognition",
     "fl_group_submit_recognition", "fl_group_collect_recognition", "fl_group_recognize",
     "fl_pipe_submit_masked", "fl_group_match_masked", "fl_match_shard_exchange_masked_async", "fl_match_shard_exchange_device_masked_async",
+    "fl_pipe_set_recognition_sharded",
 ]
 
 
@@ -913,6 +914,16 @@ class Pipe:
         crop = np.ascontiguousarray(crop_of_template, np.int32)
         pose = None if pose12 is None else np.ascontiguousarray(pose12, np.float32).reshape(-1, 12)
         _check(lib().fl_pipe_set_recognition(self._p, C.byref(params or reco_params()), _p(crop), _p(pose)), "fl_pipe_set_recognition")
+
+    def set_recognition_sharded(self, tset, crop_of_template, pose12=None, params: Optional[RecoParams] = None) -> None:
+        """fl_pipe_set_recognition_sharded (a template-sharded pipe): ``tset`` = the WHOLE set the shards were cut from, crop index and
+        pose of every template of it (order of the set; pose12 None = the first 12 floats of the set's pose13)."""
+        hdr = np.ascontiguousarray(tset.headers, np.int32)
+        co = np.ascontiguousarray(tset.class_of, np.int32)
+        crop = np.ascontiguousarray(crop_of_template, np.int32)
+        pose = np.ascontiguousarray(np.asarray(tset.pose13, np.float32).reshape(-1, 13)[:, :12] if pose12 is None else pose12, np.float32).reshape(-1, 12)
+        _check(lib().fl_pipe_set_recognition_sharded(self._p, C.byref(params or reco_params()), int(tset.n_templates), _p(hdr), _p(co), _p(crop), _p(pose)),
+               "fl_pipe_set_recognition_sharded")
 
     def submit_recognition(self, bgr, depth, K, W: Optional[int] = None, H: Optional[int] = None) -> None:
         """fl_pipe_submit_recognition (host frame; page-locked arrays are read by DMA while in flight, so they are kept referenced)."""

@@ -1089,7 +1089,7 @@ extern "C" int fl_sort_unique_device(fl_handle* h, const fl_match_t* d_in, int32
 
 extern "C" size_t fl_exchange_buffer_bytes(int32_t world, int32_t capacity) {
   if (world < 1 || capacity < 1) return 0;
-  return FL_XCHG_SIGNALS * sizeof(unsigned) + (size_t)2 * world * ((size_t)capacity + 1) * sizeof(fl_match_t);
+  return fl_reco_mailbox_offset(world, capacity) + FL_RECO_MAILBOX_WORDS * sizeof(int);   // blocks, then the result mailbox (fl_internal.cuh)
 }
 
 extern "C" int fl_exchange_sort_unique_device_async(fl_handle* h, int32_t rank, int32_t world, void* const* peer_buffers, int32_t capacity,
@@ -1684,8 +1684,9 @@ extern "C" int fl_set_recognition(fl_handle* h, const fl_reco_params_t* prm, con
 }
 
 // selection -> ICP -> finish on the sorted list in d_out.  check_big: the list came from the fused refinement + sort, which leaves
-// lists of more than 1,024 records unsorted and flagged (k_reco_select then selects nothing and reports the frame deferred)
-static int reco_enqueue(fl_handle* h, bool check_big) {
+// lists of more than 1,024 records unsorted and flagged (k_reco_select then selects nothing and reports the frame deferred).  push: the
+// other ranks' mailboxes of a template-sharded pipe's frame that this handle owns, or NULL
+static int reco_enqueue(fl_handle* h, bool check_big, const fl_reco_push* push = nullptr) {
   cudaStream_t s = h->stream.get();
   const int max_hyp = h->reco_max_hyp;
   int nl = fl_launch_reco_select(h->d_out, reinterpret_cast<const int*>(h->d_outblk.get()), h->p.max_candidates, check_big ? 1 : 0, h->d_reco_class_first.get(),
@@ -1698,7 +1699,7 @@ static int reco_enqueue(fl_handle* h, bool check_big) {
   nl = fl_launch_icp(ws, h->reco.icp, h->icpw.d_hyps.get(), h->d_in_depth.get(), h->reco_W, h->reco_H, h->reco_K, h->icpw.d_results.get(), h->icpw.d_ticket.get(), nullptr, h->n_sm, s);
   if (nl < 0) { fl_set_error("ICP kernel launch failed: %s", cudaGetErrorString(cudaGetLastError())); return FL_ERR_CUDA; }
   h->launches += nl;
-  nl = fl_launch_reco_finish(h->d_out, h->d_reco_sel.get(), h->icpw.d_results.get(), max_hyp, h->reco.th_obj_dist, h->d_reco_host, s);
+  nl = fl_launch_reco_finish(h->d_out, h->d_reco_sel.get(), h->icpw.d_results.get(), max_hyp, h->reco.th_obj_dist, h->d_reco_host, push, s);
   if (nl < 0) { fl_set_error("recognition finish launch failed: %s", cudaGetErrorString(cudaGetLastError())); return FL_ERR_CUDA; }
   h->launches += nl;
   return FL_OK;
@@ -1764,19 +1765,39 @@ int fl_reco_shard_match(fl_handle* h, int rank, int world, void* const* peers, i
   return FL_OK;
 }
 
-int fl_reco_shard_tail(fl_handle* h) {
+int fl_reco_shard_tail(fl_handle* h, const fl_reco_push* push) {
   if (!h) return FL_ERR_ARG;
   if (!h->pend_sort || !h->reco_set) { fl_set_error("no matched recognition frame on this handle"); return FL_ERR_STATE; }
   FL_CUDA(cudaSetDevice(h->p.device));
-  TRY(reco_enqueue(h, true));
+  TRY(reco_enqueue(h, true, push));
   h->pend_reco = true;
   return FL_OK;
+}
+
+int fl_reco_shard_receive(fl_handle* h, const uint8_t* own_buffer, size_t mailbox_off, uint32_t epoch, int owner) {
+  if (!h || !own_buffer) return FL_ERR_ARG;
+  if (!h->pend_sort || !h->reco_set) { fl_set_error("no matched recognition frame on this handle"); return FL_ERR_STATE; }
+  FL_CUDA(cudaSetDevice(h->p.device));
+  if (fl_launch_reco_receive(own_buffer, mailbox_off, epoch, owner, h->d_reco_host, h->stream.get()) < 0) {
+    fl_set_error("recognition receive launch failed: %s", cudaGetErrorString(cudaGetLastError())); return FL_ERR_CUDA;
+  }
+  ++h->launches;
+  h->pend_reco = true;
+  return FL_OK;
+}
+
+int fl_reco_shard_preload(fl_handle* h) {
+  if (!h || !h->reco_set) return FL_ERR_STATE;
+  FL_CUDA(cudaSetDevice(h->p.device));
+  TRY(fl_reco_preload());
+  return fl_icp_preload(h->icp.max_pts);
 }
 
 // after the frame's match wait: the tail once more on the final list when the selection ran on a list that was not sorted yet (or on a
 // frame that has been re-run since), then the results and the summary
 static int reco_results(fl_handle* h, bool rerun, fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary) {
   const volatile int* blk = h->h_reco.get();
+  if (blk[FL_RECO_MISSING_OWNER]) { fl_set_error("owner rank %d did not post its results", blk[FL_RECO_MISSING_OWNER] - 1); return FL_ERR_STATE; }
   if ((blk[4] & FL_RECO_DEFERRED) || rerun) {
     TRY(reco_enqueue(h, false));
     FL_CUDA(wait_stream(h));

@@ -185,6 +185,10 @@ struct fl_lists { const fl_match_t* in; int n_lists, list_cap, list_stride; cons
 #define FL_XCHG_MAX_WORLD 8
 #define FL_XCHG_SIGNALS 64
 struct fl_xchg { int world, rank, cap; unsigned epoch; const fl_match_t* local_block; uint8_t* peer[FL_XCHG_MAX_WORLD]; };
+#ifdef __CUDACC__
+__device__ __forceinline__ void st_release_sys(unsigned* p, unsigned v) { asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
+__device__ __forceinline__ unsigned ld_acquire_sys(const unsigned* p) { unsigned v; asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory"); return v; }
+#endif
 
 // sort + unique: result in d_out/d_out_count, summary in d_hdr[16] = {unique count, live records, flag_big, raw counts...}.
 // One launch; when flag_big comes back set the host runs fl_launch_sort_unique_big (key workspace: next_pow2(n_upper) keys
@@ -272,9 +276,33 @@ struct fl_reco_tmpl { const uint16_t* crop; fl_rect_t rect; float pose[12]; };
 int fl_launch_reco_select(const fl_match_t* matches, const int* d_hdr, int out_cap, int check_big, const int32_t* class_first, int n_classes,
                           int n_templates, const fl_reco_tmpl* tmpl, int top_k, int per_class, int max_hyp, int W, int H,
                           fl_icp_hyp* hyps, int* sel, cudaStream_t s);
-// objects that came out of ICP -> [NMS] -> fl_reco_result_t records + summary posted to mapped host memory (host_block)
+// summary word a rank that does not own a frame of a template-sharded pipe sets to 1 + owner when the owner's results never arrived
+#define FL_RECO_MISSING_OWNER 5
+// Result mailbox of a template-sharded pipe (fl_pipe_set_recognition_sharded): FL_RECO_MAILBOX_WORDS words at the end of every exchange
+// buffer (behind the candidate blocks, fl_exchange_buffer_bytes), and its signal, one of the signal words the candidate exchange leaves
+// unused (it takes words 0 .. world - 1).  A frame's owner writes [summary | records] into the mailbox of every other rank, fences, and
+// publishes the slot's exchange epoch in the signal (system-scope release); k_reco_receive acquire-waits for that epoch.
+// One mailbox per slot is enough: a rank's receive of epoch e runs on the slot's stream before its exchange launch of e + 1, and the
+// owner of e + 1 pushes only after its own exchange has seen every rank publish e + 1 - so no push overwrites a mailbox not yet read.
+#define FL_RECO_MAILBOX_WORDS (FL_RECO_SUMMARY_WORDS + FL_RECO_MAX_HYP * (int)(sizeof(fl_reco_result_t) / 4))
+#define FL_XCHG_RECO_SIGNAL (FL_XCHG_SIGNALS - 1)
+inline size_t fl_reco_mailbox_offset(int world, int capacity) {
+  return FL_XCHG_SIGNALS * sizeof(unsigned) + (size_t)2 * world * ((size_t)capacity + 1) * sizeof(fl_match_t);
+}
+// the owner's push: exchange buffers (as mapped into this process) of the n ranks that do not own the frame, and the frame's epoch
+struct fl_reco_push { int n; unsigned epoch; size_t mailbox_off; uint8_t* peer[FL_XCHG_MAX_WORLD]; };
+// objects that came out of ICP -> [NMS] -> fl_reco_result_t records + summary posted to mapped host memory (host_block), and with
+// push != NULL (push->n > 0) into the mailbox of every rank listed there
 int fl_launch_reco_finish(const fl_match_t* matches, const int* sel, const fl_icp_result_t* results, int max_hyp, float th_obj_dist,
-                          int* host_block, cudaStream_t s);
+                          int* host_block, const fl_reco_push* push, cudaStream_t s);
+// a rank that does not own the frame: wait (bounded, ~2 s) for `epoch` in its own buffer's mailbox signal, then copy the mailbox into
+// host_block; on time-out host_block gets an empty summary with word FL_RECO_MISSING_OWNER = 1 + owner
+int fl_launch_reco_receive(const uint8_t* own_buffer, size_t mailbox_off, unsigned epoch, int owner, int* host_block, cudaStream_t s);
+// load the kernels of the recognition tail and of the receive on the current device now (fl_icp_preload: k_icp_fused, with its
+// shared-memory opt-in for max_pts points): a first launch under lazy module loading may wait for the device, where an exchange kernel
+// can be spinning until this rank's peers arrive
+int fl_reco_preload();
+int fl_icp_preload(int max_pts);
 // the template set a recognition set-up covers, in upload order: class, level-0 modality-0 box and pose13 (nullable) of every template.
 // fl_set_recognition passes the handle's own upload, fl_group_set_recognition the whole set of a template-sharded group (api.cu).
 struct fl_reco_set { int n_templates; const int32_t* class_of; const fl_rect_t* box0; const float* pose13; };
@@ -286,5 +314,10 @@ int fl_reco_setup(fl_handle* h, const fl_reco_params_t* prm, const fl_reco_set& 
 int fl_reco_shard_stage(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int src_W, int src_H, int W, int H,
                         fl_intrinsics_t K_ref);
 int fl_reco_shard_match(fl_handle* h, int rank, int world, void* const* peers, int capacity, fl_match_t* block, uint32_t epoch);
-int fl_reco_shard_tail(fl_handle* h);
+int fl_reco_shard_tail(fl_handle* h, const fl_reco_push* push = nullptr);
 int fl_reco_shard_results(fl_handle* h, fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary);
+// a template-sharded pipe's rank that does not own the frame: k_reco_receive in place of the tail (own_buffer: this rank's exchange
+// buffer of the slot); fl_reco_shard_results then reads what the owner posted, or runs the tail itself on a deferred list
+int fl_reco_shard_receive(fl_handle* h, const uint8_t* own_buffer, size_t mailbox_off, uint32_t epoch, int owner);
+// after fl_reco_setup on a handle of a template-sharded pipe: every kernel the handle's recognition frames launch is loaded
+int fl_reco_shard_preload(fl_handle* h);

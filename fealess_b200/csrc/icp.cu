@@ -847,24 +847,37 @@ static int icp_smem_plan(int max_pts, int* smem_pts) {
   return fixed + *smem_pts * 16;
 }
 
+// the shared-memory opt-in of k_icp_fused on the current device, for a launch with `smem` dynamic bytes
+static cudaError_t icp_opt_in(int smem) {
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e != cudaSuccess) return e;
+  if (dev < 0 || dev >= FL_MAX_DEVICES) return cudaErrorInvalidDevice;
+  static std::mutex mu;                                             // the opt-in belongs to the (device, function) pair
+  static int configured[FL_MAX_DEVICES];
+  std::lock_guard<std::mutex> lk(mu);
+  if (smem > configured[dev]) {
+    if ((e = cudaFuncSetAttribute(k_icp_fused, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)) != cudaSuccess) return e;
+    configured[dev] = smem;
+  }
+  return cudaSuccess;
+}
+
+int fl_icp_preload(int max_pts) {
+  int smem_pts = 0;
+  cudaFuncAttributes a;
+  FL_CUDA(cudaFuncGetAttributes(&a, k_icp_fused));
+  FL_CUDA(icp_opt_in(icp_smem_plan(max_pts, &smem_pts)));
+  return FL_OK;
+}
+
 int fl_launch_icp(fl_icp_ws ws, fl_icp_params_t p, const fl_icp_hyp* hyps_or_null, const uint16_t* ref_depth, int W, int H, fl_intrinsics_t K_ref,
                   fl_icp_result_t* results, int* ticket, unsigned long long* trace, int n_sm, cudaStream_t s) {
   if (ws.n_hyp <= 0) return 0;
   fl_icp_args A;
   A.ws = ws; A.prm = p; A.hyps = hyps_or_null; A.ref_depth = ref_depth; A.W = W; A.H = H; A.Kr = K_ref; A.results = results; A.ticket = ticket; A.trace = trace;
   const int smem = icp_smem_plan(ws.max_pts, &A.smem_pts);
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) return -1;
-  if (dev < 0 || dev >= FL_MAX_DEVICES) return -1;
-  {   // the opt-in belongs to the (device, function) pair
-    static std::mutex mu;
-    static int configured[FL_MAX_DEVICES];
-    std::lock_guard<std::mutex> lk(mu);
-    if (smem > configured[dev]) {
-      if (cudaFuncSetAttribute(k_icp_fused, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return -1;
-      configured[dev] = smem;
-    }
-  }
+  if (icp_opt_in(smem) != cudaSuccess) return -1;
   if (cudaMemsetAsync(ticket, 0, sizeof(int), s) != cudaSuccess) return -1;
   k_icp_fused<<<min(ws.n_hyp, n_sm), ICP_NT, smem, s>>>(A);
   return cudaGetLastError() == cudaSuccess ? 1 : -1;

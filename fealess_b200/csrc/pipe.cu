@@ -9,7 +9,9 @@
 // frame i+1 and the result copy of frame i-1 ride on the copy engines meanwhile.  Nothing here synchronises more than one stream.
 // fl_pipe_set_exchange turns the pipe into ONE RANK of a template-sharded detector: every slot then runs the fused local match +
 // peer-memory exchange (fl_match_shard_exchange_*) with its own exchange buffers and epoch sequence, so a rank's whole per-frame host
-// loop - upload, enqueue, wait, fetch - lives in fl_pipe_match_batch.
+// loop - upload, enqueue, wait, fetch - lives in fl_pipe_match_batch.  Recognition on such a pipe (fl_pipe_set_recognition_sharded):
+// every rank matches its shard and takes part in the exchange, only the frame's owner (rank f % world) runs selection, ICP and
+// suppression, and its k_reco_finish pushes the results into the other ranks' mailboxes, where their k_reco_receive picks them up.
 #include "fl_internal.cuh"
 #include <vector>
 
@@ -23,6 +25,7 @@ struct fl_pipe {
   std::vector<void*> peers;
   std::vector<fl_match_t*> blocks;
   std::vector<uint32_t> epoch;
+  bool reco_sharded = false;        // fl_pipe_set_recognition_sharded has set up every slot
 };
 
 extern "C" int fl_pipe_destroy(fl_pipe* p) {
@@ -54,6 +57,7 @@ extern "C" int fl_pipe_upload_templates(fl_pipe* p, int32_t n_templates, const f
                                         const int32_t* class_of, const float* pose13) {
   if (!p) return FL_ERR_ARG;
   if (p->submitted != p->collected) { fl_set_error("fl_pipe_upload_templates: %lld frame(s) still in flight", p->submitted - p->collected); return FL_ERR_STATE; }
+  p->reco_sharded = false;
   for (fl_handle* h : p->h) {
     const int rc = fl_upload_templates(h, n_templates, headers, features, n_features, class_of, pose13);
     if (rc != FL_OK) return rc;
@@ -73,7 +77,7 @@ extern "C" int fl_pipe_set_exchange(fl_pipe* p, int32_t rank, int32_t world, int
     if (!local_blocks[i]) return FL_ERR_ARG;
     for (int r = 0; r < world; ++r) if (!peer_buffers[(size_t)i * world + r]) return FL_ERR_ARG;
   }
-  p->rank = rank; p->world = world; p->xcap = exchange_capacity;
+  p->rank = rank; p->world = world; p->xcap = exchange_capacity; p->reco_sharded = false;
   p->peers.assign(peer_buffers, peer_buffers + (size_t)p->depth * world);
   p->blocks.assign(local_blocks, local_blocks + p->depth);
   p->epoch.assign(p->depth, 0u);
@@ -152,6 +156,7 @@ extern "C" int fl_pipe_upload_model_depths(fl_pipe* p, int32_t n_models, const u
                                            const fl_rect_t* rect_model, int32_t W, int32_t H) {
   if (!p) return FL_ERR_ARG;
   if (p->submitted != p->collected) { fl_set_error("fl_pipe_upload_model_depths: %lld frame(s) still in flight", p->submitted - p->collected); return FL_ERR_STATE; }
+  p->reco_sharded = false;
   for (fl_handle* h : p->h) {
     const int rc = fl_upload_model_depths(h, n_models, model_depth, model_stride, rect_model, W, H);
     if (rc != FL_OK) return rc;
@@ -161,7 +166,7 @@ extern "C" int fl_pipe_upload_model_depths(fl_pipe* p, int32_t n_models, const u
 
 extern "C" int fl_pipe_set_recognition(fl_pipe* p, const fl_reco_params_t* params, const int32_t* crop_of_template, const float* pose12) {
   if (!p) return FL_ERR_ARG;
-  if (p->world > 1) { fl_set_error("fl_pipe_set_recognition: not available on a template-sharded pipe"); return FL_ERR_STATE; }
+  if (p->world > 1) { fl_set_error("fl_pipe_set_recognition: a template-sharded pipe takes fl_pipe_set_recognition_sharded"); return FL_ERR_STATE; }
   if (p->submitted != p->collected) { fl_set_error("fl_pipe_set_recognition: %lld frame(s) still in flight", p->submitted - p->collected); return FL_ERR_STATE; }
   for (fl_handle* h : p->h) {
     const int rc = fl_set_recognition(h, params, crop_of_template, pose12);
@@ -170,12 +175,63 @@ extern "C" int fl_pipe_set_recognition(fl_pipe* p, const fl_reco_params_t* param
   return FL_OK;
 }
 
+// Recognition on a template-sharded pipe.  Every slot's handle gets the selection table of the WHOLE set (the ranks hold only their
+// shards), and every kernel its frames launch is loaded here: after a rank's exchange launch nothing may wait for the device, since
+// the exchange kernel spins until the peers arrive (group.cu explains the same hazard for a group).
+extern "C" int fl_pipe_set_recognition_sharded(fl_pipe* p, const fl_reco_params_t* params, int32_t n_templates, const fl_template_hdr_t* headers,
+                                               const int32_t* class_of, const int32_t* crop_of_template, const float* pose12) {
+  if (!p || !params || n_templates < 0 || (n_templates > 0 && (!headers || !class_of)) || !crop_of_template || !pose12) return FL_ERR_ARG;
+  if (p->world <= 1) { fl_set_error("fl_pipe_set_recognition_sharded: not a template-sharded pipe (fl_pipe_set_exchange, world > 1)"); return FL_ERR_STATE; }
+  if (p->submitted != p->collected) { fl_set_error("fl_pipe_set_recognition_sharded: %lld frame(s) still in flight", p->submitted - p->collected); return FL_ERR_STATE; }
+  p->reco_sharded = false;
+  const int LM = fl_entries_per_template(p->h[0]);                 // level-0 modality-0 box of every template (current_template[0], :111)
+  std::vector<fl_rect_t> box0((size_t)n_templates);
+  for (int t = 0; t < n_templates; ++t) { const fl_template_hdr_t& b = headers[(size_t)t * LM]; box0[t] = {b.offset_x, b.offset_y, b.width, b.height}; }
+  const fl_reco_set set = {n_templates, class_of, box0.data(), nullptr};
+  for (fl_handle* h : p->h) {
+    int rc = fl_reco_setup(h, params, set, crop_of_template, pose12);
+    if (rc == FL_OK) rc = fl_reco_shard_preload(h);
+    if (rc != FL_OK) return rc;
+  }
+  p->reco_sharded = true;
+  return FL_OK;
+}
+
+// frame f of a template-sharded pipe on slot f % depth: stage, match the shard + exchange, then the tail with the push to the other
+// ranks on the frame's owner (rank f % world), the receive of the owner's results everywhere else
+static int submit_recognition_sharded(fl_pipe* p, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
+                                      int32_t src_W, int32_t src_H, int32_t W, int32_t H, fl_intrinsics_t K_ref) {
+  if (!p->reco_sharded) { fl_set_error("fl_pipe_submit_recognition: call fl_pipe_set_recognition_sharded after the template and crop uploads"); return FL_ERR_STATE; }
+  const long long f = p->submitted;
+  const int slot = (int)(f % p->depth), owner = (int)(f % p->world);
+  fl_handle* h = p->h[slot];
+  void* const* peers = p->peers.data() + (size_t)slot * p->world;
+  const size_t mbox = fl_reco_mailbox_offset(p->world, p->xcap);
+  int rc = fl_reco_shard_stage(h, bgr, bgr_stride, depth, depth_stride, src_W, src_H, W, H, K_ref);
+  if (rc != FL_OK) return rc;                                   // nothing launched that a peer waits for
+  const uint32_t e = p->epoch[slot] + 1;
+  rc = fl_reco_shard_match(h, p->rank, p->world, peers, p->xcap, p->blocks[slot], e);
+  if (rc != FL_OK) return rc;
+  p->epoch[slot] = e;
+  if (owner == p->rank) {
+    fl_reco_push push;
+    memset(&push, 0, sizeof push);
+    push.epoch = e; push.mailbox_off = mbox;
+    for (int r = 0; r < p->world; ++r) if (r != p->rank) push.peer[push.n++] = static_cast<uint8_t*>(peers[r]);
+    rc = fl_reco_shard_tail(h, &push);
+  } else {
+    rc = fl_reco_shard_receive(h, static_cast<const uint8_t*>(peers[p->rank]), mbox, e, owner);
+  }
+  if (rc != FL_OK) { fl_match_wait(h); return rc; }              // the exchange is under way: wait for it, so that the slot is free again
+  return FL_OK;
+}
+
 extern "C" int fl_pipe_submit_recognition(fl_pipe* p, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
                                           int32_t src_W, int32_t src_H, int32_t W, int32_t H, fl_intrinsics_t K_ref) {
   if (!p) return FL_ERR_ARG;
-  if (p->world > 1) { fl_set_error("fl_pipe_submit_recognition: not available on a template-sharded pipe"); return FL_ERR_STATE; }
   if (p->submitted - p->collected >= p->depth) { fl_set_error("fl_pipe_submit_recognition: %d frames in flight already - collect one first", p->depth); return FL_ERR_STATE; }
-  const int rc = fl_recognize_async(p->h[p->submitted % p->depth], bgr, bgr_stride, depth, depth_stride, src_W, src_H, W, H, K_ref);
+  const int rc = p->world > 1 ? submit_recognition_sharded(p, bgr, bgr_stride, depth, depth_stride, src_W, src_H, W, H, K_ref)
+                              : fl_recognize_async(p->h[p->submitted % p->depth], bgr, bgr_stride, depth, depth_stride, src_W, src_H, W, H, K_ref);
   if (rc != FL_OK) return rc;
   ++p->submitted;
   return FL_OK;
@@ -189,5 +245,12 @@ extern "C" int fl_pipe_collect_recognition(fl_pipe* p, fl_reco_result_t* out, in
   // the oldest frame came from fl_pipe_submit: it stays in flight for fl_pipe_collect (waiting for it here would leave nothing to fetch)
   if (!fl_recognition_pending(h)) { fl_set_error("fl_pipe_collect_recognition: the oldest frame in flight is a match frame - fl_pipe_collect it"); return FL_ERR_STATE; }
   ++p->collected;                                               // the slot is free again whatever the frame's status
+  if (p->world > 1) {
+    // a missing peer or owner, an overflowing exchange block: this frame's status only.  A deferred list (more than the 1,024 records
+    // the fused sort holds) was sorted by the wait; every rank then runs the tail itself on its copy of it (fl_reco_shard_results)
+    const int rc = fl_match_wait(h);
+    if (rc != FL_OK) return rc;
+    return fl_reco_shard_results(h, out, capacity, summary);
+  }
   return fl_recognize_wait(h, out, capacity, summary);
 }

@@ -2,7 +2,8 @@
 // list to the ICP launch and the ICP results to the caller, so that a frame needs no host round trip between its stages.
 //   k_reco_select  after k_refine_sort: hypothesis selection of the mirrors (fealess_b200/reco.py, include/fealess_b200/obj_reco.hpp)
 //   k_reco_finish  after k_icp_fused: the objects that came out of ICP, nonMaximumSuppression (ICP/NMS.cpp:6-39), Convert (:20-30),
-//                  posted to mapped pinned host memory
+//                  posted to mapped pinned host memory (on a template-sharded pipe also pushed to the other ranks' mailboxes)
+//   k_reco_receive on a template-sharded pipe's ranks that do not own the frame: the owner's results, from the mailbox to mapped host memory
 #include "fl_internal.cuh"
 
 // One warp walks the sorted list 32 matches at a time.  A match is taken while its key (its class with per_class, else one key for
@@ -77,9 +78,11 @@ static_assert(sizeof(fl_reco_result_t) % 4 == 0, "fl_reco_result_t is a sequence
 
 // One thread per hypothesis (FL_RECO_MAX_HYP threads).  The summary and the records are staged in shared memory and leave as ONE
 // run of coalesced word stores: single stores to mapped host memory cost ~0.7 us each when one thread issues them in sequence.
+// With push.n > 0 (the owner of a template-sharded pipe's frame) the same words go to the mailbox of every listed rank, and the frame's
+// epoch is published in each mailbox signal after a system-scope fence, as the candidate exchange publishes its blocks.
 __global__ void __launch_bounds__(FL_RECO_MAX_HYP) k_reco_finish(const fl_match_t* __restrict__ matches, const int* __restrict__ sel,
                                                                 const fl_icp_result_t* __restrict__ results, int max_hyp, float th,
-                                                                int* __restrict__ host_block) {
+                                                                int* __restrict__ host_block, const __grid_constant__ fl_reco_push push) {
   extern __shared__ int s_out[];                                 // [FL_RECO_SUMMARY_WORDS][records]
   __shared__ float s_t3[3 * FL_RECO_MAX_HYP], s_dist[FL_RECO_MAX_HYP];
   __shared__ int32_t s_npts[FL_RECO_MAX_HYP], s_ok[FL_RECO_MAX_HYP], s_keep[FL_RECO_MAX_HYP];
@@ -124,7 +127,43 @@ __global__ void __launch_bounds__(FL_RECO_MAX_HYP) k_reco_finish(const fl_match_
     s_out[tid] = tid < 5 ? v[tid] : 0;
   }
   __syncthreads();
-  for (int i = tid; i < FL_RECO_SUMMARY_WORDS + n_keep * RECO_REC_WORDS; i += blockDim.x) host_block[i] = s_out[i];
+  const int n_words = FL_RECO_SUMMARY_WORDS + n_keep * RECO_REC_WORDS;
+  for (int i = tid; i < n_words; i += blockDim.x) host_block[i] = s_out[i];
+  if (push.n > 0) {
+    for (int p = 0; p < push.n; ++p) {
+      int* mbox = reinterpret_cast<int*>(push.peer[p] + push.mailbox_off);
+      for (int i = tid; i < n_words; i += blockDim.x) mbox[i] = s_out[i];
+    }
+    __threadfence_system();
+    __syncthreads();
+    if (tid < push.n) st_release_sys(reinterpret_cast<unsigned*>(push.peer[tid]) + FL_XCHG_RECO_SIGNAL, push.epoch);
+  }
+}
+
+// One CTA on a rank that does not own the frame: thread 0 acquire-waits for the frame's epoch in this rank's mailbox signal (bounded as
+// the candidate exchange's wait: ~2 s of SM cycles), then the mailbox leaves for the mapped host block as one run of coalesced word stores.
+__global__ void __launch_bounds__(FL_RECO_MAX_HYP) k_reco_receive(const uint8_t* __restrict__ own, size_t mailbox_off, unsigned epoch, int owner,
+                                                                 int* __restrict__ host_block) {
+  __shared__ int s_arrived;
+  const int tid = threadIdx.x;
+  if (tid == 0) {
+    const unsigned* sig = reinterpret_cast<const unsigned*>(own) + FL_XCHG_RECO_SIGNAL;
+    const long long t0 = clock64();
+    int arrived = 1;
+    while ((int)(ld_acquire_sys(sig) - epoch) < 0) {
+      if (clock64() - t0 > (1ll << 32)) { arrived = 0; break; }
+      __nanosleep(64);
+    }
+    s_arrived = arrived;
+  }
+  __syncthreads();
+  if (!s_arrived) {                                              // an empty summary that names the owner; the host reports FL_ERR_STATE
+    if (tid < FL_RECO_SUMMARY_WORDS) host_block[tid] = tid == FL_RECO_MISSING_OWNER ? 1 + owner : 0;
+    return;
+  }
+  const int* mbox = reinterpret_cast<const int*>(own + mailbox_off);
+  const int n_keep = min(max(__ldcg(mbox + 3), 0), FL_RECO_MAX_HYP);   // L2 loads: the owner wrote these over the peer link
+  for (int i = tid; i < FL_RECO_SUMMARY_WORDS + n_keep * RECO_REC_WORDS; i += blockDim.x) host_block[i] = __ldcg(mbox + i);
 }
 
 int fl_launch_reco_select(const fl_match_t* matches, const int* d_hdr, int out_cap, int check_big, const int32_t* class_first, int n_classes,
@@ -136,7 +175,22 @@ int fl_launch_reco_select(const fl_match_t* matches, const int* d_hdr, int out_c
 }
 
 int fl_launch_reco_finish(const fl_match_t* matches, const int* sel, const fl_icp_result_t* results, int max_hyp, float th_obj_dist,
-                          int* host_block, cudaStream_t s) {
+                          int* host_block, const fl_reco_push* push, cudaStream_t s) {
   const size_t smem = (size_t)(FL_RECO_SUMMARY_WORDS + max_hyp * RECO_REC_WORDS) * sizeof(int);
-  return fl_launch(k_reco_finish, dim3(1), dim3(FL_RECO_MAX_HYP), smem, s, matches, sel, results, max_hyp, th_obj_dist, host_block) == cudaSuccess ? 1 : -1;
+  fl_reco_push P;
+  memset(&P, 0, sizeof P);
+  if (push) P = *push;
+  return fl_launch(k_reco_finish, dim3(1), dim3(FL_RECO_MAX_HYP), smem, s, matches, sel, results, max_hyp, th_obj_dist, host_block, P) == cudaSuccess ? 1 : -1;
+}
+
+int fl_launch_reco_receive(const uint8_t* own_buffer, size_t mailbox_off, unsigned epoch, int owner, int* host_block, cudaStream_t s) {
+  return fl_launch(k_reco_receive, dim3(1), dim3(FL_RECO_MAX_HYP), 0, s, own_buffer, mailbox_off, epoch, owner, host_block) == cudaSuccess ? 1 : -1;
+}
+
+int fl_reco_preload() {
+  cudaFuncAttributes a;
+  FL_CUDA(cudaFuncGetAttributes(&a, k_reco_select));
+  FL_CUDA(cudaFuncGetAttributes(&a, k_reco_finish));
+  FL_CUDA(cudaFuncGetAttributes(&a, k_reco_receive));
+  return FL_OK;
 }

@@ -354,8 +354,6 @@ __global__ void __launch_bounds__(256) k_build_keys(fl_lists L, fl_sort_key* __r
 // Common case, ONE launch of one CTA: gather the live candidates of all lists, sort, prune duplicates.  When the lists hold
 // more records than fit its shared memory it only sets *d_flag_big = 1 and the host runs the multi-kernel path (k_build_keys + global
 // bitonic steps + k_unique_big).  d_scratch = {n_live, flag_big}.
-__device__ __forceinline__ void st_release_sys(unsigned* p, unsigned v) { asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
-__device__ __forceinline__ unsigned ld_acquire_sys(const unsigned* p) { unsigned v; asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory"); return v; }
 
 // loads that must see what other CTAs of the SAME launch wrote (fused refine + sort): L2, not this SM's L1
 __device__ __forceinline__ int ld_count(const fl_lists& L, int l) { return __ldcg(L.n_in + (size_t)l * L.n_in_stride); }

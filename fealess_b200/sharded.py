@@ -16,7 +16,7 @@ from typing import List, Tuple
 
 import numpy as np
 
-from . import synth
+from . import RECO_MAX_HYP, synth
 
 RECORD_INTS = 5  # fl_match_t = 5 x int32-sized fields
 
@@ -275,7 +275,12 @@ class ShardedPipe:
 class NativeShardedPipe:
     """The same schedule as ``ShardedPipe`` with the per-frame host work inside the library: one ``fl_pipe`` per rank in template-sharded
     mode (``fl_pipe_set_exchange``).  torch only provides the symmetric-memory exchange buffers (one per slot, mapped into every process)
-    and the rendezvous; ``match_batch`` is ONE C call for any number of frames.  Peer-memory exchange only."""
+    and the rendezvous; ``match_batch`` is ONE C call for any number of frames.  Peer-memory exchange only.
+
+    Recognition (``upload_model_depths``, ``set_recognition``, then ``submit_recognition`` / ``collect_recognition`` or ``recognize``, the
+    arguments and return values of ``Pipe``'s methods): frame f is matched on every rank, refined and suppressed by rank f % world alone,
+    and its results reach every rank through peer memory (fl_pipe_set_recognition_sharded); every rank collects the single detector's
+    results for every frame."""
 
     def __init__(self, tset, rank: int, world: int, depth: int = 4, capacity: int = 2048, device=None, T=(5, 8), modality_kind=(0, 1),
                  max_width: int = 640, max_height: int = 480, max_candidates: int = 1 << 16):
@@ -285,6 +290,7 @@ class NativeShardedPipe:
         from . import Pipe, lib
         dev = device if device is not None else torch.device("cuda", torch.cuda.current_device())
         self.rank, self.world, self.depth, self.cap = rank, world, int(depth), capacity
+        self._tset, self._dev, self._reco_err = tset, dev, None        # the whole set: the recognition set-up selects from the merged list
         # Everything that can fail on ONE rank alone (device allocations, the template upload) happens before the first collective, and
         # the ranks agree on the outcome: a rank that failed must not leave its peers waiting inside the rendezvous that follows.
         self.pipe, self._xbufs, self._xhdls, self._blocks, err = None, [], [], [], None
@@ -320,6 +326,48 @@ class NativeShardedPipe:
 
     def match_batch(self, frames, threshold: float, capacity_per_frame: int = 1 << 12, out=None, copy: bool = True):
         return self.pipe.match_batch(frames, threshold, capacity_per_frame=capacity_per_frame, out=out, copy=copy)
+
+    def in_flight(self) -> int:
+        return self.pipe.in_flight()
+
+    def upload_model_depths(self, model_depths, rects_model) -> None:
+        """``Pipe.upload_model_depths`` on this rank.  A failure here is raised by ``set_recognition`` on every rank, once the ranks
+        have agreed on it: a rank that raised alone would leave its peers waiting."""
+        self._reco_err = None
+        try:
+            self.pipe.upload_model_depths(model_depths, rects_model)
+        except Exception as e:  # noqa: BLE001
+            self._reco_err = e
+
+    def set_recognition(self, crop_of_template, pose12=None, params=None) -> None:
+        """``Pipe.set_recognition_sharded`` with the whole set this pipe was built from; crop index and pose of every template of that
+        set.  Collective: the ranks agree on the outcome of the crop upload and of this set-up before any frame is submitted."""
+        import torch
+        import torch.distributed as dist
+        err, self._reco_err = self._reco_err, None
+        if err is None:
+            try:
+                self.pipe.set_recognition_sharded(self._tset, crop_of_template, pose12, params)
+            except Exception as e:  # noqa: BLE001
+                err = e
+        flag = torch.tensor([0 if err else 1], device=self._dev)
+        dist.all_reduce(flag, op=dist.ReduceOp.MIN)
+        if int(flag.item()) == 0:
+            raise RuntimeError("NativeShardedPipe: recognition set-up failed on %s: %r" % ("this rank" if err else "another rank", err))
+
+    def submit_recognition(self, bgr, depth, K, W=None, H=None) -> None:
+        self.pipe.submit_recognition(bgr, depth, K, W, H)
+
+    def collect_recognition(self, capacity: int = RECO_MAX_HYP):
+        return self.pipe.collect_recognition(capacity)
+
+    def recognize(self, bgr, depth, K, W=None, H=None, capacity: int = RECO_MAX_HYP):
+        """One frame, submitted and collected (nothing else may be in flight)."""
+        from . import FL_ERR_STATE, FealessError
+        if self.in_flight():
+            raise FealessError(FL_ERR_STATE, "NativeShardedPipe.recognize", "%d frame(s) in flight - collect them first" % self.in_flight())
+        self.submit_recognition(bgr, depth, K, W, H)
+        return self.collect_recognition(capacity)
 
     def close(self) -> None:
         import torch

@@ -236,7 +236,9 @@ int fl_sort_unique_blocks_device(fl_handle* h, const fl_match_t* d_blocks, int32
  * job (CUDA IPC, fabric handles, torch symmetric memory ...); peer_buffers[p] is the address of rank p's buffer in THIS
  * process.  The kernel pushes this rank's block [count | records] into every peer's buffer, publishes `epoch` (> 0,
  * incremented by all ranks for every frame) in the peer's signal word, waits for the epoch of all peers (bounded: a
- * missing peer yields FL_ERR_STATE after ~2 s instead of a hang), and sorts + prunes the union.  world <= 8. */
+ * missing peer yields FL_ERR_STATE after ~2 s instead of a hang), and sorts + prunes the union.  world <= 8.
+ * The buffer's layout is private.  Its size includes a result mailbox of about 40 KB at the end, which only the recognition frames of
+ * a template-sharded pipe use (fl_pipe_set_recognition_sharded); match-only frames never touch it. */
 size_t fl_exchange_buffer_bytes(int32_t world, int32_t capacity);
 int fl_exchange_sort_unique_device(fl_handle* h, int32_t rank, int32_t world, void* const* peer_buffers, int32_t capacity,
                                    const fl_match_t* d_local_block, uint32_t epoch);
@@ -401,10 +403,27 @@ int fl_recognize(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint
                  int32_t src_W, int32_t src_H, int32_t W, int32_t H, fl_intrinsics_t K_ref,
                  fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary);
 /* The same over a pipe: one host thread keeps up to `depth` frames in flight; results come back in submission order.  Setup on
- * every slot (FL_ERR_STATE while frames are in flight); FL_ERR_STATE on a template-sharded pipe (fl_pipe_set_exchange). */
+ * every slot (FL_ERR_STATE while frames are in flight).  fl_pipe_set_recognition: FL_ERR_STATE on a template-sharded pipe
+ * (fl_pipe_set_exchange with world > 1), which takes fl_pipe_set_recognition_sharded instead. */
 int fl_pipe_upload_model_depths(fl_pipe* p, int32_t n_models, const uint16_t* const* model_depth, const size_t* model_stride,
                                 const fl_rect_t* rect_model, int32_t W, int32_t H);
 int fl_pipe_set_recognition(fl_pipe* p, const fl_reco_params_t* params, const int32_t* crop_of_template, const float* pose12);
+/* Recognition on a template-sharded pipe (one process, or one pipe, per rank).  The rank holds only its shard, so the set-up takes the
+ * tables of the WHOLE set: headers and class_of in the layout of fl_upload_templates over the whole set (only the level-0
+ * modality-0 box of each template is read), crop_of_template as in fl_set_recognition (crops uploaded with
+ * fl_pipe_upload_model_depths), pose12 (required) = 12 floats per template.  Every rank passes the same set.  FL_ERR_STATE on a pipe
+ * that is not template-sharded or with frames in flight; otherwise the checks and statuses of fl_set_recognition.  Cleared by a later
+ * template or crop upload or fl_pipe_set_exchange.
+ * fl_pipe_submit_recognition then runs frame f on slot f % depth of every rank: each rank uploads [and rescales] the frame, matches
+ * its shard and takes part in the exchange; only the frame's owner, rank f % world, runs selection, ICP and suppression, and pushes
+ * the results over peer memory into every other rank's exchange buffer, where a one-CTA receive kernel waits for them (bounded: an
+ * owner that never posts gives FL_ERR_STATE after ~2 s).  One enqueue per frame; fl_pipe_collect_recognition is its only host wait
+ * and returns on EVERY rank the results of a single handle's fl_recognize over the whole set.  A list of more than 1,024 unique
+ * matches is finished by every rank on its own copy.  Collecting frees the slot whatever the frame's status (a missing peer or
+ * owner, an overflowing exchange block, FL_ERR_CAPACITY).  Match frames (fl_pipe_submit) and recognition frames may be mixed; all
+ * ranks submit the same sequence.  The first frame of a new source geometry allocates its rescale tables before its exchange. */
+int fl_pipe_set_recognition_sharded(fl_pipe* p, const fl_reco_params_t* params, int32_t n_templates, const fl_template_hdr_t* headers,
+                                    const int32_t* class_of, const int32_t* crop_of_template, const float* pose12);
 int fl_pipe_submit_recognition(fl_pipe* p, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
                                int32_t src_W, int32_t src_H, int32_t W, int32_t H, fl_intrinsics_t K_ref);
 int fl_pipe_collect_recognition(fl_pipe* p, fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary);
