@@ -33,6 +33,23 @@ struct fl_icp_bufs {
   fl_pinned_buf<uint16_t> h_model_crops; fl_pinned_buf<fl_icp_hyp> h_hyps; fl_pinned_buf<fl_icp_result_t> h_results;
 };
 
+// What d_in_bgr / d_in_depth hold: the last host frame staged on the handle (stage_host).  Its depth counts as "the matched frame" - the
+// reference depth of fl_detection_batch_resident(_device) with ref_depth == NULL - only once an enqueue that used it has succeeded.
+struct fl_staged_frame { int W = 0, H = 0; bool bgr = false, depth = false, matched = false; };
+
+// The frame in flight (fl_frame_kind), from the enqueue that starts it (frame_begin) to fl_frame_wait.  The fields stay valid after the
+// wait: a recognition frame's tail may run again on them, and a group re-runs its members' staged frames.
+struct fl_frame {
+  fl_frame_kind kind = fl_frame_kind::none;
+  // the sort half (sort_launch -> sort_finish): own = the first matches go to this handle's mapped block too; fused = the launch also
+  // refined the candidates (k_refine_sort, whose last CTA sorts at most 1,024 records)
+  fl_lists lists = {}; fl_match_t* out = nullptr; int out_cap = 0; int* out_count = nullptr; bool own = false, fused = false;
+  // what a front-end time-out re-runs; rerun = the frame was matched on this handle alone (one that exchanged with peers needs every rank)
+  bool rerun = false; const void* bgr = nullptr; const void* depth = nullptr; int W = 0, H = 0; const void* masks[FL_MAX_MODALITIES] = {};
+  float threshold = 0.f; std::vector<int32_t> filter;
+  fl_intrinsics_t K = {};                                  // recognition frames: the intrinsics of the staged frame
+};
+
 // Every resource has one owner (fl_owned.cuh); plan, icp, rz, d_out(_count), h_small, h_first, d_fe_err_host, d_reco_host point into them.
 struct fl_handle {
   fl_owned_stream stream;                                  // declared first: destroyed last, after everything used on it
@@ -65,9 +82,7 @@ struct fl_handle {
   fl_dev_buf<uint32_t> d_mass;                                         // response mass of the coarsest level (FL_MASS_*): the staged kernel's phase order
   const uint8_t* frame_mask[FL_MAX_MODALITIES] = {};               // level-0 mask (device memory) of the last frame's modality m, or NULL
   bool keep_spread = false;
-  // state between the enqueue half (fl_match_device_async, ..._async) and fl_match_wait
-  bool pend_sort = false, pend_match = false, pend_own = false, pend_masks_valid = false, pend_small_fused = false; fl_lists pend_lists = {}; fl_match_t* pend_out = nullptr; int pend_out_cap = 0; int* pend_out_count = nullptr;
-  const void* pend_bgr = nullptr; const void* pend_depth = nullptr; int pend_W = 0, pend_H = 0; float pend_threshold = 0.f; const void* pend_masks[FL_MAX_MODALITIES] = {}; std::vector<int32_t> pend_filter;
+  fl_frame frame; fl_staged_frame staged;
   fl_dev_buf<unsigned long long> d_fe_trace; int fe_trace_jobs = 0, fe_trace_kind[FL_FE_MAX_JOBS] = {}, fe_trace_ctas[FL_FE_MAX_JOBS] = {};
   bool opt_fe_waves = false, opt_split_refine = false, opt_trace = false, opt_dep_test = false, opt_no_prune = false, opt_rotate = false;   // fl_debug_option
   fl_mapped_buf<int> h_fe_err; int* d_fe_err_host = nullptr; bool fe_force_waves = false;   // in-grid dependency time-out: mapped host flag (+ its device alias); true = this handle launches one kernel per wave from now on
@@ -76,16 +91,14 @@ struct fl_handle {
   fl_dev_buf<fl_match_t> d_cand; fl_dev_buf<int> d_count; fl_dev_buf<fl_sort_key> d_keys; int key_cap = 0; fl_dev_buf<uint8_t> d_outblk; fl_match_t* d_out = nullptr; int* d_out_count = nullptr;   // d_outblk = [16-int summary][matches]
   // pinned host staging
   fl_pinned_buf<uint8_t> h_bgr; fl_pinned_buf<uint16_t> h_depth; fl_pinned_buf<uint8_t> h_mask, h_outblk, h_class_enabled; int* h_small = nullptr; fl_match_t* h_first = nullptr;   // h_small/h_first point into h_outblk
-  bool have_result = false, overflow = false;
+  bool have_result = false, overflow = false;              // the last completed frame: its list can be fetched; it overflowed a buffer
   // profiling
   bool profile = false; fl_owned_event ev[5]; float stage_ms[4] = {}; float icp_ms = 0.f;
   // ICP workspace (grown on demand)
   int icp_hyp_cap = 0, icp_pts_cap = 0;
   fl_icp_ws icp = {}; fl_icp_bufs icpw; int icp_trace_n = 0; fl_dev_buf<uint16_t> d_ref_depth;
-  // rendered template depth crops kept on the device (fl_upload_model_depths) and the geometry of the depth frame that the
-  // last host-input fl_match left in d_in_depth (0 x 0 = none)
+  // rendered template depth crops kept on the device (fl_upload_model_depths)
   fl_dev_buf<uint16_t> d_resident; std::vector<size_t> res_off; std::vector<fl_rect_t> res_rect; int res_W = 0, res_H = 0;
-  int in_depth_W = 0, in_depth_H = 0;
   fl_dev_buf<int32_t> d_nms; int nms_cap = 0;   // fl_nms workspace (hypotheses)
   bool blocking_wait = false; fl_owned_event ev_block;   // fl_set_blocking_wait
   fl_dev_buf<uint8_t> d_train;                           // fl_add_template workspace (allocated at the first call)
@@ -94,13 +107,12 @@ struct fl_handle {
   fl_dev_buf<int> rz_xofs, rz_yofs; fl_dev_buf<short2> rz_ialpha, rz_ibeta; fl_dev_buf<float2> rz_alpha, rz_beta;
   fl_dev_buf<uint8_t> d_src_bgr; fl_dev_buf<uint16_t> d_src_depth;
   // Recognition on the device (fl_set_recognition, fl_recognize_*): per-template table, per-frame selection state, mapped host block
-  // [summary | records] (+ its device alias); the frame in flight (pend_reco) and its geometry and intrinsics
-  bool custom_tids = false, reco_set = false, reco_any_crop = false, pend_reco = false; fl_reco_params_t reco = {}; int reco_max_hyp = 0;
+  // [summary | records] (+ its device alias)
+  bool custom_tids = false, reco_set = false, reco_any_crop = false; fl_reco_params_t reco = {}; int reco_max_hyp = 0;
   fl_dev_buf<fl_reco_tmpl> d_reco_tmpl; fl_dev_buf<int> d_reco_sel; fl_mapped_buf<int> h_reco; int* d_reco_host = nullptr;
-  int reco_W = 0, reco_H = 0; fl_intrinsics_t reco_K = {};
   // the template set the selection table covers: the handle's own upload, or the whole set of a template-sharded group, whose merged
   // list this handle selects from (fl_group_set_recognition)
-  int reco_n_templates = 0, reco_n_classes = 0; fl_dev_buf<int32_t> d_reco_class_first; bool reco_bgr = false;   // reco_bgr: the staged frame has colour
+  int reco_n_templates = 0, reco_n_classes = 0; fl_dev_buf<int32_t> d_reco_class_first;
 };
 
 // The host waits for the handle's stream.  Default: cudaStreamSynchronize (the runtime spins - lowest latency, one busy core per
@@ -216,7 +228,20 @@ extern "C" int fl_sync(fl_handle* h) { if (!h) return FL_ERR_ARG; FL_CUDA(cudaSt
 extern "C" void* fl_stream(fl_handle* h) { return h ? (void*)h->stream.get() : nullptr; }
 extern "C" int64_t fl_launch_count(fl_handle* h) { return h ? h->launches : 0; }
 int fl_entries_per_template(const fl_handle* h) { return h ? h->p.n_levels * h->p.n_modalities : 0; }
-bool fl_recognition_pending(const fl_handle* h) { return h && h->pend_reco; }
+fl_frame_kind fl_frame_in_flight(const fl_handle* h) { return h ? h->frame.kind : fl_frame_kind::none; }
+// One frame in flight per handle: its wait reads the frame record, and a host frame would overwrite staging buffers it may still read.
+static int frame_idle(const fl_handle* h) {
+  if (h->frame.kind == fl_frame_kind::none) return FL_OK;
+  fl_set_error("a frame is in flight on this handle: wait for it first (fl_match_wait or fl_recognize_wait)");
+  return FL_ERR_STATE;
+}
+// the start of every entry point that enqueues frame work: nothing in flight, the handle's device, and the last frame's result is gone
+static int frame_begin(fl_handle* h) {
+  TRY(frame_idle(h));
+  FL_CUDA(cudaSetDevice(h->p.device));
+  h->have_result = h->overflow = false;
+  return FL_OK;
+}
 extern "C" int fl_profile(fl_handle* h, int enable) { if (!h) return FL_ERR_ARG; h->profile = enable != 0; return FL_OK; }
 extern "C" int fl_last_icp_ms(fl_handle* h, float* ms) { if (!h || !ms) return FL_ERR_ARG; *ms = h->icp_ms; return FL_OK; }
 extern "C" int fl_debug_icp_trace(fl_handle* h, uint64_t* out, int32_t n_hyp) {
@@ -677,7 +702,6 @@ static int sort_launch(fl_handle* h, fl_lists L, fl_match_t* d_out, int out_cap,
                                          d_out, out_cap, d_out_count, d_hdr, h->h_small, own ? h->h_first : nullptr, std::min(FETCH_FIRST, out_cap), s);
     if (nl < 0) { fl_set_error("refinement + sort launch failed: %s", cudaGetErrorString(cudaGetLastError())); return FL_ERR_CUDA; }
     h->launches += nl;
-    h->pend_small_fused = true;
   } else {
     const int nl = fl_launch_sort_unique(L, X, h->key_cap, d_out, out_cap, d_out_count, d_hdr, h->h_small, own ? h->h_first : nullptr,
                                          std::min(FETCH_FIRST, out_cap), s);
@@ -686,7 +710,8 @@ static int sort_launch(fl_handle* h, fl_lists L, fl_match_t* d_out, int out_cap,
   }
   if (h->profile) cudaEventRecord(h->ev[4].get(), s);
   // what the second half (sort_finish) needs: it runs after the host has waited for the stream
-  h->pend_lists = L; h->pend_out = d_out; h->pend_out_cap = out_cap; h->pend_out_count = d_out_count; h->pend_own = own; h->pend_sort = true;
+  fl_frame& f = h->frame;
+  f.lists = L; f.out = d_out; f.out_cap = out_cap; f.out_count = d_out_count; f.own = own; f.fused = refine != nullptr;
   return FL_OK;
 }
 
@@ -694,36 +719,31 @@ static int sort_launch(fl_handle* h, fl_lists L, fl_match_t* d_out, int out_cap,
 // reported more records than it holds
 static int sort_finish(fl_handle* h) {
   cudaStream_t s = h->stream.get();
-  if (!h->pend_sort) return FL_ERR_STATE;
-  h->pend_sort = false;
-  const fl_lists L = h->pend_lists;
-  fl_match_t* d_out = h->pend_out; const int out_cap = h->pend_out_cap; int* d_out_count = h->pend_out_count; const bool own = h->pend_own;
-  const int n_lists = L.n_lists, list_cap = L.list_cap;
+  const fl_frame& f = h->frame;
+  const int n_lists = f.lists.n_lists, list_cap = f.lists.list_cap;
   FL_CUDA(wait_stream(h));
   h->overflow = false;
   int n_upper = 0;
   for (int i = 0; i < std::min(n_lists, 11); ++i) { if (h->h_small[3 + i] > list_cap) h->overflow = true; n_upper += std::min(std::max(h->h_small[3 + i], 0), list_cap); }
   if (n_lists > 11) n_upper = n_lists * list_cap;
-  if (h->h_small[2] && h->pend_small_fused && n_upper <= 8192) {
+  if (h->h_small[2] && f.fused && n_upper <= 8192) {
     // the fused refinement + sort launch sorts up to 1,024 records in its last CTA; this frame has more (already refined in
     // place): run the stand-alone one-CTA sort (8,192 keys) on them.  What the first launch reported about the exchange
     // (a peer that never arrived) survives the second launch, which knows nothing about it.
     const int keep15 = h->h_small[15];
     const bool keep_overflow = h->overflow;
-    h->pend_small_fused = false;
-    TRY(sort_launch(h, L, d_out, out_cap, d_out_count, own));
+    TRY(sort_launch(h, f.lists, f.out, f.out_cap, f.out_count, f.own));
     const int rc = sort_finish(h);
     if (keep15) h->h_small[15] = keep15;
     h->overflow |= keep_overflow;
     return rc;
   }
-  h->pend_small_fused = false;
   if (h->h_small[2]) {                                                          // more records than the one-CTA sort holds: multi-kernel sort
-    int rc = fl_launch_sort_unique_big(L, h->d_keys.get(), h->key_cap, n_upper, d_out, out_cap, d_out_count, s);
+    int rc = fl_launch_sort_unique_big(f.lists, h->d_keys.get(), h->key_cap, n_upper, f.out, f.out_cap, f.out_count, s);
     if (rc < 0) return FL_ERR_CAPACITY;
     h->launches += rc;
-    FL_CUDA(cudaMemcpyAsync(h->h_small, d_out_count, sizeof(int), cudaMemcpyDeviceToHost, s));
-    if (own) FL_CUDA(cudaMemcpyAsync(h->h_first, d_out, sizeof(fl_match_t) * (size_t)std::min(FETCH_FIRST, out_cap), cudaMemcpyDeviceToHost, s));
+    FL_CUDA(cudaMemcpyAsync(h->h_small, f.out_count, sizeof(int), cudaMemcpyDeviceToHost, s));
+    if (f.own) FL_CUDA(cudaMemcpyAsync(h->h_first, f.out, sizeof(fl_match_t) * (size_t)std::min(FETCH_FIRST, f.out_cap), cudaMemcpyDeviceToHost, s));
     if (h->profile) cudaEventRecord(h->ev[4].get(), s);
     FL_CUDA(wait_stream(h));
   }
@@ -738,47 +758,58 @@ static int run_sort_unique(fl_handle* h, fl_lists L, fl_match_t* d_out, int out_
   return sort_finish(h);
 }
 
-extern "C" int fl_match_device_async(fl_handle* h, const void* d_bgr, const void* d_depth, int32_t W, int32_t H, const void* const* d_masks,
-                                     float threshold, const int32_t* class_filter, int32_t n_filter) {
-  if (!h) return FL_ERR_ARG;
-  if (h->pend_sort) { fl_set_error("fl_match_wait has not been called for the previous frame"); return FL_ERR_STATE; }
-  h->have_result = false; h->pend_match = false;
-  // refinement and sort + unique share one launch (k_refine_sort: 256-thread CTAs, the last one to finish sorts up to 1,024
-  // records); FL_OPT_SPLIT_REFINE keeps them as separate launches (what fl_match_shard_device needs anyway: its candidates must
-  // be refined before an NCCL gather).  A variant with 1,024-thread CTAs and the 8,192-key sort inside was measured slower (those
-  // CTAs cost more to launch than the launch they save) and removed.
+// A device frame on this handle: front end + matchClass into (cand, cap, d_count), then one launch that refines those candidates and sorts
+// `lists` into the handle's output block - with the peer exchange X of a template-sharded frame in its last CTA, or X == NULL.
+// Refinement and sort + unique share that launch (k_refine_sort: 256-thread CTAs, the last one to finish sorts up to 1,024 records);
+// FL_OPT_SPLIT_REFINE keeps them as separate launches (what fl_match_shard_device needs anyway: its candidates must be refined before an
+// NCCL gather).  A variant with 1,024-thread CTAs and the 8,192-key sort inside was measured slower (those CTAs cost more to launch than
+// the launch they save) and removed.
+static int match_launch(fl_handle* h, const void* d_bgr, const void* d_depth, int W, int H, const void* const* d_masks, float threshold,
+                        const int32_t* class_filter, int n_filter, fl_match_t* cand, int cap, int* d_count, const fl_lists& lists, const fl_xchg* X) {
   const bool defer = !h->opt_split_refine && h->n_templates > 0 && h->p.n_levels > 1;
-  TRY(run_match_stages(h, (const uint8_t*)d_bgr, (const uint16_t*)d_depth, W, H, d_masks, threshold, class_filter, n_filter, h->d_cand.get(),
-                       h->p.max_candidates, h->d_count.get(), defer));
-  const fl_lists lists = {h->d_cand.get(), 1, h->p.max_candidates, h->p.max_candidates, h->d_count.get(), 1};
-  const fl_refine_req req = {threshold, h->d_cand.get(), h->p.max_candidates, h->d_count.get()};
-  TRY(sort_launch(h, lists, h->d_out, h->p.max_candidates, h->d_out_count, true, nullptr, defer ? &req : nullptr));
-  // kept for fl_match_wait: a front-end dependency time-out re-runs the frame
-  h->pend_match = true; h->pend_bgr = d_bgr; h->pend_depth = d_depth; h->pend_W = W; h->pend_H = H; h->pend_threshold = threshold;
-  h->pend_masks_valid = d_masks != nullptr;
-  for (int m = 0; m < FL_MAX_MODALITIES; ++m) h->pend_masks[m] = d_masks ? d_masks[m] : nullptr;
-  h->pend_filter.assign(class_filter && n_filter > 0 ? class_filter : nullptr, class_filter && n_filter > 0 ? class_filter + n_filter : nullptr);
+  TRY(run_match_stages(h, (const uint8_t*)d_bgr, (const uint16_t*)d_depth, W, H, d_masks, threshold, class_filter, n_filter, cand, cap, d_count, defer));
+  const fl_refine_req req = {threshold, cand, cap, d_count};
+  TRY(sort_launch(h, lists, h->d_out, h->p.max_candidates, h->d_out_count, true, X, defer ? &req : nullptr));
+  fl_frame& f = h->frame;
+  f.kind = X ? fl_frame_kind::shard : fl_frame_kind::match;
+  f.rerun = !X; f.bgr = d_bgr; f.depth = d_depth; f.W = W; f.H = H; f.threshold = threshold;
+  for (int m = 0; m < FL_MAX_MODALITIES; ++m) f.masks[m] = d_masks ? d_masks[m] : nullptr;
+  f.filter.assign(class_filter && n_filter > 0 ? class_filter : nullptr, class_filter && n_filter > 0 ? class_filter + n_filter : nullptr);
+  if (d_depth && d_depth == h->d_in_depth.get()) h->staged.matched = true;
   return FL_OK;
 }
 
-static int match_wait(fl_handle* h) {
-  if (!h->pend_sort) return FL_ERR_STATE;
-  const bool was_match = h->pend_match;
-  h->pend_match = false;
+extern "C" int fl_match_device_async(fl_handle* h, const void* d_bgr, const void* d_depth, int32_t W, int32_t H, const void* const* d_masks,
+                                     float threshold, const int32_t* class_filter, int32_t n_filter) {
+  if (!h) return FL_ERR_ARG;
+  TRY(frame_begin(h));
+  const fl_lists lists = {h->d_cand.get(), 1, h->p.max_candidates, h->p.max_candidates, h->d_count.get(), 1};
+  return match_launch(h, d_bgr, d_depth, W, H, d_masks, threshold, class_filter, n_filter, h->d_cand.get(), h->p.max_candidates, h->d_count.get(), lists,
+                      nullptr);
+}
+
+int fl_frame_wait(fl_handle* h, fl_wait_note* note) {
+  *note = fl_wait_note::done;
+  fl_frame& f = h->frame;
+  if (f.kind == fl_frame_kind::none) { fl_set_error("no frame in flight on this handle"); return FL_ERR_STATE; }
+  f.kind = fl_frame_kind::none;
   TRY(sort_finish(h));
   if (*reinterpret_cast<volatile int*>(h->h_fe_err.get())) {
     // an in-grid dependency of the single-launch front end timed out (the producer CTAs were not dispatched before their consumers:
-    // see k_front_end_wave): the frame's result is not trustworthy.  From now on this handle launches one kernel per wave; a frame
-    // submitted through fl_match / fl_match_device* is re-run right away, the shard entry points report the state.
+    // see k_front_end_wave): the frame's result is not trustworthy.  From now on this handle launches one kernel per wave.
     const int job = *h->h_fe_err.get() - 1;
     *h->h_fe_err.get() = 0;
     FL_CUDA(cudaMemsetAsync(h->d_fe_counters.get() + FL_FE_MAX_JOBS, 0, sizeof(unsigned), h->stream.get()));
     h->fe_force_waves = true;
-    if (!was_match) { fl_set_error("front end: in-grid dependency of job %d timed out; the handle now uses per-wave launches - resubmit the frame", job); return FL_ERR_STATE; }
+    if (!f.rerun) {
+      *note = fl_wait_note::resubmit;
+      fl_set_error("front end: in-grid dependency of job %d timed out; the handle now uses per-wave launches - resubmit the frame", job);
+      return FL_ERR_STATE;
+    }
+    *note = fl_wait_note::rerun;
     const fl_lists lists = {h->d_cand.get(), 1, h->p.max_candidates, h->p.max_candidates, h->d_count.get(), 1};
-    int rc = run_match_stages(h, (const uint8_t*)h->pend_bgr, (const uint16_t*)h->pend_depth, h->pend_W, h->pend_H, h->pend_masks_valid ? h->pend_masks : nullptr,
-                              h->pend_threshold, h->pend_filter.empty() ? nullptr : h->pend_filter.data(), (int)h->pend_filter.size(), h->d_cand.get(),
-                              h->p.max_candidates, h->d_count.get());
+    int rc = run_match_stages(h, (const uint8_t*)f.bgr, (const uint16_t*)f.depth, f.W, f.H, f.masks, f.threshold, f.filter.empty() ? nullptr : f.filter.data(),
+                              (int)f.filter.size(), h->d_cand.get(), h->p.max_candidates, h->d_count.get());
     if (rc == FL_OK) rc = run_sort_unique(h, lists, h->d_out, h->p.max_candidates, h->d_out_count, true);
     if (rc != FL_OK) return rc;
   }
@@ -788,8 +819,8 @@ static int match_wait(fl_handle* h) {
 }
 extern "C" int fl_match_wait(fl_handle* h) {
   if (!h) return FL_ERR_ARG;
-  h->pend_reco = false;                 // a recognition frame waited for this way has no results to collect
-  return match_wait(h);
+  fl_wait_note note;
+  return fl_frame_wait(h, &note);
 }
 
 extern "C" int fl_match_device(fl_handle* h, const void* d_bgr, const void* d_depth, int32_t W, int32_t H, const void* const* d_masks,
@@ -815,21 +846,38 @@ extern "C" int fl_match_fetch(fl_handle* h, fl_match_t* out, int32_t capacity, i
   return (n > capacity || n > h->p.max_candidates || h->overflow) ? FL_ERR_CAPACITY : FL_OK;
 }
 
-// Frame upload of the host-buffer entry points.  A caller buffer that is already page-locked (cudaHostAlloc / cudaHostRegister /
-// torch pin_memory) is DMA'd directly, strided rows included, and has to stay valid until the frame has been waited for; pageable
-// memory goes through the handle's pinned staging buffer first (copied before this returns).
-static int stage_frame(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int W, int H, const uint8_t* const* masks,
-                       const uint8_t** d_bgr_out, const uint16_t** d_depth_out, const void** d_masks, bool* any_mask) {
+static int resize_tables(fl_handle* h, int sW, int sH, int dW, int dH);
+static int resize_staging(fl_handle* h, size_t npx);
+// the device side of a staged host frame: d_in_bgr / d_in_depth (NULL when the frame has no such image) and the level-0 masks
+struct fl_dev_frame { const uint8_t* bgr; const uint16_t* depth; const void* masks[FL_MAX_MODALITIES]; };
+
+// The one upload of the host-buffer entry points: a src_W x src_H frame (bgr and depth, either may be NULL) into d_in_bgr / d_in_depth
+// as a W x H frame, rescaled on the device (cv::resize INTER_LINEAR) when the sizes differ, and the masks (NULL or n_modalities
+// pointers of W x H bytes, each NULL or not) into d_mask[0].  Same size: a caller buffer that is already page-locked (cudaHostAlloc /
+// cudaHostRegister / torch pin_memory) is DMA'd directly, strided rows included, and has to stay valid until the frame has been waited
+// for; pageable memory goes through the handle's pinned staging buffer first (copied before this returns).
+static int stage_host(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int sW, int sH, int W, int H,
+                      const uint8_t* const* masks, fl_dev_frame* d) {
   const fl_params_t& p = h->p;
   cudaStream_t s = h->stream.get();
-  *d_bgr_out = nullptr; *d_depth_out = nullptr; *any_mask = false;
+  memset(d, 0, sizeof *d);
+  h->staged = fl_staged_frame();
+  if (W <= 0 || H <= 0 || W > p.max_width || H > p.max_height) return FL_ERR_SIZE;
+  if ((bgr && bgr_stride < (size_t)sW * 3) || (depth && depth_stride < (size_t)sW * 2)) return FL_ERR_SIZE;
   auto is_pinned = [](const void* q) {
     cudaPointerAttributes a;
     if (cudaPointerGetAttributes(&a, q) != cudaSuccess) { cudaGetLastError(); return false; }
     return a.type == cudaMemoryTypeHost;
   };
-  if (depth) {                                                                     // depth first: it is the smaller image
-    if (depth_stride < (size_t)W * 2) return FL_ERR_SIZE;
+  const bool rescale = sW != W || sH != H;
+  if (rescale) {
+    TRY(resize_tables(h, sW, sH, W, H));
+    TRY(resize_staging(h, (size_t)sW * sH));
+  }
+  if (depth && rescale) {                                                          // depth first: it is the smaller image
+    FL_CUDA(cudaMemcpy2DAsync(h->d_src_depth.get(), (size_t)sW * 2, depth, depth_stride, (size_t)sW * 2, sH, cudaMemcpyHostToDevice, s));
+    fl_launch_resize_linear(h->d_src_depth.get(), sW, sH, FL_IMG_16UC1, h->d_in_depth.get(), W, H, h->rz, s); ++h->launches;
+  } else if (depth) {
     if (is_pinned(depth)) {
       // dense rows go as ONE linear DMA (a 2-D copy of the same bytes is split into row descriptors and runs at about half the rate)
       if (depth_stride == (size_t)W * 2) FL_CUDA(cudaMemcpyAsync(h->d_in_depth.get(), depth, (size_t)W * H * 2, cudaMemcpyHostToDevice, s));
@@ -838,10 +886,11 @@ static int stage_frame(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, cons
       for (int y = 0; y < H; ++y) memcpy(h->h_depth.get() + (size_t)y * W, (const uint8_t*)depth + (size_t)y * depth_stride, (size_t)W * 2);
       FL_CUDA(cudaMemcpyAsync(h->d_in_depth.get(), h->h_depth.get(), (size_t)W * H * 2, cudaMemcpyHostToDevice, s));
     }
-    *d_depth_out = h->d_in_depth.get();
   }
-  if (bgr) {
-    if (bgr_stride < (size_t)W * 3) return FL_ERR_SIZE;
+  if (bgr && rescale) {
+    FL_CUDA(cudaMemcpy2DAsync(h->d_src_bgr.get(), (size_t)sW * 3, bgr, bgr_stride, (size_t)sW * 3, sH, cudaMemcpyHostToDevice, s));
+    fl_launch_resize_linear(h->d_src_bgr.get(), sW, sH, FL_IMG_8UC3, h->d_in_bgr.get(), W, H, h->rz, s); ++h->launches;
+  } else if (bgr) {
     if (is_pinned(bgr)) {
       if (bgr_stride == (size_t)W * 3) FL_CUDA(cudaMemcpyAsync(h->d_in_bgr.get(), bgr, (size_t)W * H * 3, cudaMemcpyHostToDevice, s));
       else FL_CUDA(cudaMemcpy2DAsync(h->d_in_bgr.get(), (size_t)W * 3, bgr, bgr_stride, (size_t)W * 3, H, cudaMemcpyHostToDevice, s));
@@ -854,14 +903,14 @@ static int stage_frame(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, cons
         if (y1 > y0) FL_CUDA(cudaMemcpyAsync(h->d_in_bgr.get() + (size_t)y0 * W * 3, h->h_bgr.get() + (size_t)y0 * W * 3, (size_t)(y1 - y0) * W * 3, cudaMemcpyHostToDevice, s));
       }
     }
-    *d_bgr_out = h->d_in_bgr.get();
   }
-  for (int m = 0; m < FL_MAX_MODALITIES; ++m) d_masks[m] = nullptr;
   if (masks) for (int m = 0; m < p.n_modalities; ++m) if (masks[m]) {
     memcpy(h->h_mask.get() + (size_t)m * W * H, masks[m], (size_t)W * H);
     FL_CUDA(cudaMemcpyAsync(h->d_mask[0][m].get(), h->h_mask.get() + (size_t)m * W * H, (size_t)W * H, cudaMemcpyHostToDevice, s));
-    d_masks[m] = h->d_mask[0][m].get(); *any_mask = true;
+    d->masks[m] = h->d_mask[0][m].get();
   }
+  d->bgr = bgr ? h->d_in_bgr.get() : nullptr; d->depth = depth ? h->d_in_depth.get() : nullptr;
+  h->staged.W = W; h->staged.H = H; h->staged.bgr = bgr != nullptr; h->staged.depth = depth != nullptr;
   return FL_OK;
 }
 
@@ -894,19 +943,17 @@ static int read_quantized(fl_handle* h, int l, int m, uint8_t* dst) {
 extern "C" int fl_match_async(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int32_t W, int32_t H,
                               const uint8_t* const* masks, float threshold, const int32_t* class_filter, int32_t n_filter) {
   if (!h) return FL_ERR_ARG;
-  const fl_params_t& p = h->p;
-  // an asynchronous frame still in flight may be reading the staging buffers this call is about to overwrite
-  if (h->pend_sort) { fl_set_error("fl_match_wait has not been called for the previous frame"); return FL_ERR_STATE; }
-  h->in_depth_W = h->in_depth_H = 0;                                               // d_in_depth counts as "the matched frame" only once this call has succeeded
-  if (W <= 0 || H <= 0 || W > p.max_width || H > p.max_height) return FL_ERR_SIZE;
-  FL_CUDA(cudaSetDevice(p.device));
-  const uint8_t* d_bgr; const uint16_t* d_depth;
-  const void* d_masks[FL_MAX_MODALITIES];
-  bool any_mask;
-  TRY(stage_frame(h, bgr, bgr_stride, depth, depth_stride, W, H, masks, &d_bgr, &d_depth, d_masks, &any_mask));
-  TRY(fl_match_device_async(h, d_bgr, d_depth, W, H, any_mask ? d_masks : nullptr, threshold, class_filter, n_filter));
-  if (d_depth) { h->in_depth_W = W; h->in_depth_H = H; }
-  return FL_OK;
+  fl_dev_frame d;
+  TRY(frame_begin(h));
+  TRY(stage_host(h, bgr, bgr_stride, depth, depth_stride, W, H, W, H, masks, &d));
+  return fl_match_device_async(h, d.bgr, d.depth, W, H, d.masks, threshold, class_filter, n_filter);
+}
+
+// the end of the synchronous host-frame calls.  A frame whose wait fails leaves no matched depth frame behind.
+static int wait_fetch(fl_handle* h, fl_match_t* out, int32_t capacity, int32_t* count) {
+  const int rc = fl_match_wait(h);
+  if (rc != FL_OK) { h->staged.matched = false; return rc; }
+  return fl_match_fetch(h, out, capacity, count);
 }
 
 extern "C" int fl_match(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int32_t W, int32_t H,
@@ -915,12 +962,9 @@ extern "C" int fl_match(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, con
   if (!h || !count) return FL_ERR_ARG;
   *count = 0;
   const fl_params_t& p = h->p;
-  int rc = fl_match_async(h, bgr, bgr_stride, depth, depth_stride, W, H, masks, threshold, class_filter, n_filter);
-  if (rc != FL_OK) return rc;
-  rc = fl_match_wait(h);
-  if (rc != FL_OK) { h->in_depth_W = h->in_depth_H = 0; return rc; }
-  rc = fl_match_fetch(h, out, capacity, count);
-  if (quantized_out) {
+  TRY(fl_match_async(h, bgr, bgr_stride, depth, depth_stride, W, H, masks, threshold, class_filter, n_filter));
+  const int rc = wait_fetch(h, out, capacity, count);
+  if (quantized_out && h->have_result) {
     for (int l = 0; l < p.n_levels; ++l) for (int m = 0; m < p.n_modalities; ++m)
       if (quantized_out[l * p.n_modalities + m]) TRY(read_quantized(h, l, m, quantized_out[l * p.n_modalities + m]));
     FL_CUDA(cudaStreamSynchronize(h->stream.get()));
@@ -1075,6 +1119,7 @@ extern "C" int fl_match_shard_device(fl_handle* h, const void* d_bgr, const void
                                      float threshold, const int32_t* class_filter, int32_t n_filter, fl_match_t* d_candidates,
                                      int32_t capacity, int32_t* d_count) {
   if (!h || !d_candidates || !d_count || capacity < 1) return FL_ERR_ARG;
+  TRY(frame_begin(h));           // (its front end shares the time-out flag that the wait of a frame in flight reads; it starts no frame itself)
   return run_match_stages(h, (const uint8_t*)d_bgr, (const uint16_t*)d_depth, W, H, d_masks, threshold, class_filter, n_filter, d_candidates,
                           capacity, d_count);
 }
@@ -1082,7 +1127,7 @@ extern "C" int fl_match_shard_device(fl_handle* h, const void* d_bgr, const void
 extern "C" int fl_sort_unique_device(fl_handle* h, const fl_match_t* d_in, int32_t n_lists, int32_t list_capacity, const int32_t* d_n_in,
                                      fl_match_t* d_out, int32_t out_capacity, int32_t* d_out_count) {
   if (!h || !d_in || !d_n_in || !d_out || !d_out_count || n_lists < 1 || list_capacity < 1 || out_capacity < 1) return FL_ERR_ARG;
-  FL_CUDA(cudaSetDevice(h->p.device));
+  TRY(frame_begin(h));
   const fl_lists lists = {d_in, n_lists, list_capacity, list_capacity, d_n_in, 1};
   return run_sort_unique(h, lists, d_out, out_capacity, d_out_count, false);
 }
@@ -1092,21 +1137,29 @@ extern "C" size_t fl_exchange_buffer_bytes(int32_t world, int32_t capacity) {
   return fl_reco_mailbox_offset(world, capacity) + FL_RECO_MAILBOX_WORDS * sizeof(int);   // blocks, then the result mailbox (fl_internal.cuh)
 }
 
+// The peer exchange of a template-sharded frame: rank `rank` of `world` pushes `block` into every peer's buffer (peers: as mapped into
+// this process), and `lists` is what the multi-kernel fallback sorts - this rank's own buffer at the epoch's parity, filled by the
+// kernel's exchange.
+static int exchange_setup(int rank, int world, void* const* peers, int capacity, const fl_match_t* block, uint32_t epoch, fl_xchg* X, fl_lists* lists) {
+  if (!peers || !block || world < 1 || world > FL_XCHG_MAX_WORLD || rank < 0 || rank >= world || capacity < 1 || epoch == 0) return FL_ERR_ARG;
+  memset(X, 0, sizeof *X);
+  X->world = world; X->rank = rank; X->cap = capacity; X->epoch = epoch; X->local_block = block;
+  for (int p = 0; p < world; ++p) { if (!peers[p]) return FL_ERR_ARG; X->peer[p] = static_cast<uint8_t*>(peers[p]); }
+  const uint8_t* own = X->peer[rank] + FL_XCHG_SIGNALS * sizeof(unsigned) + (size_t)(epoch & 1u) * world * ((size_t)capacity + 1) * sizeof(fl_match_t);
+  *lists = {reinterpret_cast<const fl_match_t*>(own) + 1, world, capacity, capacity + 1, reinterpret_cast<const int*>(own), 5 * (capacity + 1)};
+  return FL_OK;
+}
+
 extern "C" int fl_exchange_sort_unique_device_async(fl_handle* h, int32_t rank, int32_t world, void* const* peer_buffers, int32_t capacity,
                                                     const fl_match_t* d_local_block, uint32_t epoch) {
-  if (!h || !peer_buffers || !d_local_block || world < 1 || world > FL_XCHG_MAX_WORLD || rank < 0 || rank >= world || capacity < 1 || epoch == 0) return FL_ERR_ARG;
-  FL_CUDA(cudaSetDevice(h->p.device));
-  if (h->pend_sort) { fl_set_error("fl_match_wait has not been called for the previous frame"); return FL_ERR_STATE; }
-  h->have_result = false; h->pend_match = false;
+  if (!h) return FL_ERR_ARG;
+  fl_xchg X; fl_lists lists;
+  TRY(exchange_setup(rank, world, peer_buffers, capacity, d_local_block, epoch, &X, &lists));
+  TRY(frame_begin(h));
   if (h->profile) for (int i = 0; i < 4; ++i) cudaEventRecord(h->ev[i].get(), h->stream.get());
-  fl_xchg X;
-  memset(&X, 0, sizeof X);
-  X.world = world; X.rank = rank; X.cap = capacity; X.epoch = epoch; X.local_block = d_local_block;
-  for (int p = 0; p < world; ++p) { if (!peer_buffers[p]) return FL_ERR_ARG; X.peer[p] = static_cast<uint8_t*>(peer_buffers[p]); }
-  // the lists the multi-kernel fallback would read: this rank's own buffer, parity of this epoch (filled by the kernel's exchange)
-  const uint8_t* own = X.peer[rank] + FL_XCHG_SIGNALS * sizeof(unsigned) + (size_t)(epoch & 1u) * world * ((size_t)capacity + 1) * sizeof(fl_match_t);
-  const fl_lists lists = {reinterpret_cast<const fl_match_t*>(own) + 1, world, capacity, capacity + 1, reinterpret_cast<const int*>(own), 5 * (capacity + 1)};
-  return sort_launch(h, lists, h->d_out, h->p.max_candidates, h->d_out_count, true, &X);
+  TRY(sort_launch(h, lists, h->d_out, h->p.max_candidates, h->d_out_count, true, &X));
+  h->frame.kind = fl_frame_kind::sort; h->frame.rerun = false;
+  return FL_OK;
 }
 
 // Template-sharded frame in one go (enqueue only): front end + matchClass on this handle's shard with the candidates written
@@ -1116,22 +1169,12 @@ extern "C" int fl_match_shard_exchange_device_masked_async(fl_handle* h, const v
                                                            const void* const* d_masks, float threshold, const int32_t* class_filter, int32_t n_filter,
                                                            int32_t rank, int32_t world, void* const* peer_buffers, int32_t capacity,
                                                            fl_match_t* d_local_block, uint32_t epoch) {
-  if (!h || !peer_buffers || !d_local_block || world < 1 || world > FL_XCHG_MAX_WORLD || rank < 0 || rank >= world || capacity < 1 || epoch == 0) return FL_ERR_ARG;
-  FL_CUDA(cudaSetDevice(h->p.device));
-  if (h->pend_sort) { fl_set_error("fl_match_wait has not been called for the previous frame"); return FL_ERR_STATE; }
-  h->have_result = false; h->pend_match = false;
-  const bool defer = !h->opt_split_refine && h->n_templates > 0 && h->p.n_levels > 1;
-  fl_match_t* recs = d_local_block + 1;
-  int* d_cnt = reinterpret_cast<int*>(d_local_block);
-  TRY(run_match_stages(h, (const uint8_t*)d_bgr, (const uint16_t*)d_depth, W, H, d_masks, threshold, class_filter, n_filter, recs, capacity, d_cnt, defer));
-  fl_xchg X;
-  memset(&X, 0, sizeof X);
-  X.world = world; X.rank = rank; X.cap = capacity; X.epoch = epoch; X.local_block = d_local_block;
-  for (int p = 0; p < world; ++p) { if (!peer_buffers[p]) return FL_ERR_ARG; X.peer[p] = static_cast<uint8_t*>(peer_buffers[p]); }
-  const uint8_t* own = X.peer[rank] + FL_XCHG_SIGNALS * sizeof(unsigned) + (size_t)(epoch & 1u) * world * ((size_t)capacity + 1) * sizeof(fl_match_t);
-  const fl_lists lists = {reinterpret_cast<const fl_match_t*>(own) + 1, world, capacity, capacity + 1, reinterpret_cast<const int*>(own), 5 * (capacity + 1)};
-  const fl_refine_req req = {threshold, recs, capacity, d_cnt};
-  return sort_launch(h, lists, h->d_out, h->p.max_candidates, h->d_out_count, true, &X, defer ? &req : nullptr);
+  if (!h) return FL_ERR_ARG;
+  fl_xchg X; fl_lists lists;
+  TRY(exchange_setup(rank, world, peer_buffers, capacity, d_local_block, epoch, &X, &lists));
+  TRY(frame_begin(h));
+  return match_launch(h, d_bgr, d_depth, W, H, d_masks, threshold, class_filter, n_filter, d_local_block + 1, capacity, reinterpret_cast<int*>(d_local_block),
+                      lists, &X);
 }
 extern "C" int fl_match_shard_exchange_device_async(fl_handle* h, const void* d_bgr, const void* d_depth, int32_t W, int32_t H, float threshold,
                                                     const int32_t* class_filter, int32_t n_filter, int32_t rank, int32_t world,
@@ -1145,18 +1188,11 @@ extern "C" int fl_match_shard_exchange_masked_async(fl_handle* h, const uint8_t*
                                                     int32_t n_filter, int32_t rank, int32_t world, void* const* peer_buffers, int32_t capacity,
                                                     fl_match_t* d_local_block, uint32_t epoch) {
   if (!h) return FL_ERR_ARG;
-  if (h->pend_sort) { fl_set_error("fl_match_wait has not been called for the previous frame"); return FL_ERR_STATE; }
-  h->in_depth_W = h->in_depth_H = 0;
-  if (W <= 0 || H <= 0 || W > h->p.max_width || H > h->p.max_height) return FL_ERR_SIZE;
-  FL_CUDA(cudaSetDevice(h->p.device));
-  const uint8_t* d_bgr; const uint16_t* d_depth;
-  const void* d_masks[FL_MAX_MODALITIES];
-  bool any_mask;
-  TRY(stage_frame(h, bgr, bgr_stride, depth, depth_stride, W, H, masks, &d_bgr, &d_depth, d_masks, &any_mask));
-  TRY(fl_match_shard_exchange_device_masked_async(h, d_bgr, d_depth, W, H, any_mask ? d_masks : nullptr, threshold, class_filter, n_filter, rank, world,
-                                                  peer_buffers, capacity, d_local_block, epoch));
-  if (d_depth) { h->in_depth_W = W; h->in_depth_H = H; }
-  return FL_OK;
+  fl_dev_frame d;
+  TRY(frame_begin(h));
+  TRY(stage_host(h, bgr, bgr_stride, depth, depth_stride, W, H, W, H, masks, &d));
+  return fl_match_shard_exchange_device_masked_async(h, d.bgr, d.depth, W, H, d.masks, threshold, class_filter, n_filter, rank, world, peer_buffers, capacity,
+                                                     d_local_block, epoch);
 }
 extern "C" int fl_match_shard_exchange_async(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int32_t W, int32_t H,
                                              float threshold, const int32_t* class_filter, int32_t n_filter, int32_t rank, int32_t world,
@@ -1174,8 +1210,7 @@ extern "C" int fl_exchange_sort_unique_device(fl_handle* h, int32_t rank, int32_
 
 extern "C" int fl_sort_unique_blocks_device(fl_handle* h, const fl_match_t* d_blocks, int32_t n_blocks, int32_t capacity) {
   if (!h || !d_blocks || n_blocks < 1 || capacity < 1) return FL_ERR_ARG;
-  FL_CUDA(cudaSetDevice(h->p.device));
-  h->have_result = false;
+  TRY(frame_begin(h));
   if (h->profile) for (int i = 0; i < 4; ++i) cudaEventRecord(h->ev[i].get(), h->stream.get());   // stage times are not defined for this entry point
   const fl_lists lists = {d_blocks + 1, n_blocks, capacity, capacity + 1, reinterpret_cast<const int*>(d_blocks), 5 * (capacity + 1)};
   TRY(run_sort_unique(h, lists, h->d_out, h->p.max_candidates, h->d_out_count, true));
@@ -1300,49 +1335,22 @@ extern "C" int fl_resize_linear(fl_handle* h, const void* src, size_t src_stride
   return FL_OK;
 }
 
-// upload of a src_W x src_H frame and its INTER_LINEAR rescale into d_in_bgr / d_in_depth (the host-input staging of W x H frames)
-static int stage_rescaled(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int sW, int sH, int W, int H,
-                          const uint8_t** d_bgr_out, const uint16_t** d_depth_out) {
-  *d_bgr_out = nullptr; *d_depth_out = nullptr;
-  if ((bgr && bgr_stride < (size_t)sW * 3) || (depth && depth_stride < (size_t)sW * 2)) return FL_ERR_SIZE;
-  cudaStream_t s = h->stream.get();
-  TRY(resize_tables(h, sW, sH, W, H));
-  TRY(resize_staging(h, (size_t)sW * sH));
-  if (depth) {
-    FL_CUDA(cudaMemcpy2DAsync(h->d_src_depth.get(), (size_t)sW * 2, depth, depth_stride, (size_t)sW * 2, sH, cudaMemcpyHostToDevice, s));
-    fl_launch_resize_linear(h->d_src_depth.get(), sW, sH, FL_IMG_16UC1, h->d_in_depth.get(), W, H, h->rz, s); ++h->launches;
-    *d_depth_out = h->d_in_depth.get();
-  }
-  if (bgr) {
-    FL_CUDA(cudaMemcpy2DAsync(h->d_src_bgr.get(), (size_t)sW * 3, bgr, bgr_stride, (size_t)sW * 3, sH, cudaMemcpyHostToDevice, s));
-    fl_launch_resize_linear(h->d_src_bgr.get(), sW, sH, FL_IMG_8UC3, h->d_in_bgr.get(), W, H, h->rz, s); ++h->launches;
-    *d_bgr_out = h->d_in_bgr.get();
-  }
-  return FL_OK;
-}
-
 extern "C" int fl_match_rescaled(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int32_t sW, int32_t sH,
                                  int32_t W, int32_t H, float threshold, const int32_t* class_filter, int32_t n_filter, fl_match_t* out, int32_t capacity,
                                  int32_t* count, uint16_t* rescaled_depth_out) {
   if (!h || !count || sW <= 0 || sH <= 0) return FL_ERR_ARG;
   *count = 0;
-  const fl_params_t& p = h->p;
-  if (h->pend_sort) { fl_set_error("fl_match_wait has not been called for the previous frame"); return FL_ERR_STATE; }
-  h->in_depth_W = h->in_depth_H = 0;
-  if (W <= 0 || H <= 0 || W > p.max_width || H > p.max_height) return FL_ERR_SIZE;
-  if (sW == W && sH == H) {                                                      // TImage2Mat resizes only when the width differs (:42)
-    int rc = fl_match(h, bgr, bgr_stride, depth, depth_stride, W, H, nullptr, threshold, class_filter, n_filter, out, capacity, count, nullptr);
-    if (rescaled_depth_out && depth) for (int y = 0; y < H; ++y) memcpy(rescaled_depth_out + (size_t)y * W, (const uint8_t*)depth + (size_t)y * depth_stride, (size_t)W * 2);
-    return rc;
+  fl_dev_frame d;
+  TRY(frame_begin(h));
+  TRY(stage_host(h, bgr, bgr_stride, depth, depth_stride, sW, sH, W, H, nullptr, &d));
+  if (rescaled_depth_out && depth) {
+    if (sW == W && sH == H)                                                      // TImage2Mat resizes only when the size differs (:42)
+      for (int y = 0; y < H; ++y) memcpy(rescaled_depth_out + (size_t)y * W, (const uint8_t*)depth + (size_t)y * depth_stride, (size_t)W * 2);
+    else
+      FL_CUDA(cudaMemcpyAsync(rescaled_depth_out, h->d_in_depth.get(), (size_t)W * H * 2, cudaMemcpyDeviceToHost, h->stream.get()));
   }
-  FL_CUDA(cudaSetDevice(p.device));
-  const uint8_t* d_bgr = nullptr; const uint16_t* d_depth = nullptr;
-  TRY(stage_rescaled(h, bgr, bgr_stride, depth, depth_stride, sW, sH, W, H, &d_bgr, &d_depth));
-  if (d_depth && rescaled_depth_out) FL_CUDA(cudaMemcpyAsync(rescaled_depth_out, h->d_in_depth.get(), (size_t)W * H * 2, cudaMemcpyDeviceToHost, h->stream.get()));
-  int rc = fl_match_device(h, d_bgr, d_depth, W, H, nullptr, threshold, class_filter, n_filter);
-  if (rc != FL_OK) return rc;
-  if (d_depth) { h->in_depth_W = W; h->in_depth_H = H; }
-  return fl_match_fetch(h, out, capacity, count);
+  TRY(fl_match_device_async(h, d.bgr, d.depth, W, H, nullptr, threshold, class_filter, n_filter));
+  return wait_fetch(h, out, capacity, count);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -1411,7 +1419,11 @@ static bool rect_inside(const fl_rect_t& a, int W, int H) {
 // host-input fl_match left in d_in_depth (Recognition hands the same image to match and to detection, obj_reco_lmicp.cpp:101, 188)
 static int icp_ref_frame(fl_handle* h, const uint16_t* ref_depth, size_t ref_stride, int W, int H, const uint16_t** d_ref) {
   if (!ref_depth) {
-    if (h->in_depth_W != W || h->in_depth_H != H) { fl_set_error("ref_depth == NULL needs a preceding fl_match of a %d x %d depth frame on this handle (have %d x %d)", W, H, h->in_depth_W, h->in_depth_H); return FL_ERR_STATE; }
+    const fl_staged_frame& st = h->staged;
+    if (!st.matched || st.W != W || st.H != H) {
+      fl_set_error("ref_depth == NULL needs a preceding fl_match of a %d x %d depth frame on this handle (have %d x %d)", W, H, st.matched ? st.W : 0, st.matched ? st.H : 0);
+      return FL_ERR_STATE;
+    }
     *d_ref = h->d_in_depth.get();
     return FL_OK;
   }
@@ -1623,7 +1635,7 @@ extern "C" void fl_default_reco_params(fl_reco_params_t* p) {
 // member's handle selects from.
 int fl_reco_setup(fl_handle* h, const fl_reco_params_t* prm, const fl_reco_set& set, const int32_t* crop_of_template, const float* pose12) {
   if (!h || !prm || !crop_of_template || prm->top_k < 1 || set.n_templates < 0 || (set.n_templates > 0 && (!set.class_of || !set.box0))) return FL_ERR_ARG;
-  if (h->pend_sort) { fl_set_error("fl_set_recognition: a frame is in flight on this handle"); return FL_ERR_STATE; }
+  TRY(frame_idle(h));
   if (set.n_templates == 0) { fl_set_error("fl_set_recognition: no templates uploaded"); return FL_ERR_STATE; }
   if (!pose12 && !set.pose13) { fl_set_error("fl_set_recognition: no pose table (pose12 NULL and no pose13 uploaded)"); return FL_ERR_ARG; }
   int nc = 0;
@@ -1669,7 +1681,7 @@ int fl_reco_setup(fl_handle* h, const fl_reco_params_t* prm, const fl_reco_set& 
 
 extern "C" int fl_set_recognition(fl_handle* h, const fl_reco_params_t* prm, const int32_t* crop_of_template, const float* pose12) {
   if (!h || !prm || !crop_of_template || prm->top_k < 1) return FL_ERR_ARG;
-  if (h->pend_sort) { fl_set_error("fl_set_recognition: a frame is in flight on this handle"); return FL_ERR_STATE; }
+  TRY(frame_idle(h));
   if (h->n_templates == 0) { fl_set_error("fl_set_recognition: no templates uploaded"); return FL_ERR_STATE; }
   // matches carry the ids of fl_set_template_ids (a shard's global ids): the template behind a match is not class_first + template_id
   if (h->custom_tids) { fl_set_error("fl_set_recognition: not available on a handle with fl_set_template_ids (template shards)"); return FL_ERR_STATE; }
@@ -1690,13 +1702,13 @@ static int reco_enqueue(fl_handle* h, bool check_big, const fl_reco_push* push =
   cudaStream_t s = h->stream.get();
   const int max_hyp = h->reco_max_hyp;
   int nl = fl_launch_reco_select(h->d_out, reinterpret_cast<const int*>(h->d_outblk.get()), h->p.max_candidates, check_big ? 1 : 0, h->d_reco_class_first.get(),
-                                 h->reco_n_classes, h->reco_n_templates, h->d_reco_tmpl.get(), h->reco.top_k, h->reco.per_class, max_hyp, h->reco_W, h->reco_H,
+                                 h->reco_n_classes, h->reco_n_templates, h->d_reco_tmpl.get(), h->reco.top_k, h->reco.per_class, max_hyp, h->staged.W, h->staged.H,
                                  h->icpw.d_hyps.get(), h->d_reco_sel.get(), s);
   if (nl < 0) { fl_set_error("hypothesis selection launch failed: %s", cudaGetErrorString(cudaGetLastError())); return FL_ERR_CUDA; }
   h->launches += nl;
   fl_icp_ws ws = h->icp;
   ws.n_hyp = max_hyp;                                                              // padding hypotheses are skipped by the kernel
-  nl = fl_launch_icp(ws, h->reco.icp, h->icpw.d_hyps.get(), h->d_in_depth.get(), h->reco_W, h->reco_H, h->reco_K, h->icpw.d_results.get(), h->icpw.d_ticket.get(), nullptr, h->n_sm, s);
+  nl = fl_launch_icp(ws, h->reco.icp, h->icpw.d_hyps.get(), h->d_in_depth.get(), h->staged.W, h->staged.H, h->frame.K, h->icpw.d_results.get(), h->icpw.d_ticket.get(), nullptr, h->n_sm, s);
   if (nl < 0) { fl_set_error("ICP kernel launch failed: %s", cudaGetErrorString(cudaGetLastError())); return FL_ERR_CUDA; }
   h->launches += nl;
   nl = fl_launch_reco_finish(h->d_out, h->d_reco_sel.get(), h->icpw.d_results.get(), max_hyp, h->reco.th_obj_dist, h->d_reco_host, push, s);
@@ -1705,36 +1717,25 @@ static int reco_enqueue(fl_handle* h, bool check_big, const fl_reco_push* push =
   return FL_OK;
 }
 
-// the upload of a recognition frame into d_in_bgr / d_in_depth, rescaled on the device when src_W x src_H differs from W x H
+// the upload of a recognition frame (rescaled on the device when src_W x src_H differs from W x H, TImage2Mat :42) and its intrinsics
 static int reco_stage(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int sW, int sH, int W, int H,
-                      fl_intrinsics_t K_ref, const uint8_t** d_bgr, const uint16_t** d_depth) {
-  const fl_params_t& p = h->p;
-  if (h->pend_sort) { fl_set_error("the previous frame of this handle has not been waited for"); return FL_ERR_STATE; }
+                      fl_intrinsics_t K_ref, fl_dev_frame* d) {
+  if (!h || !depth || sW <= 0 || sH <= 0) return FL_ERR_ARG;
+  TRY(frame_begin(h));
   if (!h->reco_set) { fl_set_error("fl_recognize: call fl_set_recognition after the template and crop uploads"); return FL_ERR_STATE; }
-  h->in_depth_W = h->in_depth_H = 0;
-  if (W <= 0 || H <= 0 || W > p.max_width || H > p.max_height) return FL_ERR_SIZE;
+  TRY(stage_host(h, bgr, bgr_stride, depth, depth_stride, sW, sH, W, H, nullptr, d));
   if (h->reco_any_crop && (W != h->res_W || H != h->res_H)) { fl_set_error("model depth crops were uploaded for %d x %d frames, not %d x %d", h->res_W, h->res_H, W, H); return FL_ERR_STATE; }
-  FL_CUDA(cudaSetDevice(p.device));
-  if (sW == W && sH == H) {                                                      // TImage2Mat resizes only when the size differs (:42)
-    const void* d_masks[FL_MAX_MODALITIES];
-    bool any_mask;
-    TRY(stage_frame(h, bgr, bgr_stride, depth, depth_stride, W, H, nullptr, d_bgr, d_depth, d_masks, &any_mask));
-  } else {
-    TRY(stage_rescaled(h, bgr, bgr_stride, depth, depth_stride, sW, sH, W, H, d_bgr, d_depth));
-  }
-  h->reco_W = W; h->reco_H = H; h->reco_K = K_ref; h->reco_bgr = *d_bgr != nullptr;
+  h->frame.K = K_ref;
   return FL_OK;
 }
 
 extern "C" int fl_recognize_async(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,
                                   int32_t sW, int32_t sH, int32_t W, int32_t H, fl_intrinsics_t K_ref) {
-  if (!h || !depth || sW <= 0 || sH <= 0) return FL_ERR_ARG;
-  const uint8_t* d_bgr; const uint16_t* d_depth;
-  TRY(reco_stage(h, bgr, bgr_stride, depth, depth_stride, sW, sH, W, H, K_ref, &d_bgr, &d_depth));
-  TRY(fl_match_device_async(h, d_bgr, d_depth, W, H, nullptr, h->reco.threshold, nullptr, 0));
-  h->in_depth_W = W; h->in_depth_H = H;
+  fl_dev_frame d;
+  TRY(reco_stage(h, bgr, bgr_stride, depth, depth_stride, sW, sH, W, H, K_ref, &d));
+  TRY(fl_match_device_async(h, d.bgr, d.depth, W, H, nullptr, h->reco.threshold, nullptr, 0));
   TRY(reco_enqueue(h, true));
-  h->pend_reco = true;
+  h->frame.kind = fl_frame_kind::reco;
   return FL_OK;
 }
 
@@ -1747,42 +1748,35 @@ extern "C" int fl_recognize_async(fl_handle* h, const uint8_t* bgr, size_t bgr_s
 // again on the frames already staged.
 int fl_reco_shard_stage(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride, int sW, int sH, int W, int H,
                         fl_intrinsics_t K_ref) {
-  if (!h || !depth || sW <= 0 || sH <= 0) return FL_ERR_ARG;
-  const uint8_t* d_bgr; const uint16_t* d_depth;
-  TRY(reco_stage(h, bgr, bgr_stride, depth, depth_stride, sW, sH, W, H, K_ref, &d_bgr, &d_depth));
-  return FL_OK;
+  fl_dev_frame d;
+  return reco_stage(h, bgr, bgr_stride, depth, depth_stride, sW, sH, W, H, K_ref, &d);
 }
 
 int fl_reco_shard_match(fl_handle* h, int rank, int world, void* const* peers, int capacity, fl_match_t* block, uint32_t epoch) {
   if (!h) return FL_ERR_ARG;
-  if (h->pend_sort || !h->reco_set || h->reco_W == 0) { fl_set_error("no staged recognition frame on this handle"); return FL_ERR_STATE; }
-  FL_CUDA(cudaSetDevice(h->p.device));
-  h->pend_reco = false;
-  const uint8_t* d_bgr = h->reco_bgr ? h->d_in_bgr.get() : nullptr;
-  TRY(fl_match_shard_exchange_device_async(h, d_bgr, h->d_in_depth.get(), h->reco_W, h->reco_H, h->reco.threshold, nullptr, 0, rank, world, peers, capacity,
-                                           block, epoch));
-  h->in_depth_W = h->reco_W; h->in_depth_H = h->reco_H;
-  return FL_OK;
+  if (!h->reco_set || !h->staged.depth) { fl_set_error("no staged recognition frame on this handle"); return FL_ERR_STATE; }
+  return fl_match_shard_exchange_device_async(h, h->staged.bgr ? h->d_in_bgr.get() : nullptr, h->d_in_depth.get(), h->staged.W, h->staged.H, h->reco.threshold,
+                                              nullptr, 0, rank, world, peers, capacity, block, epoch);
 }
 
 int fl_reco_shard_tail(fl_handle* h, const fl_reco_push* push) {
   if (!h) return FL_ERR_ARG;
-  if (!h->pend_sort || !h->reco_set) { fl_set_error("no matched recognition frame on this handle"); return FL_ERR_STATE; }
+  if (h->frame.kind != fl_frame_kind::shard || !h->reco_set) { fl_set_error("no matched recognition frame on this handle"); return FL_ERR_STATE; }
   FL_CUDA(cudaSetDevice(h->p.device));
   TRY(reco_enqueue(h, true, push));
-  h->pend_reco = true;
+  h->frame.kind = fl_frame_kind::reco;
   return FL_OK;
 }
 
 int fl_reco_shard_receive(fl_handle* h, const uint8_t* own_buffer, size_t mailbox_off, uint32_t epoch, int owner) {
   if (!h || !own_buffer) return FL_ERR_ARG;
-  if (!h->pend_sort || !h->reco_set) { fl_set_error("no matched recognition frame on this handle"); return FL_ERR_STATE; }
+  if (h->frame.kind != fl_frame_kind::shard || !h->reco_set) { fl_set_error("no matched recognition frame on this handle"); return FL_ERR_STATE; }
   FL_CUDA(cudaSetDevice(h->p.device));
   if (fl_launch_reco_receive(own_buffer, mailbox_off, epoch, owner, h->d_reco_host, h->stream.get()) < 0) {
     fl_set_error("recognition receive launch failed: %s", cudaGetErrorString(cudaGetLastError())); return FL_ERR_CUDA;
   }
   ++h->launches;
-  h->pend_reco = true;
+  h->frame.kind = fl_frame_kind::reco;
   return FL_OK;
 }
 
@@ -1825,12 +1819,11 @@ int fl_reco_shard_results(fl_handle* h, fl_reco_result_t* out, int32_t capacity,
 extern "C" int fl_recognize_wait(fl_handle* h, fl_reco_result_t* out, int32_t capacity, fl_reco_summary_t* summary) {
   if (!h || capacity < 0 || (capacity > 0 && !out)) return FL_ERR_ARG;
   if (summary) memset(summary, 0, sizeof *summary);
-  if (!h->pend_reco) { fl_set_error("fl_recognize_wait: no recognition frame in flight on this handle"); return FL_ERR_STATE; }
-  h->pend_reco = false;
-  const bool forced_before = h->fe_force_waves;
-  // the frame's one wait; the rare > 1,024-record sorts and the re-run after a front-end dependency time-out are fl_match_wait's
-  TRY(match_wait(h));
-  return reco_results(h, h->fe_force_waves && !forced_before, out, capacity, summary);
+  if (h->frame.kind != fl_frame_kind::reco) { fl_set_error("fl_recognize_wait: no recognition frame in flight on this handle"); return FL_ERR_STATE; }
+  // the frame's one wait; the rare > 1,024-record sorts and the re-run after a front-end dependency time-out are fl_frame_wait's
+  fl_wait_note note;
+  TRY(fl_frame_wait(h, &note));
+  return reco_results(h, note == fl_wait_note::rerun, out, capacity, summary);
 }
 
 extern "C" int fl_recognize(fl_handle* h, const uint8_t* bgr, size_t bgr_stride, const uint16_t* depth, size_t depth_stride,

@@ -26,7 +26,17 @@ struct fl_sort_key { unsigned long long hi, lo; };
 
 void fl_set_error(const char* fmt, ...);
 int fl_entries_per_template(const fl_handle* h);   // n_levels * n_modalities of the handle (api.cu)
-bool fl_recognition_pending(const fl_handle* h);   // a fl_recognize_async frame is in flight on the handle (api.cu)
+
+// The frame in flight on a handle (api.cu), from its enqueue to its wait.  match: fl_match_device_async and the host entry points
+// that stage into it; shard: the fused local match + peer exchange (fl_match_shard_exchange_*); sort: the stand-alone exchange + sort
+// (fl_exchange_sort_unique_device_async); reco: a frame with the recognition tail behind its sort, whose results are still to be collected.
+enum class fl_frame_kind { none, match, shard, sort, reco };
+fl_frame_kind fl_frame_in_flight(const fl_handle* h);
+// What fl_frame_wait did besides waiting for the frame in flight.  After an in-grid dependency time-out of the single-launch front end
+// the handle launches one kernel per wave from then on, and the frame's result is not trustworthy: a frame matched on this handle alone
+// has been run again (rerun); one that exchanged with peers needs every rank, so it must be submitted again (resubmit, FL_ERR_STATE).
+enum class fl_wait_note { done, rerun, resubmit };
+int fl_frame_wait(fl_handle* h, fl_wait_note* note);
 
 // ---- programmatic dependent launch (PDL) -------------------------------------------------------------------------
 // A kernel launched with cudaLaunchAttributeProgrammaticStreamSerialization may have its CTAs resident while the previous kernel

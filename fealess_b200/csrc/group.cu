@@ -20,6 +20,7 @@
 #include "fl_internal.cuh"
 #include "fl_owned.cuh"
 #include <algorithm>
+#include <functional>
 #include <vector>
 
 struct fl_group {
@@ -47,6 +48,26 @@ struct fl_group {
   } while (0)
 
 static int in_flight(const fl_group* g) { return (int)(g->submitted - g->collected); }
+
+// Waits for the frames of the first n members of a slot (hs): each one, whatever the others return; the first error counts.  A member
+// whose single-launch front end timed out on an in-grid dependency has switched itself to per-wave launches and asks for the frame again
+// (fl_frame_wait); every member has to take part in that, so `again`, when given, enqueues the frame once more on all of them.
+static int wait_members(const fl_group* g, fl_handle* const* hs, int n, const char* what = nullptr, const std::function<int()>& again = nullptr) {
+  for (int attempt = 0;; ++attempt) {
+    int first_err = FL_OK;
+    bool resubmit = false;
+    for (int m = 0; m < n; ++m) {
+      GCUDA(cudaSetDevice(g->device[m]));
+      fl_wait_note note;
+      const int rc = fl_frame_wait(hs[m], &note);
+      if (note == fl_wait_note::resubmit) resubmit = true;
+      else if (rc != FL_OK && first_err == FL_OK) first_err = rc;   // (incl. a peer that never arrived)
+    }
+    if (first_err != FL_OK || !resubmit || !again) return first_err;
+    if (attempt == 1) { fl_set_error("%s: the front end timed out twice", what); return FL_ERR_STATE; }
+    if ((first_err = again()) != FL_OK) return first_err;
+  }
+}
 
 extern "C" int fl_group_destroy(fl_group* g) {
   if (!g) return FL_ERR_ARG;
@@ -182,31 +203,19 @@ extern "C" int fl_group_match_masked(fl_group* g, const uint8_t* bgr, size_t bgr
   if (in_flight(g)) { fl_set_error("fl_group_match: %d recognition frame(s) in flight - collect them first", in_flight(g)); return FL_ERR_STATE; }
   if (W <= 0 || H <= 0 || W > g->max_w || H > g->max_h) return FL_ERR_SIZE;
   if ((bgr && bgr_stride < (size_t)W * 3) || (depth && depth_stride < (size_t)W * 2)) return FL_ERR_SIZE;
-  // (a second attempt only when a handle's single-launch front end timed out on an in-grid dependency during the first: that handle
-  //  has switched itself to per-wave launches - fl_match_wait - and asks for the frame again; every rank has to take part in it)
-  for (int attempt = 0; attempt < 2; ++attempt) {
+  auto enqueue = [&]() -> int {                                 // on every handle; nothing waits until all are under way
     const uint32_t e = ++g->epoch[0];
-    int first_err = FL_OK;
-    bool switched = false;
-    int launched = 0;
-    for (int i = 0; i < g->n; ++i) {                            // enqueue on every handle; nothing waits until all are under way
+    for (int i = 0; i < g->n; ++i) {
       GCUDA(cudaSetDevice(g->device[i]));
       const int rc = fl_match_shard_exchange_masked_async(g->h[i], bgr, bgr_stride, depth, depth_stride, W, H, masks, threshold, class_filter, n_filter,
                                                           i, g->n, g->peers.data(), g->cap, g->block[i].get(), e);
-      if (rc != FL_OK) { first_err = rc; break; }                // (the ranks already launched report the missing peer instead of hanging)
-      ++launched;
+      if (rc != FL_OK) { wait_members(g, g->h.data(), i); return rc; }   // (the ranks already launched report the missing peer instead of hanging)
     }
-    for (int i = 0; i < launched; ++i) {
-      cudaSetDevice(g->device[i]);
-      const int forced = fl_debug_option(g->h[i], FL_OPT_FE_FORCED_WAVES, 0);
-      const int rc = fl_match_wait(g->h[i]);
-      if (rc == FL_ERR_STATE && !forced && fl_debug_option(g->h[i], FL_OPT_FE_FORCED_WAVES, 0) == 1) switched = true;   // resubmit
-      else if (rc != FL_OK && first_err == FL_OK) first_err = rc;                                                        // (incl. a peer that never arrived)
-    }
-    if (first_err != FL_OK) return first_err;
-    if (!switched) break;
-    if (attempt == 1) { fl_set_error("fl_group_match: the front end timed out twice"); return FL_ERR_STATE; }
-  }
+    return FL_OK;
+  };
+  int rc = enqueue();
+  if (rc == FL_OK) rc = wait_members(g, g->h.data(), g->n, "fl_group_match", enqueue);
+  if (rc != FL_OK) return rc;
   GCUDA(cudaSetDevice(g->device[0]));
   return fl_match_fetch(g->h[0], out, capacity, count);
 }
@@ -259,16 +268,15 @@ static int enqueue_frame(fl_group* g, int s, long long f, bool restage, const ui
       if (rc != FL_OK) { for (int k = 0; k <= m; ++k) { cudaSetDevice(g->device[k]); fl_sync(hs[k]); } return rc; }   // nothing launched yet
     }
   const uint32_t e = ++g->epoch[s];
-  auto wait_all = [&](int launched) { for (int k = 0; k < launched; ++k) { cudaSetDevice(g->device[k]); fl_match_wait(hs[k]); } };
   for (int m = 0; m < g->n; ++m) {
     int rc = cudaSetDevice(g->device[m]) == cudaSuccess ? FL_OK : FL_ERR_CUDA;
     if (rc == FL_OK) rc = fl_reco_shard_match(hs[m], m, g->n, g->peers.data() + (size_t)s * g->n, g->cap, g->block[(size_t)s * g->n + m].get(), e);
     // the members already under way report the missing peer instead of hanging: wait for them, so that the slot is free again
-    if (rc != FL_OK) { wait_all(m); return rc; }
+    if (rc != FL_OK) { wait_members(g, hs, m); return rc; }
   }
   int rc = cudaSetDevice(g->device[owner]) == cudaSuccess ? FL_OK : FL_ERR_CUDA;
   if (rc == FL_OK) rc = fl_reco_shard_tail(hs[owner]);
-  if (rc != FL_OK) { wait_all(g->n); return rc; }
+  if (rc != FL_OK) { wait_members(g, hs, g->n); return rc; }
   return FL_OK;
 }
 
@@ -294,23 +302,11 @@ extern "C" int fl_group_collect_recognition(fl_group* g, fl_reco_result_t* out, 
   const long long f = g->collected++;                           // the slot is free again whatever the frame's status
   const int s = (int)(f % g->depth), owner = (int)(f % g->n);
   fl_handle* const* hs = g->h.data() + (size_t)s * g->n;
-  for (int attempt = 0; attempt < 2; ++attempt) {
-    int first_err = FL_OK;
-    bool switched = false;
-    for (int m = 0; m < g->n; ++m) {
-      GCUDA(cudaSetDevice(g->device[m]));
-      const int forced = fl_debug_option(hs[m], FL_OPT_FE_FORCED_WAVES, 0);
-      const int rc = fl_match_wait(hs[m]);
-      if (rc == FL_ERR_STATE && !forced && fl_debug_option(hs[m], FL_OPT_FE_FORCED_WAVES, 0) == 1) switched = true;
-      else if (rc != FL_OK && first_err == FL_OK) first_err = rc;
-    }
-    if (first_err != FL_OK) return first_err;
-    if (!switched) break;
-    if (attempt == 1) { fl_set_error("fl_group_collect_recognition: the front end timed out twice"); return FL_ERR_STATE; }
+  const int rc = wait_members(g, hs, g->n, "fl_group_collect_recognition", [&]() {
     const fl_intrinsics_t none = {0.f, 0.f, 0.f, 0.f};           // (restage = false: each handle keeps the frame's geometry and intrinsics)
-    const int rc = enqueue_frame(g, s, f, false, nullptr, 0, nullptr, 0, 0, 0, 0, 0, none);
-    if (rc != FL_OK) return rc;
-  }
+    return enqueue_frame(g, s, f, false, nullptr, 0, nullptr, 0, 0, 0, 0, 0, none);
+  });
+  if (rc != FL_OK) return rc;
   GCUDA(cudaSetDevice(g->device[owner]));
   return fl_reco_shard_results(hs[owner], out, capacity, summary);
 }

@@ -243,7 +243,7 @@ extern "C" int fl_pipe_collect_recognition(fl_pipe* p, fl_reco_result_t* out, in
   if (p->submitted == p->collected) { fl_set_error("fl_pipe_collect_recognition: no frame in flight"); return FL_ERR_STATE; }
   fl_handle* h = p->h[p->collected % p->depth];
   // the oldest frame came from fl_pipe_submit: it stays in flight for fl_pipe_collect (waiting for it here would leave nothing to fetch)
-  if (!fl_recognition_pending(h)) { fl_set_error("fl_pipe_collect_recognition: the oldest frame in flight is a match frame - fl_pipe_collect it"); return FL_ERR_STATE; }
+  if (fl_frame_in_flight(h) != fl_frame_kind::reco) { fl_set_error("fl_pipe_collect_recognition: the oldest frame in flight is a match frame - fl_pipe_collect it"); return FL_ERR_STATE; }
   ++p->collected;                                               // the slot is free again whatever the frame's status
   if (p->world > 1) {
     // a missing peer or owner, an overflowing exchange block: this frame's status only.  A deferred list (more than the 1,024 records
