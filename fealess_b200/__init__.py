@@ -486,12 +486,13 @@ class Handle:
         return buf[128:128 + n].astype(np.int64), buf[:128].view(np.uint32).astype(np.int64)
 
     def fe_trace(self):
-        """FL_DBG_FE_TRACE: [n_jobs, 4] int64 {kind, CTAs, first start ns, last end ns} of the front end of the last frame."""
-        buf = np.zeros(4 * 64, np.uint64)
+        """FL_DBG_FE_TRACE: [n_jobs, 6] int64 {kind, CTAs, first start ns, last end ns, summed CTA spans in SM cycles, the same in ns}
+        of the front end of the last frame."""
+        buf = np.zeros(6 * 64, np.uint64)
         n = lib().fl_debug_get(self._h, FL_DBG_FE_TRACE, 0, 0, 0, C.c_void_p(buf.ctypes.data), C.c_size_t(buf.nbytes))
         if n < 0:
             _check(n, "fl_debug_get(FL_DBG_FE_TRACE)")
-        return buf[:n * 4].reshape(n, 4).astype(np.int64)
+        return buf[:n * 6].reshape(n, 6).astype(np.int64)
 
     def keep_spread(self, enable=True):
         _check(lib().fl_debug_keep_spread(self._h, int(enable)), "fl_debug_keep_spread")

@@ -602,10 +602,10 @@ static int run_match_stages(fl_handle* h, const uint8_t* d_bgr, const uint16_t* 
         consume(is_color ? slot_color[l][m] : slot_depth[m]);
         consume_rows(is_color ? slot_color[l][m] : slot_depth[m], is_color ? 0 : l);
       }
-    if (h->opt_trace) {                                                        // developer timeline: per job first start / last end
+    if (h->opt_trace) {                                                        // developer timeline: per job first start / last end, summed CTA spans
       TRY(h->d_fe_trace.grow(2 * FL_FE_MAX_JOBS + 2 * FL_FE_MAX_JOBS));
-      unsigned long long init[2 * FL_FE_MAX_JOBS];
-      for (int i = 0; i < FL_FE_MAX_JOBS; ++i) { init[2 * i] = ~0ull; init[2 * i + 1] = 0; }
+      unsigned long long init[4 * FL_FE_MAX_JOBS];
+      for (int i = 0; i < FL_FE_MAX_JOBS; ++i) { init[2 * i] = ~0ull; init[2 * i + 1] = 0; init[2 * FL_FE_MAX_JOBS + 2 * i] = init[2 * FL_FE_MAX_JOBS + 2 * i + 1] = 0; }
       FL_CUDA(cudaMemcpyAsync(h->d_fe_trace.get(), init, sizeof init, cudaMemcpyHostToDevice, s));
       FL_CUDA(cudaStreamSynchronize(s));
       w.trace = h->d_fe_trace.get();
@@ -1262,13 +1262,16 @@ extern "C" int fl_debug_get(fl_handle* h, int what, int32_t a, int32_t b, int32_
     memcpy(host_out, h->h_small, 16 * sizeof(int));
     return FL_OK;
   }
-  if (what == FL_DBG_FE_TRACE) {                                                               // developer: front-end job timeline {kind, ctas, start, end} x jobs (FL_OPT_TRACE)
+  if (what == FL_DBG_FE_TRACE) {                                                               // developer: front-end job timeline {kind, ctas, start, end, cycles, ns} x jobs (FL_OPT_TRACE)
     if (!h->d_fe_trace.get() || h->fe_trace_jobs <= 0) return FL_ERR_STATE;
-    if (bytes < (size_t)h->fe_trace_jobs * 4 * sizeof(unsigned long long)) return FL_ERR_CAPACITY;
-    unsigned long long raw[2 * FL_FE_MAX_JOBS];
+    if (bytes < (size_t)h->fe_trace_jobs * 6 * sizeof(unsigned long long)) return FL_ERR_CAPACITY;
+    unsigned long long raw[4 * FL_FE_MAX_JOBS];
     FL_CUDA(cudaMemcpy(raw, h->d_fe_trace.get(), sizeof raw, cudaMemcpyDeviceToHost));
     unsigned long long* o = static_cast<unsigned long long*>(host_out);
-    for (int i = 0; i < h->fe_trace_jobs; ++i) { o[4 * i] = (unsigned long long)h->fe_trace_kind[i]; o[4 * i + 1] = (unsigned long long)h->fe_trace_ctas[i]; o[4 * i + 2] = raw[2 * i]; o[4 * i + 3] = raw[2 * i + 1]; }
+    for (int i = 0; i < h->fe_trace_jobs; ++i) {
+      o[6 * i] = (unsigned long long)h->fe_trace_kind[i]; o[6 * i + 1] = (unsigned long long)h->fe_trace_ctas[i]; o[6 * i + 2] = raw[2 * i]; o[6 * i + 3] = raw[2 * i + 1];
+      o[6 * i + 4] = raw[2 * FL_FE_MAX_JOBS + 2 * i]; o[6 * i + 5] = raw[2 * FL_FE_MAX_JOBS + 2 * i + 1];
+    }
     return h->fe_trace_jobs;
   }
   if (what == FL_DBG_STAGED_ORDER) {                                                           // the phase order of the last staged launch

@@ -16,10 +16,11 @@
 // tables: NORMAL_LUT depends only on (v2, v1) -> 400 bytes; response table packs the 8 per-label responses of one
 // spread byte into a uint2 (labels 0-3 in .x, 4-7 in .y), i.e. SIMILARITY_LUT (linemod.cpp:970) re-indexed by pixel value.
 // ------------------------------------------------------------------------------------------------
-__constant__ uint8_t c_normal_plane[400];
+// g_*: in global memory, copied to shared memory by every CTA that indexes them per thread (one coalesced load per thread); the
+// constant cache would serialise a warp's 32 distinct addresses
+__device__ __align__(4) uint8_t g_normal_plane[400];
 __constant__ uint2 c_resp8[256];
-__device__ uint2 g_resp8[256];          // same table in global memory: 256 threads copy it to shared memory with ONE coalesced load each
-                                        // (the constant cache serialises a warp's 32 distinct addresses)
+__device__ uint2 g_resp8[256];
 
 int fl_launch_tables_init() {
   uint8_t plane[400];
@@ -46,7 +47,7 @@ int fl_launch_tables_init() {
     }
     resp[v] = make_uint2(w[0], w[1]);
   }
-  FL_CUDA(cudaMemcpyToSymbol(c_normal_plane, plane, sizeof plane));
+  FL_CUDA(cudaMemcpyToSymbol(g_normal_plane, plane, sizeof plane));
   FL_CUDA(cudaMemcpyToSymbol(c_resp8, resp, sizeof resp));
   FL_CUDA(cudaMemcpyToSymbol(g_resp8, resp, sizeof resp));
   return FL_OK;
@@ -98,9 +99,11 @@ __device__ __forceinline__ int reflect101(int p, int n) {
 __device__ __forceinline__ int reflect101_near(int p, int n) {         // |overshoot| <= 2 and n >= 3: a single fold
   return p < 0 ? -p : (p >= n ? 2 * n - 2 - p : p);
 }
-// src_static: the source was complete before this launch (the caller's frame), so it may go through L1 (neighbouring threads
-// share every line); a level produced by an earlier job of the same launch must be read from L2.
-__device__ __forceinline__ void dev_pyrdown_bgr(const uint8_t* __restrict__ src, int W, int H, uint8_t* __restrict__ dst, int bx, bool src_static) {
+// SRC_STATIC: the source was complete before this launch (the caller's frame), so it may go through L1 (neighbouring threads
+// share every line); a level produced by an earlier job of the same launch must be read from L2.  A template argument: chosen
+// per load at run time, the two load kinds of the unrolled 5 x 5 taps did not fit 32 registers and spilled.
+template <bool SRC_STATIC>
+__device__ __forceinline__ void dev_pyrdown_bgr(const uint8_t* __restrict__ src, int W, int H, uint8_t* __restrict__ dst, int bx) {
   const int dw = W / 2, dh = H / 2;
   const int gx = (dw + PD_TW - 1) / PD_TW;
   const int by = bx / gx; bx -= by * gx;
@@ -124,7 +127,7 @@ __device__ __forceinline__ void dev_pyrdown_bgr(const uint8_t* __restrict__ src,
     for (int t = 0; t < 5; ++t) {
       const int kt = t == 0 || t == 4 ? 1 : (t == 2 ? 6 : 4);
       const uint8_t* p = row + cx[t];
-      if (src_static) { r0 += kt * __ldg(p); r1 += kt * __ldg(p + 1); r2 += kt * __ldg(p + 2); }
+      if (SRC_STATIC) { r0 += kt * __ldg(p); r1 += kt * __ldg(p + 1); r2 += kt * __ldg(p + 2); }
       else { r0 += kt * __ldcg(p); r1 += kt * __ldcg(p + 1); r2 += kt * __ldcg(p + 2); }
     }
     s0 += kj * r0; s1 += kj * r1; s2 += kj * r2;
@@ -197,7 +200,9 @@ __device__ __forceinline__ uint32_t or_window(const uint32_t* __restrict__ w, in
   return o;
 }
 
-template <int TT>
+template <int TT, bool COARSE>
+// COARSE = false: the caller guarantees lm4 == mass == nullptr (every level but the coarsest), so neither the nibble stores nor the
+// response sums are compiled in and the scatter loop fits the registers of __launch_bounds__(256, 8) without spilling.
 // mass (nullable, the coarsest level only): += this CTA's sum of every (row, cell) response of label lab into mass[lab], one atomic per label
 // per CTA - the per-frame weights by which the staged similarity kernel orders its phases (k_similarity_staged)
 // mk (nullable): the frame's mask of this modality (copyTo(dst, mask), linemod.cpp:455-459, 741-745); label (y, x) of this level is kept
@@ -295,42 +300,47 @@ __device__ __forceinline__ void dev_spread_lm(const uint8_t* __restrict__ q, con
   // response sums of labels {0, 2}, {1, 3}, {4, 6}, {5, 7}, two per word in 16-bit halves (a thread adds at most 16 per item, a warp
   // at most 32 x 16 x ceil(T^2 SL_CW / 4 / SL_THREADS) <= 8,192 per half for T <= 16)
   uint32_t m02 = 0, m13 = 0, m46 = 0, m57 = 0;
+  const size_t lab_st = g.label_stride;
+  const size_t off0 = (size_t)gy * Wd + cx0;            // this CTA's first cell in every (label, residue) run
   for (int i = tid; i < items; i += SL_THREADS) {
     const int rr = (int)(((uint32_t)i * inv_ngrp) >> 16), c4 = i - rr * ngrp;
     const int ry = (int)(((uint32_t)rr * inv_T) >> 16), rx = rr - ry * T;
-    uint32_t lo[4], hi[4];
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      const int c = c4 * 4 + k;
-      const uint2 r8 = c < ncell ? s_resp[s_sp[ry * st_pw + c * T + rx]] : make_uint2(0, 0);
-      lo[k] = r8.x; hi[k] = r8.y;
-      m02 += r8.x & 0x00FF00FFu; m13 += (r8.x >> 8) & 0x00FF00FFu; m46 += r8.y & 0x00FF00FFu; m57 += (r8.y >> 8) & 0x00FF00FFu;
-    }
-    const size_t off = (size_t)rr * cells + (size_t)gy * Wd + cx0 + c4 * 4;
     const int nvalid = min(4, ncell - c4 * 4);
+    const uint8_t* sp = s_sp + ry * st_pw + c4 * 4 * T + rx;
+    const uint2 r0 = s_resp[sp[0]];                     // c4 * 4 < ncell always
+    const uint2 r1 = nvalid > 1 ? s_resp[sp[T]] : make_uint2(0, 0);
+    const uint2 r2 = nvalid > 2 ? s_resp[sp[2 * T]] : make_uint2(0, 0);
+    const uint2 r3 = nvalid > 3 ? s_resp[sp[3 * T]] : make_uint2(0, 0);
+    if (COARSE) {
+      m02 += (r0.x & 0x00FF00FFu) + (r1.x & 0x00FF00FFu) + (r2.x & 0x00FF00FFu) + (r3.x & 0x00FF00FFu);
+      m13 += ((r0.x >> 8) & 0x00FF00FFu) + ((r1.x >> 8) & 0x00FF00FFu) + ((r2.x >> 8) & 0x00FF00FFu) + ((r3.x >> 8) & 0x00FF00FFu);
+      m46 += (r0.y & 0x00FF00FFu) + (r1.y & 0x00FF00FFu) + (r2.y & 0x00FF00FFu) + (r3.y & 0x00FF00FFu);
+      m57 += ((r0.y >> 8) & 0x00FF00FFu) + ((r1.y >> 8) & 0x00FF00FFu) + ((r2.y >> 8) & 0x00FF00FFu) + ((r3.y >> 8) & 0x00FF00FFu);
+    }
+    const size_t off = (size_t)rr * cells + off0 + c4 * 4;
+    uint8_t* dst = lm + off;
+    // one word = byte (lab & 3) of the four cells' response words, for label lab; the stride between labels is label_stride
+    const bool wide = nvalid == 4 && ((((uintptr_t)dst) | lab_st) & 3) == 0;
 #pragma unroll
-    for (int lab = 0; lab < 8; ++lab) {
-      const uint32_t* src = lab < 4 ? lo : hi;
-      // byte (lab & 3) of each of the four words -> one word
+    for (int lab = 0; lab < 8; ++lab, dst += lab_st) {
       const uint32_t sel = 0x0040u + (lab & 3) * 0x0011u;          // PRMT selector: {byte b of x, byte b of y}
-      const uint32_t w01 = __byte_perm(src[0], src[1], sel), w23 = __byte_perm(src[2], src[3], sel);
-      const uint32_t w = __byte_perm(w01, w23, 0x5410);
-      uint8_t* dst = lm + (size_t)lab * g.label_stride + off;
-      if (nvalid == 4 && (((uintptr_t)dst) & 3) == 0) *reinterpret_cast<uint32_t*>(dst) = w;
+      const uint32_t w = lab < 4 ? __byte_perm(__byte_perm(r0.x, r1.x, sel), __byte_perm(r2.x, r3.x, sel), 0x5410)
+                                 : __byte_perm(__byte_perm(r0.y, r1.y, sel), __byte_perm(r2.y, r3.y, sel), 0x5410);
+      if (wide) *reinterpret_cast<uint32_t*>(dst) = w;
       else for (int k = 0; k < nvalid; ++k) dst[k] = (uint8_t)(w >> (8 * k));
-      if (lm4) {
+      if (COARSE && lm4) {
         // the same four responses (each 0, 1, 2 or 4) as nibbles, cell j of the label in nibble j: what the staged similarity
         // kernel reads (half the bytes).  Only passed for grids of even width, so `off` is even and nvalid is 2 or 4.  `off` is
         // a multiple of 4 only when Wd and cells are: a grid width of 2 mod 4 cells puts every other row at an odd byte.
         const uint32_t p2 = (w | (w >> 4)) & 0x00FF00FFu;
         const uint32_t p4 = (p2 | (p2 >> 8)) & 0xFFFFu;
-        uint8_t* d4 = lm4 + (((size_t)lab * g.label_stride + off) >> 1);
+        uint8_t* d4 = lm4 + (((size_t)lab * lab_st + off) >> 1);
         if (nvalid == 4 && (((uintptr_t)d4) & 1) == 0) *reinterpret_cast<uint16_t*>(d4) = (uint16_t)p4;
         else { d4[0] = (uint8_t)p4; if (nvalid == 4) d4[1] = (uint8_t)(p4 >> 8); }
       }
     }
   }
-  if (mass) {                                           // (uniform over the CTA)
+  if (COARSE && mass) {                                 // (uniform over the CTA)
     m02 = __reduce_add_sync(0xffffffffu, m02); m13 = __reduce_add_sync(0xffffffffu, m13);
     m46 = __reduce_add_sync(0xffffffffu, m46); m57 = __reduce_add_sync(0xffffffffu, m57);
     if (lane == 0 && (m02 | m13 | m46 | m57)) {
@@ -342,13 +352,15 @@ __device__ __forceinline__ void dev_spread_lm(const uint8_t* __restrict__ q, con
   }
 }
 
+// Compile-time T for the pyramid of LINE-MOD's default (T = 5 below the coarsest level, T = 8 at it); every other (T, level) takes the
+// runtime-T instantiation.  Each instantiation is ~1.5 k instructions of the one front-end kernel, so fewer of them keep its code small.
 __device__ __forceinline__ void dev_spread_lm_any(const fl_fe_job& jb, int bx, int by, uint8_t* smem) {
-  switch (jb.g.T) {
-    case 5: dev_spread_lm<5>(jb.src, jb.g, jb.dst, jb.dst2, jb.dst3, jb.mass, jb.mask, jb.mask_stride, jb.mask_shift, bx, by, smem, jb.p0); break;
-    case 8: dev_spread_lm<8>(jb.src, jb.g, jb.dst, jb.dst2, jb.dst3, jb.mass, jb.mask, jb.mask_stride, jb.mask_shift, bx, by, smem, jb.p0); break;
-    case 4: dev_spread_lm<4>(jb.src, jb.g, jb.dst, jb.dst2, jb.dst3, jb.mass, jb.mask, jb.mask_stride, jb.mask_shift, bx, by, smem, jb.p0); break;
-    default: dev_spread_lm<0>(jb.src, jb.g, jb.dst, jb.dst2, jb.dst3, jb.mass, jb.mask, jb.mask_stride, jb.mask_shift, bx, by, smem, jb.p0); break;
-  }
+  if (jb.g.T == 5 && !jb.dst3 && !jb.mass)
+    dev_spread_lm<5, false>(jb.src, jb.g, jb.dst, jb.dst2, nullptr, nullptr, jb.mask, jb.mask_stride, jb.mask_shift, bx, by, smem, jb.p0);
+  else if (jb.g.T == 8)
+    dev_spread_lm<8, true>(jb.src, jb.g, jb.dst, jb.dst2, jb.dst3, jb.mass, jb.mask, jb.mask_stride, jb.mask_shift, bx, by, smem, jb.p0);
+  else
+    dev_spread_lm<0, true>(jb.src, jb.g, jb.dst, jb.dst2, jb.dst3, jb.mass, jb.mask, jb.mask_stride, jb.mask_shift, bx, by, smem, jb.p0);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -388,7 +400,12 @@ __global__ void __launch_bounds__(256, 8) k_front_end_wave(fl_fe_wave w) {
   }
   const fl_fe_job& jb = w.job[j];
   const int local = b - jb.cta_begin;
-  if (w.trace && threadIdx.x == 0) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); atomicMin(w.trace + 2 * j, t); }
+  __shared__ unsigned long long s_trace0[2];            // this CTA's start (clock64, globaltimer): kept out of registers of the hot path
+  if (w.trace && threadIdx.x == 0) {
+    unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    s_trace0[0] = (unsigned long long)clock64(); s_trace0[1] = t;
+    atomicMin(w.trace + 2 * j, t);
+  }
   if (jb.wait_row_base >= 0) {
     // row-grained wait of a spread CTA (see fl_fe_job): the producer's tile rows that hold this grid row's label rows
     if (threadIdx.x == 0) {
@@ -429,7 +446,10 @@ __global__ void __launch_bounds__(256, 8) k_front_end_wave(fl_fe_wave w) {
     __syncthreads();
   }
   switch (jb.kind) {
-    case FL_JOB_PYRDOWN: dev_pyrdown_bgr(jb.src, jb.W, jb.H, jb.dst, local, jb.p0 != 0); break;
+    case FL_JOB_PYRDOWN:
+      if (jb.p0) dev_pyrdown_bgr<true>(jb.src, jb.W, jb.H, jb.dst, local);
+      else dev_pyrdown_bgr<false>(jb.src, jb.W, jb.H, jb.dst, local);
+      break;
     case FL_JOB_RESIZE: dev_resize_nn_half(jb.src, jb.W, jb.H, jb.dst, local); break;
     case FL_JOB_SPREAD: dev_spread_lm_any(jb, local % jb.gx, local / jb.gx, smem_dyn); break;
     case FL_JOB_PREFETCH: {
@@ -443,7 +463,16 @@ __global__ void __launch_bounds__(256, 8) k_front_end_wave(fl_fe_wave w) {
                             local % abs(jb.gx), local / abs(jb.gx), smem_dyn);
       break;
   }
-  if (w.trace) { __syncthreads(); if (threadIdx.x == 0) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); atomicMax(w.trace + 2 * j + 1, t); } }
+  if (w.trace) {
+    __syncthreads();
+    if (threadIdx.x == 0) {                             // last end, and this CTA's span (dependency wait included) added to the job's SM time
+      unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+      const unsigned long long c = (unsigned long long)clock64();
+      atomicMax(w.trace + 2 * j + 1, t);
+      atomicAdd(w.trace + 2 * FL_FE_MAX_JOBS + 2 * j, c - s_trace0[0]);
+      atomicAdd(w.trace + 2 * FL_FE_MAX_JOBS + 2 * j + 1, t - s_trace0[1]);
+    }
+  }
   if (jb.signal_slot >= 0) {
     __syncthreads();                                    // every thread's stores of this CTA ...
     if (threadIdx.x == 0) {                             // ... are visible before the counts

@@ -198,6 +198,7 @@ __device__ __forceinline__ void dev_color_quantize_v2(const uint8_t* __restrict_
 //   s_d [30][48] u16   depth, rows y0-7.., columns x0-8.. (0 outside the image)
 //   s_t [20][40] u8    thermometer-coded raw labels, (ry, lx) <-> (y0-2+ry, x0-4+lx)
 //   s_c [3][16][10]    bit-sliced vertical counts (0..5) of the five rows oy..oy+4, per bit position
+//   s_p [20][20] u8    the normal-plane table (g_normal_plane): indexed per pixel, which the constant cache would serialise
 // ------------------------------------------------------------------------------------------------
 #define D2_TW 32
 #define D2_TH 16
@@ -207,16 +208,19 @@ __device__ __forceinline__ void dev_color_quantize_v2(const uint8_t* __restrict_
 #define D2_LW 40
 #define D2_OFF_T (D2_SH * D2_SW * 2)
 #define D2_OFF_C (D2_OFF_T + D2_LH * D2_LW)
-#define D2_SMEM_BYTES (D2_OFF_C + 3 * D2_TH * (D2_LW / 4) * 4)
+#define D2_OFF_P (D2_OFF_C + 3 * D2_TH * (D2_LW / 4) * 4)
+#define D2_SMEM_BYTES (D2_OFF_P + 400)
 
 __device__ __forceinline__ void dev_depth_quantize_v2(const uint16_t* __restrict__ depth, int W, int H, int dist_thr, int diff_thr,
                                                       uint8_t* __restrict__ q, const fl_fe_wave& wv, int pyr_slot, int bx, int by, uint8_t* smem) {
   uint16_t* s_d = reinterpret_cast<uint16_t*>(smem);
   uint8_t* s_t = smem + D2_OFF_T;
   uint32_t* s_c = reinterpret_cast<uint32_t*>(smem + D2_OFF_C);
+  uint8_t* s_p = smem + D2_OFF_P;
   const int x0 = bx * D2_TW, y0 = by * D2_TH;
   const int tid = threadIdx.x;
   const bool aligned = ((reinterpret_cast<uintptr_t>(depth) & 7) | (uintptr_t)(W & 3)) == 0;
+  if (tid < 100) reinterpret_cast<uint32_t*>(s_p)[tid] = reinterpret_cast<const uint32_t*>(g_normal_plane)[tid];
 #pragma unroll
   for (int u = 0; u < (D2_SH * (D2_SW / 4) + 255) / 256; ++u) {     // unrolled: both passes' loads in flight together
     const int i = tid + 256 * u;
@@ -272,7 +276,7 @@ __device__ __forceinline__ void dev_depth_quantize_v2(const uint16_t* __restrict
           nx = __fmul_rn(nx, inv); ny = __fmul_rn(ny, inv);
           const int v1 = (int)__fadd_rn(__fmul_rn(nx, 10.f), 10.f);   // C truncation :665-667
           const int v2 = (int)__fadd_rn(__fmul_rn(ny, 10.f), 10.f);
-          const uint32_t lab = c_normal_plane[clampi(v2, 0, 19) * 20 + clampi(v1, 0, 19)];   // one-hot, table is v3-independent
+          const uint32_t lab = s_p[clampi(v2, 0, 19) * 20 + clampi(v1, 0, 19)];   // one-hot, table is v3-independent
           th = (lab << 1) - 1u;                                 // thermometer: bits 0..k for label 1 << k
         }
       }

@@ -460,8 +460,9 @@ enum {
   FL_DBG_STAGED_TRACE = 4,  /* ()                        -> 8 u64 per CTA of the staged similarity kernel {t_start, t_ready, t_first_data,
                                t_loop_end, t_end (globaltimer ns), smid, 0, 0}; only after fl_debug_option(h, FL_OPT_TRACE, 1);
                                returns the number of CTAs */
-  FL_DBG_FE_TRACE = 6,      /* ()                        -> 4 u64 per front-end job {kind, CTAs, first CTA start, last CTA end (globaltimer ns)};
-                               only after fl_debug_option(h, FL_OPT_TRACE, 1); returns the number of jobs */
+  FL_DBG_FE_TRACE = 6,      /* ()                        -> 6 u64 per front-end job {kind, CTAs, first CTA start, last CTA end (globaltimer ns),
+                               sum over the job's CTAs of the CTA's span in SM clock cycles (clock64) and in globaltimer ns}: the job's SM
+                               time, dependency waits included; only after fl_debug_option(h, FL_OPT_TRACE, 1); returns the number of jobs */
   FL_DBG_STAGED_ORDER = 7   /* ()                        -> the phase order of the last staged similarity launch: 32 u32 response sums of the
                                coarsest level it ordered by (word 8 m + l = modality m, label l), then one u8 per visit step: the phase
                                CTA 0 visited at that step; returns the number of phases */

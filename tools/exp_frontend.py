@@ -35,13 +35,11 @@ for it in range(104):
         if it < 8:
             print("frame %d: unique %d live %d raw %d | sort body ns: counts %d gather %d sort %d output %d" % (it % 4, cnt[0], cnt[1], cnt[3], cnt[4], cnt[5], cnt[6], cnt[7]))
 if TRACE:
-    fe = np.zeros(64, np.uint64)
-    nj = fb.lib().fl_debug_get(h._h, 6, 0, 0, 0, C.c_void_p(fe.ctypes.data), C.c_size_t(fe.nbytes))
-    if nj > 0:
-        fe = fe[:4 * nj].reshape(nj, 4).astype(np.int64)
+    fe = h.fe_trace()
+    if len(fe):
         t0 = fe[:, 2].min()
         names = {2: "pyrDown", 3: "resize", 4: "spread+LM", 5: "colour", 6: "depth", 7: "prefetch"}
-        for k, c, a, b in fe:
+        for k, c, a, b, _, _ in fe:
             print("FE job %-10s %5d CTAs: first start %6.2f us, last end %6.2f us" % (names.get(int(k), "?"), c, (a - t0) / 1e3, (b - t0) / 1e3))
 st /= n
 tl /= n
