@@ -50,7 +50,7 @@ struct fl_frame {
   fl_intrinsics_t K = {};                                  // recognition frames: the intrinsics of the staged frame
 };
 
-// Every resource has one owner (fl_owned.cuh); plan, icp, rz, d_out(_count), h_small, h_first, d_fe_err_host, d_reco_host point into them.
+// Every resource has one owner (fl_owned.cuh); plan, icp, rz, d_out(_count), h_small, h_first, d_reco_host point into them.
 struct fl_handle {
   fl_owned_stream stream;                                  // declared first: destroyed last, after everything used on it
   fl_params_t p = {};
@@ -75,7 +75,7 @@ struct fl_handle {
   fl_dev_buf<uint8_t> d_bgr[FL_MAX_LEVELS];                        // colour pyramid, levels >= 1
   fl_dev_buf<uint8_t> d_q[FL_MAX_LEVELS][FL_MAX_MODALITIES];       // quantised images (unmasked: a frame's masks apply in the spread jobs and at read-back)
   // masks, sized at fl_create: level 0 = the staged masks of host-input frames, levels >= 1 = the NN mask pyramid of a geometry that
-  // does not halve exactly (run_match_stages)
+  // does not halve exactly (the resize jobs of the front end, frontend.cu)
   fl_dev_buf<uint8_t> d_mask[FL_MAX_LEVELS][FL_MAX_MODALITIES];
   fl_dev_buf<uint8_t> d_spread[FL_MAX_LEVELS][FL_MAX_MODALITIES];  // debug only
   fl_dev_buf<uint8_t> d_lm[FL_MAX_LEVELS]; fl_dev_buf<uint8_t> d_lm4;   // d_lm4: 4-bit copy of the coarsest level's linear memories
@@ -83,10 +83,8 @@ struct fl_handle {
   const uint8_t* frame_mask[FL_MAX_MODALITIES] = {};               // level-0 mask (device memory) of the last frame's modality m, or NULL
   bool keep_spread = false;
   fl_frame frame; fl_staged_frame staged;
-  fl_dev_buf<unsigned long long> d_fe_trace; int fe_trace_jobs = 0, fe_trace_kind[FL_FE_MAX_JOBS] = {}, fe_trace_ctas[FL_FE_MAX_JOBS] = {};
-  bool opt_fe_waves = false, opt_split_refine = false, opt_trace = false, opt_dep_test = false, opt_no_prune = false, opt_rotate = false;   // fl_debug_option
-  fl_mapped_buf<int> h_fe_err; int* d_fe_err_host = nullptr; bool fe_force_waves = false;   // in-grid dependency time-out: mapped host flag (+ its device alias); true = this handle launches one kernel per wave from now on
-  fl_dev_buf<unsigned> d_fe_counters; unsigned fe_counter_base[FL_FE_MAX_JOBS] = {}; unsigned fe_row_base[FL_FE_MAX_JOBS] = {};   // in-grid dependency counters of the single-launch front end (+ 1 error word)
+  fl_fe_owned fe;                                           // the front end's dependency counters, time-out flag, timeline and switches
+  bool opt_split_refine = false, opt_trace = false, opt_no_prune = false, opt_rotate = false;   // fl_debug_option
   // candidates / matches
   fl_dev_buf<fl_match_t> d_cand; fl_dev_buf<int> d_count; fl_dev_buf<fl_sort_key> d_keys; int key_cap = 0; fl_dev_buf<uint8_t> d_outblk; fl_match_t* d_out = nullptr; int* d_out_count = nullptr;   // d_outblk = [16-int summary][matches]
   // pinned host staging
@@ -186,11 +184,7 @@ extern "C" int fl_create(const fl_params_t* params, fl_handle** out) {
   FL_CUDA(cudaMemset(h->d_mass.get(), 0, FL_MASS_WORDS * sizeof(uint32_t)));
   TRY(h->d_cand.alloc((size_t)p.max_candidates)); TRY(h->d_count.alloc(4));   // [0] candidate count, [1] CTA ticket counter of k_refine_sort
   FL_CUDA(cudaMemset(h->d_count.get(), 0, 4 * sizeof(int)));
-  // [FL_FE_MAX_JOBS job counters][1 error word][FL_FE_MAX_JOBS x FL_FE_MAX_TILE_ROWS tile-row counters]
-  TRY(h->d_fe_counters.alloc(FL_FE_MAX_JOBS + 1 + FL_FE_MAX_JOBS * FL_FE_MAX_TILE_ROWS));
-  FL_CUDA(cudaMemset(h->d_fe_counters.get(), 0, (FL_FE_MAX_JOBS + 1 + FL_FE_MAX_JOBS * FL_FE_MAX_TILE_ROWS) * sizeof(unsigned)));
-  TRY(h->h_fe_err.alloc(16)); *h->h_fe_err.get() = 0;
-  FL_CUDA(cudaHostGetDevicePointer((void**)&h->d_fe_err_host, h->h_fe_err.get(), 0));
+  TRY(fl_fe_create(&h->fe));
   int kc = 2; while (kc < p.max_candidates) kc <<= 1;
   h->key_cap = kc;
   TRY(h->d_keys.alloc((size_t)kc + 1));      // + room for the two scratch ints behind the keys
@@ -276,11 +270,9 @@ extern "C" int fl_debug_plan_staged(int W, int H, int T, int n_modalities, int n
 extern "C" int fl_debug_option(fl_handle* h, int option, int value) {
   if (!h) return FL_ERR_ARG;
   switch (option) {
-    case FL_OPT_FE_WAVES: h->opt_fe_waves = value != 0; return FL_OK;
+    case FL_OPT_FE_WAVES: case FL_OPT_FE_DEP_TIMEOUT_TEST: case FL_OPT_FE_FORCED_WAVES: return fl_fe_option(h->fe.get(), option, value);
     case FL_OPT_SPLIT_REFINE: h->opt_split_refine = value != 0; return FL_OK;
     case FL_OPT_TRACE: h->opt_trace = value != 0; h->packed = false; return FL_OK;     // (the staged plan allocates its timeline at planning time)
-    case FL_OPT_FE_DEP_TIMEOUT_TEST: h->opt_dep_test = value != 0; return FL_OK;
-    case FL_OPT_FE_FORCED_WAVES: return h->fe_force_waves ? 1 : 0;                      // query: has a dependency time-out switched this handle to wave launches?
     case FL_OPT_SIM_NO_PRUNE: h->opt_no_prune = value != 0; return FL_OK;
     case FL_OPT_SIM_ROTATE: h->opt_rotate = value != 0; return FL_OK;
   }
@@ -419,10 +411,7 @@ static int ensure_geometry(fl_handle* h, int W, int H) {
     h->gW = W; h->gH = H; h->packed = false;
   }
   if (!h->packed) {
-    // the front end's tile-row counters are per job SLOT and advance by "tiles per row" every frame; a new geometry or template
-    // set can change the job layout, so they restart from zero (stream-ordered with the launches that follow)
-    FL_CUDA(cudaMemsetAsync(h->d_fe_counters.get() + FL_FE_MAX_JOBS + 1, 0, (size_t)FL_FE_MAX_JOBS * FL_FE_MAX_TILE_ROWS * sizeof(unsigned), h->stream.get()));
-    memset(h->fe_row_base, 0, sizeof h->fe_row_base);
+    TRY(fl_fe_forget_rows(h->fe.get(), h->stream.get()));
     if (h->n_templates == 0) h->packed = true;
   }
   if (!h->packed && h->n_templates > 0) {
@@ -449,16 +438,6 @@ static int ensure_geometry(fl_handle* h, int W, int H) {
     h->packed = true;
   }
   return FL_OK;
-}
-
-// the 4-bit linear memories of (level, modality): only the coarsest level has them, and only grids of even width (two cells per byte)
-static uint8_t* lm4_of(fl_handle* h, int l, int m) {
-  return (l == h->p.n_levels - 1 && (h->geom[l].Wd & 1) == 0) ? h->d_lm4.get() + (((size_t)m * h->geom[l].mod_stride) >> 1) : nullptr;
-}
-// the response sums of (level, modality) that order the staged kernel's phases: only the coarsest level, and only when that kernel runs
-// (it clears them; nothing else would)
-static uint32_t* mass_of(fl_handle* h, int l, int m) {
-  return (l == h->p.n_levels - 1 && h->use_staged && h->n_templates > 0) ? h->d_mass.get() + 8 * m : nullptr;
 }
 
 // front end + matchClass on the handle's templates; candidates land in (cand, count)
@@ -490,170 +469,28 @@ static int run_match_stages(fl_handle* h, const uint8_t* d_bgr, const uint16_t* 
     }
   }
   if (h->profile) cudaEventRecord(h->ev[0].get(), s);
-  const float thr_sq = p.weak_threshold * p.weak_threshold;
-  // the frame's masks (level 0, device memory): applied where the spread jobs read the labels (dev_spread_lm), so a masked frame takes
-  // the same schedule and launches as an unmasked one
-  const uint8_t* mask0[FL_MAX_MODALITIES] = {};
-  for (int m = 0; m < p.n_modalities; ++m) { mask0[m] = d_masks ? static_cast<const uint8_t*>(d_masks[m]) : nullptr; h->frame_mask[m] = mask0[m]; }
-  int first_color = -1;
-  for (int m = 0; m < p.n_modalities; ++m) if (p.modality_kind[m] == FL_MODALITY_COLOR_GRADIENT && first_color < 0) first_color = m;
-  // wave schedule (frontend.cu): L + 1 launches for the whole front end; wave l produces the labels of level l and the
-  // linear memories of level l - 1.  Jobs are added longest first: the kernel ends with its slowest CTA, and CTAs are
-  // scheduled in job order.  (Measured alternative: slicing the level-0 colour quantisation over the waves and moving
-  // every spread to the last wave - 16.6 + 10.8 + 9.2 us instead of 17.7 + 9.4 + 6.0 us, i.e. no gain: each wave has a
-  // latency floor of one colour-tile CTA, about 8 us.)
-  const int L = p.n_levels;
-  fl_fe_wave w;
-  auto wave_begin = [&](bool zero) { w.n_jobs = 0; w.n_ctas = 0; w.smem = 0; w.n_pyr = 0; w.zero_me = zero ? d_count : nullptr; w.counters = nullptr; w.dep_error = nullptr; w.dep_error_host = nullptr; w.trace = nullptr; };
-  bool launch_ok = true;
-  auto wave_flush = [&]() { if (w.n_jobs > 0) { launch_ok &= fl_launch_fe_wave(w, s) == cudaSuccess; ++h->launches; } w.n_jobs = 0; w.n_ctas = 0; w.smem = 0; w.n_pyr = 0; w.zero_me = nullptr; };
-  // word-parallel quantisers (frontend_v2.cuh).  The depth job also writes the NN-downsampled label pyramid when every level
-  // halves exactly (then dst_l(y,x) = src(2^l y, 2^l x)).
-  bool depth_pyr_fused[FL_MAX_MODALITIES] = {false, false, false, false};
-  bool halves = true;
-  for (int l = 0; l + 1 < L; ++l) halves &= (h->geom[l].W % 2 == 0) && (h->geom[l].H % 2 == 0);
-  auto wave_room = [&]() { if (w.n_jobs == FL_FE_MAX_JOBS) wave_flush(); };     // jobs of one wave are independent: splitting is always safe
-  // spread + response maps + linear memories of (level l, modality m).  A masked modality's spread job reads the level-0 mask at a
-  // shift of l when every level halves exactly (NN-halving then picks src(2y, 2x)); otherwise only the per-wave schedule runs, and it
-  // builds the mask pyramid in d_mask with resize jobs next to the depth labels'.
-  auto add_spread = [&](int l, int m) -> int {
-    uint8_t* spread = nullptr;
-    if (h->keep_spread) { TRY(h->d_spread[l][m].grow((size_t)(p.max_width >> l) * (p.max_height >> l))); spread = h->d_spread[l][m].get(); }
-    const bool pyr = mask0[m] && l > 0 && !halves;
-    fl_fe_add_spread(&w, h->d_q[l][m].get(), h->geom[l], h->d_lm[l].get() + (size_t)m * h->geom[l].mod_stride, spread, lm4_of(h, l, m), mass_of(h, l, m),
-                     pyr ? h->d_mask[l][m].get() : mask0[m], pyr ? h->geom[l].W : h->geom[0].W, pyr ? 0 : l);
-    return FL_OK;
-  };
-  // ---- single-launch front end: every job of the frame in ONE grid, producers before consumers, dependencies resolved by
-  // per-job CTA counters inside the kernel (k_front_end_wave).  Removes L launches + their dependency gaps and lets the
-  // level-0 work fill the machine while the short critical chain pyrDown -> colour L(top) -> spread L(top) runs.
-  const bool fe_waves = h->opt_fe_waves;                                       // FL_OPT_FE_WAVES: one launch per wave (also the fallback after a dependency time-out)
-  int n_color = 0, n_depth = 0;
-  for (int m = 0; m < p.n_modalities; ++m) { n_color += p.modality_kind[m] == FL_MODALITY_COLOR_GRADIENT; n_depth += p.modality_kind[m] == FL_MODALITY_DEPTH_NORMAL; }
-  const int n_jobs_single = (n_color ? L - 1 : 0) + n_color * L + n_depth + p.n_modalities * L;
-  const bool single = !fe_waves && !h->fe_force_waves && n_jobs_single <= FL_FE_MAX_JOBS && n_depth <= FL_FE_MAX_DPYR && (L == 1 || (halves && L - 1 <= FL_FE_MAX_PYR));
-  if (single) {
-    wave_begin(true);                                                            // wave 0 resets the candidate counter: no memset node between the kernels
-    w.counters = h->d_fe_counters.get(); w.dep_error = reinterpret_cast<int*>(h->d_fe_counters.get() + FL_FE_MAX_JOBS); w.dep_error_host = h->d_fe_err_host;
-    int slot_pyr[FL_MAX_LEVELS], slot_color[FL_MAX_LEVELS][FL_MAX_MODALITIES], slot_depth[FL_MAX_MODALITIES];
-    auto last_job = [&]() -> fl_fe_job& { return w.job[w.n_jobs - 1]; };
-    auto job_ctas = [&](int idx) { return (idx + 1 < w.n_jobs ? w.job[idx + 1].cta_begin : w.n_ctas) - w.job[idx].cta_begin; };
-    auto produce = [&]() { last_job().signal_slot = w.n_jobs - 1; return w.n_jobs - 1; };
-    // tile jobs (32 x 16 tiles) also count per tile row; returns false when the image has more tile rows than counters
-    auto produce_rows = [&](int slot) {
-      fl_fe_job& jb = w.job[slot];
-      const int rows = (jb.H + 15) / 16;
-      if (rows > FL_FE_MAX_TILE_ROWS) return;                 // (then the consumers wait for the whole job)
-      jb.row_base = FL_FE_MAX_JOBS + 1 + slot * FL_FE_MAX_TILE_ROWS;
-    };
-    auto consume_rows = [&](int slot, int shift) {      // spread job: wait per tile row of producer `slot` (level shift for the depth pyramid)
-      const fl_fe_job& pj = w.job[slot];
-      if (pj.row_base < 0) return;
-      fl_fe_job& jb = last_job();
-      jb.wait_row_base = pj.row_base; jb.wait_row_shift = shift; jb.wait_row_count = (pj.H + 15) / 16;
-      jb.wait_row_target = h->fe_row_base[slot] + (unsigned)abs(pj.gx);
-    };
-    // FL_OPT_FE_DEP_TIMEOUT_TEST: the next frame waits for one CTA more than its producer has, i.e. the wait times out (test of the fallback)
-    const unsigned dep_test = h->opt_dep_test ? 1u : 0u;
-    h->opt_dep_test = false;
-    auto consume = [&](int slot) { last_job().wait_slot = slot; last_job().wait_target = h->fe_counter_base[slot] + (unsigned)job_ctas(slot) + dep_test; };
-    // 0. the staged similarity kernel's per-template feature lists -> L2 (they would otherwise cost its prologue DRAM round trips)
-    if (h->use_staged && h->n_templates > 0 && n_jobs_single + 3 <= FL_FE_MAX_JOBS) {
-      fl_fe_add_prefetch(&w, h->plan.gfeat, (size_t)h->n_templates * 64 * sizeof(uint32_t));
-      fl_fe_add_prefetch(&w, h->plan.gpre, (size_t)h->n_templates * h->plan.pre_stride);
-      fl_fe_add_prefetch(&w, h->plan.gmeta, (size_t)h->n_templates * sizeof(int4));
-      if (n_jobs_single + 6 <= FL_FE_MAX_JOBS) {                               // the prologue's dependent lookups: template -> class -> enabled
-        fl_fe_add_prefetch(&w, h->d_class_of.get(), (size_t)h->n_templates * sizeof(int32_t));
-        fl_fe_add_prefetch(&w, h->d_class_enabled.get(), (size_t)std::max(h->n_classes, 1));
-        fl_fe_add_prefetch(&w, h->d_tid_of.get(), (size_t)h->n_templates * sizeof(int32_t));
-      }
+  fl_fe_frame fe = {};
+  fe.n_levels = p.n_levels; fe.n_modalities = p.n_modalities; fe.modality_kind = p.modality_kind; fe.geom = h->geom; fe.bgr = d_bgr; fe.depth = d_depth;
+  for (int l = 0; l < p.n_levels; ++l) {
+    fe.bgr_pyr[l] = h->d_bgr[l].get(); fe.lm[l] = h->d_lm[l].get();
+    for (int m = 0; m < p.n_modalities; ++m) {
+      fe.q[l][m] = h->d_q[l][m].get(); fe.mask_pyr[l][m] = h->d_mask[l][m].get();
+      if (h->keep_spread) { TRY(h->d_spread[l][m].grow((size_t)(p.max_width >> l) * (p.max_height >> l))); fe.spread[l][m] = h->d_spread[l][m].get(); }
     }
-    // 1. colour pyramid chain (short jobs, on the critical path of the coarsest level)
-    if (first_color >= 0)
-      for (int l = 0; l + 1 < L; ++l) {
-        fl_fe_add_pyrdown(&w, l == 0 ? d_bgr : h->d_bgr[l].get(), h->geom[l].W, h->geom[l].H, h->d_bgr[l + 1].get(), l == 0);
-        slot_pyr[l + 1] = produce();
-        if (l > 0) consume(slot_pyr[l]);
-      }
-    // 2. depth labels of every level (one job per depth modality)
-    for (int m = 0; m < p.n_modalities; ++m)
-      if (p.modality_kind[m] == FL_MODALITY_DEPTH_NORMAL) {
-        fl_depth_pyr pyr; memset(&pyr, 0, sizeof pyr);
-        pyr.n = L - 1;
-        for (int k = 1; k < L; ++k) { pyr.W[k - 1] = h->geom[k].W; pyr.H[k - 1] = h->geom[k].H; pyr.dst[k - 1] = h->d_q[k][m].get(); }
-        fl_fe_add_depth_v2(&w, d_depth, h->geom[0].W, h->geom[0].H, p.distance_threshold, p.difference_threshold, h->d_q[0][m].get(), pyr.n > 0 ? &pyr : nullptr);
-        slot_depth[m] = produce();
-        produce_rows(slot_depth[m]);
-      }
-    // 3. colour labels, coarsest level first
-    for (int l = L - 1; l >= 0; --l)
-      for (int m = 0; m < p.n_modalities; ++m)
-        if (p.modality_kind[m] == FL_MODALITY_COLOR_GRADIENT) {
-          fl_fe_add_color_v2(&w, l == 0 ? d_bgr : h->d_bgr[l].get(), h->geom[l].W, h->geom[l].H, thr_sq, h->d_q[l][m].get());
-          slot_color[l][m] = produce();
-          produce_rows(slot_color[l][m]);
-          if (l > 0) consume(slot_pyr[l]);
-        }
-    // 4. spread + response maps + linear memories, coarsest level first (the similarity kernel needs only that one)
-    for (int l = L - 1; l >= 0; --l)
-      for (int m = 0; m < p.n_modalities; ++m) {
-        TRY(add_spread(l, m));
-        const bool is_color = p.modality_kind[m] == FL_MODALITY_COLOR_GRADIENT;
-        consume(is_color ? slot_color[l][m] : slot_depth[m]);
-        consume_rows(is_color ? slot_color[l][m] : slot_depth[m], is_color ? 0 : l);
-      }
-    if (h->opt_trace) {                                                        // developer timeline: per job first start / last end, summed CTA spans
-      TRY(h->d_fe_trace.grow(2 * FL_FE_MAX_JOBS + 2 * FL_FE_MAX_JOBS));
-      unsigned long long init[4 * FL_FE_MAX_JOBS];
-      for (int i = 0; i < FL_FE_MAX_JOBS; ++i) { init[2 * i] = ~0ull; init[2 * i + 1] = 0; init[2 * FL_FE_MAX_JOBS + 2 * i] = init[2 * FL_FE_MAX_JOBS + 2 * i + 1] = 0; }
-      FL_CUDA(cudaMemcpyAsync(h->d_fe_trace.get(), init, sizeof init, cudaMemcpyHostToDevice, s));
-      FL_CUDA(cudaStreamSynchronize(s));
-      w.trace = h->d_fe_trace.get();
-      h->fe_trace_jobs = w.n_jobs;
-      for (int i = 0; i < w.n_jobs; ++i) { h->fe_trace_kind[i] = w.job[i].kind; h->fe_trace_ctas[i] = job_ctas(i); }
-    }
-    // the monotonic counter bases advance only when the launch really went out (a failed launch bumps no counter)
-    unsigned add_ctr[FL_FE_MAX_JOBS] = {0}, add_row[FL_FE_MAX_JOBS] = {0};
-    for (int i = 0; i < w.n_jobs; ++i) { if (w.job[i].signal_slot >= 0) add_ctr[i] = (unsigned)job_ctas(i); if (w.job[i].row_base >= 0) add_row[i] = (unsigned)abs(w.job[i].gx); }
-    wave_flush();
-    if (!launch_ok) { fl_set_error("front-end launch failed: %s", cudaGetErrorString(cudaGetLastError())); return FL_ERR_CUDA; }
-    for (int i = 0; i < FL_FE_MAX_JOBS; ++i) { h->fe_counter_base[i] += add_ctr[i]; h->fe_row_base[i] += add_row[i]; }
-  } else
-  for (int wv = 0; wv <= L; ++wv) {
-    wave_begin(wv == 0);                                                        // the candidate counter is reset by the first wave
-    const int l = wv;                                                             // level whose labels this wave produces
-    if (l < L) {
-      const fl_level_geom& g = h->geom[l];
-      for (int m = 0; m < p.n_modalities; ++m)
-        if (p.modality_kind[m] == FL_MODALITY_COLOR_GRADIENT) {
-          wave_room();
-          fl_fe_add_color_v2(&w, l == 0 ? d_bgr : h->d_bgr[l].get(), g.W, g.H, thr_sq, h->d_q[l][m].get());
-        }
-      for (int m = 0; m < p.n_modalities; ++m)
-        if (p.modality_kind[m] == FL_MODALITY_DEPTH_NORMAL && l == 0) {
-          wave_room();
-          fl_depth_pyr pyr; memset(&pyr, 0, sizeof pyr);
-          if (halves && L > 1 && L - 1 <= FL_FE_MAX_PYR) {
-            pyr.n = L - 1;
-            for (int k = 1; k < L; ++k) { pyr.W[k - 1] = h->geom[k].W; pyr.H[k - 1] = h->geom[k].H; pyr.dst[k - 1] = h->d_q[k][m].get(); }
-          }
-          if (pyr.n > 0 && fl_fe_add_depth_v2(&w, d_depth, g.W, g.H, p.distance_threshold, p.difference_threshold, h->d_q[0][m].get(), &pyr)) depth_pyr_fused[m] = true;
-          else fl_fe_add_depth_v2(&w, d_depth, g.W, g.H, p.distance_threshold, p.difference_threshold, h->d_q[0][m].get(), nullptr);
-        }
-    }
-    if (l >= 1) {
-      for (int m = 0; m < p.n_modalities; ++m) { wave_room(); TRY(add_spread(l - 1, m)); }
-    }
-    if (l < L) {
-      const fl_level_geom& g = h->geom[l];
-      if (first_color >= 0 && l + 1 < L) { wave_room(); fl_fe_add_pyrdown(&w, l == 0 ? d_bgr : h->d_bgr[l].get(), g.W, g.H, h->d_bgr[l + 1].get(), true); }   // shared by all colour modalities
-      for (int m = 0; m < p.n_modalities; ++m)
-        if (p.modality_kind[m] == FL_MODALITY_DEPTH_NORMAL && l > 0 && !depth_pyr_fused[m]) { wave_room(); fl_fe_add_resize(&w, h->d_q[l - 1][m].get(), h->geom[l - 1].W, h->geom[l - 1].H, h->d_q[l][m].get()); }
-      for (int m = 0; m < p.n_modalities; ++m)
-        if (mask0[m] && l > 0 && !halves) { wave_room(); fl_fe_add_resize(&w, l == 1 ? mask0[m] : h->d_mask[l - 1][m].get(), h->geom[l - 1].W, h->geom[l - 1].H, h->d_mask[l][m].get()); }
-    }
-    wave_flush();
   }
+  // the frame's masks (level 0, device memory): applied where the spread jobs read the labels, so a masked frame takes the same launches
+  for (int m = 0; m < p.n_modalities; ++m) fe.mask[m] = h->frame_mask[m] = d_masks ? static_cast<const uint8_t*>(d_masks[m]) : nullptr;
+  fe.lm4 = (h->geom[p.n_levels - 1].Wd & 1) == 0 ? h->d_lm4.get() : nullptr;            // two cells per byte: grids of even width only
+  if (h->use_staged && h->n_templates > 0) {                                   // the response sums order the staged kernel's phases; it clears them
+    fe.mass = h->d_mass.get();
+    const void* pf[6] = {h->plan.gfeat, h->plan.gpre, h->plan.gmeta, h->d_class_of.get(), h->d_class_enabled.get(), h->d_tid_of.get()};
+    const size_t nt = (size_t)h->n_templates;
+    const size_t pb[6] = {nt * 64 * sizeof(uint32_t), nt * h->plan.pre_stride, nt * sizeof(int4), nt * sizeof(int32_t), (size_t)std::max(h->n_classes, 1), nt * sizeof(int32_t)};
+    memcpy(fe.prefetch, pf, sizeof pf); memcpy(fe.prefetch_bytes, pb, sizeof pb);
+  }
+  fe.thr_sq = p.weak_threshold * p.weak_threshold; fe.dist_thr = p.distance_threshold; fe.diff_thr = p.difference_threshold;
+  fe.zero_me = d_count; fe.trace = h->opt_trace;
+  TRY(fl_fe_run(h->fe.get(), fe, s, &h->launches));
   if (h->profile) cudaEventRecord(h->ev[1].get(), s);
   if (h->n_templates > 0) {
     fl_tdb db = make_tdb(h);
@@ -794,13 +631,11 @@ int fl_frame_wait(fl_handle* h, fl_wait_note* note) {
   if (f.kind == fl_frame_kind::none) { fl_set_error("no frame in flight on this handle"); return FL_ERR_STATE; }
   f.kind = fl_frame_kind::none;
   TRY(sort_finish(h));
-  if (*reinterpret_cast<volatile int*>(h->h_fe_err.get())) {
+  int job;
+  TRY(fl_fe_take_timeout(h->fe.get(), h->stream.get(), &job));
+  if (job >= 0) {
     // an in-grid dependency of the single-launch front end timed out (the producer CTAs were not dispatched before their consumers:
     // see k_front_end_wave): the frame's result is not trustworthy.  From now on this handle launches one kernel per wave.
-    const int job = *h->h_fe_err.get() - 1;
-    *h->h_fe_err.get() = 0;
-    FL_CUDA(cudaMemsetAsync(h->d_fe_counters.get() + FL_FE_MAX_JOBS, 0, sizeof(unsigned), h->stream.get()));
-    h->fe_force_waves = true;
     if (!f.rerun) {
       *note = fl_wait_note::resubmit;
       fl_set_error("front end: in-grid dependency of job %d timed out; the handle now uses per-wave launches - resubmit the frame", job);
@@ -1262,18 +1097,7 @@ extern "C" int fl_debug_get(fl_handle* h, int what, int32_t a, int32_t b, int32_
     memcpy(host_out, h->h_small, 16 * sizeof(int));
     return FL_OK;
   }
-  if (what == FL_DBG_FE_TRACE) {                                                               // developer: front-end job timeline {kind, ctas, start, end, cycles, ns} x jobs (FL_OPT_TRACE)
-    if (!h->d_fe_trace.get() || h->fe_trace_jobs <= 0) return FL_ERR_STATE;
-    if (bytes < (size_t)h->fe_trace_jobs * 6 * sizeof(unsigned long long)) return FL_ERR_CAPACITY;
-    unsigned long long raw[4 * FL_FE_MAX_JOBS];
-    FL_CUDA(cudaMemcpy(raw, h->d_fe_trace.get(), sizeof raw, cudaMemcpyDeviceToHost));
-    unsigned long long* o = static_cast<unsigned long long*>(host_out);
-    for (int i = 0; i < h->fe_trace_jobs; ++i) {
-      o[6 * i] = (unsigned long long)h->fe_trace_kind[i]; o[6 * i + 1] = (unsigned long long)h->fe_trace_ctas[i]; o[6 * i + 2] = raw[2 * i]; o[6 * i + 3] = raw[2 * i + 1];
-      o[6 * i + 4] = raw[2 * FL_FE_MAX_JOBS + 2 * i]; o[6 * i + 5] = raw[2 * FL_FE_MAX_JOBS + 2 * i + 1];
-    }
-    return h->fe_trace_jobs;
-  }
+  if (what == FL_DBG_FE_TRACE) return fl_fe_trace(h->fe.get(), host_out, bytes);   // developer: front-end job timeline (FL_OPT_TRACE)
   if (what == FL_DBG_STAGED_ORDER) {                                                           // the phase order of the last staged launch
     if (!h->use_staged) return FL_ERR_STATE;
     if (bytes < 32 * sizeof(uint32_t) + (size_t)h->plan.n_phases) return FL_ERR_CAPACITY;

@@ -4,6 +4,7 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
+#include <memory>
 #include "../../include/fealess_b200.h"
 
 #define FL_MAX_DEVICES 64        // devices of one process (per-device kernel attribute tables)
@@ -103,22 +104,50 @@ struct fl_fe_job {
 struct fl_depth_pyr { int n; int W[FL_FE_MAX_PYR], H[FL_FE_MAX_PYR]; uint8_t* dst[FL_FE_MAX_PYR]; };
 #define FL_FE_MAX_JOBS 16
 #define FL_FE_MAX_DPYR 2
+// the argument of one k_front_end_wave launch.  zero_me: int reset by CTA 0 (the candidate counter), or NULL.  pyr: the NN pyramids the
+// depth jobs write (a depth job's thr_sq holds its slot).  counters (single launch only, else NULL): FL_FE_MAX_JOBS monotonic CTA
+// counters, one error word (dep_error), FL_FE_MAX_JOBS x FL_FE_MAX_TILE_ROWS tile-row counters; dep_error_host: the same flag in mapped
+// host memory, written only on a time-out.  trace (FL_OPT_TRACE, or NULL): per job {first CTA start, last CTA end} in globaltimer ns,
+// then per job the sums of its CTAs' spans {SM cycles, ns}.
 struct fl_fe_wave { int n_jobs, n_ctas; size_t smem; int* zero_me; fl_fe_job job[FL_FE_MAX_JOBS]; int n_pyr; fl_depth_pyr pyr[FL_FE_MAX_DPYR];
-                    unsigned* counters; int* dep_error; int* dep_error_host;   // dep_error_host: the same flag in mapped host memory (written only on a time-out)
-                    unsigned long long* trace; };   // trace (FL_OPT_TRACE): per job {first CTA start, last CTA end} in globaltimer ns   // zero_me: int reset by CTA 0 (candidate counter), or NULL; counters: FL_FE_MAX_JOBS monotonic CTA counters
-// word-parallel quantisers (frontend_v2.cuh); pyr (nullable, at most FL_FE_MAX_DPYR per wave): also write the NN pyramid of the labels
-void fl_fe_add_color_v2(fl_fe_wave* w, const uint8_t* bgr, int W, int H, float thr_sq, uint8_t* q);
-bool fl_fe_add_depth_v2(fl_fe_wave* w, const uint16_t* depth, int W, int H, int dist_thr, int diff_thr, uint8_t* q, const fl_depth_pyr* pyr);
-void fl_fe_add_pyrdown(fl_fe_wave* w, const uint8_t* src, int W, int H, uint8_t* dst, bool src_static);
-// pull `bytes` at src towards L2 (one 128-byte line per thread): the similarity kernel's per-template feature lists, touched
-// in the shadow of the front end so that its prologue does not start with DRAM round trips
-void fl_fe_add_prefetch(fl_fe_wave* w, const void* src, size_t bytes);
-void fl_fe_add_resize(fl_fe_wave* w, const uint8_t* src, int W, int H, uint8_t* dst);
-// mass_or_null: the coarsest level's response sums of this modality (8 words, see FL_MASS_*), or NULL.  mask_or_null: labels (y, x) are
-// kept where mask[(y << mask_shift) * mask_stride + (x << mask_shift)] != 0
-void fl_fe_add_spread(fl_fe_wave* w, const uint8_t* q, fl_level_geom g, uint8_t* lm_mod, uint8_t* spread_or_null, uint8_t* lm4_mod_or_null,
-                      uint32_t* mass_or_null, const uint8_t* mask_or_null, int mask_stride, int mask_shift);
-cudaError_t fl_launch_fe_wave(const fl_fe_wave& w, cudaStream_t s);
+                    unsigned* counters; int* dep_error; int* dep_error_host;
+                    unsigned long long* trace; };
+
+// What one frame's front end reads and writes: the frame's level-0 images and masks, and the handle's buffers for its geometry.
+struct fl_fe_frame {
+  int n_levels, n_modalities; const int32_t* modality_kind; const fl_level_geom* geom;
+  const uint8_t* bgr; const uint16_t* depth;                 // level 0 (NULL when no modality reads it)
+  uint8_t* bgr_pyr[FL_MAX_LEVELS];                           // colour pyramid, levels >= 1
+  uint8_t* q[FL_MAX_LEVELS][FL_MAX_MODALITIES];              // labels
+  uint8_t* lm[FL_MAX_LEVELS];                                // linear memories of a level, modality m at m * mod_stride
+  uint8_t* lm4; uint32_t* mass;                              // coarsest level: 4-bit linear memories, response sums (FL_MASS_*); NULL = not written
+  uint8_t* spread[FL_MAX_LEVELS][FL_MAX_MODALITIES];         // spread images (NULL = not kept)
+  const uint8_t* mask[FL_MAX_MODALITIES];                    // level-0 masks (NULL = unmasked)
+  uint8_t* mask_pyr[FL_MAX_LEVELS][FL_MAX_MODALITIES];       // levels >= 1 of the NN mask pyramid of a geometry that does not halve exactly
+  float thr_sq; int dist_thr, diff_thr;                      // colour magnitude threshold squared, depth distance / difference thresholds
+  // pulled towards L2 in the single launch (one 128-byte line per thread): the staged similarity kernel's per-template feature lists, and
+  // then its prologue's lookups (template -> class -> enabled), so that it does not start with DRAM round trips.  The first three
+  // ranges go in when the launch has room for three more jobs, all six when it has room for six; empty ranges are skipped.
+  const void* prefetch[6]; size_t prefetch_bytes[6];
+  int* zero_me;                                              // reset by the first launch (the candidate counter)
+  bool trace;                                                // FL_OPT_TRACE: record the single launch's job timeline
+};
+// Per-handle state of the front end (frontend.cu): the in-grid dependency counters and their bases, the time-out flag, the job timeline
+// and the front end's switches.  Owned by the handle through fl_fe_owned.
+struct fl_fe_state;
+struct fl_fe_free { void operator()(fl_fe_state* s) const; };
+typedef std::unique_ptr<fl_fe_state, fl_fe_free> fl_fe_owned;
+int fl_fe_create(fl_fe_owned* out);                          // on the current device
+// a new geometry or template set can change the job layout: the tile-row counters restart from zero (stream-ordered)
+int fl_fe_forget_rows(fl_fe_state* fe, cudaStream_t s);
+// enqueue the whole front end of one frame: one launch, or one per wave (FL_OPT_FE_WAVES, after a time-out, and for geometries the
+// single launch does not take); *launches grows by the number of launches
+int fl_fe_run(fl_fe_state* fe, const fl_fe_frame& f, cudaStream_t s, int64_t* launches);
+// after the frame's wait: *job = the job whose in-grid dependency timed out, or -1.  On a time-out the flag and the error word are
+// cleared and the handle launches one kernel per wave from then on.
+int fl_fe_take_timeout(fl_fe_state* fe, cudaStream_t s, int* job);
+int fl_fe_trace(const fl_fe_state* fe, void* host_out, size_t bytes);     // FL_DBG_FE_TRACE
+int fl_fe_option(fl_fe_state* fe, int option, int value);                  // FL_OPT_FE_WAVES, FL_OPT_FE_DEP_TIMEOUT_TEST, FL_OPT_FE_FORCED_WAVES
 
 // ---- template training, per-pixel half (train.cu) -----------------------------------------------
 void fl_launch_train_magnitude(const uint8_t* bgr, int W, int H, float* mag, cudaStream_t s);

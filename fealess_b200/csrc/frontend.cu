@@ -10,7 +10,9 @@
 //   spread / computeResponseMaps / linearize                  linemod.cpp:950-965, 979-1048, 1060-1088
 // Compiled with -fmad=false: the fp32 expressions below must round exactly like the (uncontracted) reference.
 #include "fl_internal.cuh"
+#include "fl_owned.cuh"
 #include <math.h>
+#include <new>
 
 // ------------------------------------------------------------------------------------------------
 // tables: NORMAL_LUT depends only on (v2, v1) -> 400 bytes; response table packs the 8 per-label responses of one
@@ -365,11 +367,8 @@ __device__ __forceinline__ void dev_spread_lm_any(const fl_fe_job& jb, int bx, i
 
 // ------------------------------------------------------------------------------------------------
 // Wave kernel: at VGA every stage above moves a few hundred KB, i.e. ~1 us of HBM time against ~5-8 us of launch +
-// dependency latency, so the front end is launch bound.  All stages that are independent of each other at one point of
-// the pyramid recursion are therefore issued as ONE launch: the grid is the concatenation of the jobs' grids.
-//   wave 0      : colour quantise L0 | depth quantise L0 | pyrDown L0->L1
-//   wave k >= 1 : colour quantise Lk | NN-downsample depth labels Lk | pyrDown Lk->Lk+1 | spread+LM of level k-1 (all modalities)
-//   last wave   : spread+LM of the coarsest level
+// dependency latency, so the front end is launch bound.  Jobs are therefore issued together: the grid is the concatenation
+// of the jobs' grids (the whole frame, or one wave of it: fe_build, fe_run_single, fe_run_waves below).
 // ------------------------------------------------------------------------------------------------
 // bounded in-grid wait: true = stop waiting (this CTA timed out, or another one already did); see k_front_end_wave
 __device__ __forceinline__ bool fe_dep_give_up(const fl_fe_wave& w, int job, long long t0) {
@@ -483,64 +482,240 @@ __global__ void __launch_bounds__(256, 8) k_front_end_wave(fl_fe_wave w) {
   }
 }
 
-void fl_fe_add_color_v2(fl_fe_wave* w, const uint8_t* bgr, int W, int H, float thr_sq, uint8_t* q) {
-  fl_fe_job& j = w->job[w->n_jobs++];
-  j.wait_slot = -1; j.signal_slot = -1; j.wait_target = 0; j.row_base = -1; j.wait_row_base = -1; j.wait_row_shift = 0; j.wait_row_count = 0; j.wait_row_target = 0;
-  j.kind = FL_JOB_COLOR2; j.src = bgr; j.dst = q; j.dst2 = nullptr; j.W = W; j.H = H; j.thr_sq = thr_sq;
-  j.gx = (W + C2_TW - 1) / C2_TW; j.p0 = j.p1 = 0; j.cta_begin = w->n_ctas; w->n_ctas += j.gx * ((H + C2_TH - 1) / C2_TH);
-  w->smem = w->smem > (size_t)C2_SMEM_BYTES ? w->smem : (size_t)C2_SMEM_BYTES;
+// ---- host side: a frame's front end is ONE list of jobs (fe_build), launched as one grid with in-grid dependencies (fe_run_single)
+// or cut into waves, one launch each (fe_run_waves)
+
+// One job of a frame, with what only the host needs: the launch of the per-wave schedule it belongs to (the labels, pyrDown and resize jobs
+// of level l are in wave l, the spread job of level l in wave l + 1), the jobs whose output it reads (its labels, and a level of the mask
+// pyramid; -1 = none), and for a spread job the level shift of its label rows in the producer's tile rows (-1: waits for the whole job).
+struct fe_item { fl_fe_job j; int ctas; size_t smem; int wave, prod[2], row_shift; };
+#define FE_LIST_MAX (FL_MAX_LEVELS * (1 + 3 * FL_MAX_MODALITIES))
+struct fe_list { int n, n_depth, n_pyr; bool halves; fe_item it[FE_LIST_MAX]; fl_depth_pyr pyr[FL_FE_MAX_DPYR]; };
+struct fl_fe_state {
+  // the single launch's [FL_FE_MAX_JOBS job counters][1 error word][FL_FE_MAX_JOBS x FL_FE_MAX_TILE_ROWS tile-row counters], never reset between
+  // frames: slot i reaches counter_base[i] + its job's CTAs (row_base[i] + tiles per row); the bases advance after every launch that went out
+  fl_dev_buf<unsigned> counters; unsigned counter_base[FL_FE_MAX_JOBS] = {}, row_base[FL_FE_MAX_JOBS] = {};
+  fl_mapped_buf<int> err; int* err_dev = nullptr;       // 1 + the job whose wait timed out, in mapped host memory (+ its device alias)
+  bool force_waves = false, opt_waves = false, opt_dep_test = false;   // a wait timed out (one launch per wave from then on); FL_OPT_FE_*
+  fl_dev_buf<unsigned long long> trace; int trace_jobs = 0, trace_kind[FL_FE_MAX_JOBS] = {}, trace_ctas[FL_FE_MAX_JOBS] = {};   // FL_DBG_FE_TRACE
+  fe_list list;                                         // the current frame's jobs (20 KB: kept off the enqueue's stack)
+};
+void fl_fe_free::operator()(fl_fe_state* s) const { delete s; }
+int fl_fe_create(fl_fe_owned* out) {
+  fl_fe_owned fe(new (std::nothrow) fl_fe_state());
+  if (!fe) return FL_ERR_ARG;
+  const size_t n = (FL_FE_MAX_JOBS + 1) + FL_FE_MAX_JOBS * FL_FE_MAX_TILE_ROWS;
+  int rc;
+  if ((rc = fe->counters.alloc(n)) != FL_OK || (rc = fe->err.alloc(16)) != FL_OK) return rc;
+  FL_CUDA(cudaMemset(fe->counters.get(), 0, n * sizeof(unsigned)));
+  *fe->err.get() = 0;
+  FL_CUDA(cudaHostGetDevicePointer((void**)&fe->err_dev, fe->err.get(), 0));
+  *out = std::move(fe);
+  return FL_OK;
 }
-// returns false (nothing added) when a pyramid is requested but the wave has no free pyramid slot
-bool fl_fe_add_depth_v2(fl_fe_wave* w, const uint16_t* depth, int W, int H, int dist_thr, int diff_thr, uint8_t* q, const fl_depth_pyr* pyr) {
-  int slot = -1;
-  if (pyr && pyr->n > 0) {
-    if (w->n_pyr >= FL_FE_MAX_DPYR) return false;
-    slot = w->n_pyr++;
-    w->pyr[slot] = *pyr;
-  }
-  fl_fe_job& j = w->job[w->n_jobs++];
-  j.wait_slot = -1; j.signal_slot = -1; j.wait_target = 0; j.row_base = -1; j.wait_row_base = -1; j.wait_row_shift = 0; j.wait_row_count = 0; j.wait_row_target = 0;
-  j.kind = FL_JOB_DEPTH2; j.src = reinterpret_cast<const uint8_t*>(depth); j.dst = q; j.dst2 = nullptr; j.W = W; j.H = H; j.p0 = dist_thr; j.p1 = diff_thr;
-  const int gx = (W + D2_TW - 1) / D2_TW;
-  j.gx = slot < 0 ? -gx : gx; j.thr_sq = (float)(slot < 0 ? 0 : slot);            // gx < 0: no pyramid; thr_sq carries the pyramid slot
-  j.cta_begin = w->n_ctas; w->n_ctas += gx * ((H + D2_TH - 1) / D2_TH);
-  w->smem = w->smem > (size_t)D2_SMEM_BYTES ? w->smem : (size_t)D2_SMEM_BYTES;
-  return true;
+int fl_fe_forget_rows(fl_fe_state* fe, cudaStream_t s) {
+  FL_CUDA(cudaMemsetAsync(fe->counters.get() + (FL_FE_MAX_JOBS + 1), 0, (size_t)FL_FE_MAX_JOBS * FL_FE_MAX_TILE_ROWS * sizeof(unsigned), s));
+  memset(fe->row_base, 0, sizeof fe->row_base);
+  return FL_OK;
 }
-void fl_fe_add_pyrdown(fl_fe_wave* w, const uint8_t* src, int W, int H, uint8_t* dst, bool src_static) {
-  fl_fe_job& j = w->job[w->n_jobs++];
-  j.wait_slot = -1; j.signal_slot = -1; j.wait_target = 0; j.row_base = -1; j.wait_row_base = -1; j.wait_row_shift = 0; j.wait_row_count = 0; j.wait_row_target = 0;
-  j.kind = FL_JOB_PYRDOWN; j.src = src; j.dst = dst; j.dst2 = nullptr; j.W = W; j.H = H; j.gx = 1; j.p0 = src_static ? 1 : 0;
-  j.cta_begin = w->n_ctas; w->n_ctas += pyrdown_ctas(W, H);
+static fl_fe_job& fe_init(fe_item& it, int kind, int wave, int ctas, size_t smem, int prod0 = -1, int prod1 = -1, int row_shift = -1) {
+  memset(&it, 0, sizeof it);
+  it.j.kind = kind; it.j.wait_slot = it.j.signal_slot = it.j.row_base = it.j.wait_row_base = -1;
+  it.ctas = ctas; it.smem = smem; it.wave = wave; it.prod[0] = prod0; it.prod[1] = prod1; it.row_shift = row_shift;
+  return it.j;
 }
-void fl_fe_add_prefetch(fl_fe_wave* w, const void* src, size_t bytes) {
-  const int lines = (int)((bytes + 127) / 128);
-  if (lines <= 0 || w->n_jobs >= FL_FE_MAX_JOBS) return;
-  fl_fe_job& j = w->job[w->n_jobs++];
-  j.wait_slot = -1; j.signal_slot = -1; j.wait_target = 0; j.row_base = -1; j.wait_row_base = -1; j.wait_row_shift = 0; j.wait_row_count = 0; j.wait_row_target = 0;
-  j.kind = FL_JOB_PREFETCH; j.src = static_cast<const uint8_t*>(src); j.dst = nullptr; j.dst2 = nullptr; j.W = lines; j.H = 0; j.gx = 1;
-  j.cta_begin = w->n_ctas; w->n_ctas += (lines + 255) / 256;
-}
-void fl_fe_add_resize(fl_fe_wave* w, const uint8_t* src, int W, int H, uint8_t* dst) {
-  fl_fe_job& j = w->job[w->n_jobs++];
-  j.wait_slot = -1; j.signal_slot = -1; j.wait_target = 0; j.row_base = -1; j.wait_row_base = -1; j.wait_row_shift = 0; j.wait_row_count = 0; j.wait_row_target = 0;
-  j.kind = FL_JOB_RESIZE; j.src = src; j.dst = dst; j.dst2 = nullptr; j.W = W; j.H = H; j.gx = 1;
-  j.cta_begin = w->n_ctas; w->n_ctas += ((W / 2) * (H / 2) + 255) / 256;
-}
-void fl_fe_add_spread(fl_fe_wave* w, const uint8_t* q, fl_level_geom g, uint8_t* lm_mod, uint8_t* spread_or_null, uint8_t* lm4_mod_or_null,
-                      uint32_t* mass_or_null, const uint8_t* mask_or_null, int mask_stride, int mask_shift) {
-  fl_fe_job& j = w->job[w->n_jobs++];
-  j.wait_slot = -1; j.signal_slot = -1; j.wait_target = 0; j.row_base = -1; j.wait_row_base = -1; j.wait_row_shift = 0; j.wait_row_count = 0; j.wait_row_target = 0;
-  j.kind = FL_JOB_SPREAD; j.src = q; j.dst = lm_mod; j.dst2 = spread_or_null; j.dst3 = lm4_mod_or_null; j.mass = mass_or_null; j.g = g; j.W = g.W; j.H = g.H;
-  j.mask = mask_or_null; j.mask_stride = mask_stride; j.mask_shift = mask_shift;
-  int cw = SL_CW;                                       // small levels: narrower CTAs so that the job still fills the SMs
-  while (cw > 8 && ((g.Wd + cw - 1) / cw) * g.Hd < 148) cw >>= 1;
-  j.p0 = cw;
-  j.gx = (g.Wd + cw - 1) / cw; j.cta_begin = w->n_ctas; w->n_ctas += j.gx * g.Hd;
-  size_t sm = spread_smem_bytes(g.T);
-  w->smem = w->smem > sm ? w->smem : sm;
-}
-cudaError_t fl_launch_fe_wave(const fl_fe_wave& w, cudaStream_t s) {
-  return w.n_ctas > 0 ? fl_launch(k_front_end_wave, dim3(w.n_ctas), dim3(256), w.smem, s, w) : cudaSuccess;
+// nearest-neighbour x1/2 of a level-(l - 1) image into level l; returns the job's index
+static int fe_add_resize(fe_list& F, int l, const uint8_t* src, const fl_level_geom& g, uint8_t* dst, int prod) {
+  fl_fe_job& j = fe_init(F.it[F.n++], FL_JOB_RESIZE, l, ((g.W / 2) * (g.H / 2) + 255) / 256, 0, prod);
+  j.src = src; j.dst = dst; j.W = g.W; j.H = g.H; j.gx = 1;
+  return F.n - 1;
 }
 
+// Every job of the frame, once, in the order of the single launch: the colour pyramid chain (short jobs, on the critical path of the
+// coarsest level), the depth labels, the colour labels coarsest level first, then spread + response maps + linear memories coarsest level
+// first (the similarity kernel needs only that one).  The resize jobs, which only the per-wave schedule takes, follow the depth labels.
+static void fe_build(const fl_fe_frame& f, fe_list& F) {
+  const int L = f.n_levels, M = f.n_modalities;
+  F.n = F.n_depth = F.n_pyr = 0; F.halves = true;
+  for (int l = 0; l + 1 < L; ++l) F.halves &= f.geom[l].W % 2 == 0 && f.geom[l].H % 2 == 0;
+  bool color = false;
+  for (int m = 0; m < M; ++m) color |= f.modality_kind[m] == FL_MODALITY_COLOR_GRADIENT;
+  // the producing jobs: of colour level l, of the labels of (l, m), of mask level l of modality m
+  int bgr[FL_MAX_LEVELS] = {-1}, lab[FL_MAX_LEVELS][FL_MAX_MODALITIES], msk[FL_MAX_LEVELS][FL_MAX_MODALITIES];
+  if (color)                                            // one chain, shared by all colour modalities
+    for (int l = 0; l + 1 < L; ++l) {
+      const fl_level_geom& g = f.geom[l];
+      fl_fe_job& j = fe_init(F.it[F.n++], FL_JOB_PYRDOWN, l, pyrdown_ctas(g.W, g.H), 0, bgr[l]);
+      j.src = l == 0 ? f.bgr : f.bgr_pyr[l]; j.dst = f.bgr_pyr[l + 1]; j.W = g.W; j.H = g.H; j.gx = 1;
+      j.p0 = l == 0; bgr[l + 1] = F.n - 1;              // p0: the source was complete before the launch (see dev_pyrdown_bgr)
+    }
+  // The depth job also writes the NN-downsampled pyramid of its labels when every level halves exactly (then dst_l(y, x) = src(2^l y, 2^l x))
+  // and the launch has a pyramid slot left; otherwise resize jobs halve the labels level by level.
+  for (int m = 0; m < M; ++m) {
+    if (f.modality_kind[m] != FL_MODALITY_DEPTH_NORMAL) continue;
+    const fl_level_geom& g = f.geom[0];
+    const bool pyr = L > 1 && F.halves && L - 1 <= FL_FE_MAX_PYR && F.n_pyr < FL_FE_MAX_DPYR;
+    const int gx = (g.W + D2_TW - 1) / D2_TW;
+    fl_fe_job& j = fe_init(F.it[F.n++], FL_JOB_DEPTH2, 0, gx * ((g.H + D2_TH - 1) / D2_TH), D2_SMEM_BYTES);
+    j.src = reinterpret_cast<const uint8_t*>(f.depth); j.dst = f.q[0][m]; j.W = g.W; j.H = g.H; j.p0 = f.dist_thr; j.p1 = f.diff_thr;
+    j.gx = pyr ? gx : -gx;                              // gx < 0: no pyramid; thr_sq carries the pyramid slot
+    if (pyr) {
+      fl_depth_pyr& P = F.pyr[F.n_pyr];
+      memset(&P, 0, sizeof P); P.n = L - 1;
+      for (int k = 1; k < L; ++k) { P.W[k - 1] = f.geom[k].W; P.H[k - 1] = f.geom[k].H; P.dst[k - 1] = f.q[k][m]; }
+      j.thr_sq = (float)F.n_pyr++;
+    }
+    ++F.n_depth; lab[0][m] = F.n - 1;
+    for (int l = 1; l < L; ++l) lab[l][m] = pyr ? lab[0][m] : fe_add_resize(F, l, f.q[l - 1][m], f.geom[l - 1], f.q[l][m], lab[l - 1][m]);
+  }
+  // A masked modality's spread job reads the level-0 mask at a shift of l when every level halves exactly (NN-halving then picks
+  // src(2y, 2x)); otherwise resize jobs build the mask pyramid next to the depth labels'.
+  for (int m = 0; m < M; ++m)
+    for (int l = 0; l < L; ++l)
+      msk[l][m] = l > 0 && f.mask[m] && !F.halves ? fe_add_resize(F, l, l == 1 ? f.mask[m] : f.mask_pyr[l - 1][m], f.geom[l - 1], f.mask_pyr[l][m], msk[l - 1][m]) : -1;
+  for (int l = L - 1; l >= 0; --l)
+    for (int m = 0; m < M; ++m) {
+      if (f.modality_kind[m] != FL_MODALITY_COLOR_GRADIENT) continue;
+      const fl_level_geom& g = f.geom[l];
+      const int gx = (g.W + C2_TW - 1) / C2_TW;
+      fl_fe_job& j = fe_init(F.it[F.n++], FL_JOB_COLOR2, l, gx * ((g.H + C2_TH - 1) / C2_TH), C2_SMEM_BYTES, bgr[l]);
+      j.src = l == 0 ? f.bgr : f.bgr_pyr[l]; j.dst = f.q[l][m]; j.W = g.W; j.H = g.H; j.thr_sq = f.thr_sq; j.gx = gx;
+      lab[l][m] = F.n - 1;
+    }
+  for (int l = L - 1; l >= 0; --l)
+    for (int m = 0; m < M; ++m) {
+      const fl_level_geom& g = f.geom[l];
+      int cw = SL_CW;                                   // small levels: narrower CTAs so that the job still fills the SMs
+      while (cw > 8 && ((g.Wd + cw - 1) / cw) * g.Hd < 148) cw >>= 1;
+      const int gx = (g.Wd + cw - 1) / cw;
+      // labels that the level-0 job wrote (the depth job's own pyramid): row y of level l is its row y << l
+      fl_fe_job& j = fe_init(F.it[F.n++], FL_JOB_SPREAD, l + 1, gx * g.Hd, spread_smem_bytes(g.T), lab[l][m], msk[l][m], lab[l][m] == lab[0][m] ? l : 0);
+      const bool coarsest = l == L - 1, mpyr = msk[l][m] >= 0;
+      j.src = f.q[l][m]; j.dst = f.lm[l] + (size_t)m * g.mod_stride; j.dst2 = f.spread[l][m];
+      j.dst3 = coarsest && f.lm4 ? f.lm4 + (((size_t)m * g.mod_stride) >> 1) : nullptr; j.mass = coarsest && f.mass ? f.mass + 8 * m : nullptr;
+      j.mask = mpyr ? f.mask_pyr[l][m] : f.mask[m]; j.mask_stride = mpyr ? g.W : f.geom[0].W; j.mask_shift = mpyr ? 0 : l;
+      j.g = g; j.W = g.W; j.H = g.H; j.p0 = cw; j.gx = gx;
+    }
+}
+static void fe_wave_begin(fl_fe_wave& w, const fe_list& F, int* zero_me) {
+  w.n_jobs = w.n_ctas = 0; w.smem = 0; w.zero_me = zero_me; w.counters = nullptr; w.dep_error = w.dep_error_host = nullptr; w.trace = nullptr;
+  w.n_pyr = F.n_pyr; memcpy(w.pyr, F.pyr, sizeof w.pyr);
+}
+static void fe_append(fl_fe_wave& w, const fe_item& it) {
+  fl_fe_job& j = w.job[w.n_jobs++] = it.j;
+  j.cta_begin = w.n_ctas; w.n_ctas += it.ctas; w.smem = w.smem > it.smem ? w.smem : it.smem;
+}
+static int fe_ctas(const fl_fe_wave& w, int i) { return (i + 1 < w.n_jobs ? w.job[i + 1].cta_begin : w.n_ctas) - w.job[i].cta_begin; }
+static int fe_launch(const fl_fe_wave& w, cudaStream_t s, int64_t* launches) {
+  ++*launches;
+  if ((w.n_ctas > 0 ? fl_launch(k_front_end_wave, dim3(w.n_ctas), dim3(256), w.smem, s, w) : cudaSuccess) == cudaSuccess) return FL_OK;
+  fl_set_error("front-end launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+  return FL_ERR_CUDA;
+}
+
+// Single launch: every job of the frame in ONE grid, producers before consumers, dependencies resolved by per-job CTA counters inside the
+// kernel (k_front_end_wave).  Removes L launches and their dependency gaps, and lets the level-0 work fill the machine while the short
+// critical chain pyrDown -> colour L(top) -> spread L(top) runs.
+static int fe_run_single(fl_fe_state& S, const fl_fe_frame& f, const fe_list& F, cudaStream_t s, int64_t* launches) {
+  fl_fe_wave w;
+  fe_wave_begin(w, F, f.zero_me);                       // resets the candidate counter: no memset node between the kernels
+  w.counters = S.counters.get(); w.dep_error = reinterpret_cast<int*>(w.counters + FL_FE_MAX_JOBS); w.dep_error_host = S.err_dev;
+  for (int i = 0, room = FL_FE_MAX_JOBS - F.n; i < (room >= 6 ? 6 : room >= 3 ? 3 : 0); ++i) {
+    const int lines = (int)((f.prefetch_bytes[i] + 127) / 128);
+    if (lines <= 0) continue;
+    fe_item it;
+    fl_fe_job& j = fe_init(it, FL_JOB_PREFETCH, 0, (lines + 255) / 256, 0);
+    j.src = static_cast<const uint8_t*>(f.prefetch[i]); j.W = lines; j.gx = 1;
+    fe_append(w, it);
+  }
+  const int off = w.n_jobs;                             // list job i is job off + i of the grid and owns counter slot off + i
+  for (int i = 0; i < F.n; ++i) fe_append(w, F.it[i]);
+  // FL_OPT_FE_DEP_TIMEOUT_TEST: this frame's waits for whole jobs ask for one CTA more than the producer has, i.e. they time out
+  const unsigned dep_test = S.opt_dep_test ? 1u : 0u;
+  S.opt_dep_test = false;
+  for (int i = 0; i < F.n; ++i) {                       // (no job of a single launch has a second producer: that is a mask pyramid level)
+    const int p = off + F.it[i].prod[0];
+    if (p < off) continue;
+    fl_fe_job& j = w.job[off + i]; fl_fe_job& pj = w.job[p];
+    pj.signal_slot = p;
+    j.wait_slot = p; j.wait_target = S.counter_base[p] + (unsigned)fe_ctas(w, p) + dep_test;
+    // a spread job waits only for the tile rows of the producer that hold its label rows (see fl_fe_job), if the producer has few enough
+    const int rows = (pj.H + 15) / 16;
+    if (F.it[i].row_shift < 0 || rows > FL_FE_MAX_TILE_ROWS) continue;
+    pj.row_base = (FL_FE_MAX_JOBS + 1) + p * FL_FE_MAX_TILE_ROWS;
+    j.wait_row_base = pj.row_base; j.wait_row_shift = F.it[i].row_shift; j.wait_row_count = rows; j.wait_row_target = S.row_base[p] + (unsigned)abs(pj.gx);
+  }
+  if (f.trace) {                                        // developer timeline: per job first start / last end, summed CTA spans
+    if (int rc = S.trace.grow(4 * FL_FE_MAX_JOBS)) return rc;
+    unsigned long long init[4 * FL_FE_MAX_JOBS] = {};
+    for (int i = 0; i < FL_FE_MAX_JOBS; ++i) init[2 * i] = ~0ull;   // first CTA start (min), then last end (max), then the span sums
+    FL_CUDA(cudaMemcpyAsync(S.trace.get(), init, sizeof init, cudaMemcpyHostToDevice, s));
+    FL_CUDA(cudaStreamSynchronize(s));
+    w.trace = S.trace.get(); S.trace_jobs = w.n_jobs;
+    for (int i = 0; i < w.n_jobs; ++i) { S.trace_kind[i] = w.job[i].kind; S.trace_ctas[i] = fe_ctas(w, i); }
+  }
+  if (int rc = fe_launch(w, s, launches)) return rc;
+  for (int i = 0; i < w.n_jobs; ++i) {                  // the bases advance only when the launch went out (a failed launch bumps no counter)
+    if (w.job[i].signal_slot >= 0) S.counter_base[i] += (unsigned)fe_ctas(w, i);
+    if (w.job[i].row_base >= 0) S.row_base[i] += (unsigned)abs(w.job[i].gx);
+  }
+  return FL_OK;
+}
+
+// Per wave: L + 1 launches, no in-grid waits; wave l produces the labels of level l and the linear memories of level l - 1.  Within a wave
+// the longest jobs go first: the kernel ends with its slowest CTA, and CTAs are scheduled in job order.  (Measured alternative: slicing the
+// level-0 colour quantisation over the waves and moving every spread to the last wave - 16.6 + 10.8 + 9.2 us instead of 17.7 + 9.4 + 6.0
+// us, i.e. no gain: each wave has a latency floor of one colour-tile CTA, about 8 us.)
+static int fe_run_waves(const fl_fe_frame& f, const fe_list& F, cudaStream_t s, int64_t* launches) {
+  static const int order[] = {FL_JOB_COLOR2, FL_JOB_DEPTH2, FL_JOB_SPREAD, FL_JOB_PYRDOWN, FL_JOB_RESIZE};
+  fl_fe_wave w;
+  fe_wave_begin(w, F, f.zero_me);                       // the first launch resets the candidate counter
+  auto flush = [&]() { const int rc = fe_launch(w, s, launches); fe_wave_begin(w, F, nullptr); return rc; };
+  int rc = FL_OK;
+  for (int wave = 0; wave <= f.n_levels && rc == FL_OK; ++wave) {
+    for (int kind : order)
+      for (int i = 0; i < F.n && rc == FL_OK; ++i) {
+        if (F.it[i].wave != wave || F.it[i].j.kind != kind) continue;
+        if (w.n_jobs == FL_FE_MAX_JOBS && (rc = flush()) != FL_OK) break;   // jobs of one wave are independent: splitting a wave is safe
+        fe_append(w, F.it[i]);
+        if (kind == FL_JOB_PYRDOWN) w.job[w.n_jobs - 1].p0 = 1;   // its source was written by an earlier launch
+      }
+    if (rc == FL_OK && w.n_jobs > 0) rc = flush();
+  }
+  return rc;
+}
+int fl_fe_run(fl_fe_state* fe, const fl_fe_frame& f, cudaStream_t s, int64_t* launches) {
+  fe_list& F = fe->list;
+  fe_build(f, F);
+  // The in-grid waits know one producer per job and the depth pyramid's tile rows at a shift of the level.  So the single launch takes a
+  // list in which every level halves exactly and every depth job writes its own pyramid (no resize job), and that fits one grid.
+  const bool single = !fe->opt_waves && !fe->force_waves && F.halves && F.n_depth <= FL_FE_MAX_DPYR && F.n <= FL_FE_MAX_JOBS;
+  return single ? fe_run_single(*fe, f, F, s, launches) : fe_run_waves(f, F, s, launches);
+}
+int fl_fe_take_timeout(fl_fe_state* fe, cudaStream_t s, int* job) {
+  *job = *reinterpret_cast<volatile int*>(fe->err.get()) - 1;
+  if (*job < 0) return FL_OK;
+  *fe->err.get() = 0; fe->force_waves = true;
+  FL_CUDA(cudaMemsetAsync(fe->counters.get() + FL_FE_MAX_JOBS, 0, sizeof(unsigned), s));
+  return FL_OK;
+}
+int fl_fe_trace(const fl_fe_state* fe, void* host_out, size_t bytes) {
+  if (!fe->trace.get() || fe->trace_jobs <= 0) return FL_ERR_STATE;
+  if (bytes < (size_t)fe->trace_jobs * 6 * sizeof(unsigned long long)) return FL_ERR_CAPACITY;
+  unsigned long long raw[4 * FL_FE_MAX_JOBS];
+  FL_CUDA(cudaMemcpy(raw, fe->trace.get(), sizeof raw, cudaMemcpyDeviceToHost));
+  unsigned long long* o = static_cast<unsigned long long*>(host_out);
+  for (int i = 0; i < fe->trace_jobs; ++i) {
+    o[6 * i] = (unsigned long long)fe->trace_kind[i]; o[6 * i + 1] = (unsigned long long)fe->trace_ctas[i]; o[6 * i + 2] = raw[2 * i]; o[6 * i + 3] = raw[2 * i + 1];
+    o[6 * i + 4] = raw[2 * FL_FE_MAX_JOBS + 2 * i]; o[6 * i + 5] = raw[2 * FL_FE_MAX_JOBS + 2 * i + 1];
+  }
+  return fe->trace_jobs;
+}
+int fl_fe_option(fl_fe_state* fe, int option, int value) {
+  switch (option) {
+    case FL_OPT_FE_WAVES: fe->opt_waves = value != 0; return FL_OK;
+    case FL_OPT_FE_DEP_TIMEOUT_TEST: fe->opt_dep_test = value != 0; return FL_OK;
+    case FL_OPT_FE_FORCED_WAVES: return fe->force_waves ? 1 : 0;   // query: has a time-out switched this handle to wave launches?
+  }
+  return FL_ERR_ARG;
+}

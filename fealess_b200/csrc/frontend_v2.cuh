@@ -1,5 +1,5 @@
-// Word-parallel colour-gradient and depth-normal quantisers (included by frontend.cu; same reference semantics as the
-// byte-granular kernels there, which remain as the masked-path / A-B fallback).
+// Word-parallel colour-gradient and depth-normal quantisers, the colour and depth jobs of k_front_end_wave (included by
+// frontend.cu; they replaced the byte-granular first versions, which are deleted).
 //
 // The first versions spent ~900 (colour) and ~550 (depth) instructions per pixel on byte-granular shared-memory tiles.
 // Here every stage works on 32-bit words of four pixels:
